@@ -406,8 +406,30 @@ def verify_against_single_context(torch, dist, rig, scenes, inv, voxel, bricks, 
     return bool(flag.item())
 
 
+DUMP_DRAWS = 1 << 21           # seeded voxel draws of --dump-outputs over the whole volume (about 2.1 M distinct voxels, 25 MB with their indices)
+
+
+def dump_outputs(out_dir, fu):
+    """--dump-outputs: what the last timed step left for a caller of rr_fuse_frame, as float32 / float64 .npy files, about 55 MB.
+    The TSDF (537 MB at 512^3) is written in two parts. `tsdf_occupied_bricks` is every voxel the integration wrote: the
+    occupied bricks in `occupied_bricks` order, each brick as tsdf[z0:z1, y0:y1, x0:x1] flattened (ranges from
+    rr_get_brick_ranges). `tsdf_sample` is a fixed, seeded sample of the whole volume, cleared space included, and
+    `tsdf_sample_index` holds the sample's flat indices (z*Y*X + y*X + x). `brick_counters` and `occupied_bricks` are whole."""
+    os.makedirs(out_dir, exist_ok=True)
+    tsdf = fu.download_tsdf()
+    idx = np.unique(np.random.default_rng(2024).integers(0, tsdf.size, DUMP_DRAWS))
+    counters, occupied = fu.download_bricks()
+    rr = fu.brick_ranges()[occupied]
+    in_bricks = np.concatenate([tsdf[z0:z1, y0:y1, x0:x1].reshape(-1) for x0, x1, y0, y1, z0, z1 in rr] or [np.zeros(0, np.float32)])
+    for name, a in (("tsdf_occupied_bricks", in_bricks), ("tsdf_sample", tsdf.reshape(-1)[idx]), ("tsdf_sample_index", idx.astype(np.float64)),
+                    ("brick_counters", counters.astype(np.float64)), ("occupied_bricks", occupied.astype(np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single-GPU run (each rank of a sharded run holds only its slab)")
     import torch
     from rrpy import capi, multigpu, synth
     rank = int(os.environ.get("RANK", "0"))
@@ -434,6 +456,8 @@ def run_ours(args):
     sampler = ClockSampler(local, args.clock_ms) if (rank == 0 and args.clock_ms > 0) else None
     ms_total = rig.timed(rig.step_device, args.steps, args.warmup)
     gpu_launches, host_enqueue_ms = rig.launches, rig.host_ms
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, fu)
     # stage breakdown and the dominant kernel's launch duration: the same steps again with CUDA-event stage timers on the
     # context's stream (timers need direct launches, so this pass is not the one `value` comes from)
     stage_steps = max(10, min(args.steps, 100))
@@ -817,7 +841,12 @@ def main():
     ap.add_argument("--no-subrecords", dest="subrecords", action="store_false", help="skip the dense and config5 sub-records")
     ap.add_argument("--tune", default="", help="integrator tunables k=v,k=v applied on every rank (A/B measurements; results never depend on them)")
     ap.add_argument("--clock-ms", type=int, default=100, help="nvidia-smi sampling period during the timed regions (0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
     global _RESULT_FD
     sys.stdout.flush()

@@ -12,13 +12,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import bits_equal
-
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-
-
-def gold(name):
-    return np.load(os.path.join(GOLD, name))
+from conftest import GOLD, assert_points, assert_raymarch, assert_trigrid, bits_equal, gold
 
 
 @pytest.fixture(scope="module")
@@ -362,27 +356,6 @@ def test_oracle_against_reference_shader_goldens(O):
         _assert_stage(key, got, g[key], 2e-5 * 0.01)
 
 
-def _assert_raymarch(got, want_rgba, want_depth, want_samples, want_hit, what, proj, sample_flips=0.0):
-    """Oracle raymarch vs the reference's tsdf_raymarch.fs: same fragments kept, same sample counts; surface depth within
-    0.1 mm in eye space (BASELINE's bar is 1 mm) and 1e-5 in window depth; colours within 2e-3 (bilinear RGB8 lookups and
-    gradient normals amplify the ~1e-7 differences of the hit position)."""
-    hit = got["depth"] < 1.0
-    assert np.array_equal(hit, want_hit > 0), f"{what}: hit masks differ on {(hit != (want_hit > 0)).sum()} pixels"
-    assert hit.sum() > 100
-    assert (got["samples"] != want_samples).mean() <= sample_flips, f"{what}: sample counts differ on {(got['samples'] != want_samples).sum()} pixels"
-    assert np.abs(got["depth"] - want_depth).max() <= 1e-5, what
-    p22, p32 = np.float64(proj.reshape(16)[10]), np.float64(proj.reshape(16)[14])
-
-    def eye_z(d):                                                       # inverse of gl_FragDepth = ((p22 z + p32) / -z) / 2 + 1/2
-        return p32 / (-(2.0 * d.astype(np.float64) - 1.0) - p22)
-
-    dz_mm = np.abs(eye_z(got["depth"][hit]) - eye_z(want_depth[hit])) * 1000.0
-    assert dz_mm.max() <= 0.1, f"{what}: surface differs by {dz_mm.max():.4f} mm"
-    assert (np.isnan(got["rgba"]) == np.isnan(want_rgba)).all(), what
-    ok = np.isfinite(got["rgba"]) & np.isfinite(want_rgba)
-    assert np.abs(got["rgba"][ok] - want_rgba[ok]).max() <= 2e-3, what
-
-
 def test_oracle_raymarch_matches_the_reference_shader_run_on_cpu(O, small_scene, small_frame):
     import ref_glsl_py as G
     if not G.available():
@@ -396,20 +369,7 @@ def test_oracle_raymarch_matches_the_reference_shader_run_on_cpu(O, small_scene,
         for mode in range(4):
             want = G.raymarch(tsdf, 0.01, inv, sc, pre, mv, pr, VW, VH, mode)
             got = O.raymarch(tsdf, 0.01, inv, sc, pre, grid, occ, mv, pr, VW, VH, mode, skip_space=False)
-            _assert_raymarch(got, want["rgba"], want["depth"], want["samples"], want["hit"], f"eye {eye} mode {mode}", np.asarray(pr))
-
-
-def _assert_points(got, want, what):
-    """Point renderings agree when coverage is the same up to a handful of boundary pixels (the fixed-function stage is fp64 in
-    the shader harness, fp32 in the oracle) and, where the same point won, depth to 2e-7 and colour to 2e-5."""
-    (rgba, depth), (w_rgba, w_depth) = got, want
-    cov, w_cov = depth < 1.0, w_depth < 1.0
-    assert w_cov.sum() > 50, what
-    assert (cov != w_cov).sum() <= max(2, int(0.002 * w_cov.sum())), f"{what}: coverage differs on {(cov != w_cov).sum()} pixels"
-    both = cov & w_cov
-    same = both & (np.abs(depth - w_depth) <= 2e-7)
-    assert same.sum() >= 0.995 * both.sum(), f"{what}: another point won on {both.sum() - same.sum()} pixels"
-    assert np.abs(rgba - w_rgba)[same].max() <= 2e-5, what
+            assert_raymarch(got, want["rgba"], want["depth"], want["samples"], want["hit"], f"eye {eye} mode {mode}", np.asarray(pr))
 
 
 def test_oracle_point_renderers_match_the_reference_shaders_run_on_cpu(O, small_scene, small_frame):
@@ -426,11 +386,11 @@ def test_oracle_point_renderers_match_the_reference_shaders_run_on_cpu(O, small_
     for eye in ((1.6, 1.5, 2.2), (0.7, 1.3, 0.75)):
         mv, pr = synth.look_at(eye, (0.0, 1.1, 0.0)), synth.perspective(50.0, VW / VH, 0.1, 10.0)
         for mode in range(4):
-            _assert_points(O.draw_points(sc, pre, mv, pr, VW, VH, mode), G.draw_points(sc, pre, mv, pr, VW, VH, mode), f"points eye {eye} mode {mode}")
+            assert_points(O.draw_points(sc, pre, mv, pr, VW, VH, mode), G.draw_points(sc, pre, mv, pr, VW, VH, mode), f"points eye {eye} mode {mode}")
         IZ, IY, IX = inv.shape[1:4]
         for limit in (0.01, 0.005):
-            _assert_points(O.draw_calibs(tsdf, (IX, IY, IZ), limit, sc.bbox_min, sc.bbox_max, mv, pr, VW, VH),
-                           G.draw_calibs(tsdf, inv, sc, 1, limit, mv, pr, VW, VH), f"calibs eye {eye} limit {limit}")
+            assert_points(O.draw_calibs(tsdf, (IX, IY, IZ), limit, sc.bbox_min, sc.bbox_max, mv, pr, VW, VH),
+                          G.draw_calibs(tsdf, inv, sc, 1, limit, mv, pr, VW, VH), f"calibs eye {eye} limit {limit}")
 
 
 def test_oracle_point_renderers_against_the_committed_shader_outputs(O):
@@ -449,21 +409,8 @@ def test_oracle_point_renderers_against_the_committed_shader_outputs(O):
     V = dict(eye=(1.2, 1.4, 1.6), at=(0.0, 1.1, 0.0), fovy=50.0, w=160, h=90)                  # make_golden.py::RM_VIEW
     mv, pr = synth.look_at(V["eye"], V["at"]), synth.perspective(V["fovy"], V["w"] / V["h"], 0.1, 10.0)
     for mode in range(4):
-        _assert_points(O.draw_points(sc, pre, mv, pr, V["w"], V["h"], mode), (g[f"points_rgba{mode}"], g[f"points_depth{mode}"]), f"points mode {mode}")
-    _assert_points(O.draw_calibs(tsdf, (20, 22, 20), 0.01, sc.bbox_min, sc.bbox_max, mv, pr, V["w"], V["h"]), (g["calibs_rgba"], g["calibs_depth"]), "calibs")
-
-
-def _assert_trigrid(got, want, what):
-    """Triangle-mesh renderings agree when coverage is the same up to a handful of pixels (a fragment test that lands on the
-    other side of a threshold), depth to 2e-5 (window depth of triangles cut by the near plane) and colour to 5e-5."""
-    (rgba, depth), (w_rgba, w_depth) = got, want
-    cov, w_cov = depth < 1.0, w_depth < 1.0
-    assert w_cov.sum() > 100, what
-    assert (cov != w_cov).sum() <= max(2, int(0.002 * w_cov.sum())), f"{what}: coverage differs on {(cov != w_cov).sum()} pixels"
-    both = cov & w_cov
-    assert np.abs(depth - w_depth)[both].max() <= 2e-5, what
-    d = np.abs(rgba - w_rgba)[both]
-    assert (d > 5e-5).any(axis=-1).sum() <= max(2, int(0.002 * both.sum())), f"{what}: colour differs by up to {d.max()}"
+        assert_points(O.draw_points(sc, pre, mv, pr, V["w"], V["h"], mode), (g[f"points_rgba{mode}"], g[f"points_depth{mode}"]), f"points mode {mode}")
+    assert_points(O.draw_calibs(tsdf, (20, 22, 20), 0.01, sc.bbox_min, sc.bbox_max, mv, pr, V["w"], V["h"]), (g["calibs_rgba"], g["calibs_depth"]), "calibs")
 
 
 def test_oracle_trigrid_matches_the_reference_shaders_run_on_cpu(O, small_scene, small_frame):
@@ -479,8 +426,8 @@ def test_oracle_trigrid_matches_the_reference_shaders_run_on_cpu(O, small_scene,
     for eye in ((1.6, 1.5, 2.2), (0.2, 1.2, 0.3)):
         mv, pr = synth.look_at(eye, (0.0, 1.1, 0.0)), synth.perspective(50.0, VW / VH, 0.1, 10.0)
         for mode in range(4):
-            _assert_trigrid(O.draw_trigrid(sc, pre, mv, pr, VW, VH, mode, min_length=0.06), G.draw_trigrid(sc, pre, mv, pr, VW, VH, mode, min_length=0.06),
-                            f"trigrid eye {eye} mode {mode}")
+            assert_trigrid(O.draw_trigrid(sc, pre, mv, pr, VW, VH, mode, min_length=0.06), G.draw_trigrid(sc, pre, mv, pr, VW, VH, mode, min_length=0.06),
+                           f"trigrid eye {eye} mode {mode}")
 
 
 def test_oracle_trigrid_against_the_committed_shader_outputs(O):
@@ -498,8 +445,8 @@ def test_oracle_trigrid_against_the_committed_shader_outputs(O):
     for tag, eye in (("", V["eye"]), ("in_", tuple(float(x) for x in g["eye_in"]))):
         mv = synth.look_at(eye, V["at"])
         for mode in range(4):
-            _assert_trigrid(O.draw_trigrid(sc, pre, mv, pr, V["w"], V["h"], mode, min_length=float(g["min_length"])),
-                            (g[f"{tag}rgba{mode}"], g[f"{tag}depth{mode}"]), f"trigrid {tag}mode {mode}")
+            assert_trigrid(O.draw_trigrid(sc, pre, mv, pr, V["w"], V["h"], mode, min_length=float(g["min_length"])),
+                           (g[f"{tag}rgba{mode}"], g[f"{tag}depth{mode}"]), f"trigrid {tag}mode {mode}")
 
 
 def test_the_rasteriser_partitions_a_shared_edge(O):
@@ -570,7 +517,7 @@ def test_oracle_space_skipping_matches_the_reference_shader_on_rasterised_peels(
                  else G.depth_peels(sc, grid, occ, mv, pr, VW, VH, 0.01))
         want = G.raymarch(tsdf, 0.01, inv, sc, pre, mv, pr, VW, VH, 1, depth_peels=peels)
         got = O.raymarch(tsdf, 0.01, inv, sc, pre, grid, occ, mv, pr, VW, VH, 1, skip_space=True)
-        _assert_raymarch(got, want["rgba"], want["depth"], want["samples"], want["hit"], f"skipSpace eye {eye}", np.asarray(pr), sample_flips=0.01)
+        assert_raymarch(got, want["rgba"], want["depth"], want["samples"], want["hit"], f"skipSpace eye {eye}", np.asarray(pr), sample_flips=0.01)
 
 
 def test_reference_cube_proxy_faces_are_front_facing_outward():
@@ -613,9 +560,9 @@ def test_oracle_raymarch_against_reference_shader_golden(O):
     mv, pr = synth.look_at((1.2, 1.4, 1.6), (0.0, 1.1, 0.0)), synth.perspective(50.0, 160 / 90, 0.1, 10.0)   # make_golden.py::RM_VIEW
     for mode in range(4):
         got = O.raymarch(tsdf, 0.01, inv, sc, pre, grid, occ, mv, pr, 160, 90, mode, skip_space=False)
-        _assert_raymarch(got, g[f"rgba{mode}"], g["depth"], g["samples"], g["hit"], f"golden mode {mode}", np.asarray(pr))
+        assert_raymarch(got, g[f"rgba{mode}"], g["depth"], g["samples"], g["hit"], f"golden mode {mode}", np.asarray(pr))
     got = O.raymarch(tsdf, 0.01, inv, sc, pre, grid, occ, mv, pr, 160, 90, 1, skip_space=True)
-    _assert_raymarch(got, g["skip_rgba"], g["skip_depth"], g["skip_samples"], g["skip_hit"], "golden skipSpace", np.asarray(pr), sample_flips=0.01)
+    assert_raymarch(got, g["skip_rgba"], g["skip_depth"], g["skip_samples"], g["skip_hit"], "golden skipSpace", np.asarray(pr), sample_flips=0.01)
 
 
 def _assert_colorfill(O, rgba, depth, want_filled, want_atlas_c, want_atlas_d, what):

@@ -1,11 +1,111 @@
 """GPU vs the reference's own shaders, directly (no oracle in between). Runs last in the suite (file name) so that its
-looser, formulation-dependent bars can never mask a result of the bit-exact parity tests."""
+looser, formulation-dependent bars can never mask a result of the bit-exact parity tests.
+
+The shaders run live where oracle/_ref/libref_glsl.so was built from the reference tree; everywhere else the kernels are
+compared with what those shaders computed for tools/make_golden.py::glsl_scene (tests/golden/ref_glsl_*.npz)."""
+import hashlib
+
 import numpy as np
 import pytest
 
-from conftest import bits_equal
+from conftest import assert_points, assert_raymarch, assert_trigrid, bits_equal, gold
 
 pytestmark = pytest.mark.gpu
+
+GOLDEN_VIEW = dict(eye=(1.2, 1.4, 1.6), at=(0.0, 1.1, 0.0), fovy=50.0, w=160, h=90)      # tools/make_golden.py::RM_VIEW
+
+
+def _sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def _golden_frame(use_bricks=True, skip_space=False):
+    """One fused frame of tools/make_golden.py::glsl_scene on the GPU, with the golden's voxel size and inverse volume."""
+    from rrpy import capi, synth
+    g = gold("ref_glsl_stages.npz")
+    sc = synth.make_scene(N=1, W=128, H=106, CW=160, CH=135, cv_res=(24, 24, 48), seed=77)
+    fu = capi.Fusion(sc.N, sc.W, sc.H, sc.CW, sc.CH)
+    capi.load_scene(fu, sc, g["inv"])
+    fu.configure(limit=0.01, voxel_size=float(g["voxel"]), brick_size=0.1, min_voxels=10, use_bricks=use_bricks, skip_space=skip_space)
+    fu.upload_frames(sc.color, sc.depth)
+    fu.frame(sync_bricks=True)
+    return fu, g
+
+
+def _golden_view():
+    from rrpy import synth
+    V = GOLDEN_VIEW
+    return synth.look_at(V["eye"], V["at"]), synth.perspective(V["fovy"], V["w"] / V["h"], 0.1, 10.0)
+
+
+def test_kernels_against_the_reference_shader_outputs():
+    """The CUDA path's full chain against the reference shaders' full chain as committed (ref_glsl_stages.npz, every stage fed
+    by the shaders' own previous stage), bricked and dense: the stages with the bars of the live comparison below, the volume
+    with the oracle's bar on the same golden. The bricked volume is also the oracle's, bit for bit (the raymarch golden's hash)."""
+    for use_bricks, key in ((True, "tsdf_bricks"), (False, "tsdf_dense")):
+        fu, g = _golden_frame(use_bricks)
+        got = {k: fu.download_stage(k) for k in ("morph", "depth", "lab", "depth_b", "sil", "normal", "quality")}
+        counters, occupied = fu.download_bricks()
+        tsdf = fu.download_tsdf()
+        fu.close()
+        if use_bricks:
+            assert np.array_equal(counters, g["pre_bricks"]) and np.array_equal(occupied, g["occupied"]) and len(occupied) > 10
+            assert _sha(tsdf) == str(gold("ref_glsl_raymarch.npz")["tsdf_sha"]), "the kernels' volume differs from the oracle's"
+        assert bits_equal(got["morph"], g["pre_morph"]).all() and bits_equal(got["sil"], g["pre_sil"]).all()
+        for k, tol in dict(depth=2e-6, lab=2e-4, depth_b=2e-6, normal=2e-4, quality=4e-5).items():
+            want = g["pre_" + k]
+            assert ((got[k] != got[k]) == (want != want)).all(), k
+            ok = np.isfinite(got[k]) & np.isfinite(want)
+            assert np.abs(got[k][ok] - want[ok]).max() <= tol, f"{k}: {np.abs(got[k][ok] - want[ok]).max()}"
+        want = g[key]
+        assert (np.abs(want) < 0.0099).sum() > 200, "the golden volume must hold in-band voxels"
+        assert (np.isnan(tsdf) == np.isnan(want)).all(), key
+        ok = np.isfinite(tsdf) & np.isfinite(want)
+        # the oracle's bar on the same golden (test_oracle_against_reference_shader_goldens): the kernels match the oracle bit for bit
+        assert np.abs(tsdf[ok].astype(np.float64) - want[ok]).max() <= 2e-5 * 0.01, key
+
+
+def test_raymarch_kernel_against_the_reference_shader_outputs():
+    """rr_raymarch against tsdf_raymarch.fs + shading.glsl as committed (ref_glsl_raymarch.npz: the shader run on the oracle's
+    volume, which the kernels reproduce bit for bit), every shade mode with the cube-proxy march, and the skipSpace branch fed
+    the reference's rasterised brick depth peels against the kernels' brick hull."""
+    g = gold("ref_glsl_raymarch.npz")
+    mv, pr = _golden_view()
+    W, H = GOLDEN_VIEW["w"], GOLDEN_VIEW["h"]
+    fu, _ = _golden_frame(skip_space=False)
+    assert _sha(fu.download_tsdf()) == str(g["tsdf_sha"]), "the kernels' volume differs from the golden's input volume"
+    for mode in range(4):
+        rgba, depth = fu.raymarch(mv, pr, W, H, shade_mode=mode)
+        got = dict(rgba=rgba, depth=depth, samples=fu.download_num_samples(W, H))
+        assert_raymarch(got, g[f"rgba{mode}"], g["depth"], g["samples"], g["hit"], f"mode {mode}", np.asarray(pr))
+    fu.close()
+    fu, _ = _golden_frame(skip_space=True)
+    rgba, depth = fu.raymarch(mv, pr, W, H, shade_mode=1)
+    got = dict(rgba=rgba, depth=depth, samples=fu.download_num_samples(W, H))
+    fu.close()
+    assert_raymarch(got, g["skip_rgba"], g["skip_depth"], g["skip_samples"], g["skip_hit"], "skipSpace", np.asarray(pr), sample_flips=0.01)
+
+
+def test_point_and_trigrid_kernels_against_the_reference_shader_outputs():
+    """rr_draw_points, rr_draw_calibs and rr_draw_trigrid against points.{vs,gs,fs}, calib_vis.{vs,fs} and trigrid_accum.{vs,gs,fs}
+    + trigrid_normalize.fs as committed (ref_glsl_points.npz, ref_glsl_trigrid.npz: the shaders run on the oracle's maps and
+    volume, which the kernels reproduce bit for bit), every shade mode, the triangle mesh also from inside the volume."""
+    gp, gt = gold("ref_glsl_points.npz"), gold("ref_glsl_trigrid.npz")
+    from rrpy import synth
+    mv, pr = _golden_view()
+    W, H = GOLDEN_VIEW["w"], GOLDEN_VIEW["h"]
+    fu, _ = _golden_frame()
+    assert _sha(fu.download_stage("quality")) == str(gt["quality_sha"]), "the kernels' maps differ from the golden's input maps"
+    assert _sha(fu.download_tsdf()) == str(gp["tsdf_sha"]), "the kernels' volume differs from the golden's input volume"
+    for mode in range(4):
+        assert_points(fu.draw_points(mv, pr, W, H, shade_mode=mode), (gp[f"points_rgba{mode}"], gp[f"points_depth{mode}"]), f"points mode {mode}")
+    assert_points(fu.draw_calibs(mv, pr, W, H, active_kinect=0, limit=0.01), (gp["calibs_rgba"], gp["calibs_depth"]), "calibs")
+    for tag, eye in (("", GOLDEN_VIEW["eye"]), ("in_", tuple(float(x) for x in gt["eye_in"]))):
+        mv = synth.look_at(eye, GOLDEN_VIEW["at"])
+        for mode in range(4):
+            assert_trigrid(fu.draw_trigrid(mv, pr, W, H, shade_mode=mode, min_length=float(gt["min_length"])),
+                           (gt[f"{tag}rgba{mode}"], gt[f"{tag}depth{mode}"]), f"trigrid {tag}mode {mode}")
+    fu.close()
 
 
 def test_kernels_against_the_reference_shaders_directly(small_scene):

@@ -311,6 +311,9 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
   const bool new_volume = !c->configured || res[0] != c->res[0] || res[1] != c->res[1] || res[2] != c->res[2] ||
                           (cfg->store_weight == RR_VOXELS_F32_WEIGHT) != (c->d_weight != nullptr);
   const bool new_bricks = new_volume || bs != c->bricks.brick_size;
+  // the staged integrator's tables depend on the volume, the brick grid, bricks mode and the voxel format; plain setters
+  // (limit, min_voxels, skip_space) keep them, and the next integrate needs no synchronising rebuild
+  const bool restage = new_bricks || cfg->use_bricks != c->cfg.use_bricks || cfg->store_weight != c->cfg.store_weight;
   if (new_volume) {
     const size_t nvox = (size_t)res[0] * res[1] * res[2];
     RR_TRY(dev_alloc(c, &c->d_tsdf, nvox, "tsdf volume"));
@@ -365,7 +368,7 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
   }
   c->cfg = *cfg;
   c->configured = true;
-  c->sti.dirty = true;
+  if (restage) c->sti.dirty = true;
   return RR_OK;
 }
 
@@ -933,6 +936,12 @@ int rr_integrator_info(rr_ctx* c, uint32_t* out) {
     RR_TRY(check(c, cudaMemcpy(e, s.d_err, sizeof(e), cudaMemcpyDeviceToHost), "integrator flags"));
     out[13] = (e[0] ? 1u : 0u) | (e[1] ? 2u : 0u);
   }
+  return RR_OK;
+}
+
+int rr_integrator_last(const rr_ctx* c, uint32_t* out) {
+  if (!c || !out) return RR_ERR_INVALID;
+  std::memcpy(out, c->last_integrate, sizeof(c->last_integrate));
   return RR_OK;
 }
 

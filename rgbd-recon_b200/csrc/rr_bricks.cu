@@ -99,6 +99,7 @@ __global__ void __launch_bounds__(1024) k_bricks_update(const uint32_t* __restri
 
 int launch_bricks_clear(rr_ctx* c) {
   cudaError_t e = cudaMemsetAsync(c->d_counters, 0, sizeof(uint32_t) * ((size_t)c->bricks.num + RR_CLASS_COUNTERS), c->stream);
+  c->sti.lists_key = 0;
   return check(c, e, "bricks clear");
 }
 
@@ -121,6 +122,7 @@ int launch_bricks_update(rr_ctx* c) {
   RR_LAUNCH_CHECK(c, "k_bricks_update");
   timer_end(c, "bricks");
   c->work_fresh = true;
+  if (classify) c->sti.lists_key = staged_lists_key(c);
   cudaError_t e = cudaMemcpyAsync(c->h_num_occ, c->d_num_occ, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream);
   return check(c, e, "bricks count copy");
 }

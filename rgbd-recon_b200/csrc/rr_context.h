@@ -114,6 +114,7 @@ struct rr_ctx {
   float4* d_normal = nullptr;
   float* d_quality = nullptr;
   float4* d_gather = nullptr;
+  bool gather_packed = false;      // d_gather holds the texels of the last rr_preprocess (k_pack_gather ran for it)
   float2* d_pairs = nullptr;       // [N][H+2][pair_pitch]
   int pair_pitch = 0;              // W+2 rounded up to even (TMA strides are multiples of 16 bytes)
   uint32_t* d_flags = nullptr;     // [0] pack-encoding violation counter
@@ -150,8 +151,11 @@ struct rr_ctx {
   struct IpcView { std::string key; uint32_t* step; float4* rgba; float* zbuf; float* nsamp; };
   std::vector<IpcView> ipc_views;
   bool graphs_broken = false;      // a capture failed once: stay on direct launches
+  // the last launch_integrate (rr_integrator_last): path (0 none, 1 staged, 2 fused, 3 k_fill + k_integrate_bricks, 4 dense),
+  // sensors, voxel mode, CTA threads or consumer warps, repairs (bit 0 stale item lists declined, bit 1 gather packed late)
+  uint32_t last_integrate[8] = {};
   // staged (TMA) integrator, rr_integrate_staged.cu. `dirty` is set by everything its tables depend on (inverse volumes,
-  // volume / brick grid, tunables); they are rebuilt lazily by the next integrate or pre-process call.
+  // volume / brick grid, bricks mode, voxel format, tunables); they are rebuilt lazily by the next integrate or pre-process call.
   struct StagedIntegrator {
     bool dirty = true;             // tables below do not match the current calibration / configuration
     bool ok = false;               // the configuration fits the staged kernel
@@ -165,6 +169,9 @@ struct rr_ctx {
     uint2* d_fp = nullptr;         // [items][N]: tile origin tx0 | ty0 << 16, footprint rectangle inside the tile (bit 7 of .y: exceeds the tile)
     uint32_t n_oversize = 0;       // (item, sensor) pairs of the whole brick grid whose footprint exceeds the tile
     uint2* d_list = nullptr;       // [N + 1][list_stride]: this frame's occupied items by cost class (item, verdict), k_bricks_update
+    unsigned tables = 0;           // bumped by every table rebuild
+    uint64_t lists_key = 0;        // staged_lists_key() the lists were classified for; 0: no valid lists (cleared by a table
+                                   // rebuild, rr_bricks_clear and rr_preprocess, whose new pair image the verdicts do not describe)
     uint32_t list_stride = 0;
     float2* d_zr = nullptr;        // [items][N]: exact range of pos_calib.z over the item (k_footprints)
     uint32_t* d_err = nullptr;     // [4] device-side consistency flags (must stay 0)
@@ -237,6 +244,7 @@ SensorTables sensor_tables(const rr_ctx* c);
 
 // kernels' host launchers (one translation unit each)
 int launch_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, int refine);
+int launch_pack_gather(rr_ctx* c);    // the gather texels of the direct integrators from the last pre-process's stage images
 int launch_bricks_clear(rr_ctx* c);
 int launch_bricks_update(rr_ctx* c);
 int launch_integrate(rr_ctx* c);
@@ -254,6 +262,7 @@ int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines
 void staged_release(rr_ctx* c);
 bool staged_selected(const rr_ctx* c); // after staged_prepare: the next bricks-mode integrate runs the staged kernel
+uint64_t staged_lists_key(const rr_ctx* c);   // what the item lists depend on besides the frame: table rebuild, limit
 void drop_frame_graphs(rr_ctx* c);
 
 // host geometry (rr_host_geom.cpp)

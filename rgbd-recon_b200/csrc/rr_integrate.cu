@@ -225,6 +225,7 @@ static int launch_bricks_n(rr_ctx* c, const IntegrateParams& p, int mode) {
   }
   const int zchunk = 9;
   const dim3 grd(148 * std::max(1, tunables().brick_grid), 1, 1);
+  c->last_integrate[0] = 3; c->last_integrate[3] = (uint32_t)threads;
   if (mode == 1) k_integrate_bricks<N, 1, 2><<<grd, threads, 0, c->stream>>>(p, max_cols, max_nz, zchunk);
   else if (mode == 2) k_integrate_bricks<N, 2, 2><<<grd, threads, 0, c->stream>>>(p, max_cols, max_nz, zchunk);
   else k_integrate_bricks<N, 0, 2><<<grd, threads, 0, c->stream>>>(p, max_cols, max_nz, zchunk);
@@ -252,6 +253,8 @@ static int launch_n(rr_ctx* c, const IntegrateParams& p, bool bricks, int mode, 
       f.chunk = tn.chunk > 0 ? tn.chunk : (max_cols + 31) / 32;
       cudaMemsetAsync(c->d_work, 0, 4 * sizeof(uint32_t), c->stream);
       const dim3 grd(148 * std::min(2, std::max(1, tn.ctas)), 1, 1);
+      c->last_integrate[0] = 2;
+      c->last_integrate[3] = N > 4 ? 256u : (mode == 0 && tn.threads != 384 ? 512u : 384u);
       if constexpr (N > 4) {
         // 6 registers of plane state per sensor: more than 4 sensors get 256-thread CTAs (128 registers)
         if (mode == 1) k_integrate_fused<N, 1, 256><<<grd, 256, 0, c->stream>>>(f);
@@ -270,6 +273,7 @@ static int launch_n(rr_ctx* c, const IntegrateParams& p, bool bricks, int mode, 
   } else {
     const int nz = p.z_end - p.z_begin;
     const dim3 grd((p.X + 31) / 32, (p.Y + 7) / 8, (nz + p.z_chunk - 1) / p.z_chunk);
+    c->last_integrate[0] = 4; c->last_integrate[3] = blk.x * blk.y;
     if (mode == 1) k_integrate_dense<N, 1><<<grd, blk, 0, c->stream>>>(p);
     else if (mode == 2) k_integrate_dense<N, 2><<<grd, blk, 0, c->stream>>>(p);
     else k_integrate_dense<N, 0><<<grd, blk, 0, c->stream>>>(p);
@@ -316,6 +320,8 @@ int launch_integrate(rr_ctx* c) {
   const int mode = c->cfg.store_weight == RR_VOXELS_HALF2 ? 2 : (c->cfg.store_weight != 0 ? 1 : 0);
   const bool weight = mode == 1;
   const bool bricks = c->cfg.use_bricks != 0;
+  std::memset(c->last_integrate, 0, sizeof(c->last_integrate));
+  c->last_integrate[1] = (uint32_t)c->N; c->last_integrate[2] = (uint32_t)mode;
   timer_begin(c, "2integrate");
   const size_t plane = (size_t)p.X * p.Y;
   const size_t nslab = plane * (size_t)(p.z_end - p.z_begin);
@@ -324,8 +330,13 @@ int launch_integrate(rr_ctx* c) {
   int rc = RR_OK;
   bool done = false;
   // first choice in bricks mode: the TMA-staged persistent kernel (rr_integrate_staged.cu); it declines (done = false) when
-  // the configuration does not fit its shared-memory stages, and the direct kernels below take over
+  // the configuration does not fit its shared-memory stages or its item lists are stale, and the direct kernels below take over
   if (fused && nslab && tunables().staged != 0) rc = launch_integrate_staged(c, p, mode, &done);
+  if (!done && rc == RR_OK && nslab && !c->gather_packed) {
+    // the last pre-process left the gather texels to the staged kernel, which is not the one running now
+    rc = launch_pack_gather(c);
+    c->last_integrate[4] |= 2u;
+  }
   if (!done && rc == RR_OK) {
     if (bricks && !fused && nslab) {
       // dense mode overwrites every voxel, so only the brick path needs the clear
@@ -350,6 +361,7 @@ int launch_integrate(rr_ctx* c) {
         default: return fail(c, RR_ERR_UNSUPPORTED, "integrate: 1..8 sensors supported");
       }
     }
+    c->work_fresh = false;   // the fused kernel draws from the work counters too
   }
   timer_end(c, "2integrate");
   return rc;

@@ -627,6 +627,13 @@ void staged_release(rr_ctx* c) {
   cudaFree(c->sti.d_fp); cudaFree(c->sti.d_list); cudaFree(c->sti.d_err); cudaFree(c->sti.d_zr);
   c->sti.d_fp = nullptr; c->sti.d_list = nullptr; c->sti.d_err = nullptr; c->sti.d_zr = nullptr;
   c->sti.ok = false; c->sti.dirty = true;
+  c->sti.lists_key = 0;
+}
+
+uint64_t staged_lists_key(const rr_ctx* c) {
+  uint32_t limit;
+  std::memcpy(&limit, &c->cfg.limit, sizeof(limit));
+  return ((uint64_t)c->sti.tables << 32) | limit;
 }
 
 // the tunables the staged tables depend on, as one key (other knobs change launch shapes of the direct kernels only)
@@ -663,6 +670,8 @@ int staged_prepare(rr_ctx* c) {
   if (!st.dirty && st.generation == staged_key()) return RR_OK;
   st.ok = false;
   st.n_oversize = 0;
+  // declined before any table is built: stay dirty, so that returning to the current tunables rebuilds the tables
+  st.dirty = true;
   if (!c->configured || !c->cfg.use_bricks || !c->fused_ok || !tn.staged || !tn.fused || !c->d_inv) return RR_OK;
   for (int i = 0; i < c->N; ++i) if (!c->have_inv[i]) return RR_OK;
   st.dirty = false;
@@ -790,6 +799,7 @@ int staged_prepare(rr_ctx* c) {
     }
   staged_release(c);
   st.dirty = false;
+  ++st.tables;
   st.d_zr = d_zr;
   st.list_stride = (uint32_t)items;
   RR_TRY_RC(check(c, cudaMalloc((void**)&st.d_list, (size_t)(N + 1) * items * sizeof(uint2)), "item lists"));
@@ -839,6 +849,10 @@ int launch_integrate_staged(rr_ctx* c, const IntegrateParams& p, int mode, bool*
   RR_TRY_RC(staged_prepare(c));
   const auto& st = c->sti;
   if (!staged_selected(c)) return RR_OK;
+  // The item lists hold the verdicts of the last rr_bricks_update. Tables rebuilt since, a limit changed since, a newer
+  // pre-process (the verdicts describe the pair image they were classified on) or rr_bricks_clear (it zeroes the class
+  // counters) leave them stale: the direct kernels integrate the occupied list instead.
+  if (st.lists_key != staged_lists_key(c)) { c->last_integrate[4] |= 1u; return RR_OK; }
   StagedParams sp{};
   setup_fill(c, p, mode, tunables().stage_fill_rows, sp.f);
   sp.cy = st.cy; sp.cz = st.cz; sp.n_yc = st.n_yc; sp.n_zc = st.n_zc;
@@ -872,6 +886,7 @@ int launch_integrate_staged(rr_ctx* c, const IntegrateParams& p, int mode, bool*
     default: return fail(c, RR_ERR_UNSUPPORTED, "integrate: 1..8 sensors supported");
   }
   if (rc != RR_OK) return rc;
+  c->last_integrate[0] = 1; c->last_integrate[3] = (uint32_t)st.cwarps;
   *done = true;
   return RR_OK;
 }

@@ -574,6 +574,8 @@ int launch_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, i
   // The staged integrator reads the pair image k_quality writes on its way out; the 32-byte gather texels of the direct
   // kernels (dense mode, configurations the staged kernel declines) cost one more pass and are built only when needed.
   const bool staged = staged_selected(c);
+  c->sti.lists_key = 0;                    // the item lists describe the previous pair image
+  c->gather_packed = false;
   if (tunables().fuse_nq) {
     timer_begin(c, "quality");
     k_normal_quality<<<grd, blk, 0, s>>>(c->d_depth_b, c->d_normal, c->d_counters, c->d_quality, c->d_sil, c->d_pairs, c->pair_pitch,
@@ -588,14 +590,19 @@ int launch_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, i
     k_quality<<<grd, blk, 0, s>>>(c->d_depth_b, c->d_normal, c->d_quality, c->d_sil, c->d_pairs, c->pair_pitch, c->d_flags, W, H, st);
     RR_LAUNCH_CHECK(c, "k_quality");
   }
-  if (!staged) {
-    const dim3 grd_g((W + 1 + TILE_X - 1) / TILE_X, (H + 1 + TILE_Y - 1) / TILE_Y, N);
-    k_pack_gather<<<grd_g, blk, 0, s>>>(c->d_depth_b, c->d_quality, c->d_sil, c->d_gather, c->d_flags, W, H);
-    RR_LAUNCH_CHECK(c, "k_pack_gather");
-  }
+  if (!staged) RR_TRY_RC(launch_pack_gather(c));
   timer_end(c, "quality");
 
   timer_end(c, "1preprocess");
+  return RR_OK;
+}
+
+int launch_pack_gather(rr_ctx* c) {
+  const dim3 blk(TILE_X, TILE_Y, 1);
+  const dim3 grd_g((c->W + 1 + TILE_X - 1) / TILE_X, (c->H + 1 + TILE_Y - 1) / TILE_Y, c->N);
+  k_pack_gather<<<grd_g, blk, 0, c->stream>>>(c->d_depth_b, c->d_quality, c->d_sil, c->d_gather, c->d_flags, c->W, c->H);
+  RR_LAUNCH_CHECK(c, "k_pack_gather");
+  c->gather_packed = true;
   return RR_OK;
 }
 

@@ -27,6 +27,9 @@ class Config(C.Structure):
 # rr_voxel_format (rr_config.store_weight)
 VOXELS_F32, VOXELS_F32_WEIGHT, VOXELS_HALF2 = 0, 1, 2
 
+# rr_integrator_last()[0]
+INTEGRATE_PATHS = ("none", "staged", "fused", "two_kernel", "dense")
+
 
 class View(C.Structure):
     _fields_ = [("modelview", C.c_float * 16), ("projection", C.c_float * 16), ("viewport", C.c_int32 * 4),
@@ -94,6 +97,7 @@ def lib():
     L.rr_get_stage_stats.argtypes = [vp, C.c_char_p, f32, u32]
     L.rr_integrator_info.argtypes = [vp, u32]
     L.rr_integrator_profile.argtypes = [vp, C.POINTER(C.c_uint64)]
+    L.rr_integrator_last.argtypes = [vp, u32]
     L.rr_draw_points.argtypes = [vp, C.POINTER(View), f32, f32]
     L.rr_draw_calibs.argtypes = [vp, C.POINTER(View), C.c_int, C.c_float, f32, f32]
     L.rr_draw_trigrid.argtypes = [vp, C.POINTER(View), C.c_float, f32, f32]
@@ -480,6 +484,13 @@ class Fusion:
                 "smem_bytes", "consumer_warps", "fill_warps", "flags", "slots", "slot_bytes")
         return {k: int(v) for k, v in zip(keys, out)}
 
+    def integrator_last(self):
+        """rr_integrator_last as a dict: the kernel the last integrate launched (path name), its sensors, voxel format, CTA
+        threads (consumer warps for the staged kernel) and repair bits (1: stale staged item lists, 2: gather packed late)."""
+        out = np.zeros(8, np.uint32)
+        self._ck(self.L.rr_integrator_last(self.h, _u32(out)))
+        return dict(path=INTEGRATE_PATHS[int(out[0])], sensors=int(out[1]), voxel_mode=int(out[2]), threads=int(out[3]), repairs=int(out[4]))
+
     def integrator_profile(self):
         """rr_integrator_profile: cycle counters of the staged integrator's roles (stage_debug bit 7), reset on read."""
         out = np.zeros(16, np.uint64)
@@ -589,12 +600,25 @@ class Group:
 
     def frame(self, filter_textures=True, use_processed_depth=True, refine=True):
         """The per-frame sequence call by call (kinect_client.cpp:572-600) on every member; returns (occupied, ratio)."""
+        self.bricks_clear()
+        self.preprocess(filter_textures, use_processed_depth, refine)
+        r = self.bricks_update()
+        self.integrate()
+        return r
+
+    def bricks_clear(self):
         self._ck(self.L.rr_group_bricks_clear(self.h))
+
+    def preprocess(self, filter_textures=True, use_processed_depth=True, refine=True):
         self._ck(self.L.rr_group_preprocess(self.h, int(filter_textures), int(use_processed_depth), int(refine)))
+
+    def bricks_update(self):
         n, r = C.c_uint32(), C.c_float()
         self._ck(self.L.rr_group_bricks_update(self.h, C.byref(n), C.byref(r)))
-        self._ck(self.L.rr_group_integrate(self.h))
         return int(n.value), float(r.value)
+
+    def integrate(self):
+        self._ck(self.L.rr_group_integrate(self.h))
 
     def fuse_frame(self, filter_textures=True, use_processed_depth=True, refine=True):
         self._ck(self.L.rr_group_fuse_frame(self.h, int(filter_textures), int(use_processed_depth), int(refine)))

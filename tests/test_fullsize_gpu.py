@@ -1,7 +1,7 @@
 """Parity at BASELINE.json's full size (4 sensors, 512x424 depth, 512^3 volume) through size-independent properties —
 the scalar oracle would need minutes per frame here, so it checks a sample of bricks and the rest is covered by
 identities between independent GPU paths:
-  * fused clear+integrate == k_fill + k_integrate_bricks (two different kernels), bit for bit;
+  * the TMA-staged clear+integrate kernel == k_fill + k_integrate_bricks (two different kernels), bit for bit;
   * dense integration == brick integration inside occupied bricks; outside them the brick path holds exactly -limit;
   * 2 z-slabs + composite == single volume (integration slices and the 1280x720 raymarched image);
   * the oracle, run on a random sample of occupied bricks only, agrees bit for bit with the volume."""
@@ -32,21 +32,25 @@ def _ctx(full, use_bricks=True):
     return fu
 
 
-def test_fullsize_paths_agree(full, monkeypatch):
+def test_fullsize_paths_agree(full):
     import oracle_py as O
-    b, sc = full["bench"], full["scene"]
+    b, capi, sc = full["bench"], full["capi"], full["scene"]
     fu = _ctx(full)
     assert tuple(fu.volume_res()) == (512, 512, 512)
     n_occ, ratio = fu.frame(sync_bricks=True)
+    assert fu.integrator_last()["path"] == "staged", fu.integrator_last()
     fused = fu.download_tsdf()
     counters, occ = fu.download_bricks()
     ranges = fu.brick_ranges()
     assert 100 < n_occ < 2000 and len(occ) == n_occ
     # (1) the two-kernel path
-    monkeypatch.setenv("RR_INTEGRATE_FUSED", "0")
-    fu.frame(sync_bricks=True)
-    unfused = fu.download_tsdf()
-    monkeypatch.delenv("RR_INTEGRATE_FUSED")
+    capi.set_tunable("fused", 0)
+    try:
+        fu.frame(sync_bricks=True)
+        assert fu.integrator_last()["path"] == "two_kernel", fu.integrator_last()
+        unfused = fu.download_tsdf()
+    finally:
+        capi.set_tunable("fused", 1)
     assert bits_equal(fused, unfused).all(), f"{(~bits_equal(fused, unfused)).sum()} voxels differ between fused and two-kernel paths"
     del unfused
     # (2) dense vs bricks

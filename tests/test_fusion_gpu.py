@@ -30,6 +30,7 @@ def _run_both(scene, voxel_size, inv_res, use_bricks, flags=(True, True, True), 
     got["res"] = fu.volume_res()
     got["brick_info"] = fu.brick_info()
     got["ranges"] = fu.brick_ranges()
+    got["last"] = fu.integrator_last()
     fu.close()
 
     grid = O.brick_grid(scene.bbox_min, scene.bbox_max, voxel_size, 0.1)
@@ -66,9 +67,15 @@ def _assert_frame(got, want, stages=("morph", "depth", "lab", "depth_b", "sil", 
 
 
 @pytest.mark.parametrize("fused", ["1", "0"])
-def test_frame_bricks_small(small_scene, fused, monkeypatch):
-    monkeypatch.setenv("RR_INTEGRATE_FUSED", fused)     # fused clear+integrate kernel vs k_fill + k_integrate_bricks
-    got, want = _run_both(small_scene, 0.02, (50, 55, 50), use_bricks=True)
+def test_frame_bricks_small(small_scene, fused):
+    # tunable fused: the staged / fused clear+integrate kernels (1) vs k_fill + k_integrate_bricks (0)
+    from rrpy import capi
+    capi.set_tunable("fused", int(fused))
+    try:
+        got, want = _run_both(small_scene, 0.02, (50, 55, 50), use_bricks=True)
+    finally:
+        capi.set_tunable("fused", 1)
+    assert got["last"]["path"] == ("staged" if fused == "1" else "two_kernel"), got["last"]
     assert len(want["occupied"]) > 20, "synthetic scene should occupy bricks"
     assert ((want["tsdf"] > -0.01) & (want["tsdf"] < 0.01)).sum() > 1000, "scene should produce a TSDF band"
     _assert_frame(got, want)

@@ -283,6 +283,43 @@ int rr_group_download_tsdf(rr_group* g, float* out);
 int rr_view_export(rr_ctx* ctx, int width, int height, void* out_handle);
 int rr_composite_peers(rr_ctx* ctx, const void* peer_handles, int n_peers, int width, int height, float* out_rgba, float* out_depth);
 
+/* ---- surface extraction (no reference counterpart: the reference only raymarches the volume) ---------------------------
+ * The fused surface as an indexed triangle mesh with per-vertex normals and colours, by marching cubes on the device.
+ *   Grid      corner (x, y, z) = the voxel centre; its value v is the density rr_raymarch reads (R32F, or the low half of a
+ *             half2 voxel widened; F32_WEIGHT: the tsdf volume only). Cell = the cube of corners x..x+1, y..y+1, z..z+1 for
+ *             x < X-1, y < Y-1, z < Z-1. Inside: v > 0 (the raymarch's hit test); outside: v <= 0. A cell with a
+ *             non-finite corner emits nothing.
+ *   Cases     generated from a rule, not transcribed: on each cube face two crossed edges give one segment, four crossed
+ *             edges the two segments that cut off the inside corners (so neighbouring cells agree along every face and the
+ *             mesh is crack-free); the segments are chained into loops oriented counter-clockwise seen from the outside,
+ *             so geometric normals point to free space; each loop is a fan from its lowest edge, loops by lowest edge.
+ *   Vertices  one per crossed edge (one end > 0, the other <= 0, both finite, on at least one emitting cell), ordered by
+ *             edge key (linear index of the lower corner a, then axis x < y < z). Along axis k from a to b:
+ *             t = va / (va - vb); texture coordinate q_k = ((float)i_k + 0.5f + t) / (float)R_k, the other two the voxel
+ *             centre ((float)i + 0.5f) * (1.0f / (float)R); position (metres) = bbox_min + q * (bbox_max - bbox_min),
+ *             binary32 without fused multiply-adds.
+ *             normal = normalize(g / (bbox_max - bbox_min)) with g the raymarch's gradient at q (step limit / 2, normalised,
+ *             negated; NaN where it vanishes); rgba = blendColors at q (shade mode 0's diffuse colour; alpha 1 when
+ *             quality-weighted, -1 for the fallback blend) from the limit, stage images and colour rr_raymarch would use now.
+ *   Triangles three uint32 vertex indices, ordered by cell linear index (z, y, x), then by table order within the cell.
+ * The order is canonical: it depends neither on scheduling, on the occupied-brick shortcut (in bricks mode only cells
+ * near occupied bricks are visited while the brick tables are the ones the volume was integrated with; otherwise every
+ * cell is) nor on the number of devices. The result always equals marching cubes over the volume rr_download_tsdf returns.
+ *
+ * rr_extract_mesh   extracts on the context's stream and synchronises once; returns the counts. RR_ERR_INVALID before any
+ *                   integrate into the current volume (an rr_configure that changes the resolution or the voxel format
+ *                   starts a new one; a new limit does not) and on a context restricted by rr_set_slab (use
+ *                   rr_group_extract_mesh); RR_ERR_UNSUPPORTED for 2^31 or more vertices or triangles. Changes nothing
+ *                   else: volume, view images, brick tables and captured frame graphs stay as they are.
+ * rr_download_mesh  the last extraction: positions float32 [V][3], normals float32 [V][3], rgba float32 [V][4], triangles
+ *                   uint32 [T][3], host, each may be NULL. RR_ERR_INVALID if nothing was extracted from the current volume.
+ * rr_group_extract_mesh  the same for a group, bit for bit: member 0 receives the other members' slabs by peer copies (one
+ *                   volume per call; its own unowned slices are overwritten, which nothing else reads) and extracts; read
+ *                   the mesh with rr_download_mesh(rr_group_member(g, 0), ...). */
+int rr_extract_mesh(rr_ctx* ctx, uint32_t* out_num_vertices, uint32_t* out_num_triangles);
+int rr_download_mesh(rr_ctx* ctx, float* positions, float* normals, float* rgba, uint32_t* triangles);
+int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out_num_triangles);
+
 /* ---- read-back (tests, debug views) ------------------------------------------------------------------------ */
 int rr_download_tsdf(rr_ctx* ctx, float* out);
 int rr_download_weight(rr_ctx* ctx, float* out);

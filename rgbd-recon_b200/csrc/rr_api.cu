@@ -142,6 +142,7 @@ int rr_create(rr_ctx** out, int device, int num_sensors, int depth_w, int depth_
   if (rc == RR_OK) rc = dev_alloc(c, &c->d_num_occ, 1, "num_occ");
   if (rc == RR_OK) rc = dev_alloc(c, &c->d_work, 4, "work counters");
   if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_num_occ, sizeof(uint32_t)), "pinned count");
+  if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_mesh_totals, 2 * sizeof(unsigned long long)), "pinned mesh totals");
   if (rc == RR_OK) {
     cudaMemsetAsync(c->d_flags, 0, 4 * sizeof(uint32_t), c->stream);
     cudaMemsetAsync(c->d_pairs, 0, (size_t)c->N * (c->H + 2) * c->pair_pitch * sizeof(float2), c->stream);
@@ -173,6 +174,7 @@ void rr_destroy(rr_ctx* c) {
   cudaFree(c->d_lab); cudaFree(c->d_depth_b); cudaFree(c->d_sil); cudaFree(c->d_normal); cudaFree(c->d_quality);
   staged_release(c);
   trigrid_release(c);
+  mesh_release(c);
   for (auto& v : c->ipc_views) { cudaIpcCloseMemHandle(v.step); cudaIpcCloseMemHandle(v.rgba); cudaIpcCloseMemHandle(v.zbuf); cudaIpcCloseMemHandle(v.nsamp); }
   cudaGetLastError();
   cudaFree(c->d_pairs);
@@ -321,7 +323,12 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     for (int a = 0; a < 3; ++a) c->res[a] = res[a];
     c->slab_z0 = 0; c->slab_z1 = res[2];
   }
+  if (new_volume || cfg->store_weight != c->cfg.store_weight) {   // a new volume allocation as far as extraction goes
+    c->volume_integrated = false;
+    c->mesh_valid = false;
+  }
   if (new_bricks) {
+    c->mesh_rows_ok = false;
     uint32_t rb[3];
     const uint32_t nb = host_divide_box(c->bbox_min, c->bbox_max, bs, res, rb, &c->h_ranges);
     c->bricks.brick_size = bs; c->bricks.num = nb;
@@ -572,6 +579,8 @@ int rr_fuse_frame(rr_ctx* c, int filter_textures, int use_processed_depth, int r
   for (auto& g : c->frame_graphs)
     if (g.key == key) {
       c->launches += g.launches;
+      c->volume_integrated = true;                 // the captured frame ends with the integrate launch_integrate recorded
+      c->mesh_rows_ok = mesh_rows_usable(c);
       return check(c, cudaGraphLaunch(g.exec, c->stream), "frame graph launch");
     }
   if (c->frame_graphs.size() >= 16) drop_frame_graphs(c);          // stale tunable generations
@@ -880,6 +889,28 @@ int rr_download_hit_positions(rr_ctx* c, float* out) {
   if (!c) return RR_ERR_INVALID;
   RR_REQUIRE(c, out && c->d_pos, "rr_download_hit_positions: no raymarch yet");
   return download(c, out, c->d_pos, (size_t)c->view_w * c->view_h * sizeof(float4), "positions download");
+}
+
+int rr_extract_mesh(rr_ctx* c, uint32_t* out_num_vertices, uint32_t* out_num_triangles) {
+  if (!c) return RR_ERR_INVALID;
+  RR_TRY(require_ready(c, true));
+  RR_REQUIRE(c, c->volume_integrated, "rr_extract_mesh: nothing has been integrated into the current volume");
+  RR_REQUIRE(c, c->slab_z0 == 0 && c->slab_z1 == c->res[2],
+             "rr_extract_mesh: this context holds only its z-slab (rr_set_slab); extract through rr_group_extract_mesh");
+  RR_SET_DEVICE(c);
+  return launch_extract_mesh(c, out_num_vertices, out_num_triangles);
+}
+
+int rr_download_mesh(rr_ctx* c, float* positions, float* normals, float* rgba, uint32_t* triangles) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, c->mesh_valid, "rr_download_mesh: no mesh extracted from the current volume (rr_extract_mesh first)");
+  RR_SET_DEVICE(c);
+  const size_t nv = c->mesh_nv, nt = c->mesh_nt;
+  if (positions && nv) RR_TRY(check(c, cudaMemcpyAsync(positions, c->d_mesh_pos, nv * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
+  if (normals && nv) RR_TRY(check(c, cudaMemcpyAsync(normals, c->d_mesh_nrm, nv * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
+  if (rgba && nv) RR_TRY(check(c, cudaMemcpyAsync(rgba, c->d_mesh_rgba, nv * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
+  if (triangles && nt) RR_TRY(check(c, cudaMemcpyAsync(triangles, c->d_mesh_tri, nt * 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
+  return check(c, cudaStreamSynchronize(c->stream), "mesh download sync");
 }
 
 int rr_set_timing(rr_ctx* c, int level) {

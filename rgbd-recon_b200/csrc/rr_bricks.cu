@@ -122,6 +122,7 @@ int launch_bricks_update(rr_ctx* c) {
   RR_LAUNCH_CHECK(c, "k_bricks_update");
   timer_end(c, "bricks");
   c->work_fresh = true;
+  c->mesh_rows_ok = false;     // new row tables: the volume was cleared by the previous ones
   if (classify) c->sti.lists_key = staged_lists_key(c);
   cudaError_t e = cudaMemcpyAsync(c->h_num_occ, c->d_num_occ, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream);
   return check(c, e, "bricks count copy");

@@ -197,6 +197,19 @@ struct rr_ctx {
   float4* d_tg_frag_rgba = nullptr; float4* d_tg_frag_pos = nullptr; uint2* d_tg_frag_link = nullptr; size_t tg_frag_cap = 0;
   uint32_t* d_tg_count = nullptr;
 
+  // surface extraction (rr_mesh.cu)
+  bool volume_integrated = false;  // an integrate has run into the current volume allocation
+  bool mesh_rows_ok = false;       // rowany / cand_y / cand_z are the tables the last integrate cleared the volume by
+  bool mesh_table = false;         // the case table is in this device's constant memory
+  bool mesh_valid = false;         // the d_mesh_* arrays hold an extraction of the current volume allocation
+  uint32_t mesh_nv = 0, mesh_nt = 0;
+  unsigned long long* d_mesh_rows = nullptr; size_t mesh_rows_cap = 0;   // per row: counts and offsets of vertices, triangles
+  uint8_t* d_mesh_scratch = nullptr; size_t mesh_scratch_cap = 0;        // CUB scan storage
+  unsigned long long* d_mesh_keys = nullptr;   // [V] edge key = linear index of the lower corner * 3 + axis
+  float* d_mesh_pos = nullptr; float* d_mesh_nrm = nullptr; float4* d_mesh_rgba = nullptr; size_t mesh_v_cap = 0;
+  uint32_t* d_mesh_tri = nullptr; size_t mesh_t_cap = 0;
+  unsigned long long* h_mesh_totals = nullptr;   // pinned [2]: vertices, triangles
+
   // colour hole filling (rr_colorfill.cu): atlas right of column W, squeezed copy, filled colour
   int fill_w = 0, fill_h = 0;
   float4* d_fill_fc = nullptr; float* d_fill_fd = nullptr;
@@ -257,6 +270,9 @@ int launch_fill_colors(rr_ctx* c);
 int launch_draw_points(rr_ctx* c, const rr_view* v, int mode, float calib_limit);   // rr_points.cu
 int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length);             // rr_trigrid.cu
 void trigrid_release(rr_ctx* c);
+int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt);   // rr_mesh.cu: the whole volume, ignoring the slab
+bool mesh_rows_usable(const rr_ctx* c);   // the last integrate cleared everything outside the occupied bricks of the row tables
+void mesh_release(rr_ctx* c);
 int launch_unpack_frames(rr_ctx* c, int slot);
 int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4* d_out);
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines

@@ -12,8 +12,7 @@
 // Filtering is software fp32 (x -> y -> z lerps), see rr_math.cuh.
 #include "rr_context.h"
 #include "rr_math.cuh"
-
-#include <cuda_fp16.h>
+#include "rr_sample.cuh"
 
 #include <cmath>
 
@@ -55,68 +54,9 @@ __device__ __forceinline__ bool slab(float3 o, float3 invd, float3 lo, float3 hi
   return t0 <= t1;
 }
 
-// One voxel's density: R32F, or the low half of a half2 (tsdf, weight) voxel widened exactly (warp-uniform branch).
-__device__ __forceinline__ float ld_density(const RayParams& p, unsigned i) {
-  if (p.half2) {
-    const uint32_t u = __ldg(reinterpret_cast<const uint32_t*>(p.tsdf) + i);
-    return __half2float(__ushort_as_half((unsigned short)(u & 0xffffu)));
-  }
-  return __ldg(p.tsdf + i);
-}
-
-__device__ __forceinline__ float sample_tsdf(const RayParams& p, float3 q) {
-  int x0, x1, y0, y1, z0, z1; float a, b, g;
-  lin_coord(q.x, p.X, x0, x1, a);
-  lin_coord(q.y, p.Y, y0, y1, b);
-  lin_coord(q.z, p.Z, z0, z1, g);
-  const unsigned sy = (unsigned)p.X, sz = (unsigned)(p.X * p.Y);
-  const float c00 = lerpf(ld_density(p, z0 * sz + y0 * sy + x0), ld_density(p, z0 * sz + y0 * sy + x1), a);
-  const float c10 = lerpf(ld_density(p, z0 * sz + y1 * sy + x0), ld_density(p, z0 * sz + y1 * sy + x1), a);
-  const float c01 = lerpf(ld_density(p, z1 * sz + y0 * sy + x0), ld_density(p, z1 * sz + y0 * sy + x1), a);
-  const float c11 = lerpf(ld_density(p, z1 * sz + y1 * sy + x0), ld_density(p, z1 * sz + y1 * sy + x1), a);
-  return lerpf(lerpf(c00, c10, b), lerpf(c01, c11, b), g);
-}
-
-__device__ __forceinline__ float tex_nearest_depth(const float2* img, int W, int H, float s, float t) {
-  return __ldg(img + (size_t)near_coord(t, H) * W + near_coord(s, W)).x;
-}
-
-__device__ __forceinline__ float tex_linear_1(const float* img, int W, int H, float s, float t) {
-  int x0, x1, y0, y1; float a, b;
-  lin_coord(s, W, x0, x1, a);
-  lin_coord(t, H, y0, y1, b);
-  const float v00 = __ldg(img + (size_t)y0 * W + x0), v10 = __ldg(img + (size_t)y0 * W + x1);
-  const float v01 = __ldg(img + (size_t)y1 * W + x0), v11 = __ldg(img + (size_t)y1 * W + x1);
-  return lerpf(lerpf(v00, v10, a), lerpf(v01, v11, a), b);
-}
-
 __constant__ float kCameraColors[5][3] = {{228.f / 255.f, 26.f / 255.f, 28.f / 255.f}, {55.f / 255.f, 126.f / 255.f, 184.f / 255.f},
                                           {77.f / 255.f, 175.f / 255.f, 74.f / 255.f}, {152.f / 255.f, 78.f / 255.f, 163.f / 255.f},
                                           {255.f / 255.f, 127.f / 255.f, 0.f / 255.f}};
-
-// tsdf_raymarch.fs:303-338 blendColors
-__device__ float4 blend_colors(const RayParams& p, float3 q) {
-  float3 tc = make_float3(0.f, 0.f, 0.f), tc2 = make_float3(0.f, 0.f, 0.f);
-  float tw = 0.0f, tw2 = 0.0f;
-  const size_t inv_stride = (size_t)p.IX * p.IY * p.IZ, img = (size_t)p.W * p.H;
-  for (int i = 0; i < p.N; ++i) {
-    const float3 pc = tex3d_xyz(p.inv + inv_stride * i, p.IX, p.IY, p.IZ, q.x, q.y, q.z);
-    const float2 uv = tex3d_uv(p.uv[i], p.cx[i], p.cy[i], p.cz[i], pc.x, pc.y, pc.z);
-    const float3 col = tex2d_rgb8(p.color + (size_t)p.CW * p.CH * 3 * i, p.CW, p.CH, uv.x, uv.y);
-    const float depth = tex_nearest_depth(p.depth_b + img * i, p.W, p.H, pc.x, pc.y);
-    const float dist = fabsf(depth - pc.z);
-    float quality = 0.0f;
-    if (dist < p.limit) quality = tex_linear_1(p.quality + img * i, p.W, p.H, pc.x, pc.y);
-    const float den = dist + 0.01f;
-    tc = tc + (col * quality) / den;
-    tw += quality / den;
-    tc2 = tc2 + col / dist;
-    tw2 += 1.0f / dist;
-  }
-  if (tw > 0.0f) { tc = tc / tw; return make_float4(tc.x, tc.y, tc.z, 1.0f); }
-  tc2 = tc2 / tw2;
-  return make_float4(tc2.x, tc2.y, tc2.z, -1.0f);
-}
 
 // tsdf_raymarch.fs:354-369 blendCameras (+ getWeights :159-174)
 __device__ float3 blend_cameras(const RayParams& p, float3 q) {
@@ -305,11 +245,8 @@ __global__ void __launch_bounds__(64) k_raymarch(const __grid_constant__ RayPara
       hit_step = num_samples;
       // submitFragment (tsdf_raymarch.fs:116-142); get_gradient :148-157
       const float3 q = sample_pos;
-      const float3 gv = make_float3(sample_tsdf(p, make_float3(q.x + sd, q.y, q.z)) - sample_tsdf(p, make_float3(q.x - sd, q.y, q.z)),
-                                    sample_tsdf(p, make_float3(q.x, q.y + sd, q.z)) - sample_tsdf(p, make_float3(q.x, q.y - sd, q.z)),
-                                    sample_tsdf(p, make_float3(q.x, q.y, q.z + sd)) - sample_tsdf(p, make_float3(q.x, q.y, q.z - sd)));
-      const float3 gn = normalize3(gv);
-      const float4 vn4 = mulv(p.normal_matrix, make_float4(-gn.x, -gn.y, -gn.z, 0.0f));
+      const float3 gn = get_gradient(p, q, sd);
+      const float4 vn4 = mulv(p.normal_matrix, make_float4(gn.x, gn.y, gn.z, 0.0f));
       const float3 view_normal = normalize3(make_float3(vn4.x, vn4.y, vn4.z));
       const float4 vp4 = mulv(p.mv_v2w, make_float4(q.x, q.y, q.z, 1.0f));
       const float3 view_pos = make_float3(vp4.x, vp4.y, vp4.z);

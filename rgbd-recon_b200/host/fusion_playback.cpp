@@ -1,8 +1,9 @@
 // fusion_playback — headless equivalent of kinect_client's init() + frame loop (source/kinect_client.cpp:194-279,
 // 572-617) for the TSDF-integration mode: plays .stream files through NetKinectArray, fuses every frame set and
-// raymarches it. Prints the TimerDatabase stage means; optionally dumps the last TSDF volume and image.
+// raymarches it. Prints the TimerDatabase stage means; optionally dumps the last TSDF volume, image and surface mesh.
 //   fusion_playback <file.ks> (--streams "s0;s1;..." | --messages file) [--depth W H --color CW CH] [--frames K] [--voxel m]
 //                   [--limit l] [--eye x y z | --matrices file] [--view W H] [--shade m] [--dump-tsdf file] [--dump-image file] [--dense]
+//                   [--dump-mesh file.ply]
 //                   [--gpus N | --devices a,b,...] [--recon points|trigrid|calibs [--min-length m] [--dump-recon file]]
 // --recon: like kinect_client's reconstruction list (source/kinect_client.cpp:251-257, key-selected g_recon_mode), one of the
 // other reconstructions also draws the last frame set's maps - ReconPoints, ReconTrigrid (min_length from the sensor .yml
@@ -10,6 +11,7 @@
 // --gpus N / --devices: the volume is split into z-slabs over several devices in this one process (rr_group: frame sets by
 // peer copies from the first device, per-slab integration, the view composited on the first device); after the first frame
 // the slabs are re-cut to equal integrate cost. A device may be named more than once (slabs sharing a GPU).
+// --dump-mesh: the last frame set's fused surface (ReconIntegration::extractMesh) as a binary PLY with normals and colours.
 // Without --depth/--color the sizes and stream formats (DXT1 colour, 8-bit depth, near/far) come from the sensors' .yml
 // files like in the reference (CalibrationFiles, calibration_files.cpp:7-34). --messages plays a file of back-to-back
 // server messages (the ZMQ payload layout of NetKinectArray::readLoop, :511-538) through NetKinectArray::pushMessage.
@@ -44,7 +46,7 @@ static void perspective(float fovy_deg, float aspect, float n, float f, float m[
 }
 
 int main(int argc, char** argv) {
-  std::string ks, streams, messages, dump_tsdf, dump_image, matrices, recon_mode, dump_recon;
+  std::string ks, streams, messages, dump_tsdf, dump_image, dump_mesh, matrices, recon_mode, dump_recon;
   float min_length = 0.0f;
   bool explicit_sizes = false;
   unsigned W = 512, H = 424, CW = 1280, CH = 1080, VW = 1280, VH = 720;
@@ -66,6 +68,7 @@ int main(int argc, char** argv) {
     else if (!std::strcmp(argv[i], "--shade")) shade = std::atoi(argv[++i]);
     else if (!std::strcmp(argv[i], "--dump-tsdf")) dump_tsdf = argv[++i];
     else if (!std::strcmp(argv[i], "--dump-image")) dump_image = argv[++i];
+    else if (!std::strcmp(argv[i], "--dump-mesh")) dump_mesh = argv[++i];
     else if (!std::strcmp(argv[i], "--dense")) dense = true;
     else if (!std::strcmp(argv[i], "--gpus")) { devices.clear(); for (int d = 0, n = std::atoi(argv[++i]); d < n; ++d) devices.push_back(d); }
     else if (!std::strcmp(argv[i], "--devices")) {
@@ -145,6 +148,12 @@ int main(int argc, char** argv) {
       std::vector<float> tsdf;
       recon.downloadTsdf(tsdf);
       std::ofstream(dump_tsdf, std::ios::binary).write(reinterpret_cast<char const*>(tsdf.data()), (std::streamsize)(tsdf.size() * sizeof(float)));
+    }
+    if (!dump_mesh.empty()) {
+      Mesh mesh;
+      recon.extractMesh(mesh);
+      writePly(dump_mesh, mesh);
+      std::cout << "mesh vertices " << mesh.positions.size() / 3 << " triangles " << mesh.triangles.size() / 3 << std::endl;
     }
     if (!recon_mode.empty()) {
       // the other reconstructions consume the maps of the last processTextures() (and, ReconCalibs, the fused volume)

@@ -380,6 +380,45 @@ void ReconIntegration::downloadTsdf(std::vector<float>& out) const {
   gk(rr_group_download_tsdf(grp(), out.data()), "rr_download_tsdf");
 }
 
+void ReconIntegration::extractMesh(Mesh& out) const {
+  uint32_t nv = 0, nt = 0;
+  if (gpu::Context::current().numDevices() > 1) gk(rr_group_extract_mesh(grp(), &nv, &nt), "rr_group_extract_mesh");
+  else ck(rr_extract_mesh(ctx(), &nv, &nt), "rr_extract_mesh");
+  out.positions.resize((std::size_t)nv * 3); out.normals.resize((std::size_t)nv * 3); out.rgba.resize((std::size_t)nv * 4);
+  out.triangles.resize((std::size_t)nt * 3);
+  ck(rr_download_mesh(ctx(), out.positions.data(), out.normals.data(), out.rgba.data(), out.triangles.data()), "rr_download_mesh");
+}
+
+void writePly(std::string const& path, Mesh const& mesh) {
+  const std::size_t nv = mesh.positions.size() / 3, nt = mesh.triangles.size() / 3;
+  std::ofstream o(path, std::ios::binary);
+  if (!o) throw std::runtime_error("cannot write " + path);
+  o << "ply\nformat binary_little_endian 1.0\ncomment fused surface (rr_extract_mesh)\n"
+    << "element vertex " << nv << "\nproperty float x\nproperty float y\nproperty float z\n"
+    << "property float nx\nproperty float ny\nproperty float nz\n"
+    << "property uchar red\nproperty uchar green\nproperty uchar blue\n"
+    << "element face " << nt << "\nproperty list uchar uint vertex_indices\nend_header\n";
+  static_assert(sizeof(float) == 4 && sizeof(uint32_t) == 4, "PLY float / uint are 4 bytes");
+  std::vector<char> buf;
+  buf.reserve(nv * 27 + nt * 13);
+  auto put = [&](void const* p, std::size_t n) { buf.insert(buf.end(), static_cast<char const*>(p), static_cast<char const*>(p) + n); };
+  for (std::size_t i = 0; i < nv; ++i) {
+    put(&mesh.positions[i * 3], 12);
+    put(&mesh.normals[i * 3], 12);
+    for (int c = 0; c < 3; ++c) {
+      float v = mesh.rgba[i * 4 + c];
+      v = v > 0.0f ? v : 0.0f;                 // NaN -> 0
+      v = v < 1.0f ? v : 1.0f;
+      const uint8_t b = (uint8_t)(v * 255.0f + 0.5f);
+      put(&b, 1);
+    }
+  }
+  const uint8_t three = 3;
+  for (std::size_t t = 0; t < nt; ++t) { put(&three, 1); put(&mesh.triangles[t * 3], 12); }
+  o.write(buf.data(), (std::streamsize)buf.size());
+  if (!o) throw std::runtime_error("cannot write " + path);
+}
+
 // ---------------------------------------------------------------------------------------------------- TimerDatabase
 TimerDatabase& TimerDatabase::instance() { static TimerDatabase t; return t; }
 void TimerDatabase::enable(int level) const { gk(rr_group_set_timing(grp(), level), "rr_set_timing"); }

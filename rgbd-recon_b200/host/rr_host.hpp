@@ -284,6 +284,18 @@ class Reconstruction {
   rr_view m_view;
 };
 
+// ---- surface extraction (no reference counterpart): the fused surface as an indexed, coloured triangle mesh ---------------
+// The arrays of rr_download_mesh (include/rgbd_recon_b200.h states what they hold).
+struct Mesh {
+  std::vector<float> positions;      // [V][3] metres
+  std::vector<float> normals;        // [V][3] unit length, or NaN where the gradient vanishes
+  std::vector<float> rgba;           // [V][4] blendColors; alpha 1 quality-weighted, -1 the fallback blend
+  std::vector<uint32_t> triangles;   // [T][3] vertex indices, counter-clockwise seen from free space
+};
+// Binary little-endian PLY: vertex "float x y z nx ny nz uchar red green blue", face "list uchar uint vertex_indices".
+// Colour byte = (uint8)(min(max(c, 0), 1) * 255 + 0.5f), a NaN channel counting as 0. Throws if the file cannot be written.
+void writePly(std::string const& path, Mesh const& mesh);
+
 // ---- framework/reconstruction/recon_integration.hpp:33-107 ------------------------------------------------------------
 class ReconIntegration : public Reconstruction {
  public:
@@ -309,6 +321,8 @@ class ReconIntegration : public Reconstruction {
   std::vector<float> const& colorImage() const { return m_rgba; }   // RGBA32F, viewport w*h, row 0 = bottom (GL window coords)
   std::vector<float> const& depthImage() const { return m_depth; }  // gl_FragDepth, 1.0 where no surface
   void downloadTsdf(std::vector<float>& out) const;
+  // marching cubes over the fused volume on the device (rr_extract_mesh; with several devices rr_group_extract_mesh)
+  void extractMesh(Mesh& out) const;
  private:
   void configure();
   rr_config m_cfg;

@@ -135,6 +135,9 @@ def lib():
     L.rr_group_raymarch.argtypes = [vp, C.POINTER(View), f32, f32]
     L.rr_group_fill_colors.argtypes = [vp, f32]
     L.rr_group_download_tsdf.argtypes = [vp, f32]
+    L.rr_extract_mesh.argtypes = [vp, u32, u32]
+    L.rr_download_mesh.argtypes = [vp, f32, f32, f32, u32]
+    L.rr_group_extract_mesh.argtypes = [vp, u32, u32]
     L.rr_launch_count.argtypes = [vp]
     L.rr_launch_count.restype = C.c_uint64
     L.rr_version.restype = C.c_int
@@ -462,6 +465,24 @@ class Fusion:
         self._ck(self.L.rr_download_hit_positions(self.h, _f32(out)))
         return out
 
+    def extract_mesh_counts(self):
+        """rr_extract_mesh alone: extracts the surface on the device and returns (vertices, triangles)."""
+        nv, nt = C.c_uint32(), C.c_uint32()
+        self._ck(self.L.rr_extract_mesh(self.h, C.byref(nv), C.byref(nt)))
+        return int(nv.value), int(nt.value)
+
+    def download_mesh(self, nv, nt):
+        """rr_download_mesh of the last extraction (nv, nt: its counts)."""
+        pos, nrm = np.zeros((nv, 3), np.float32), np.zeros((nv, 3), np.float32)
+        rgba, tri = np.zeros((nv, 4), np.float32), np.zeros((nt, 3), np.uint32)
+        self._ck(self.L.rr_download_mesh(self.h, _f32(pos), _f32(nrm), _f32(rgba), _u32(tri)))
+        return pos, nrm, rgba, tri
+
+    def extract_mesh(self):
+        """The fused surface as a mesh (rr_extract_mesh + rr_download_mesh): positions float32 [V, 3] (metres), normals
+        float32 [V, 3], rgba float32 [V, 4] (alpha 1 quality-weighted colour, -1 fallback blend), triangles uint32 [T, 3]."""
+        return self.download_mesh(*self.extract_mesh_counts())
+
     def set_timing(self, level=1):
         self._ck(self.L.rr_set_timing(self.h, int(level)))
 
@@ -659,6 +680,16 @@ class Group:
         out = np.zeros((int(r[2]), int(r[1]), int(r[0])), np.float32)
         self._ck(self.L.rr_group_download_tsdf(self.h, _f32(out)))
         return out
+
+    def extract_mesh_counts(self):
+        """rr_group_extract_mesh: the whole volume's surface, extracted on member 0; returns (vertices, triangles)."""
+        nv, nt = C.c_uint32(), C.c_uint32()
+        self._ck(self.L.rr_group_extract_mesh(self.h, C.byref(nv), C.byref(nt)))
+        return int(nv.value), int(nt.value)
+
+    def extract_mesh(self):
+        """As Fusion.extract_mesh, equal to a single context's bit for bit: (positions, normals, rgba, triangles)."""
+        return self.member(0).download_mesh(*self.extract_mesh_counts())
 
 
 def load_scene(fu: "Fusion", scene, inv=None):

@@ -320,6 +320,49 @@ int rr_extract_mesh(rr_ctx* ctx, uint32_t* out_num_vertices, uint32_t* out_num_t
 int rr_download_mesh(rr_ctx* ctx, float* positions, float* normals, float* rgba, uint32_t* triangles);
 int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out_num_triangles);
 
+/* ---- queries (no reference counterpart: a reference user renders a view and reads pixels back) ------------------------
+ * The fused volume evaluated at points and along rays the caller chooses: picking, collision tests, measurements.
+ *   space      RR_QUERY_WORLD: coordinates in metres; a point becomes q = (p - bbox_min) / (bbox_max - bbox_min) (one IEEE
+ *              division per component, no fused multiply-add), a direction normalize(d / (bbox_max - bbox_min)).
+ *              RR_QUERY_VOLUME: volume texture coordinates, [0,1]^3 over the bbox (as rr_download_hit_positions); points
+ *              are used as given, directions are normalised. normalize is the raymarch's (v * (1 / sqrt(dot(v, v)))).
+ *   rr_sample_points  per point: value = the density rr_raymarch reads at q (trilinear; the low half of a half2 voxel);
+ *              normal = normalize(g / (bbox_max - bbox_min)) with g the raymarch's gradient at q (step limit / 2), always
+ *              in world space (the mesh vertex normal; NaN where it vanishes); rgba = blendColors at q (alpha 1 when
+ *              quality-weighted, -1 for the fallback blend). Outside the closed unit cube, or for a non-finite input, value
+ *              and normal are NaN and rgba is 0. Arrays: points float32 [n][3]; values [n], normals [n][3], rgba [n][4].
+ *   rr_cast_rays  per ray: rr_raymarch's own march from origin q0 along the normalised direction - live only if the ray
+ *              meets the unit cube ahead of q0; it starts at the cube entry (at q0 when q0 is inside), or runs over the
+ *              occupied-brick hull when the raymarch would skip space; steps of limit / 2, the raymarch's hit refinement and
+ *              empty-space fetch skipping, with the brick tables rr_raymarch would use now. positions = the refined hit in the
+ *              input's space (world: bbox_min + q * (bbox_max - bbox_min), no fused multiply-add); normals and rgba as for
+ *              points, at the hit; steps = the raymarch's sample count at the hit. Any finite non-zero direction is a ray:
+ *              when dot(d, d) (after the division by the bbox size in world space) overflows binary32 or falls below 2^-100,
+ *              d is first scaled by an exact power of two (2^-70; or 2^64, at most twice), so it casts as the same direction
+ *              of ordinary length. A ray without a hit - also one with a zero or non-finite direction or origin, or an origin
+ *              farther than 2^24 bbox sizes (|q0_k| > 2^24), whose march length binary32 cannot resolve - gets NaN positions
+ *              and normals, rgba 0 and step 0xFFFFFFFF. Never shaded. Arrays: origins, directions float32 [n][3]; positions [n][3], normals [n][3], rgba [n][4], steps
+ *              uint32 [n].
+ * Every pointer may be host memory (pageable or pinned) or device memory of the context's GPU (for a group: of member 0's
+ * GPU); each output may be NULL. The call runs on the context's stream and returns after one synchronisation. count == 0
+ * does nothing and returns RR_OK. RR_ERR_INVALID for a bad space, NULL inputs, a call before anything was integrated into
+ * the current volume (as rr_extract_mesh) and a context restricted by rr_set_slab (use the group form);
+ * RR_ERR_UNSUPPORTED for count >= 2^31. A query is not a setting: the volume, brick tables, view images (rr_fill_colors
+ * still fills the last view), mesh and captured frame graphs stay as they are.
+ * rr_group_sample_points / rr_group_cast_rays  the same for a group, equal to a single context bit for bit without moving the
+ *              volume: every member marches every ray over the samples it owns and evaluates its own first hit, and one
+ *              kernel on member 0 keeps each ray's smallest step (lowest member on ties); a point is evaluated by the member
+ *              owning its nearest z slice. Member 0 reads the other members' results through peer memory: RR_ERR_UNSUPPORTED
+ *              when it cannot address a member's device. */
+#define RR_QUERY_WORLD 0
+#define RR_QUERY_VOLUME 1
+int rr_sample_points(rr_ctx* ctx, int space, const float* points, uint32_t count, float* values, float* normals, float* rgba);
+int rr_cast_rays(rr_ctx* ctx, int space, const float* origins, const float* directions, uint32_t count,
+                 float* positions, float* normals, float* rgba, uint32_t* steps);
+int rr_group_sample_points(rr_group* g, int space, const float* points, uint32_t count, float* values, float* normals, float* rgba);
+int rr_group_cast_rays(rr_group* g, int space, const float* origins, const float* directions, uint32_t count,
+                       float* positions, float* normals, float* rgba, uint32_t* steps);
+
 /* ---- read-back (tests, debug views) ------------------------------------------------------------------------ */
 int rr_download_tsdf(rr_ctx* ctx, float* out);
 int rr_download_weight(rr_ctx* ctx, float* out);

@@ -175,6 +175,7 @@ void rr_destroy(rr_ctx* c) {
   staged_release(c);
   trigrid_release(c);
   mesh_release(c);
+  query_release(c);
   for (auto& v : c->ipc_views) { cudaIpcCloseMemHandle(v.step); cudaIpcCloseMemHandle(v.rgba); cudaIpcCloseMemHandle(v.zbuf); cudaIpcCloseMemHandle(v.nsamp); }
   cudaGetLastError();
   cudaFree(c->d_pairs);
@@ -899,6 +900,45 @@ int rr_extract_mesh(rr_ctx* c, uint32_t* out_num_vertices, uint32_t* out_num_tri
              "rr_extract_mesh: this context holds only its z-slab (rr_set_slab); extract through rr_group_extract_mesh");
   RR_SET_DEVICE(c);
   return launch_extract_mesh(c, out_num_vertices, out_num_triangles);
+}
+
+}  // extern "C"
+
+// The checks rr_sample_points / rr_cast_rays share with their group forms (whole_volume = false: a group member, which
+// holds only its slab). RR_OK: go ahead with count > 0 entries.
+int rr::query_check(rr_ctx* c, int space, uint32_t count, bool have_inputs, bool whole_volume, const char* who) {
+  const std::string w(who);
+  RR_REQUIRE(c, space == RR_QUERY_WORLD || space == RR_QUERY_VOLUME, w + ": space must be RR_QUERY_WORLD or RR_QUERY_VOLUME");
+  RR_REQUIRE(c, have_inputs, w + ": null inputs");
+  if (count >= (1u << 31)) return fail(c, RR_ERR_UNSUPPORTED, w + ": 2^31 or more entries are not supported");
+  RR_TRY(require_ready(c, true));
+  RR_REQUIRE(c, c->volume_integrated, w + ": nothing has been integrated into the current volume");
+  if (whole_volume)
+    RR_REQUIRE(c, c->slab_z0 == 0 && c->slab_z1 == c->res[2], w + ": this context holds only its z-slab (rr_set_slab); use the group form");
+  return RR_OK;
+}
+
+extern "C" {
+
+int rr_sample_points(rr_ctx* c, int space, const float* points, uint32_t count, float* values, float* normals, float* rgba) {
+  if (!c) return RR_ERR_INVALID;
+  if (count == 0 && (space == RR_QUERY_WORLD || space == RR_QUERY_VOLUME)) return RR_OK;
+  RR_TRY(query_check(c, space, count, points != nullptr, true, "rr_sample_points"));
+  RR_SET_DEVICE(c);
+  RR_TRY(query_upload(c, points, nullptr, count));
+  RR_TRY(launch_sample_points(c, space, count));
+  return query_download(c, count, false, values, normals, rgba, nullptr);
+}
+
+int rr_cast_rays(rr_ctx* c, int space, const float* origins, const float* directions, uint32_t count,
+                 float* positions, float* normals, float* rgba, uint32_t* steps) {
+  if (!c) return RR_ERR_INVALID;
+  if (count == 0 && (space == RR_QUERY_WORLD || space == RR_QUERY_VOLUME)) return RR_OK;
+  RR_TRY(query_check(c, space, count, origins && directions, true, "rr_cast_rays"));
+  RR_SET_DEVICE(c);
+  RR_TRY(query_upload(c, origins, directions, count));
+  RR_TRY(launch_cast_rays(c, space, count));
+  return query_download(c, count, true, positions, normals, rgba, steps);
 }
 
 int rr_download_mesh(rr_ctx* c, float* positions, float* normals, float* rgba, uint32_t* triangles) {

@@ -29,6 +29,7 @@
 #include "../../include/rgbd_recon_b200.h"
 
 #define RR_MAX_SENSORS 8
+#define RR_MAX_GROUP 16           // members of an rr_group
 
 namespace rr {
 
@@ -210,6 +211,11 @@ struct rr_ctx {
   uint32_t* d_mesh_tri = nullptr; size_t mesh_t_cap = 0;
   unsigned long long* h_mesh_totals = nullptr;   // pinned [2]: vertices, triangles
 
+  // queries (rr_query.cu): inputs (points [n][3], or origins [n][3] then directions [n][3]) and per-entry results, one
+  // capacity in entries, grown on demand
+  float* d_q_in = nullptr; float* d_q_val = nullptr; float* d_q_pos = nullptr; float* d_q_nrm = nullptr;
+  float4* d_q_rgba = nullptr; uint32_t* d_q_step = nullptr; size_t q_cap = 0;
+
   // colour hole filling (rr_colorfill.cu): atlas right of column W, squeezed copy, filled colour
   int fill_w = 0, fill_h = 0;
   float4* d_fill_fc = nullptr; float* d_fill_fd = nullptr;
@@ -273,6 +279,17 @@ void trigrid_release(rr_ctx* c);
 int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt);   // rr_mesh.cu: the whole volume, ignoring the slab
 bool mesh_rows_usable(const rr_ctx* c);   // the last integrate cleared everything outside the occupied bricks of the row tables
 void mesh_release(rr_ctx* c);
+// rr_query.cu: rr_sample_points / rr_cast_rays. query_upload copies the inputs (b: the directions, NULL for points) into
+// d_q_in, the launchers evaluate the context's own slab (a group member evaluates only what it owns), query_download
+// copies the requested results out and synchronises once.
+int query_check(rr_ctx* c, int space, uint32_t count, bool have_inputs, bool whole_volume, const char* who);   // rr_api.cu
+int query_reserve(rr_ctx* c, uint32_t count);
+int query_upload(rr_ctx* c, const float* a, const float* b, uint32_t count);
+int launch_sample_points(rr_ctx* c, int space, uint32_t count);
+int launch_cast_rays(rr_ctx* c, int space, uint32_t count);
+int launch_query_composite(rr_ctx* const* members, int n, bool rays, int space, uint32_t count);   // on member 0's stream
+int query_download(rr_ctx* c, uint32_t count, bool rays, float* values_or_positions, float* normals, float* rgba, uint32_t* steps);
+void query_release(rr_ctx* c);
 int launch_unpack_frames(rr_ctx* c, int slot);
 int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4* d_out);
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines

@@ -20,8 +20,6 @@
 #include <string>
 #include <vector>
 
-#define RR_MAX_GROUP 16
-
 struct rr_group {
   std::vector<rr_ctx*> m;
   std::vector<int> dev;
@@ -557,6 +555,65 @@ int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out
   // synchronised member 0's stream, unless it failed before)
   RR_G_TRY(g, cudaStreamSynchronize(c0->stream));
   return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
+// Queries: member 0 takes the caller's inputs, every other member peer-copies them from member 0 and evaluates what its
+// slab owns (the halo covers the gradient and refinement taps), and one kernel on member 0 picks each entry's result from
+// the members' arrays through peer memory. No volume moves.
+static int group_query(rr_group* g, bool rays, int space, const float* a, const float* b, uint32_t count, float* out_a,
+                       float* normals, float* rgba, uint32_t* steps) {
+  const char* who = rays ? "rr_group_cast_rays" : "rr_group_sample_points";
+  const size_t n = g->m.size();
+  rr_ctx* c0 = g->m[0];
+  if (n == 1) {
+    const int rc = rays ? rr_cast_rays(c0, space, a, b, count, out_a, normals, rgba, steps) : rr_sample_points(c0, space, a, count, out_a, normals, rgba);
+    return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+  }
+  if (count == 0 && (space == RR_QUERY_WORLD || space == RR_QUERY_VOLUME)) return RR_OK;
+  RR_G_REQUIRE(g, g->bounds.size() == n + 1, std::string(who) + ": configure the group first");
+  for (size_t i = 0; i < n; ++i) {
+    const int rc = rr::query_check(g->m[i], space, count, a && (!rays || b), false, who);
+    if (rc != RR_OK) return member_fail(g, i, rc);
+  }
+  for (size_t i = 1; i < n; ++i)
+    if (!g->peer[i])
+      return gfail(g, RR_ERR_UNSUPPORTED, std::string(who) + ": member 0's device cannot address member " + std::to_string(i) + "'s memory");
+  RR_G_TRY(g, cudaSetDevice(c0->device));
+  int rc = rr::query_upload(c0, a, b, count);
+  if (rc != RR_OK) return member_fail(g, 0, rc);
+  RR_G_TRY(g, cudaEventRecord(g->ev_view[0], c0->stream));
+  const size_t bytes = (size_t)count * (rays ? 6 : 3) * sizeof(float);
+  for (size_t i = 0; i < n; ++i) {
+    rr_ctx* c = g->m[i];
+    RR_G_TRY(g, cudaSetDevice(c->device));
+    if (i > 0) {
+      rc = rr::query_reserve(c, count);
+      if (rc != RR_OK) return member_fail(g, i, rc);
+      RR_G_TRY(g, cudaStreamWaitEvent(c->stream, g->ev_view[0], 0));
+      // the directions follow the origins at offset 3 * count in both members' input arrays
+      RR_G_TRY(g, cudaMemcpyPeerAsync(c->d_q_in, c->device, c0->d_q_in, c0->device, bytes, c->stream));
+    }
+    rc = rays ? rr::launch_cast_rays(c, space, count) : rr::launch_sample_points(c, space, count);
+    if (rc != RR_OK) return member_fail(g, i, rc);
+    if (i > 0) RR_G_TRY(g, cudaEventRecord(g->ev_view[i], c->stream));
+  }
+  RR_G_TRY(g, cudaSetDevice(c0->device));
+  for (size_t i = 1; i < n; ++i) RR_G_TRY(g, cudaStreamWaitEvent(c0->stream, g->ev_view[i], 0));
+  rc = rr::launch_query_composite(g->m.data(), (int)n, rays, space, count);
+  // the download synchronises member 0's stream: the composite has read the members' arrays before the call returns
+  if (rc == RR_OK) rc = rr::query_download(c0, count, rays, out_a, normals, rgba, steps);
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
+int rr_group_sample_points(rr_group* g, int space, const float* points, uint32_t count, float* values, float* normals, float* rgba) {
+  if (!g) return RR_ERR_INVALID;
+  return group_query(g, false, space, points, nullptr, count, values, normals, rgba, nullptr);
+}
+
+int rr_group_cast_rays(rr_group* g, int space, const float* origins, const float* directions, uint32_t count,
+                       float* positions, float* normals, float* rgba, uint32_t* steps) {
+  if (!g) return RR_ERR_INVALID;
+  return group_query(g, true, space, origins, directions, count, positions, normals, rgba, steps);
 }
 
 // The whole volume, assembled from the slices each member owns. out: float32 [Z][Y][X], as rr_download_tsdf returns it

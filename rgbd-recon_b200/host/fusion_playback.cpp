@@ -3,7 +3,7 @@
 // raymarches it. Prints the TimerDatabase stage means; optionally dumps the last TSDF volume, image and surface mesh.
 //   fusion_playback <file.ks> (--streams "s0;s1;..." | --messages file) [--depth W H --color CW CH] [--frames K] [--voxel m]
 //                   [--limit l] [--eye x y z | --matrices file] [--view W H] [--shade m] [--dump-tsdf file] [--dump-image file] [--dense]
-//                   [--dump-mesh file.ply]
+//                   [--dump-mesh file.ply] [--pick PX PY]
 //                   [--gpus N | --devices a,b,...] [--recon points|trigrid|calibs [--min-length m] [--dump-recon file]]
 // --recon: like kinect_client's reconstruction list (source/kinect_client.cpp:251-257, key-selected g_recon_mode), one of the
 // other reconstructions also draws the last frame set's maps - ReconPoints, ReconTrigrid (min_length from the sensor .yml
@@ -12,14 +12,20 @@
 // peer copies from the first device, per-slab integration, the view composited on the first device); after the first frame
 // the slabs are re-cut to equal integrate cost. A device may be named more than once (slabs sharing a GPU).
 // --dump-mesh: the last frame set's fused surface (ReconIntegration::extractMesh) as a binary PLY with normals and colours.
+// --pick PX PY: picking as kinect_client's view would do it - the world ray through the centre of view pixel (PX, PY) (GL window
+// coordinates, row 0 = bottom) of the playback camera, cast into the last frame set's volume (ReconIntegration::castRays).
+// Prints one line: "pick origin x y z direction x y z hit x y z normal x y z rgba r g b a step s", %.9g so every binary32
+// value round-trips (NaN hit and normal, rgba 0 and step 4294967295 when the ray hits nothing).
 // Without --depth/--color the sizes and stream formats (DXT1 colour, 8-bit depth, near/far) come from the sensors' .yml
 // files like in the reference (CalibrationFiles, calibration_files.cpp:7-34). --messages plays a file of back-to-back
 // server messages (the ZMQ payload layout of NetKinectArray::readLoop, :511-538) through NetKinectArray::pushMessage.
 #include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
 #include <iostream>
+#include <utility>
 
 #include "rr_host.hpp"
 
@@ -45,8 +51,47 @@ static void perspective(float fovy_deg, float aspect, float n, float f, float m[
   m[0] = t / aspect; m[5] = t; m[10] = (f + n) / (n - f); m[11] = -1.f; m[14] = 2.f * f * n / (n - f);
 }
 
+// inverse of a column-major 4x4 matrix by Gauss-Jordan elimination with partial pivoting, in double
+static bool invert4(const double* m, double* out) {
+  double a[4][8];
+  for (int r = 0; r < 4; ++r)
+    for (int c = 0; c < 4; ++c) { a[r][c] = m[c * 4 + r]; a[r][c + 4] = r == c ? 1.0 : 0.0; }
+  for (int c = 0; c < 4; ++c) {
+    int p = c;
+    for (int r = c + 1; r < 4; ++r) if (std::fabs(a[r][c]) > std::fabs(a[p][c])) p = r;
+    if (a[p][c] == 0.0) return false;
+    for (int k = 0; k < 8; ++k) std::swap(a[c][k], a[p][k]);
+    const double d = a[c][c];
+    for (int k = 0; k < 8; ++k) a[c][k] /= d;
+    for (int r = 0; r < 4; ++r)
+      if (r != c) { const double f = a[r][c]; for (int k = 0; k < 8; ++k) a[r][k] -= f * a[c][k]; }
+  }
+  for (int r = 0; r < 4; ++r) for (int c = 0; c < 4; ++c) out[c * 4 + r] = a[r][c + 4];
+  return true;
+}
+
+// The world ray through the centre of window pixel (px, py) of a vw x vh view: from the eye (inverse modelview applied to the
+// origin) towards the pixel's point on the far plane (inverse projection, then inverse modelview), in double, rounded once.
+static void pick_ray(const float* mv, const float* pr, unsigned vw, unsigned vh, int px, int py, std::vector<float>& origin,
+                     std::vector<float>& direction) {
+  double M[16], P[16], iM[16], iP[16];
+  for (int i = 0; i < 16; ++i) { M[i] = mv[i]; P[i] = pr[i]; }
+  if (!invert4(M, iM) || !invert4(P, iP)) throw std::runtime_error("--pick: singular view matrices");
+  const double ndc[4] = {(px + 0.5) / vw * 2.0 - 1.0, (py + 0.5) / vh * 2.0 - 1.0, 1.0, 1.0};
+  double eye[4], world[4];
+  for (int r = 0; r < 4; ++r) eye[r] = iP[r] * ndc[0] + iP[4 + r] * ndc[1] + iP[8 + r] * ndc[2] + iP[12 + r] * ndc[3];
+  for (int r = 0; r < 4; ++r) world[r] = iM[r] * eye[0] + iM[4 + r] * eye[1] + iM[8 + r] * eye[2] + iM[12 + r] * eye[3];
+  origin.assign(3, 0.0f); direction.assign(3, 0.0f);
+  for (int a = 0; a < 3; ++a) {
+    const double o = iM[12 + a] / iM[15];
+    origin[a] = (float)o;
+    direction[a] = (float)(world[a] / world[3] - o);
+  }
+}
+
 int main(int argc, char** argv) {
   std::string ks, streams, messages, dump_tsdf, dump_image, dump_mesh, matrices, recon_mode, dump_recon;
+  int pick[2] = {-1, -1};
   float min_length = 0.0f;
   bool explicit_sizes = false;
   unsigned W = 512, H = 424, CW = 1280, CH = 1080, VW = 1280, VH = 720;
@@ -69,6 +114,7 @@ int main(int argc, char** argv) {
     else if (!std::strcmp(argv[i], "--dump-tsdf")) dump_tsdf = argv[++i];
     else if (!std::strcmp(argv[i], "--dump-image")) dump_image = argv[++i];
     else if (!std::strcmp(argv[i], "--dump-mesh")) dump_mesh = argv[++i];
+    else if (!std::strcmp(argv[i], "--pick")) { pick[0] = std::atoi(argv[i + 1]); pick[1] = std::atoi(argv[i + 2]); i += 2; }
     else if (!std::strcmp(argv[i], "--dense")) dense = true;
     else if (!std::strcmp(argv[i], "--gpus")) { devices.clear(); for (int d = 0, n = std::atoi(argv[++i]); d < n; ++d) devices.push_back(d); }
     else if (!std::strcmp(argv[i], "--devices")) {
@@ -154,6 +200,16 @@ int main(int argc, char** argv) {
       recon.extractMesh(mesh);
       writePly(dump_mesh, mesh);
       std::cout << "mesh vertices " << mesh.positions.size() / 3 << " triangles " << mesh.triangles.size() / 3 << std::endl;
+    }
+    if (pick[0] >= 0) {
+      std::vector<float> origin, direction, hit, normal, rgba;
+      std::vector<uint32_t> step;
+      pick_ray(mv, pr, VW, VH, pick[0], pick[1], origin, direction);
+      recon.castRays(origin, direction, hit, normal, rgba, step);
+      std::printf("pick origin %.9g %.9g %.9g direction %.9g %.9g %.9g hit %.9g %.9g %.9g normal %.9g %.9g %.9g rgba %.9g %.9g %.9g %.9g step %u\n",
+                  origin[0], origin[1], origin[2], direction[0], direction[1], direction[2], hit[0], hit[1], hit[2],
+                  normal[0], normal[1], normal[2], rgba[0], rgba[1], rgba[2], rgba[3], (unsigned)step[0]);
+      std::fflush(stdout);
     }
     if (!recon_mode.empty()) {
       // the other reconstructions consume the maps of the last processTextures() (and, ReconCalibs, the fused volume)

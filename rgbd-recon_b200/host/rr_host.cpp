@@ -389,6 +389,32 @@ void ReconIntegration::extractMesh(Mesh& out) const {
   ck(rr_download_mesh(ctx(), out.positions.data(), out.normals.data(), out.rgba.data(), out.triangles.data()), "rr_download_mesh");
 }
 
+void ReconIntegration::samplePoints(std::vector<float> const& points, std::vector<float>& values, std::vector<float>& normals,
+                                    std::vector<float>& rgba) const {
+  if (points.size() % 3) throw std::runtime_error("samplePoints: points must hold whole [x, y, z] triples");
+  const std::size_t n = points.size() / 3;
+  if (n >= (std::size_t(1) << 31)) throw std::runtime_error("samplePoints: 2^31 or more points");
+  values.resize(n); normals.resize(n * 3); rgba.resize(n * 4);
+  if (gpu::Context::current().numDevices() > 1)
+    gk(rr_group_sample_points(grp(), RR_QUERY_WORLD, points.data(), (uint32_t)n, values.data(), normals.data(), rgba.data()), "rr_group_sample_points");
+  else
+    ck(rr_sample_points(ctx(), RR_QUERY_WORLD, points.data(), (uint32_t)n, values.data(), normals.data(), rgba.data()), "rr_sample_points");
+}
+
+void ReconIntegration::castRays(std::vector<float> const& origins, std::vector<float> const& directions, std::vector<float>& positions,
+                                std::vector<float>& normals, std::vector<float>& rgba, std::vector<uint32_t>& steps) const {
+  if (origins.size() % 3 || origins.size() != directions.size()) throw std::runtime_error("castRays: origins and directions must be equal-length [n][3]");
+  const std::size_t n = origins.size() / 3;
+  if (n >= (std::size_t(1) << 31)) throw std::runtime_error("castRays: 2^31 or more rays");
+  positions.resize(n * 3); normals.resize(n * 3); rgba.resize(n * 4); steps.resize(n);
+  if (gpu::Context::current().numDevices() > 1)
+    gk(rr_group_cast_rays(grp(), RR_QUERY_WORLD, origins.data(), directions.data(), (uint32_t)n, positions.data(), normals.data(), rgba.data(),
+                          steps.data()), "rr_group_cast_rays");
+  else
+    ck(rr_cast_rays(ctx(), RR_QUERY_WORLD, origins.data(), directions.data(), (uint32_t)n, positions.data(), normals.data(), rgba.data(),
+                    steps.data()), "rr_cast_rays");
+}
+
 void writePly(std::string const& path, Mesh const& mesh) {
   const std::size_t nv = mesh.positions.size() / 3, nt = mesh.triangles.size() / 3;
   std::ofstream o(path, std::ios::binary);

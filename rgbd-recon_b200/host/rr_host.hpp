@@ -323,6 +323,12 @@ class ReconIntegration : public Reconstruction {
   void downloadTsdf(std::vector<float>& out) const;
   // marching cubes over the fused volume on the device (rr_extract_mesh; with several devices rr_group_extract_mesh)
   void extractMesh(Mesh& out) const;
+  // Queries of the fused volume in metres (rr_sample_points / rr_cast_rays; with several devices their group forms).
+  // points, origins, directions, normals, positions: [n][3]; values [n]; rgba [n][4]; steps [n] (0xFFFFFFFF: no hit, with
+  // NaN positions and normals). The outputs are resized to n.
+  void samplePoints(std::vector<float> const& points, std::vector<float>& values, std::vector<float>& normals, std::vector<float>& rgba) const;
+  void castRays(std::vector<float> const& origins, std::vector<float> const& directions, std::vector<float>& positions,
+                std::vector<float>& normals, std::vector<float>& rgba, std::vector<uint32_t>& steps) const;
  private:
   void configure();
   rr_config m_cfg;

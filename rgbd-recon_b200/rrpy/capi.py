@@ -138,6 +138,10 @@ def lib():
     L.rr_extract_mesh.argtypes = [vp, u32, u32]
     L.rr_download_mesh.argtypes = [vp, f32, f32, f32, u32]
     L.rr_group_extract_mesh.argtypes = [vp, u32, u32]
+    L.rr_sample_points.argtypes = [vp, C.c_int, vp, C.c_uint32, vp, vp, vp]
+    L.rr_cast_rays.argtypes = [vp, C.c_int, vp, vp, C.c_uint32, vp, vp, vp, vp]
+    L.rr_group_sample_points.argtypes = [vp, C.c_int, vp, C.c_uint32, vp, vp, vp]
+    L.rr_group_cast_rays.argtypes = [vp, C.c_int, vp, vp, C.c_uint32, vp, vp, vp, vp]
     L.rr_launch_count.argtypes = [vp]
     L.rr_launch_count.restype = C.c_uint64
     L.rr_version.restype = C.c_int
@@ -157,6 +161,61 @@ def _f32(a):
 
 def _u32(a):
     return a.ctypes.data_as(C.POINTER(C.c_uint32))
+
+
+# rr_sample_points / rr_cast_rays: RR_QUERY_WORLD (metres) or RR_QUERY_VOLUME (texture coordinates over the bbox)
+QUERY_SPACES = dict(world=0, volume=1)
+
+
+def _query_inputs(*arrays):
+    """[n, 3] float32 query inputs as (pointers, n, keep-alive, torch device or None). numpy-like inputs go as host memory;
+    torch tensors by data_ptr(), on the host or on the context's GPU (the caller's stream is synchronised first, as the
+    library reads them on its own stream)."""
+    ptrs, keep, device = [], [], None
+    for a in arrays:
+        if type(a).__module__.startswith("torch"):
+            import torch
+            t = a.detach().to(torch.float32).contiguous().reshape(-1, 3)
+            if t.is_cuda:
+                torch.cuda.current_stream(t.device).synchronize()
+                device = t.device
+            ptrs.append(t.data_ptr())
+            keep.append(t)
+        else:
+            arr = np.ascontiguousarray(a, np.float32).reshape(-1, 3)
+            ptrs.append(arr.ctypes.data)
+            keep.append(arr)
+    n = keep[0].shape[0]
+    if any(k.shape[0] != n for k in keep):
+        raise ValueError("origins and directions differ in length")
+    return ptrs, n, keep, device
+
+
+def _query_outputs(device, *shapes_and_types):
+    """Output arrays: torch tensors on `device` when the inputs were CUDA tensors, numpy arrays otherwise; and their pointers."""
+    outs = []
+    for shape, dt in shapes_and_types:
+        if device is not None:
+            import torch
+            outs.append(torch.empty(shape, dtype=dict(f4=torch.float32, u4=torch.uint32)[dt], device=device))
+        else:
+            outs.append(np.empty(shape, np.dtype(dt)))
+    ptrs = [o.data_ptr() if device is not None else o.ctypes.data for o in outs]
+    return outs, ptrs
+
+
+def _sample_points(call, points, space):
+    ptrs, n, keep, device = _query_inputs(points)
+    outs, op = _query_outputs(device, ((n,), "f4"), ((n, 3), "f4"), ((n, 4), "f4"))
+    call(QUERY_SPACES[space], ptrs[0], n, *op)
+    return tuple(outs)
+
+
+def _cast_rays(call, origins, directions, space):
+    ptrs, n, keep, device = _query_inputs(origins, directions)
+    outs, op = _query_outputs(device, ((n, 3), "f4"), ((n, 3), "f4"), ((n, 4), "f4"), ((n,), "u4"))
+    call(QUERY_SPACES[space], ptrs[0], ptrs[1], n, *op)
+    return tuple(outs)
 
 
 class RRError(RuntimeError):
@@ -483,6 +542,16 @@ class Fusion:
         float32 [V, 3], rgba float32 [V, 4] (alpha 1 quality-weighted colour, -1 fallback blend), triangles uint32 [T, 3]."""
         return self.download_mesh(*self.extract_mesh_counts())
 
+    def sample_points(self, points, space="world"):
+        """rr_sample_points at points [n, 3] ("world": metres, "volume": texture coordinates over the bbox): (values [n],
+        normals [n, 3], rgba [n, 4]) float32 - numpy arrays, or torch tensors on the inputs' GPU when given CUDA tensors."""
+        return _sample_points(lambda *a: self._ck(self.L.rr_sample_points(self.h, *a)), points, space)
+
+    def cast_rays(self, origins, directions, space="world"):
+        """rr_cast_rays along rays origins [n, 3] + t * directions [n, 3]: (positions [n, 3], normals [n, 3], rgba [n, 4],
+        steps uint32 [n]; 0xFFFFFFFF and NaN positions where a ray hits nothing), as numpy arrays or CUDA tensors."""
+        return _cast_rays(lambda *a: self._ck(self.L.rr_cast_rays(self.h, *a)), origins, directions, space)
+
     def set_timing(self, level=1):
         self._ck(self.L.rr_set_timing(self.h, int(level)))
 
@@ -690,6 +759,14 @@ class Group:
     def extract_mesh(self):
         """As Fusion.extract_mesh, equal to a single context's bit for bit: (positions, normals, rgba, triangles)."""
         return self.member(0).download_mesh(*self.extract_mesh_counts())
+
+    def sample_points(self, points, space="world"):
+        """As Fusion.sample_points (CUDA tensors on member 0's GPU), equal to a single context's bit for bit."""
+        return _sample_points(lambda *a: self._ck(self.L.rr_group_sample_points(self.h, *a)), points, space)
+
+    def cast_rays(self, origins, directions, space="world"):
+        """As Fusion.cast_rays (CUDA tensors on member 0's GPU), equal to a single context's bit for bit."""
+        return _cast_rays(lambda *a: self._ck(self.L.rr_group_cast_rays(self.h, *a)), origins, directions, space)
 
 
 def load_scene(fu: "Fusion", scene, inv=None):

@@ -320,6 +320,33 @@ int rr_extract_mesh(rr_ctx* ctx, uint32_t* out_num_vertices, uint32_t* out_num_t
 int rr_download_mesh(rr_ctx* ctx, float* positions, float* normals, float* rgba, uint32_t* triangles);
 int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out_num_triangles);
 
+/* ---- point clouds (no reference counterpart: a reference user draws the points and reads pixels back) -------------------
+ * The pre-processed, registered sensor points: every kept depth pixel of the sensors in sensor_mask, lifted to the world.
+ * For sensor i (bit i of sensor_mask) and pixel (x, y) of its W x H depth image, id = i*W*H + y*W + x:
+ *   sx = (float)((x + 0.5) * (double)(1.0f / W)), sy likewise with y and H (the vertex buffer rr_draw_points draws);
+ *   d  = depth_b.x of the last rr_preprocess / rr_fuse_frame at the pixel (RR_STAGE_DEPTH_B);
+ *   p  = trilinear cv_xyz_i at (sx, sy, d) in metres, t = trilinear cv_uv_i there, with the calibration volumes in effect.
+ * The point is kept iff d > 0, bbox_min <= p <= bbox_max componentwise (the bbox in effect) and 0.01 <= t.x, t.y <= 0.99:
+ * exactly the vertices rr_draw_points keeps before the view transform. A non-finite p or d is never kept. Per kept point:
+ *   positions = p, float32 [n][3];  normals = the normal stage at the pixel (xyz, as RR_STAGE_NORMAL), float32 [n][3];
+ *   colors = the bilinear RGB8 fetch of the current colour frame at t (the colour rr_draw_points shades with in shade mode 0),
+ *   float32 [n][3] in [0, 1];  quality = the quality stage at the pixel, float32 [n];  pixels = id, uint32 [n].
+ * Order: ascending id (sensor, row, column); it depends neither on scheduling nor on the number of devices.
+ *
+ * rr_extract_points  extracts on the context's stream and synchronises once; returns the count. sensor_mask == 0 gives 0
+ *                   points. RR_ERR_INVALID for a mask bit at or above the sensor count, a NULL count pointer, a sensor of the
+ *                   mask without rr_calib_upload, and a call before any rr_preprocess / rr_fuse_frame on this context. A
+ *                   context restricted by rr_set_slab is fine (its stage images are complete). Not a setting: the volume,
+ *                   stage images, brick tables, view images (rr_fill_colors still fills the last view), mesh and captured
+ *                   frame graphs stay as they are.
+ * rr_download_points  the last extraction; each pointer may be NULL, host memory (pageable or pinned) or device memory of the
+ *                   context's GPU. Returns after one synchronisation. RR_ERR_INVALID if nothing was extracted yet.
+ * rr_group_extract_points  the same on member 0 of a group (pre-processing is replicated, so no peer traffic), equal to a
+ *                   single context bit for bit; read it with rr_download_points(rr_group_member(g, 0), ...). */
+int rr_extract_points(rr_ctx* ctx, uint32_t sensor_mask, uint32_t* out_num_points);
+int rr_download_points(rr_ctx* ctx, float* positions, float* normals, float* colors, float* quality, uint32_t* pixels);
+int rr_group_extract_points(rr_group* g, uint32_t sensor_mask, uint32_t* out_num_points);
+
 /* ---- queries (no reference counterpart: a reference user renders a view and reads pixels back) ------------------------
  * The fused volume evaluated at points and along rays the caller chooses: picking, collision tests, measurements.
  *   space      RR_QUERY_WORLD: coordinates in metres; a point becomes q = (p - bbox_min) / (bbox_max - bbox_min) (one IEEE

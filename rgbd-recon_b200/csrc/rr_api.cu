@@ -143,6 +143,7 @@ int rr_create(rr_ctx** out, int device, int num_sensors, int depth_w, int depth_
   if (rc == RR_OK) rc = dev_alloc(c, &c->d_work, 4, "work counters");
   if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_num_occ, sizeof(uint32_t)), "pinned count");
   if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_mesh_totals, 2 * sizeof(unsigned long long)), "pinned mesh totals");
+  if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_cloud_count, sizeof(uint32_t)), "pinned cloud count");
   if (rc == RR_OK) {
     cudaMemsetAsync(c->d_flags, 0, 4 * sizeof(uint32_t), c->stream);
     cudaMemsetAsync(c->d_pairs, 0, (size_t)c->N * (c->H + 2) * c->pair_pitch * sizeof(float2), c->stream);
@@ -176,6 +177,7 @@ void rr_destroy(rr_ctx* c) {
   trigrid_release(c);
   mesh_release(c);
   query_release(c);
+  cloud_release(c);
   for (auto& v : c->ipc_views) { cudaIpcCloseMemHandle(v.step); cudaIpcCloseMemHandle(v.rgba); cudaIpcCloseMemHandle(v.zbuf); cudaIpcCloseMemHandle(v.nsamp); }
   cudaGetLastError();
   cudaFree(c->d_pairs);
@@ -535,7 +537,9 @@ int rr_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, int r
   if (!c) return RR_ERR_INVALID;
   RR_TRY(require_ready(c, false));
   RR_SET_DEVICE(c);
-  return launch_preprocess(c, filter_textures, use_processed_depth, refine_boundary);
+  RR_TRY(launch_preprocess(c, filter_textures, use_processed_depth, refine_boundary));
+  c->preprocessed = true;
+  return RR_OK;
 }
 
 int rr_bricks_update(rr_ctx* c, uint32_t* out_num, float* out_ratio) {
@@ -571,6 +575,7 @@ int rr_fuse_frame(rr_ctx* c, int filter_textures, int use_processed_depth, int r
   RR_SET_DEVICE(c);
   const int f = filter_textures ? 1 : 0, p = use_processed_depth ? 1 : 0, r = refine_boundary ? 1 : 0;
   RR_TRY(staged_prepare(c));       // table rebuilds synchronise: never inside a capture
+  c->preprocessed = true;          // every path below pre-processes (direct, captured or replayed)
   // capture needs a launch sequence without allocations or event timers: the z table exists (first frame ran direct)
   // and stage timing is off
   const bool ready = rr::tunables().graph != 0 && !c->graphs_broken && c->timing == 0 && c->d_ztab &&
@@ -939,6 +944,30 @@ int rr_cast_rays(rr_ctx* c, int space, const float* origins, const float* direct
   RR_TRY(query_upload(c, origins, directions, count));
   RR_TRY(launch_cast_rays(c, space, count));
   return query_download(c, count, true, positions, normals, rgba, steps);
+}
+
+int rr_extract_points(rr_ctx* c, uint32_t sensor_mask, uint32_t* out_num_points) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, out_num_points, "rr_extract_points: null count pointer");
+  RR_REQUIRE(c, (sensor_mask >> c->N) == 0, "rr_extract_points: sensor mask names a sensor at or above the sensor count");
+  *out_num_points = 0;
+  if (sensor_mask == 0) {
+    c->cloud_n = 0;
+    c->cloud_valid = true;
+    return RR_OK;
+  }
+  for (int i = 0; i < c->N; ++i)
+    if ((sensor_mask >> i) & 1u) RR_REQUIRE(c, c->have_calib[i], "rr_extract_points: missing forward calibration volume (rr_calib_upload)");
+  RR_REQUIRE(c, c->preprocessed, "rr_extract_points: no stage images yet (rr_preprocess / rr_fuse_frame first)");
+  RR_SET_DEVICE(c);
+  return launch_extract_points(c, sensor_mask, out_num_points);
+}
+
+int rr_download_points(rr_ctx* c, float* positions, float* normals, float* colors, float* quality, uint32_t* pixels) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, c->cloud_valid, "rr_download_points: nothing extracted yet (rr_extract_points first)");
+  RR_SET_DEVICE(c);
+  return cloud_download(c, positions, normals, colors, quality, pixels);
 }
 
 int rr_download_mesh(rr_ctx* c, float* positions, float* normals, float* rgba, uint32_t* triangles) {

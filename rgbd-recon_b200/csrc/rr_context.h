@@ -216,6 +216,17 @@ struct rr_ctx {
   float* d_q_in = nullptr; float* d_q_val = nullptr; float* d_q_pos = nullptr; float* d_q_nrm = nullptr;
   float4* d_q_rgba = nullptr; uint32_t* d_q_step = nullptr; size_t q_cap = 0;
 
+  // point-cloud export (rr_cloud.cu): per depth pixel a keep flag, then its exclusive scan; per kept point the outputs, one
+  // capacity in points, grown on demand
+  bool preprocessed = false;       // an rr_preprocess / rr_fuse_frame has defined the stage images
+  bool cloud_valid = false;        // the d_cloud_* arrays hold the last extraction (cloud_n points)
+  uint32_t cloud_n = 0;
+  uint32_t* d_cloud_flags = nullptr; size_t cloud_flags_cap = 0;   // [2][N * W * H + 1]: flags, offsets
+  uint8_t* d_cloud_scratch = nullptr; size_t cloud_scratch_cap = 0; // CUB scan storage
+  float* d_cloud_pos = nullptr; float* d_cloud_nrm = nullptr; float* d_cloud_rgb = nullptr; float* d_cloud_q = nullptr;
+  uint32_t* d_cloud_pix = nullptr; size_t cloud_cap = 0;
+  uint32_t* h_cloud_count = nullptr;   // pinned
+
   // colour hole filling (rr_colorfill.cu): atlas right of column W, squeezed copy, filled colour
   int fill_w = 0, fill_h = 0;
   float4* d_fill_fc = nullptr; float* d_fill_fd = nullptr;
@@ -290,6 +301,11 @@ int launch_cast_rays(rr_ctx* c, int space, uint32_t count);
 int launch_query_composite(rr_ctx* const* members, int n, bool rays, int space, uint32_t count);   // on member 0's stream
 int query_download(rr_ctx* c, uint32_t count, bool rays, float* values_or_positions, float* normals, float* rgba, uint32_t* steps);
 void query_release(rr_ctx* c);
+// rr_cloud.cu: rr_extract_points over the sensors of `mask` (checked by the caller); cloud_download copies the last extraction
+// out and synchronises once
+int launch_extract_points(rr_ctx* c, uint32_t mask, uint32_t* out_n);
+int cloud_download(rr_ctx* c, float* positions, float* normals, float* colors, float* quality, uint32_t* pixels);
+void cloud_release(rr_ctx* c);
 int launch_unpack_frames(rr_ctx* c, int slot);
 int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4* d_out);
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines

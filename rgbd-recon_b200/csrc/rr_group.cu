@@ -557,6 +557,14 @@ int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out
   return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
 }
 
+// Pre-processing is replicated on every member (rr_group_preprocess / rr_group_fuse_frame), so member 0's stage images are
+// the whole frame set's: the cloud is extracted there, with no peer traffic.
+int rr_group_extract_points(rr_group* g, uint32_t sensor_mask, uint32_t* out_num_points) {
+  if (!g) return RR_ERR_INVALID;
+  const int rc = rr_extract_points(g->m[0], sensor_mask, out_num_points);
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
 // Queries: member 0 takes the caller's inputs, every other member peer-copies them from member 0 and evaluates what its
 // slab owns (the halo covers the gradient and refinement taps), and one kernel on member 0 picks each entry's result from
 // the members' arrays through peer memory. No volume moves.

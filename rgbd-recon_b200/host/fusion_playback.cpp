@@ -3,7 +3,7 @@
 // raymarches it. Prints the TimerDatabase stage means; optionally dumps the last TSDF volume, image and surface mesh.
 //   fusion_playback <file.ks> (--streams "s0;s1;..." | --messages file) [--depth W H --color CW CH] [--frames K] [--voxel m]
 //                   [--limit l] [--eye x y z | --matrices file] [--view W H] [--shade m] [--dump-tsdf file] [--dump-image file] [--dense]
-//                   [--dump-mesh file.ply] [--pick PX PY]
+//                   [--dump-mesh file.ply] [--dump-points file.ply] [--pick PX PY]
 //                   [--gpus N | --devices a,b,...] [--recon points|trigrid|calibs [--min-length m] [--dump-recon file]]
 // --recon: like kinect_client's reconstruction list (source/kinect_client.cpp:251-257, key-selected g_recon_mode), one of the
 // other reconstructions also draws the last frame set's maps - ReconPoints, ReconTrigrid (min_length from the sensor .yml
@@ -12,6 +12,8 @@
 // peer copies from the first device, per-slab integration, the view composited on the first device); after the first frame
 // the slabs are re-cut to equal integrate cost. A device may be named more than once (slabs sharing a GPU).
 // --dump-mesh: the last frame set's fused surface (ReconIntegration::extractMesh) as a binary PLY with normals and colours.
+// --dump-points: the last frame set's pre-processed sensor points (ReconPoints::extractPoints) as a binary PLY with normals,
+// colours and quality (with --gpus N through the group call: pre-processing is replicated on every member).
 // --pick PX PY: picking as kinect_client's view would do it - the world ray through the centre of view pixel (PX, PY) (GL window
 // coordinates, row 0 = bottom) of the playback camera, cast into the last frame set's volume (ReconIntegration::castRays).
 // Prints one line: "pick origin x y z direction x y z hit x y z normal x y z rgba r g b a step s", %.9g so every binary32
@@ -90,7 +92,7 @@ static void pick_ray(const float* mv, const float* pr, unsigned vw, unsigned vh,
 }
 
 int main(int argc, char** argv) {
-  std::string ks, streams, messages, dump_tsdf, dump_image, dump_mesh, matrices, recon_mode, dump_recon;
+  std::string ks, streams, messages, dump_tsdf, dump_image, dump_mesh, dump_points, matrices, recon_mode, dump_recon;
   int pick[2] = {-1, -1};
   float min_length = 0.0f;
   bool explicit_sizes = false;
@@ -114,6 +116,7 @@ int main(int argc, char** argv) {
     else if (!std::strcmp(argv[i], "--dump-tsdf")) dump_tsdf = argv[++i];
     else if (!std::strcmp(argv[i], "--dump-image")) dump_image = argv[++i];
     else if (!std::strcmp(argv[i], "--dump-mesh")) dump_mesh = argv[++i];
+    else if (!std::strcmp(argv[i], "--dump-points")) dump_points = argv[++i];
     else if (!std::strcmp(argv[i], "--pick")) { pick[0] = std::atoi(argv[i + 1]); pick[1] = std::atoi(argv[i + 2]); i += 2; }
     else if (!std::strcmp(argv[i], "--dense")) dense = true;
     else if (!std::strcmp(argv[i], "--gpus")) { devices.clear(); for (int d = 0, n = std::atoi(argv[++i]); d < n; ++d) devices.push_back(d); }
@@ -200,6 +203,12 @@ int main(int argc, char** argv) {
       recon.extractMesh(mesh);
       writePly(dump_mesh, mesh);
       std::cout << "mesh vertices " << mesh.positions.size() / 3 << " triangles " << mesh.triangles.size() / 3 << std::endl;
+    }
+    if (!dump_points.empty()) {
+      PointCloud cloud;
+      ReconPoints(calib_files, &cv, sc.bbox).extractPoints(cloud);
+      writePly(dump_points, cloud);
+      std::cout << "points " << cloud.pixels.size() << std::endl;
     }
     if (pick[0] >= 0) {
       std::vector<float> origin, direction, hit, normal, rgba;

@@ -364,6 +364,16 @@ void ReconPoints::draw() {                                   // recon_points.cpp
   m_rgba.resize(n * 4); m_depth.resize(n);
   ck(rr_draw_points(ctx(), &m_view, m_rgba.data(), m_depth.data()), "rr_draw_points");
 }
+void ReconPoints::extractPoints(PointCloud& out, uint32_t sensor_mask) const {
+  if (sensor_mask == 0xFFFFFFFFu && m_num_kinects < 32) sensor_mask = (1u << m_num_kinects) - 1u;   // the default: every sensor
+  uint32_t n = 0;
+  if (gpu::Context::current().numDevices() > 1) gk(rr_group_extract_points(grp(), sensor_mask, &n), "rr_group_extract_points");
+  else ck(rr_extract_points(ctx(), sensor_mask, &n), "rr_extract_points");
+  out.positions.resize((std::size_t)n * 3); out.normals.resize((std::size_t)n * 3); out.colors.resize((std::size_t)n * 3);
+  out.quality.resize(n); out.pixels.resize(n);
+  ck(rr_download_points(ctx(), out.positions.data(), out.normals.data(), out.colors.data(), out.quality.data(), out.pixels.data()),
+     "rr_download_points");
+}
 void ReconTrigrid::draw() {                                  // recon_trigrid.cpp:82-149
   const std::size_t n = (std::size_t)m_view.viewport[2] * m_view.viewport[3];
   m_rgba.resize(n * 4); m_depth.resize(n);
@@ -415,6 +425,12 @@ void ReconIntegration::castRays(std::vector<float> const& origins, std::vector<f
                     steps.data()), "rr_cast_rays");
 }
 
+static uint8_t ply_byte(float v) {
+  v = v > 0.0f ? v : 0.0f;                     // NaN -> 0
+  v = v < 1.0f ? v : 1.0f;
+  return (uint8_t)(v * 255.0f + 0.5f);
+}
+
 void writePly(std::string const& path, Mesh const& mesh) {
   const std::size_t nv = mesh.positions.size() / 3, nt = mesh.triangles.size() / 3;
   std::ofstream o(path, std::ios::binary);
@@ -431,16 +447,31 @@ void writePly(std::string const& path, Mesh const& mesh) {
   for (std::size_t i = 0; i < nv; ++i) {
     put(&mesh.positions[i * 3], 12);
     put(&mesh.normals[i * 3], 12);
-    for (int c = 0; c < 3; ++c) {
-      float v = mesh.rgba[i * 4 + c];
-      v = v > 0.0f ? v : 0.0f;                 // NaN -> 0
-      v = v < 1.0f ? v : 1.0f;
-      const uint8_t b = (uint8_t)(v * 255.0f + 0.5f);
-      put(&b, 1);
-    }
+    for (int c = 0; c < 3; ++c) { const uint8_t b = ply_byte(mesh.rgba[i * 4 + c]); put(&b, 1); }
   }
   const uint8_t three = 3;
   for (std::size_t t = 0; t < nt; ++t) { put(&three, 1); put(&mesh.triangles[t * 3], 12); }
+  o.write(buf.data(), (std::streamsize)buf.size());
+  if (!o) throw std::runtime_error("cannot write " + path);
+}
+
+void writePly(std::string const& path, PointCloud const& cloud) {
+  const std::size_t n = cloud.positions.size() / 3;
+  std::ofstream o(path, std::ios::binary);
+  if (!o) throw std::runtime_error("cannot write " + path);
+  o << "ply\nformat binary_little_endian 1.0\ncomment pre-processed sensor points (rr_extract_points)\n"
+    << "element vertex " << n << "\nproperty float x\nproperty float y\nproperty float z\n"
+    << "property float nx\nproperty float ny\nproperty float nz\n"
+    << "property uchar red\nproperty uchar green\nproperty uchar blue\nproperty float quality\nend_header\n";
+  std::vector<char> buf;
+  buf.reserve(n * 31);
+  auto put = [&](void const* p, std::size_t k) { buf.insert(buf.end(), static_cast<char const*>(p), static_cast<char const*>(p) + k); };
+  for (std::size_t i = 0; i < n; ++i) {
+    put(&cloud.positions[i * 3], 12);
+    put(&cloud.normals[i * 3], 12);
+    for (int c = 0; c < 3; ++c) { const uint8_t b = ply_byte(cloud.colors[i * 3 + c]); put(&b, 1); }
+    put(&cloud.quality[i], 4);
+  }
   o.write(buf.data(), (std::streamsize)buf.size());
   if (!o) throw std::runtime_error("cannot write " + path);
 }

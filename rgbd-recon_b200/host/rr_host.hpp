@@ -296,6 +296,19 @@ struct Mesh {
 // Colour byte = (uint8)(min(max(c, 0), 1) * 255 + 0.5f), a NaN channel counting as 0. Throws if the file cannot be written.
 void writePly(std::string const& path, Mesh const& mesh);
 
+// ---- point clouds (no reference counterpart): the pre-processed, registered sensor points --------------------------------
+// The arrays of rr_download_points (include/rgbd_recon_b200.h states what they hold).
+struct PointCloud {
+  std::vector<float> positions;      // [n][3] metres
+  std::vector<float> normals;        // [n][3] the normal stage at the pixel
+  std::vector<float> colors;         // [n][3] in [0, 1], the bilinear colour-frame fetch
+  std::vector<float> quality;        // [n]
+  std::vector<uint32_t> pixels;      // [n] sensor * W * H + y * W + x, ascending
+};
+// Binary little-endian PLY: vertex "float x y z nx ny nz uchar red green blue float quality", no faces. Colour bytes as the
+// mesh writer's: (uint8)(min(max(c, 0), 1) * 255 + 0.5f), a NaN channel counting as 0. Throws if the file cannot be written.
+void writePly(std::string const& path, PointCloud const& cloud);
+
 // ---- framework/reconstruction/recon_integration.hpp:33-107 ------------------------------------------------------------
 class ReconIntegration : public Reconstruction {
  public:
@@ -346,6 +359,9 @@ class ReconPoints : public Reconstruction {
   void setShadeMode(int mode) { m_view.shade_mode = mode; }
   std::vector<float> const& colorImage() const { return m_rgba; }
   std::vector<float> const& depthImage() const { return m_depth; }
+  // the points draw() keeps before the view transform, of the sensors in sensor_mask, as a point cloud (rr_extract_points;
+  // with several devices rr_group_extract_points)
+  void extractPoints(PointCloud& out, uint32_t sensor_mask = 0xFFFFFFFFu) const;
  private:
   std::vector<float> m_rgba, m_depth;
 };

@@ -142,6 +142,9 @@ def lib():
     L.rr_cast_rays.argtypes = [vp, C.c_int, vp, vp, C.c_uint32, vp, vp, vp, vp]
     L.rr_group_sample_points.argtypes = [vp, C.c_int, vp, C.c_uint32, vp, vp, vp]
     L.rr_group_cast_rays.argtypes = [vp, C.c_int, vp, vp, C.c_uint32, vp, vp, vp, vp]
+    L.rr_extract_points.argtypes = [vp, C.c_uint32, u32]
+    L.rr_download_points.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.rr_group_extract_points.argtypes = [vp, C.c_uint32, u32]
     L.rr_launch_count.argtypes = [vp]
     L.rr_launch_count.restype = C.c_uint64
     L.rr_version.restype = C.c_int
@@ -218,6 +221,20 @@ def _cast_rays(call, origins, directions, space):
     return tuple(outs)
 
 
+def _sensor_mask(sensors, n_sensors):
+    """rr_extract_points' sensor_mask of an iterable of sensor indices (None: every sensor). Indices at or above the sensor
+    count are left for the library to refuse."""
+    if sensors is None:
+        return (1 << n_sensors) - 1
+    mask = 0
+    for i in sensors:
+        i = int(i)
+        if not 0 <= i < 32:
+            raise ValueError(f"sensor index {i} out of range")
+        mask |= 1 << i
+    return mask
+
+
 class RRError(RuntimeError):
     pass
 
@@ -229,6 +246,7 @@ class Fusion:
         self.L = lib()
         self.h = C.c_void_p()
         self.N, self.W, self.H, self.CW, self.CH = N, W, H, CW, CH
+        self.device = int(device)
         rc = self.L.rr_create(C.byref(self.h), device, N, W, H, CW, CH)
         if rc != 0:
             raise RRError(f"rr_create failed with status {rc} (no CUDA device? there is no CPU fallback)")
@@ -552,6 +570,30 @@ class Fusion:
         steps uint32 [n]; 0xFFFFFFFF and NaN positions where a ray hits nothing), as numpy arrays or CUDA tensors."""
         return _cast_rays(lambda *a: self._ck(self.L.rr_cast_rays(self.h, *a)), origins, directions, space)
 
+    def extract_points_count(self, sensors=None):
+        """rr_extract_points alone: extracts the point cloud of `sensors` (indices; None: all) and returns its size."""
+        n = C.c_uint32()
+        self._ck(self.L.rr_extract_points(self.h, _sensor_mask(sensors, self.N), C.byref(n)))
+        return int(n.value)
+
+    def download_points(self, n, device=False):
+        """rr_download_points of the last extraction (n: its size), as numpy arrays or, with device, CUDA tensors on the
+        context's GPU: (positions [n, 3], normals [n, 3], colors [n, 3], quality [n], pixels uint32 [n])."""
+        dev = None
+        if device:
+            import torch
+            dev = torch.device("cuda", self.device)
+        outs, op = _query_outputs(dev, ((n, 3), "f4"), ((n, 3), "f4"), ((n, 3), "f4"), ((n,), "f4"), ((n,), "u4"))
+        self._ck(self.L.rr_download_points(self.h, *op))
+        return tuple(outs)
+
+    def extract_points(self, sensors=None, device=False):
+        """The pre-processed sensor points of the last preprocess as a point cloud (rr_extract_points + rr_download_points):
+        positions float32 [n, 3] (metres), normals float32 [n, 3], colors float32 [n, 3] in [0, 1], quality float32 [n] and
+        pixel ids uint32 [n] (sensor * W * H + y * W + x, ascending). sensors: iterable of sensor indices, default all;
+        device: return torch tensors on the context's GPU instead of numpy arrays."""
+        return self.download_points(self.extract_points_count(sensors), device)
+
     def set_timing(self, level=1):
         self._ck(self.L.rr_set_timing(self.h, int(level)))
 
@@ -608,6 +650,7 @@ class Group:
         if rc != 0:
             raise RRError(f"rr_group_create failed with status {rc}")
         self.n = len(dev)
+        self.devices = [int(d) for d in dev]
 
     def close(self):
         if self.h:
@@ -629,6 +672,7 @@ class Group:
         fu = Fusion.__new__(Fusion)
         fu.L, fu.h = self.L, C.c_void_p(self.L.rr_group_member(self.h, i))
         fu.N, fu.W, fu.H, fu.CW, fu.CH = self.N, self.W, self.H, self.CW, self.CH
+        fu.device = self.devices[i]
         fu.close = lambda: None
         return fu
 
@@ -759,6 +803,13 @@ class Group:
     def extract_mesh(self):
         """As Fusion.extract_mesh, equal to a single context's bit for bit: (positions, normals, rgba, triangles)."""
         return self.member(0).download_mesh(*self.extract_mesh_counts())
+
+    def extract_points(self, sensors=None, device=False):
+        """As Fusion.extract_points (rr_group_extract_points on member 0; CUDA tensors on member 0's GPU), equal to a single
+        context's bit for bit."""
+        n = C.c_uint32()
+        self._ck(self.L.rr_group_extract_points(self.h, _sensor_mask(sensors, self.N), C.byref(n)))
+        return self.member(0).download_points(int(n.value), device)
 
     def sample_points(self, points, space="world"):
         """As Fusion.sample_points (CUDA tensors on member 0's GPU), equal to a single context's bit for bit."""

@@ -320,6 +320,44 @@ int rr_extract_mesh(rr_ctx* ctx, uint32_t* out_num_vertices, uint32_t* out_num_t
 int rr_download_mesh(rr_ctx* ctx, float* positions, float* normals, float* rgba, uint32_t* triangles);
 int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out_num_triangles);
 
+/* ---- connected parts (no reference counterpart) -------------------------------------------------------------------------
+ * What is in the volume: its separate objects, where each is, and which mesh triangles belong to which.
+ *   Values   the grid of the surface extraction: voxel (x, y, z) has the value v rr_raymarch reads there (R32F; the low
+ *            half of a half2 voxel, widened; F32_WEIGHT: the tsdf volume only).
+ *   Inside   v > 0 and v finite (the raymarch's hit test, the mesh's inside); NaN and +-inf are never inside.
+ *   Part     a maximal set of inside voxels connected through shared faces (6-neighbourhood): voxels that touch only along
+ *            an edge or at a corner are in different parts, as the mesh's face rule separates them, so the surfaces of two
+ *            parts never share a vertex.
+ *   Order    a part's key is the smallest linear index z*X*Y + y*X + x of its voxels; parts are numbered 0..P-1 by
+ *            ascending key. The order depends neither on scheduling, on the occupied-brick shortcut nor on the number of
+ *            devices. Every voxel of the volume counts, whatever rr_set_slab says.
+ *   Per part voxels uint32 [P] (the count); boxes int32 [P][6] = x0, x1, y0, y1, z0, z1, half-open voxel index ranges;
+ *            centroids float32 [P][3] in metres: with S_k the exact integer sum of voxel index k over the part and n its
+ *            count, c_k = (float)(bmin_k + ((S_k / n) + 0.5) / R_k * (bmax_k - bmin_k)), evaluated in binary64 in that
+ *            order without fused multiply-adds, every operand widened from its binary32 or integer value.
+ *   Labels   uint32 [Z][Y][X]: the part of every inside voxel, 0xFFFFFFFF everywhere else.
+ *   Mesh     vertex_parts uint32 [V]: the part of the inside end of the vertex's edge (exactly one end is > 0 by the mesh's
+ *            vertex rule); triangle_parts uint32 [T]: the part its three vertices share (every triangle's edges have their
+ *            inside ends in one face-connected group of its cell's inside corners, so there is one).
+ *
+ * rr_label_parts   labels on the context's stream and synchronises once; returns the part count. RR_ERR_INVALID for a NULL
+ *                  count pointer, before any integrate into the current volume (as rr_extract_mesh) and on a context
+ *                  restricted by rr_set_slab (use rr_group_label_parts). Not a setting: the volume, brick tables, view
+ *                  images (rr_fill_colors still fills the last view), mesh, cloud, query buffers, captured frame graphs and
+ *                  rr_integrator_last stay as they are.
+ * rr_download_parts  the last labelling. rr_download_mesh_parts  the parts of the last mesh; RR_ERR_INVALID unless the mesh
+ *                  and the last labelling were taken from the same volume state (no integrate and no new volume between
+ *                  them). rr_download_parts: RR_ERR_INVALID before any labelling of the current volume. For both, each
+ *                  pointer may be NULL, host memory (pageable or pinned) or device memory of the context's GPU; they return
+ *                  after one synchronisation.
+ * rr_group_label_parts  the same for a group, bit for bit: member 0 receives the other members' slabs by peer copies (as
+ *                  rr_group_extract_mesh) and labels; read with rr_download_parts(rr_group_member(g, 0), ...) and, after
+ *                  rr_group_extract_mesh, rr_download_mesh_parts on member 0. */
+int rr_label_parts(rr_ctx* ctx, uint32_t* out_num_parts);
+int rr_download_parts(rr_ctx* ctx, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels);
+int rr_download_mesh_parts(rr_ctx* ctx, uint32_t* vertex_parts, uint32_t* triangle_parts);
+int rr_group_label_parts(rr_group* g, uint32_t* out_num_parts);
+
 /* ---- point clouds (no reference counterpart: a reference user draws the points and reads pixels back) -------------------
  * The pre-processed, registered sensor points: every kept depth pixel of the sensors in sensor_mask, lifted to the world.
  * For sensor i (bit i of sensor_mask) and pixel (x, y) of its W x H depth image, id = i*W*H + y*W + x:

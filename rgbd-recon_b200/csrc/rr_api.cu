@@ -144,6 +144,7 @@ int rr_create(rr_ctx** out, int device, int num_sensors, int depth_w, int depth_
   if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_num_occ, sizeof(uint32_t)), "pinned count");
   if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_mesh_totals, 2 * sizeof(unsigned long long)), "pinned mesh totals");
   if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_cloud_count, sizeof(uint32_t)), "pinned cloud count");
+  if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_parts_count, sizeof(uint32_t)), "pinned part count");
   if (rc == RR_OK) {
     cudaMemsetAsync(c->d_flags, 0, 4 * sizeof(uint32_t), c->stream);
     cudaMemsetAsync(c->d_pairs, 0, (size_t)c->N * (c->H + 2) * c->pair_pitch * sizeof(float2), c->stream);
@@ -178,6 +179,8 @@ void rr_destroy(rr_ctx* c) {
   mesh_release(c);
   query_release(c);
   cloud_release(c);
+  parts_release(c);
+  if (c->h_parts_count) cudaFreeHost(c->h_parts_count);
   for (auto& v : c->ipc_views) { cudaIpcCloseMemHandle(v.step); cudaIpcCloseMemHandle(v.rgba); cudaIpcCloseMemHandle(v.zbuf); cudaIpcCloseMemHandle(v.nsamp); }
   cudaGetLastError();
   cudaFree(c->d_pairs);
@@ -329,7 +332,10 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
   if (new_volume || cfg->store_weight != c->cfg.store_weight) {   // a new volume allocation as far as extraction goes
     c->volume_integrated = false;
     c->mesh_valid = false;
+    c->parts_valid = false;
+    ++c->volume_epoch;
   }
+  if (new_volume) parts_release(c);   // the label array is sized by the volume
   if (new_bricks) {
     c->mesh_rows_ok = false;
     uint32_t rb[3];
@@ -586,6 +592,7 @@ int rr_fuse_frame(rr_ctx* c, int filter_textures, int use_processed_depth, int r
     if (g.key == key) {
       c->launches += g.launches;
       c->volume_integrated = true;                 // the captured frame ends with the integrate launch_integrate recorded
+      ++c->volume_epoch;
       c->mesh_rows_ok = mesh_rows_usable(c);
       return check(c, cudaGraphLaunch(g.exec, c->stream), "frame graph launch");
     }
@@ -905,6 +912,32 @@ int rr_extract_mesh(rr_ctx* c, uint32_t* out_num_vertices, uint32_t* out_num_tri
              "rr_extract_mesh: this context holds only its z-slab (rr_set_slab); extract through rr_group_extract_mesh");
   RR_SET_DEVICE(c);
   return launch_extract_mesh(c, out_num_vertices, out_num_triangles);
+}
+
+int rr_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, out_num_parts, "rr_label_parts: null count pointer");
+  RR_REQUIRE(c, c->configured && c->volume_integrated, "rr_label_parts: nothing has been integrated into the current volume");
+  RR_REQUIRE(c, c->slab_z0 == 0 && c->slab_z1 == c->res[2],
+             "rr_label_parts: this context holds only its z-slab (rr_set_slab); label through rr_group_label_parts");
+  RR_SET_DEVICE(c);
+  return launch_label_parts(c, out_num_parts);
+}
+
+int rr_download_parts(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, c->parts_valid, "rr_download_parts: nothing labelled in the current volume (rr_label_parts first)");
+  RR_SET_DEVICE(c);
+  return parts_download(c, voxels, boxes, centroids, labels);
+}
+
+int rr_download_mesh_parts(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle_parts) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, c->mesh_valid && c->parts_valid && c->mesh_epoch == c->parts_epoch,
+             "rr_download_mesh_parts: needs a mesh and a labelling of the same volume state (rr_extract_mesh and rr_label_parts "
+             "with no integrate in between)");
+  RR_SET_DEVICE(c);
+  return mesh_parts_download(c, vertex_parts, triangle_parts);
 }
 
 }  // extern "C"

@@ -202,7 +202,7 @@ struct rr_ctx {
   bool volume_integrated = false;  // an integrate has run into the current volume allocation
   bool mesh_rows_ok = false;       // rowany / cand_y / cand_z are the tables the last integrate cleared the volume by
   bool mesh_table = false;         // the case table is in this device's constant memory
-  bool mesh_valid = false;         // the d_mesh_* arrays hold an extraction of the current volume allocation
+  bool mesh_valid = false;         // the d_mesh_* arrays hold an extraction of the current volume allocation (of mesh_epoch)
   uint32_t mesh_nv = 0, mesh_nt = 0;
   unsigned long long* d_mesh_rows = nullptr; size_t mesh_rows_cap = 0;   // per row: counts and offsets of vertices, triangles
   uint8_t* d_mesh_scratch = nullptr; size_t mesh_scratch_cap = 0;        // CUB scan storage
@@ -226,6 +226,19 @@ struct rr_ctx {
   float* d_cloud_pos = nullptr; float* d_cloud_nrm = nullptr; float* d_cloud_rgb = nullptr; float* d_cloud_q = nullptr;
   uint32_t* d_cloud_pix = nullptr; size_t cloud_cap = 0;
   uint32_t* h_cloud_count = nullptr;   // pinned
+
+  // connected parts (rr_parts.cu). The volume epoch advances with every integrate and every new volume allocation; the
+  // mesh and the labelling record the epoch they were computed from, so rr_download_mesh_parts pairs only those of one state.
+  uint64_t volume_epoch = 0, mesh_epoch = 0, parts_epoch = 0;
+  bool parts_valid = false;        // d_parts_* hold the last labelling (parts_n parts)
+  uint32_t parts_n = 0;
+  uint32_t* d_parts_labels = nullptr; size_t parts_labels_cap = 0;   // [Z][Y][X]: union-find forest, then part labels
+  uint32_t* d_parts_rows = nullptr; size_t parts_rows_cap = 0;       // [2][rows + 1]: roots per row, their offsets
+  uint8_t* d_parts_scratch = nullptr; size_t parts_scratch_cap = 0;  // CUB scan storage
+  uint32_t* d_parts_voxels = nullptr; int32_t* d_parts_boxes = nullptr; unsigned long long* d_parts_sums = nullptr;
+  float* d_parts_centroids = nullptr; size_t parts_cap = 0;          // per part, one capacity in parts
+  uint32_t* d_mesh_parts = nullptr; size_t mesh_parts_cap = 0;       // [V] vertex parts, then [T] triangle parts
+  uint32_t* h_parts_count = nullptr;   // pinned
 
   // colour hole filling (rr_colorfill.cu): atlas right of column W, squeezed copy, filled colour
   int fill_w = 0, fill_h = 0;
@@ -306,6 +319,11 @@ void query_release(rr_ctx* c);
 int launch_extract_points(rr_ctx* c, uint32_t mask, uint32_t* out_n);
 int cloud_download(rr_ctx* c, float* positions, float* normals, float* colors, float* quality, uint32_t* pixels);
 void cloud_release(rr_ctx* c);
+// rr_parts.cu: rr_label_parts over the whole volume, ignoring the slab; the downloads copy out and synchronise once
+int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts);
+int parts_download(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels);
+int mesh_parts_download(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle_parts);   // the mesh and labelling of one epoch
+void parts_release(rr_ctx* c);
 int launch_unpack_frames(rr_ctx* c, int slot);
 int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4* d_out);
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines

@@ -524,20 +524,22 @@ int rr_composite_peers(rr_ctx* c, const void* peer_handles, int n_peers, int wid
   return RR_OK;
 }
 
-// Member 0 receives every other member's owned slices by peer copies (one volume over NVLink per call) and extracts over
-// the whole z range. Member 0's integrate and raymarch read only its slab and halo, and the halo slices equal the owners'
-// bit for bit (integration is pure), so overwriting its unowned slices changes nothing it computes later.
-int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out_num_triangles) {
-  if (!g) return RR_ERR_INVALID;
-  RR_G_REQUIRE(g, g->bounds.size() == g->m.size() + 1, "rr_group_extract_mesh: configure the group first");
+// Member 0 receives every other member's owned slices by peer copies (one volume over NVLink per call), so that it holds
+// the whole volume. Member 0's integrate and raymarch read only its slab and halo, and the halo slices equal the owners'
+// bit for bit (integration is pure), so overwriting its unowned slices changes nothing it computes later. The caller works
+// on member 0's stream and synchronises it before returning: the copies read the members' volumes, which must not
+// integrate again before the copies are done.
+// need_calib: refuse unless member 0 has every sensor's calibration volumes (the mesh's colours and normals read them).
+static int group_gather_volume(rr_group* g, const std::string& who, bool need_calib) {
+  RR_G_REQUIRE(g, g->bounds.size() == g->m.size() + 1, who + ": configure the group first");
   rr_ctx* c0 = g->m[0];
   for (size_t i = 0; i < g->m.size(); ++i) {
     rr_ctx* c = g->m[i];
     if (!c->configured || !c->volume_integrated)
-      return gfail(g, RR_ERR_INVALID, "rr_group_extract_mesh: nothing has been integrated into the current volume");
+      return gfail(g, RR_ERR_INVALID, who + ": nothing has been integrated into the current volume");
   }
-  for (int s = 0; s < c0->N; ++s)
-    RR_G_REQUIRE(g, c0->have_calib[s] && c0->have_inv[s], "rr_group_extract_mesh: upload every sensor's calibration volumes first");
+  for (int s = 0; need_calib && s < c0->N; ++s)
+    RR_G_REQUIRE(g, c0->have_calib[s] && c0->have_inv[s], who + ": upload every sensor's calibration volumes first");
   const size_t plane = (size_t)c0->res[0] * c0->res[1];
   for (size_t i = 1; i < g->m.size(); ++i) {
     rr_ctx* c = g->m[i];
@@ -550,10 +552,25 @@ int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out
       RR_G_TRY(g, cudaMemcpyPeerAsync(c0->d_tsdf + plane * z0, c0->device, c->d_tsdf + plane * z0, c->device, plane * (z1 - z0) * sizeof(float), c0->stream));
   }
   RR_G_TRY(g, cudaSetDevice(c0->device));
+  return RR_OK;
+}
+
+int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out_num_triangles) {
+  if (!g) return RR_ERR_INVALID;
+  rr_ctx* c0 = g->m[0];
+  RR_TRY_RC(group_gather_volume(g, "rr_group_extract_mesh", true));
   const int rc = rr::launch_extract_mesh(c0, out_num_vertices, out_num_triangles);
-  // the copies read the members' volumes: they must not integrate again before the copies are done (the extraction's read-back
-  // synchronised member 0's stream, unless it failed before)
   RR_G_TRY(g, cudaStreamSynchronize(c0->stream));
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
+// The same gather, then member 0 labels the whole volume; read the parts with rr_download_parts(rr_group_member(g, 0), ...).
+int rr_group_label_parts(rr_group* g, uint32_t* out_num_parts) {
+  if (!g) return RR_ERR_INVALID;
+  RR_G_REQUIRE(g, out_num_parts, "rr_group_label_parts: null count pointer");
+  RR_TRY_RC(group_gather_volume(g, "rr_group_label_parts", false));
+  const int rc = rr::launch_label_parts(g->m[0], out_num_parts);
+  RR_G_TRY(g, cudaStreamSynchronize(g->m[0]->stream));
   return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
 }
 

@@ -364,7 +364,7 @@ int launch_integrate(rr_ctx* c) {
     c->work_fresh = false;   // the fused kernel draws from the work counters too
   }
   timer_end(c, "2integrate");
-  if (rc == RR_OK) { c->volume_integrated = true; c->mesh_rows_ok = mesh_rows_usable(c); }
+  if (rc == RR_OK) { c->volume_integrated = true; ++c->volume_epoch; c->mesh_rows_ok = mesh_rows_usable(c); }
   return rc;
 }
 

@@ -431,6 +431,7 @@ int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt) {
     RR_LAUNCH_CHECK(c, "k_mesh_triangles");
   }
   c->mesh_nv = (uint32_t)nv; c->mesh_nt = (uint32_t)nt;
+  c->mesh_epoch = c->volume_epoch;
   c->mesh_valid = true;
   if (out_nv) *out_nv = c->mesh_nv;
   if (out_nt) *out_nt = c->mesh_nt;

@@ -3,7 +3,7 @@
 // raymarches it. Prints the TimerDatabase stage means; optionally dumps the last TSDF volume, image and surface mesh.
 //   fusion_playback <file.ks> (--streams "s0;s1;..." | --messages file) [--depth W H --color CW CH] [--frames K] [--voxel m]
 //                   [--limit l] [--eye x y z | --matrices file] [--view W H] [--shade m] [--dump-tsdf file] [--dump-image file] [--dense]
-//                   [--dump-mesh file.ply] [--dump-points file.ply] [--pick PX PY]
+//                   [--dump-mesh file.ply [--min-part-voxels N]] [--dump-points file.ply] [--pick PX PY] [--parts]
 //                   [--gpus N | --devices a,b,...] [--recon points|trigrid|calibs [--min-length m] [--dump-recon file]]
 // --recon: like kinect_client's reconstruction list (source/kinect_client.cpp:251-257, key-selected g_recon_mode), one of the
 // other reconstructions also draws the last frame set's maps - ReconPoints, ReconTrigrid (min_length from the sensor .yml
@@ -12,6 +12,10 @@
 // peer copies from the first device, per-slab integration, the view composited on the first device); after the first frame
 // the slabs are re-cut to equal integrate cost. A device may be named more than once (slabs sharing a GPU).
 // --dump-mesh: the last frame set's fused surface (ReconIntegration::extractMesh) as a binary PLY with normals and colours.
+// --min-part-voxels N: with --dump-mesh, only the triangles of connected parts of at least N voxels, and the vertices they
+//   use, in their original order and re-indexed (drops the small floating blobs sensor noise leaves in front of the surface).
+// --parts: one line per connected part of the last frame set's volume (ReconIntegration::labelParts): index, voxels, box
+//   (x0 x1 y0 y1 z0 z1, half-open voxel ranges) and centroid (metres).
 // --dump-points: the last frame set's pre-processed sensor points (ReconPoints::extractPoints) as a binary PLY with normals,
 // colours and quality (with --gpus N through the group call: pre-processing is replicated on every member).
 // --pick PX PY: picking as kinect_client's view would do it - the world ray through the centre of view pixel (PX, PY) (GL window
@@ -101,6 +105,8 @@ int main(int argc, char** argv) {
   float voxel = 0.01f, limit = 0.01f, eye[3] = {1.6f, 1.5f, 2.2f};
   bool dense = false;
   std::vector<int> devices(1, 0);
+  bool print_parts = false;
+  long long min_part_voxels = -1;
   for (int i = 1; i < argc; ++i) {
     auto next = [&](int k) { return std::atof(argv[i + k]); };
     if (!std::strcmp(argv[i], "--depth")) { W = (unsigned)next(1); H = (unsigned)next(2); i += 2; explicit_sizes = true; }
@@ -119,6 +125,8 @@ int main(int argc, char** argv) {
     else if (!std::strcmp(argv[i], "--dump-points")) dump_points = argv[++i];
     else if (!std::strcmp(argv[i], "--pick")) { pick[0] = std::atoi(argv[i + 1]); pick[1] = std::atoi(argv[i + 2]); i += 2; }
     else if (!std::strcmp(argv[i], "--dense")) dense = true;
+    else if (!std::strcmp(argv[i], "--parts")) print_parts = true;
+    else if (!std::strcmp(argv[i], "--min-part-voxels")) min_part_voxels = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--gpus")) { devices.clear(); for (int d = 0, n = std::atoi(argv[++i]); d < n; ++d) devices.push_back(d); }
     else if (!std::strcmp(argv[i], "--devices")) {
       devices.clear();
@@ -198,9 +206,41 @@ int main(int argc, char** argv) {
       recon.downloadTsdf(tsdf);
       std::ofstream(dump_tsdf, std::ios::binary).write(reinterpret_cast<char const*>(tsdf.data()), (std::streamsize)(tsdf.size() * sizeof(float)));
     }
+    Parts parts;
+    if (print_parts || (!dump_mesh.empty() && min_part_voxels >= 0)) recon.labelParts(parts);
+    if (print_parts)
+      for (std::size_t k = 0; k < parts.voxels.size(); ++k) {
+        const int32_t* b = &parts.boxes[k * 6];
+        const float* c = &parts.centroids[k * 3];
+        std::printf("part %zu voxels %u box %d %d %d %d %d %d centroid %.9g %.9g %.9g\n", k, (unsigned)parts.voxels[k], b[0], b[1], b[2],
+                    b[3], b[4], b[5], c[0], c[1], c[2]);
+      }
+    std::fflush(stdout);
     if (!dump_mesh.empty()) {
       Mesh mesh;
       recon.extractMesh(mesh);
+      if (min_part_voxels >= 0) {
+        std::vector<uint32_t> vparts, tparts;
+        recon.meshParts(vparts, tparts);
+        Mesh kept;
+        std::vector<uint32_t> index(vparts.size(), 0xFFFFFFFFu);
+        std::vector<char> used(vparts.size(), 0);
+        for (std::size_t t = 0; t < tparts.size(); ++t)
+          if (parts.voxels[tparts[t]] >= (unsigned long long)min_part_voxels)
+            for (int j = 0; j < 3; ++j) used[mesh.triangles[t * 3 + j]] = 1;
+        for (std::size_t v = 0; v < used.size(); ++v) {
+          if (!used[v]) continue;
+          index[v] = (uint32_t)(kept.positions.size() / 3);
+          kept.positions.insert(kept.positions.end(), &mesh.positions[v * 3], &mesh.positions[v * 3] + 3);
+          kept.normals.insert(kept.normals.end(), &mesh.normals[v * 3], &mesh.normals[v * 3] + 3);
+          kept.rgba.insert(kept.rgba.end(), &mesh.rgba[v * 4], &mesh.rgba[v * 4] + 4);
+        }
+        for (std::size_t t = 0; t < tparts.size(); ++t)
+          if (parts.voxels[tparts[t]] >= (unsigned long long)min_part_voxels)
+            for (int j = 0; j < 3; ++j) kept.triangles.push_back(index[mesh.triangles[t * 3 + j]]);
+        mesh.positions.swap(kept.positions); mesh.normals.swap(kept.normals); mesh.rgba.swap(kept.rgba);
+        mesh.triangles.swap(kept.triangles);
+      }
       writePly(dump_mesh, mesh);
       std::cout << "mesh vertices " << mesh.positions.size() / 3 << " triangles " << mesh.triangles.size() / 3 << std::endl;
     }

@@ -397,6 +397,20 @@ void ReconIntegration::extractMesh(Mesh& out) const {
   out.positions.resize((std::size_t)nv * 3); out.normals.resize((std::size_t)nv * 3); out.rgba.resize((std::size_t)nv * 4);
   out.triangles.resize((std::size_t)nt * 3);
   ck(rr_download_mesh(ctx(), out.positions.data(), out.normals.data(), out.rgba.data(), out.triangles.data()), "rr_download_mesh");
+  m_mesh_nv = nv; m_mesh_nt = nt;
+}
+
+void ReconIntegration::labelParts(Parts& out) const {
+  uint32_t n = 0;
+  if (gpu::Context::current().numDevices() > 1) gk(rr_group_label_parts(grp(), &n), "rr_group_label_parts");
+  else ck(rr_label_parts(ctx(), &n), "rr_label_parts");
+  out.voxels.resize(n); out.boxes.resize((std::size_t)n * 6); out.centroids.resize((std::size_t)n * 3);
+  ck(rr_download_parts(ctx(), out.voxels.data(), out.boxes.data(), out.centroids.data(), nullptr), "rr_download_parts");
+}
+
+void ReconIntegration::meshParts(std::vector<uint32_t>& vertex_parts, std::vector<uint32_t>& triangle_parts) const {
+  vertex_parts.resize(m_mesh_nv); triangle_parts.resize(m_mesh_nt);
+  ck(rr_download_mesh_parts(ctx(), vertex_parts.data(), triangle_parts.data()), "rr_download_mesh_parts");
 }
 
 void ReconIntegration::samplePoints(std::vector<float> const& points, std::vector<float>& values, std::vector<float>& normals,

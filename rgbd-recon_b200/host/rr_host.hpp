@@ -296,6 +296,14 @@ struct Mesh {
 // Colour byte = (uint8)(min(max(c, 0), 1) * 255 + 0.5f), a NaN channel counting as 0. Throws if the file cannot be written.
 void writePly(std::string const& path, Mesh const& mesh);
 
+// ---- connected parts (no reference counterpart): the separate objects in the fused volume -------------------------------
+// The per-part arrays of rr_download_parts (include/rgbd_recon_b200.h states what they hold), in ascending key order.
+struct Parts {
+  std::vector<uint32_t> voxels;      // [P] inside voxels of the part
+  std::vector<int32_t> boxes;        // [P][6] x0, x1, y0, y1, z0, z1, half-open voxel index ranges
+  std::vector<float> centroids;      // [P][3] metres
+};
+
 // ---- point clouds (no reference counterpart): the pre-processed, registered sensor points --------------------------------
 // The arrays of rr_download_points (include/rgbd_recon_b200.h states what they hold).
 struct PointCloud {
@@ -336,6 +344,10 @@ class ReconIntegration : public Reconstruction {
   void downloadTsdf(std::vector<float>& out) const;
   // marching cubes over the fused volume on the device (rr_extract_mesh; with several devices rr_group_extract_mesh)
   void extractMesh(Mesh& out) const;
+  // the 6-connected parts of the fused volume (rr_label_parts; with several devices rr_group_label_parts), and the part of
+  // every vertex [V] and triangle [T] of the last extractMesh, which must come from the same volume state
+  void labelParts(Parts& out) const;
+  void meshParts(std::vector<uint32_t>& vertex_parts, std::vector<uint32_t>& triangle_parts) const;
   // Queries of the fused volume in metres (rr_sample_points / rr_cast_rays; with several devices their group forms).
   // points, origins, directions, normals, positions: [n][3]; values [n]; rgba [n][4]; steps [n] (0xFFFFFFFF: no hit, with
   // NaN positions and normals). The outputs are resized to n.
@@ -348,6 +360,7 @@ class ReconIntegration : public Reconstruction {
   bool m_fill_holes = true;
   float m_ratio_occupied = 0.0f;
   std::vector<float> m_rgba, m_depth;
+  mutable uint32_t m_mesh_nv = 0, m_mesh_nt = 0;   // counts of the last extractMesh (meshParts sizes its outputs by them)
 };
 
 // ---- framework/reconstruction/recon_points.hpp: every depth pixel of every sensor as a shaded, depth-tested point sprite -----

@@ -145,6 +145,10 @@ def lib():
     L.rr_extract_points.argtypes = [vp, C.c_uint32, u32]
     L.rr_download_points.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rr_group_extract_points.argtypes = [vp, C.c_uint32, u32]
+    L.rr_label_parts.argtypes = [vp, u32]
+    L.rr_download_parts.argtypes = [vp, vp, vp, vp, vp]
+    L.rr_download_mesh_parts.argtypes = [vp, vp, vp]
+    L.rr_group_label_parts.argtypes = [vp, u32]
     L.rr_launch_count.argtypes = [vp]
     L.rr_launch_count.restype = C.c_uint64
     L.rr_version.restype = C.c_int
@@ -546,7 +550,8 @@ class Fusion:
         """rr_extract_mesh alone: extracts the surface on the device and returns (vertices, triangles)."""
         nv, nt = C.c_uint32(), C.c_uint32()
         self._ck(self.L.rr_extract_mesh(self.h, C.byref(nv), C.byref(nt)))
-        return int(nv.value), int(nt.value)
+        self._mesh_n = (int(nv.value), int(nt.value))
+        return self._mesh_n
 
     def download_mesh(self, nv, nt):
         """rr_download_mesh of the last extraction (nv, nt: its counts)."""
@@ -593,6 +598,50 @@ class Fusion:
         pixel ids uint32 [n] (sensor * W * H + y * W + x, ascending). sensors: iterable of sensor indices, default all;
         device: return torch tensors on the context's GPU instead of numpy arrays."""
         return self.download_points(self.extract_points_count(sensors), device)
+
+    def label_parts_count(self):
+        """rr_label_parts alone: labels the connected parts of the volume on the device and returns their count."""
+        n = C.c_uint32()
+        self._ck(self.L.rr_label_parts(self.h, C.byref(n)))
+        return int(n.value)
+
+    def download_parts(self, n):
+        """rr_download_parts of the last labelling (n: its part count): (voxels uint32 [n], boxes int32 [n, 6], centroids
+        float32 [n, 3])."""
+        voxels, boxes, centroids = np.empty(n, np.uint32), np.empty((n, 6), np.int32), np.empty((n, 3), np.float32)
+        self._ck(self.L.rr_download_parts(self.h, voxels.ctypes.data, boxes.ctypes.data, centroids.ctypes.data, None))
+        return voxels, boxes, centroids
+
+    def label_parts(self):
+        """The 6-connected parts of the inside voxels (v > 0, finite), numbered by ascending smallest linear index
+        (rr_label_parts + rr_download_parts): (voxels uint32 [P], boxes int32 [P, 6] = x0, x1, y0, y1, z0, z1 half-open
+        voxel ranges, centroids float32 [P, 3] in metres)."""
+        return self.download_parts(self.label_parts_count())
+
+    def part_labels(self, device=False):
+        """The labels of the last labelling: uint32 [Z, Y, X], the part of every inside voxel and 0xFFFFFFFF elsewhere; a
+        numpy array, or with device a CUDA tensor on the context's GPU."""
+        X, Y, Z = (int(v) for v in self.volume_res())
+        dev = None
+        if device:
+            import torch
+            dev = torch.device("cuda", self.device)
+        (labels,), (ptr,) = _query_outputs(dev, ((Z, Y, X), "u4"))
+        self._ck(self.L.rr_download_parts(self.h, None, None, None, ptr))
+        return labels
+
+    def mesh_parts(self, device=False, counts=None):
+        """rr_download_mesh_parts: (vertex_parts uint32 [V], triangle_parts uint32 [T]) of the last mesh, which must come
+        from the same volume state as the last labelling; numpy arrays, or with device CUDA tensors. counts: the mesh's
+        (V, T), by default those of this object's last extract_mesh."""
+        nv, nt = counts if counts is not None else getattr(self, "_mesh_n", (0, 0))
+        dev = None
+        if device:
+            import torch
+            dev = torch.device("cuda", self.device)
+        outs, ptrs = _query_outputs(dev, ((nv,), "u4"), ((nt,), "u4"))
+        self._ck(self.L.rr_download_mesh_parts(self.h, *ptrs))
+        return tuple(outs)
 
     def set_timing(self, level=1):
         self._ck(self.L.rr_set_timing(self.h, int(level)))
@@ -798,7 +847,8 @@ class Group:
         """rr_group_extract_mesh: the whole volume's surface, extracted on member 0; returns (vertices, triangles)."""
         nv, nt = C.c_uint32(), C.c_uint32()
         self._ck(self.L.rr_group_extract_mesh(self.h, C.byref(nv), C.byref(nt)))
-        return int(nv.value), int(nt.value)
+        self._mesh_n = (int(nv.value), int(nt.value))
+        return self._mesh_n
 
     def extract_mesh(self):
         """As Fusion.extract_mesh, equal to a single context's bit for bit: (positions, normals, rgba, triangles)."""
@@ -810,6 +860,21 @@ class Group:
         n = C.c_uint32()
         self._ck(self.L.rr_group_extract_points(self.h, _sensor_mask(sensors, self.N), C.byref(n)))
         return self.member(0).download_points(int(n.value), device)
+
+    def label_parts(self):
+        """As Fusion.label_parts (rr_group_label_parts: the whole volume, labelled on member 0), equal to a single context
+        bit for bit: (voxels, boxes, centroids)."""
+        n = C.c_uint32()
+        self._ck(self.L.rr_group_label_parts(self.h, C.byref(n)))
+        return self.member(0).download_parts(int(n.value))
+
+    def part_labels(self, device=False):
+        """As Fusion.part_labels, from member 0 (CUDA tensors on member 0's GPU)."""
+        return self.member(0).part_labels(device)
+
+    def mesh_parts(self, device=False):
+        """As Fusion.mesh_parts, for the group's last extract_mesh and label_parts (member 0)."""
+        return self.member(0).mesh_parts(device, getattr(self, "_mesh_n", (0, 0)))
 
     def sample_points(self, points, space="world"):
         """As Fusion.sample_points (CUDA tensors on member 0's GPU), equal to a single context's bit for bit."""

@@ -19,12 +19,15 @@ u32p = np.ctypeslib.ndpointer(np.uint32, flags="C_CONTIGUOUS")
 i32p = np.ctypeslib.ndpointer(np.int32, flags="C_CONTIGUOUS")
 u8p = np.ctypeslib.ndpointer(np.uint8, flags="C_CONTIGUOUS")
 
+# the volume block that ro_extract_mesh, ro_sample_points and ro_cast_rays start with (VolumeArgs)
+_VOLUME_ARGS = [f32p, u32p, C.c_float, C.c_int, C.c_void_p, i32p, C.c_void_p, i32p, C.c_void_p, C.c_int, C.c_int,
+                C.c_void_p, C.c_void_p, C.c_int, C.c_int, f32p, f32p]
 
-def build(force=False):
-    so = os.path.join(_HERE, "librr_oracle.so")
-    if force or not os.path.exists(so):
-        subprocess.check_call(["make", "-s", "-C", _HERE, "librr_oracle.so"])
-    return so
+
+def build():
+    """make tracks the sources: a library older than any of them is rebuilt, a current one is left as it is."""
+    subprocess.check_call(["make", "-s", "-C", _HERE, "librr_oracle.so"])
+    return os.path.join(_HERE, "librr_oracle.so")
 
 
 def lib():
@@ -75,8 +78,44 @@ def lib():
     L.ro_fill_num_lods.argtypes = [C.c_int, C.c_int]
     L.ro_fill_num_lods.restype = C.c_int
     L.ro_fill_colors.argtypes = [f32p, f32p, C.c_int, C.c_int, f32p, C.c_void_p, C.c_void_p]
+    L.ro_mesh_case_table.argtypes = [i32p, i32p]
+    L.ro_mesh_case_table.restype = C.c_int
+    L.ro_extract_mesh.argtypes = _VOLUME_ARGS + [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.ro_sample_points.argtypes = _VOLUME_ARGS + [C.c_int, f32p, C.c_uint32, f32p, f32p, f32p]
+    L.ro_cast_rays.argtypes = _VOLUME_ARGS + [C.c_int, C.c_void_p, C.c_uint32, u32p, C.c_float, C.c_int, f32p, f32p, C.c_uint32,
+                                              f32p, f32p, f32p, u32p]
+    L.ro_extract_points.argtypes = [C.c_int, C.c_int, C.c_int, f32p, f32p, f32p, u8p, C.c_int, C.c_int, f32p, f32p, i32p, f32p, f32p,
+                                    C.c_uint32, C.POINTER(C.c_uint32), f32p, f32p, f32p, f32p, u32p]
     _LIB = L
     return L
+
+
+class VolumeArgs:
+    """The volume block of ro_extract_mesh, ro_sample_points and ro_cast_rays (`args`): tsdf float32 [Z][Y][X] (res = (X, Y, Z)),
+    and optionally the inverse volumes, scene (cv_uv, colour) and pre-processed stage images blendColors reads (all three or
+    none). Holds the arrays the raw pointers of `args` point into."""
+
+    def __init__(self, tsdf, res, limit, inv, scene, pre, bbox_min, bbox_max):
+        self.keep = []
+        tsdf = np.ascontiguousarray(tsdf, np.float32)
+        bmin = np.ascontiguousarray(bbox_min, np.float32)
+        bmax = np.ascontiguousarray(bbox_max, np.float32)
+        head = (tsdf, np.ascontiguousarray(res, np.uint32), np.float32(limit))
+        if inv is not None:
+            N, IZ, IY, IX, _ = inv.shape
+            X, Y, Z = scene.cv_res
+            _, H, W = pre["quality"].shape
+            self.args = head + (N, self._ptr(inv, np.float32), np.array([IX, IY, IZ], np.int32), self._ptr(scene.cv_uv, np.float32),
+                                np.array([X, Y, Z], np.int32), self._ptr(scene.color, np.uint8), scene.CW, scene.CH,
+                                self._ptr(pre["depth_b"], np.float32), self._ptr(pre["quality"], np.float32), W, H, bmin, bmax)
+        else:
+            z3 = np.zeros(3, np.int32)
+            self.args = head + (0, None, z3, None, z3, None, 0, 0, None, None, 0, 0, bmin, bmax)
+
+    def _ptr(self, a, dt):
+        a = np.ascontiguousarray(a, dt)
+        self.keep.append(a)
+        return a.ctypes.data
 
 
 def set_threads(n):

@@ -3,7 +3,7 @@
 // vertex buffer, glsl/points.gs:39-41 bbox / depth cull, points.fs:38-41 colour-view border cut), in draw order, with the
 // attributes at the pixel and the colour points.fs shades with. The lookups are ro_points.cpp's, through the same
 // tex3d_linear (ro_math.h) and fetch_rgb8 (ro_draw.h).
-#include "ro_cloud.h"
+#include "rr_oracle.h"
 
 #include "ro_draw.h"
 #include "ro_math.h"

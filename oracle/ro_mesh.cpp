@@ -1,10 +1,9 @@
 // ORACLE (test infrastructure, NOT product code): scalar restatement of the library's surface extraction (rr_extract_mesh,
 // rgbd-recon_b200/csrc/rr_mesh.cu; the contract is stated in include/rgbd_recon_b200.h). Marching cubes over every cell in
-// canonical order, with its own generator of the case table. The sample functions are the raymarch oracle's (ro_sample.h). Built
-// into its own library (mesh.mk, oracle_mesh.py).
+// canonical order, with its own generator of the case table. The sample functions are the raymarch oracle's (ro_sample.h).
 #include "ro_math.h"
 #include "ro_sample.h"
-#include "ro_mesh.h"
+#include "rr_oracle.h"
 
 #include <algorithm>
 #include <cmath>

@@ -1,10 +1,10 @@
 // ORACLE (test infrastructure, NOT product code): scalar restatement of the library's volume queries (rr_sample_points /
 // rr_cast_rays, rgbd-recon_b200/csrc/rr_query.cu; the contract is stated in include/rgbd_recon_b200.h). The sample
 // functions are the raymarch oracle's (ro_sample.h); the march is ro_raymarch.cpp's with the brute-force brick hull, from
-// the caller's origin and direction instead of a pixel's. Built into its own library (query.mk, oracle_query.py).
+// the caller's origin and direction instead of a pixel's.
 #include "ro_math.h"
 #include "ro_sample.h"
-#include "ro_query.h"
+#include "rr_oracle.h"
 
 #include <cmath>
 #include <vector>

@@ -1,8 +1,7 @@
 // ORACLE (test infrastructure, NOT product code): what the raymarch reads from the volume and the stage images at a point of
-// volume space (tsdf_raymarch.fs:148-157 getGradient, :303-338 blendColors) for ro_mesh.cpp: the functions of ro_raymarch.cpp,
-// restated word for word. The library shares one implementation between its raymarch and its mesh (csrc/rr_sample.cuh), and
-// the GPU tests hold the raymarch to ro_raymarch.cpp and the mesh to ro_mesh.cpp, bit for bit, so the two oracle copies
-// cannot drift apart without a test failing.
+// volume space (tsdf_raymarch.fs:148-157 getGradient, :303-338 blendColors). One copy, shared by the raymarch (ro_raymarch.cpp),
+// the mesh (ro_mesh.cpp) and the queries (ro_query.cpp), as the library shares csrc/rr_sample.cuh between its raymarch, mesh
+// and queries.
 #ifndef RO_SAMPLE_H
 #define RO_SAMPLE_H
 

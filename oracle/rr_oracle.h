@@ -87,6 +87,44 @@ void ro_depth8_to_float(const uint8_t* in, size_t n, float* out);
 int ro_fill_num_lods(int W, int H);
 void ro_fill_colors(const float* rgba, const float* depth, int W, int H, float* out_rgba, float* atlas_rgba, float* atlas_depth);
 
+/* Surface extraction (rr_extract_mesh), see ro_mesh.cpp.
+ * ro_mesh_case_table: ntri int32[256], tri int32[256][30] (cube edges, -1 past the case's triangles); returns the most
+ * triangles any case needs, -1 if the rule is inconsistent.
+ * ro_extract_mesh: counts[2] = vertices, triangles; positions [V][3], normals [V][3], rgba [V][4], triangles uint32 [T][3],
+ * each may be null (a first call with all null gives the counts). tsdf float32 [Z][Y][X] as rr_download_tsdf returns it;
+ * inv, cv_uv, color, depth_b and quality may be null when normals and rgba are. */
+int ro_mesh_case_table(int32_t* ntri, int32_t* tri);
+void ro_extract_mesh(const float* tsdf, const uint32_t* res, float limit, int N, const float* inv, const int32_t* inv_res,
+                     const float* cv_uv, const int32_t* cv_res, const uint8_t* color, int CW, int CH,
+                     const float* depth_b, const float* quality, int W, int H, const float* bbox_min, const float* bbox_max,
+                     uint64_t* counts, float* positions, float* normals, float* rgba, uint32_t* triangles);
+
+/* Volume queries (rr_sample_points / rr_cast_rays), see ro_query.cpp. tsdf float32 [Z][Y][X] as rr_download_tsdf returns
+ * it; N may be 0 (inv, cv_uv, color, depth_b and quality null) when the colours are not wanted. space: 0 world (metres),
+ * 1 volume texture coordinates.
+ * ro_cast_rays: skip_space selects the march over the occupied-brick hull (occupied: the ordered list of
+ * rr_download_bricks, brick_res / brick_size as rr_get_brick_info). Outputs as the library's: values [n] or positions
+ * [n][3], normals [n][3], rgba [n][4], steps uint32 [n]. */
+void ro_sample_points(const float* tsdf, const uint32_t* res, float limit, int N, const float* inv, const int32_t* inv_res,
+                      const float* cv_uv, const int32_t* cv_res, const uint8_t* color, int CW, int CH,
+                      const float* depth_b, const float* quality, int W, int H, const float* bbox_min, const float* bbox_max,
+                      int space, const float* points, uint32_t count, float* values, float* normals, float* rgba);
+void ro_cast_rays(const float* tsdf, const uint32_t* res, float limit, int N, const float* inv, const int32_t* inv_res,
+                  const float* cv_uv, const int32_t* cv_res, const uint8_t* color, int CW, int CH,
+                  const float* depth_b, const float* quality, int W, int H, const float* bbox_min, const float* bbox_max,
+                  int skip_space, const uint32_t* occupied, uint32_t n_occ, const uint32_t* brick_res, float brick_size,
+                  int space, const float* origins, const float* directions, uint32_t count,
+                  float* positions, float* normals, float* rgba, uint32_t* steps);
+
+/* Point-cloud export (rr_extract_points), see ro_cloud.cpp. depth_b float32 [N][H][W][2], normal float32 [N][H][W][3],
+ * quality float32 [N][H][W], colour uint8 [N][CH][CW][3], cv_xyz float32 [N][Z][Y][X][3], cv_uv float32 [N][Z][Y][X][2]
+ * (cv_res = X, Y, Z, one resolution for all sensors). Outputs hold up to N*W*H points: positions [n][3], normals [n][3],
+ * colours [n][3], quality [n], pixel ids uint32 [n]; *out_n receives n. */
+void ro_extract_points(int N, int W, int H, const float* depth_b, const float* normal, const float* quality, const uint8_t* color,
+                       int CW, int CH, const float* cv_xyz, const float* cv_uv, const int32_t* cv_res, const float* bmin,
+                       const float* bmax, uint32_t sensor_mask, uint32_t* out_n, float* positions, float* normals, float* colors,
+                       float* quality_out, uint32_t* pixels);
+
 #ifdef __cplusplus
 }
 #endif

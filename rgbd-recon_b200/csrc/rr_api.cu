@@ -141,10 +141,7 @@ int rr_create(rr_ctx** out, int device, int num_sensors, int depth_w, int depth_
   if (rc == RR_OK) rc = dev_alloc(c, &c->d_flags, 4, "flags");
   if (rc == RR_OK) rc = dev_alloc(c, &c->d_num_occ, 1, "num_occ");
   if (rc == RR_OK) rc = dev_alloc(c, &c->d_work, 4, "work counters");
-  if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_num_occ, sizeof(uint32_t)), "pinned count");
-  if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_mesh_totals, 2 * sizeof(unsigned long long)), "pinned mesh totals");
-  if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_cloud_count, sizeof(uint32_t)), "pinned cloud count");
-  if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->h_parts_count, sizeof(uint32_t)), "pinned part count");
+  if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->pinned, sizeof(rr::PinnedScalars)), "pinned scalars");
   if (rc == RR_OK) {
     cudaMemsetAsync(c->d_flags, 0, 4 * sizeof(uint32_t), c->stream);
     cudaMemsetAsync(c->d_pairs, 0, (size_t)c->N * (c->H + 2) * c->pair_pitch * sizeof(float2), c->stream);
@@ -153,7 +150,7 @@ int rr_create(rr_ctx** out, int device, int num_sensors, int depth_w, int depth_
       cudaMemsetAsync(c->d_color_slot[b], 0, (size_t)c->N * c->CW * c->CH * 3, c->stream);
       cudaMemsetAsync(c->d_depth_slot[b], 0, px * sizeof(float), c->stream);
     }
-    *c->h_num_occ = 0;
+    c->pinned->num_occ = 0;
     rc = check(c, cudaStreamSynchronize(c->stream), "create sync");
   }
   if (rc != RR_OK) { rr_destroy(c); return rc; }
@@ -175,12 +172,6 @@ void rr_destroy(rr_ctx* c) {
   cudaFree(c->d_inv); cudaFree(c->d_morph); cudaFree(c->d_depth);
   cudaFree(c->d_lab); cudaFree(c->d_depth_b); cudaFree(c->d_sil); cudaFree(c->d_normal); cudaFree(c->d_quality);
   staged_release(c);
-  trigrid_release(c);
-  mesh_release(c);
-  query_release(c);
-  cloud_release(c);
-  parts_release(c);
-  if (c->h_parts_count) cudaFreeHost(c->h_parts_count);
   for (auto& v : c->ipc_views) { cudaIpcCloseMemHandle(v.step); cudaIpcCloseMemHandle(v.rgba); cudaIpcCloseMemHandle(v.zbuf); cudaIpcCloseMemHandle(v.nsamp); }
   cudaGetLastError();
   cudaFree(c->d_pairs);
@@ -188,7 +179,7 @@ void rr_destroy(rr_ctx* c) {
   cudaFree(c->d_num_occ); cudaFree(c->d_work); cudaFree(c->d_ztab); cudaFree(c->d_rowmask); cudaFree(c->d_rowany); cudaFree(c->d_cand_y); cudaFree(c->d_cand_z); cudaFree(c->d_near_occ); cudaFree(c->d_occ_mask); cudaFree(c->d_pos); cudaFree(c->d_step); cudaFree(c->d_tsdf); cudaFree(c->d_weight);
   cudaFree(c->d_rgba); cudaFree(c->d_zbuf); cudaFree(c->d_nsamples); cudaFree(c->d_point_keys);
   cudaFree(c->d_fill_fc); cudaFree(c->d_fill_fd); cudaFree(c->d_fill_sc); cudaFree(c->d_fill_sd); cudaFree(c->d_filled);
-  if (c->h_num_occ) cudaFreeHost(c->h_num_occ);
+  if (c->pinned) cudaFreeHost(c->pinned);
   for (auto& kv : c->timers) {
     for (cudaEvent_t e : kv.second.beg) cudaEventDestroy(e);
     for (cudaEvent_t e : kv.second.end) cudaEventDestroy(e);
@@ -335,7 +326,10 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     c->parts_valid = false;
     ++c->volume_epoch;
   }
-  if (new_volume) parts_release(c);   // the label array is sized by the volume
+  if (new_volume) {   // the label and row arrays are sized by the volume
+    c->d_parts_labels.release();
+    c->d_parts_rows.release();
+  }
   if (new_bricks) {
     c->mesh_rows_ok = false;
     uint32_t rb[3];
@@ -379,7 +373,7 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     cudaMemsetAsync(c->d_near_occ, 0, nb, c->stream);
     cudaMemsetAsync(c->d_occ_mask, 0, nb, c->stream);
     cudaMemsetAsync(c->d_num_occ, 0, sizeof(uint32_t), c->stream);
-    *c->h_num_occ = 0;
+    c->pinned->num_occ = 0;
     RR_TRY(check(c, cudaStreamSynchronize(c->stream), "brick table upload"));
   }
   c->cfg = *cfg;
@@ -555,8 +549,8 @@ int rr_bricks_update(rr_ctx* c, uint32_t* out_num, float* out_ratio) {
   RR_TRY(launch_bricks_update(c));
   if (out_num || out_ratio) {
     RR_TRY(check(c, cudaStreamSynchronize(c->stream), "bricks update sync"));
-    if (out_num) *out_num = *c->h_num_occ;
-    if (out_ratio) *out_ratio = float(*c->h_num_occ) / float(c->bricks.num);
+    if (out_num) *out_num = c->pinned->num_occ;
+    if (out_ratio) *out_ratio = float(c->pinned->num_occ) / float(c->bricks.num);
   }
   return RR_OK;
 }
@@ -626,8 +620,8 @@ int rr_bricks_count(rr_ctx* c, uint32_t* out_num, float* out_ratio) {
   RR_REQUIRE(c, c->configured, "rr_bricks_count: call rr_configure first");
   RR_SET_DEVICE(c);
   RR_TRY(check(c, cudaStreamSynchronize(c->stream), "bricks count sync"));
-  if (out_num) *out_num = *c->h_num_occ;
-  if (out_ratio) *out_ratio = float(*c->h_num_occ) / float(c->bricks.num);
+  if (out_num) *out_num = c->pinned->num_occ;
+  if (out_ratio) *out_ratio = float(c->pinned->num_occ) / float(c->bricks.num);
   return RR_OK;
 }
 
@@ -1008,10 +1002,10 @@ int rr_download_mesh(rr_ctx* c, float* positions, float* normals, float* rgba, u
   RR_REQUIRE(c, c->mesh_valid, "rr_download_mesh: no mesh extracted from the current volume (rr_extract_mesh first)");
   RR_SET_DEVICE(c);
   const size_t nv = c->mesh_nv, nt = c->mesh_nt;
-  if (positions && nv) RR_TRY(check(c, cudaMemcpyAsync(positions, c->d_mesh_pos, nv * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
-  if (normals && nv) RR_TRY(check(c, cudaMemcpyAsync(normals, c->d_mesh_nrm, nv * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
-  if (rgba && nv) RR_TRY(check(c, cudaMemcpyAsync(rgba, c->d_mesh_rgba, nv * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
-  if (triangles && nt) RR_TRY(check(c, cudaMemcpyAsync(triangles, c->d_mesh_tri, nt * 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
+  if (positions && nv) RR_TRY(check(c, cudaMemcpyAsync(positions, c->d_mesh_pos.ptr, nv * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
+  if (normals && nv) RR_TRY(check(c, cudaMemcpyAsync(normals, c->d_mesh_nrm.ptr, nv * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
+  if (rgba && nv) RR_TRY(check(c, cudaMemcpyAsync(rgba, c->d_mesh_rgba.ptr, nv * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
+  if (triangles && nt) RR_TRY(check(c, cudaMemcpyAsync(triangles, c->d_mesh_tri.ptr, nt * 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream), "mesh download"));
   return check(c, cudaStreamSynchronize(c->stream), "mesh download sync");
 }
 

@@ -124,7 +124,7 @@ int launch_bricks_update(rr_ctx* c) {
   c->work_fresh = true;
   c->mesh_rows_ok = false;     // new row tables: the volume was cleared by the previous ones
   if (classify) c->sti.lists_key = staged_lists_key(c);
-  cudaError_t e = cudaMemcpyAsync(c->h_num_occ, c->d_num_occ, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream);
+  cudaError_t e = cudaMemcpyAsync(&c->pinned->num_occ, c->d_num_occ, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream);
   return check(c, e, "bricks count copy");
 }
 

@@ -56,48 +56,17 @@ __global__ void __launch_bounds__(256) k_cloud_write(const __grid_constant__ Clo
   p.pix[o] = id;
 }
 
-template <typename T>
-int grow(rr_ctx* c, T** ptr, size_t* cap, size_t need, const char* what) {
-  if (need <= *cap && *ptr) return RR_OK;
-  if (*ptr) {
-    RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), what));   // the last extraction's copies may still read it
-    cudaFree(*ptr);
-  }
-  *ptr = nullptr; *cap = 0;
-  const size_t n = need + need / 8 + 1;
-  RR_TRY_RC(check(c, cudaMalloc((void**)ptr, n * sizeof(T)), what));
-  *cap = n;
-  return RR_OK;
-}
-
-// the per-point arrays share one capacity (in points), grown with 1/8 slack like the query buffers
-int grow_points(rr_ctx* c, size_t n_points) {
-  if (n_points <= c->cloud_cap && c->d_cloud_pos) return RR_OK;
-  RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "cloud buffers"));
-  cudaFree(c->d_cloud_pos); cudaFree(c->d_cloud_nrm); cudaFree(c->d_cloud_rgb); cudaFree(c->d_cloud_q); cudaFree(c->d_cloud_pix);
-  c->d_cloud_pos = nullptr; c->d_cloud_nrm = nullptr; c->d_cloud_rgb = nullptr; c->d_cloud_q = nullptr; c->d_cloud_pix = nullptr;
-  c->cloud_cap = 0;
-  const size_t n = n_points + n_points / 8 + 1;
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_cloud_pos, n * 3 * sizeof(float)), "cloud positions"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_cloud_nrm, n * 3 * sizeof(float)), "cloud normals"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_cloud_rgb, n * 3 * sizeof(float)), "cloud colours"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_cloud_q, n * sizeof(float)), "cloud quality"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_cloud_pix, n * sizeof(uint32_t)), "cloud pixel ids"));
-  c->cloud_cap = n;
-  return RR_OK;
-}
-
 }  // namespace
 
 int launch_extract_points(rr_ctx* c, uint32_t mask, uint32_t* out_n) {
   c->cloud_valid = false;
   const uint32_t n_px = (uint32_t)((size_t)c->N * c->W * c->H);
-  RR_TRY_RC(grow(c, &c->d_cloud_flags, &c->cloud_flags_cap, 2 * ((size_t)n_px + 1), "cloud flags"));
-  uint32_t* flags = c->d_cloud_flags;
+  RR_TRY_RC(c->d_cloud_flags.reserve(c, 2 * ((size_t)n_px + 1), "cloud flags"));
+  uint32_t* flags = c->d_cloud_flags.ptr;
   uint32_t* offsets = flags + (n_px + 1);
   size_t scan_bytes = 0;
   RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, flags, offsets, (int)(n_px + 1), c->stream), "cloud scan size"));
-  RR_TRY_RC(grow(c, &c->d_cloud_scratch, &c->cloud_scratch_cap, scan_bytes, "cloud scan scratch"));
+  RR_TRY_RC(c->d_cloud_scratch.reserve(c, scan_bytes, "cloud scan scratch"));
 
   CloudParams p{};
   p.st = sensor_tables(c);
@@ -109,15 +78,19 @@ int launch_extract_points(rr_ctx* c, uint32_t mask, uint32_t* out_n) {
 
   k_cloud_flags<<<(n_px + 1 + 255) / 256, 256, 0, c->stream>>>(p);
   RR_LAUNCH_CHECK(c, "k_cloud_flags");
-  size_t bytes = c->cloud_scratch_cap;
-  RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(c->d_cloud_scratch, bytes, flags, offsets, (int)(n_px + 1), c->stream), "cloud scan"));
+  size_t bytes = c->d_cloud_scratch.cap;
+  RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(c->d_cloud_scratch.ptr, bytes, flags, offsets, (int)(n_px + 1), c->stream), "cloud scan"));
   ++c->launches;
-  RR_TRY_RC(check(c, cudaMemcpyAsync(c->h_cloud_count, offsets + n_px, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream), "cloud count"));
+  RR_TRY_RC(check(c, cudaMemcpyAsync(&c->pinned->cloud_count, offsets + n_px, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream), "cloud count"));
   RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "cloud count sync"));
-  const uint32_t n = *c->h_cloud_count;
+  const uint32_t n = c->pinned->cloud_count;
   if (n) {
-    RR_TRY_RC(grow_points(c, n));
-    p.pos = c->d_cloud_pos; p.nrm = c->d_cloud_nrm; p.rgb = c->d_cloud_rgb; p.q = c->d_cloud_q; p.pix = c->d_cloud_pix;
+    RR_TRY_RC(c->d_cloud_pos.reserve(c, 3 * (size_t)n, "cloud positions"));
+    RR_TRY_RC(c->d_cloud_nrm.reserve(c, 3 * (size_t)n, "cloud normals"));
+    RR_TRY_RC(c->d_cloud_rgb.reserve(c, 3 * (size_t)n, "cloud colours"));
+    RR_TRY_RC(c->d_cloud_q.reserve(c, n, "cloud quality"));
+    RR_TRY_RC(c->d_cloud_pix.reserve(c, n, "cloud pixel ids"));
+    p.pos = c->d_cloud_pos.ptr; p.nrm = c->d_cloud_nrm.ptr; p.rgb = c->d_cloud_rgb.ptr; p.q = c->d_cloud_q.ptr; p.pix = c->d_cloud_pix.ptr;
     k_cloud_write<<<(n_px + 255) / 256, 256, 0, c->stream>>>(p);
     RR_LAUNCH_CHECK(c, "k_cloud_write");
   }
@@ -130,19 +103,13 @@ int launch_extract_points(rr_ctx* c, uint32_t mask, uint32_t* out_n) {
 int cloud_download(rr_ctx* c, float* positions, float* normals, float* colors, float* quality, uint32_t* pixels) {
   const size_t n = c->cloud_n;
   if (n) {
-    if (positions) RR_TRY_RC(check(c, cudaMemcpyAsync(positions, c->d_cloud_pos, n * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "cloud download"));
-    if (normals) RR_TRY_RC(check(c, cudaMemcpyAsync(normals, c->d_cloud_nrm, n * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "cloud download"));
-    if (colors) RR_TRY_RC(check(c, cudaMemcpyAsync(colors, c->d_cloud_rgb, n * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "cloud download"));
-    if (quality) RR_TRY_RC(check(c, cudaMemcpyAsync(quality, c->d_cloud_q, n * sizeof(float), cudaMemcpyDefault, c->stream), "cloud download"));
-    if (pixels) RR_TRY_RC(check(c, cudaMemcpyAsync(pixels, c->d_cloud_pix, n * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "cloud download"));
+    if (positions) RR_TRY_RC(check(c, cudaMemcpyAsync(positions, c->d_cloud_pos.ptr, n * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "cloud download"));
+    if (normals) RR_TRY_RC(check(c, cudaMemcpyAsync(normals, c->d_cloud_nrm.ptr, n * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "cloud download"));
+    if (colors) RR_TRY_RC(check(c, cudaMemcpyAsync(colors, c->d_cloud_rgb.ptr, n * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "cloud download"));
+    if (quality) RR_TRY_RC(check(c, cudaMemcpyAsync(quality, c->d_cloud_q.ptr, n * sizeof(float), cudaMemcpyDefault, c->stream), "cloud download"));
+    if (pixels) RR_TRY_RC(check(c, cudaMemcpyAsync(pixels, c->d_cloud_pix.ptr, n * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "cloud download"));
   }
   return check(c, cudaStreamSynchronize(c->stream), "cloud download sync");
-}
-
-void cloud_release(rr_ctx* c) {
-  cudaFree(c->d_cloud_flags); cudaFree(c->d_cloud_scratch);
-  cudaFree(c->d_cloud_pos); cudaFree(c->d_cloud_nrm); cudaFree(c->d_cloud_rgb); cudaFree(c->d_cloud_q); cudaFree(c->d_cloud_pix);
-  if (c->h_cloud_count) cudaFreeHost(c->h_cloud_count);
 }
 
 }  // namespace rr

@@ -61,6 +61,29 @@ struct StageTimer {            // one CUDA-event pair per recorded interval; sum
   float last_ms = 0.0f;        // the newest folded interval (rr_get_stage_ms right after a fold)
 };
 
+// A device array of the context that grows on demand to the size of a result (reserve, defined below rr_ctx); freed by the
+// context's destructor, on the context's device.
+template <typename T>
+struct DeviceArray {
+  T* ptr = nullptr;
+  size_t cap = 0;              // in elements
+  DeviceArray() = default;
+  DeviceArray(const DeviceArray&) = delete;
+  DeviceArray& operator=(const DeviceArray&) = delete;
+  ~DeviceArray() { cudaFree(ptr); }
+  int reserve(rr_ctx* c, size_t need, const char* what);
+  void release() { cudaFree(ptr); ptr = nullptr; cap = 0; }
+};
+
+// Host scalars that device-to-host copies land in, one slot per reader: num_occ is filled by an asynchronous copy in
+// rr_bricks_update and read by a later call, so no other copy may reuse its slot.
+struct PinnedScalars {
+  uint32_t num_occ;
+  uint32_t cloud_count;
+  uint32_t parts_count;
+  unsigned long long mesh_totals[2];   // vertices, triangles
+};
+
 }  // namespace rr
 
 struct rr_ctx {
@@ -178,7 +201,7 @@ struct rr_ctx {
     uint32_t* d_err = nullptr;     // [4] device-side consistency flags (must stay 0)
     CUtensorMap map_inv, map_pairs;
   } sti;
-  uint32_t* h_num_occ = nullptr;   // pinned
+  rr::PinnedScalars* pinned = nullptr;   // one cudaMallocHost allocation for the context's lifetime
   float* d_tsdf = nullptr;
   float* d_weight = nullptr;
 
@@ -192,11 +215,11 @@ struct rr_ctx {
   unsigned long long* d_point_keys = nullptr;   // rr_draw_points / rr_draw_calibs: per pixel (depth bits << 32 | vertex id), atomicMin
 
   // rr_draw_trigrid (rr_trigrid.cu): vertex records, pass-1 depth bits, per-pixel fragment lists (grown on demand)
-  float4* d_tg_verts = nullptr; size_t tg_verts_cap = 0;
-  uint32_t* d_tg_depth = nullptr; size_t tg_depth_cap = 0;
-  uint32_t* d_tg_head = nullptr; size_t tg_head_cap = 0;
-  float4* d_tg_frag_rgba = nullptr; float4* d_tg_frag_pos = nullptr; uint2* d_tg_frag_link = nullptr; size_t tg_frag_cap = 0;
-  uint32_t* d_tg_count = nullptr;
+  rr::DeviceArray<float4> d_tg_verts;
+  rr::DeviceArray<uint32_t> d_tg_depth, d_tg_head;
+  rr::DeviceArray<float4> d_tg_frag_rgba, d_tg_frag_pos;
+  rr::DeviceArray<uint2> d_tg_frag_link;
+  rr::DeviceArray<uint32_t> d_tg_count;
 
   // surface extraction (rr_mesh.cu)
   bool volume_integrated = false;  // an integrate has run into the current volume allocation
@@ -204,41 +227,40 @@ struct rr_ctx {
   bool mesh_table = false;         // the case table is in this device's constant memory
   bool mesh_valid = false;         // the d_mesh_* arrays hold an extraction of the current volume allocation (of mesh_epoch)
   uint32_t mesh_nv = 0, mesh_nt = 0;
-  unsigned long long* d_mesh_rows = nullptr; size_t mesh_rows_cap = 0;   // per row: counts and offsets of vertices, triangles
-  uint8_t* d_mesh_scratch = nullptr; size_t mesh_scratch_cap = 0;        // CUB scan storage
-  unsigned long long* d_mesh_keys = nullptr;   // [V] edge key = linear index of the lower corner * 3 + axis
-  float* d_mesh_pos = nullptr; float* d_mesh_nrm = nullptr; float4* d_mesh_rgba = nullptr; size_t mesh_v_cap = 0;
-  uint32_t* d_mesh_tri = nullptr; size_t mesh_t_cap = 0;
-  unsigned long long* h_mesh_totals = nullptr;   // pinned [2]: vertices, triangles
+  rr::DeviceArray<unsigned long long> d_mesh_rows;   // per row: counts and offsets of vertices, triangles
+  rr::DeviceArray<uint8_t> d_mesh_scratch;           // CUB scan storage
+  rr::DeviceArray<unsigned long long> d_mesh_keys;   // [V] edge key = linear index of the lower corner * 3 + axis
+  rr::DeviceArray<float> d_mesh_pos, d_mesh_nrm;     // [V][3]
+  rr::DeviceArray<float4> d_mesh_rgba;               // [V]
+  rr::DeviceArray<uint32_t> d_mesh_tri;              // [T][3]
 
-  // queries (rr_query.cu): inputs (points [n][3], or origins [n][3] then directions [n][3]) and per-entry results, one
-  // capacity in entries, grown on demand
-  float* d_q_in = nullptr; float* d_q_val = nullptr; float* d_q_pos = nullptr; float* d_q_nrm = nullptr;
-  float4* d_q_rgba = nullptr; uint32_t* d_q_step = nullptr; size_t q_cap = 0;
+  // queries (rr_query.cu): inputs (points [n][3], or origins [n][3] then directions [n][3]) and per-entry results
+  rr::DeviceArray<float> d_q_in, d_q_val, d_q_pos, d_q_nrm;
+  rr::DeviceArray<float4> d_q_rgba;
+  rr::DeviceArray<uint32_t> d_q_step;
 
-  // point-cloud export (rr_cloud.cu): per depth pixel a keep flag, then its exclusive scan; per kept point the outputs, one
-  // capacity in points, grown on demand
+  // point-cloud export (rr_cloud.cu): per depth pixel a keep flag, then its exclusive scan; per kept point the outputs
   bool preprocessed = false;       // an rr_preprocess / rr_fuse_frame has defined the stage images
   bool cloud_valid = false;        // the d_cloud_* arrays hold the last extraction (cloud_n points)
   uint32_t cloud_n = 0;
-  uint32_t* d_cloud_flags = nullptr; size_t cloud_flags_cap = 0;   // [2][N * W * H + 1]: flags, offsets
-  uint8_t* d_cloud_scratch = nullptr; size_t cloud_scratch_cap = 0; // CUB scan storage
-  float* d_cloud_pos = nullptr; float* d_cloud_nrm = nullptr; float* d_cloud_rgb = nullptr; float* d_cloud_q = nullptr;
-  uint32_t* d_cloud_pix = nullptr; size_t cloud_cap = 0;
-  uint32_t* h_cloud_count = nullptr;   // pinned
+  rr::DeviceArray<uint32_t> d_cloud_flags;           // [2][N * W * H + 1]: flags, offsets
+  rr::DeviceArray<uint8_t> d_cloud_scratch;          // CUB scan storage
+  rr::DeviceArray<float> d_cloud_pos, d_cloud_nrm, d_cloud_rgb, d_cloud_q;
+  rr::DeviceArray<uint32_t> d_cloud_pix;
 
   // connected parts (rr_parts.cu). The volume epoch advances with every integrate and every new volume allocation; the
   // mesh and the labelling record the epoch they were computed from, so rr_download_mesh_parts pairs only those of one state.
   uint64_t volume_epoch = 0, mesh_epoch = 0, parts_epoch = 0;
   bool parts_valid = false;        // d_parts_* hold the last labelling (parts_n parts)
   uint32_t parts_n = 0;
-  uint32_t* d_parts_labels = nullptr; size_t parts_labels_cap = 0;   // [Z][Y][X]: union-find forest, then part labels
-  uint32_t* d_parts_rows = nullptr; size_t parts_rows_cap = 0;       // [2][rows + 1]: roots per row, their offsets
-  uint8_t* d_parts_scratch = nullptr; size_t parts_scratch_cap = 0;  // CUB scan storage
-  uint32_t* d_parts_voxels = nullptr; int32_t* d_parts_boxes = nullptr; unsigned long long* d_parts_sums = nullptr;
-  float* d_parts_centroids = nullptr; size_t parts_cap = 0;          // per part, one capacity in parts
-  uint32_t* d_mesh_parts = nullptr; size_t mesh_parts_cap = 0;       // [V] vertex parts, then [T] triangle parts
-  uint32_t* h_parts_count = nullptr;   // pinned
+  rr::DeviceArray<uint32_t> d_parts_labels;          // [Z][Y][X]: union-find forest, then part labels
+  rr::DeviceArray<uint32_t> d_parts_rows;            // [2][rows + 1]: roots per row, their offsets
+  rr::DeviceArray<uint8_t> d_parts_scratch;          // CUB scan storage
+  rr::DeviceArray<uint32_t> d_parts_voxels;          // per part
+  rr::DeviceArray<int32_t> d_parts_boxes;            // [P][6]
+  rr::DeviceArray<unsigned long long> d_parts_sums;  // [P][3]
+  rr::DeviceArray<float> d_parts_centroids;          // [P][3]
+  rr::DeviceArray<uint32_t> d_mesh_parts;            // [V] vertex parts, then [T] triangle parts
 
   // colour hole filling (rr_colorfill.cu): atlas right of column W, squeezed copy, filled colour
   int fill_w = 0, fill_h = 0;
@@ -299,10 +321,8 @@ int launch_partial_keep(rr_ctx* c, float4* d_rec, const long long* d_keys_min, i
 int launch_fill_colors(rr_ctx* c);
 int launch_draw_points(rr_ctx* c, const rr_view* v, int mode, float calib_limit);   // rr_points.cu
 int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length);             // rr_trigrid.cu
-void trigrid_release(rr_ctx* c);
 int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt);   // rr_mesh.cu: the whole volume, ignoring the slab
 bool mesh_rows_usable(const rr_ctx* c);   // the last integrate cleared everything outside the occupied bricks of the row tables
-void mesh_release(rr_ctx* c);
 // rr_query.cu: rr_sample_points / rr_cast_rays. query_upload copies the inputs (b: the directions, NULL for points) into
 // d_q_in, the launchers evaluate the context's own slab (a group member evaluates only what it owns), query_download
 // copies the requested results out and synchronises once.
@@ -313,17 +333,14 @@ int launch_sample_points(rr_ctx* c, int space, uint32_t count);
 int launch_cast_rays(rr_ctx* c, int space, uint32_t count);
 int launch_query_composite(rr_ctx* const* members, int n, bool rays, int space, uint32_t count);   // on member 0's stream
 int query_download(rr_ctx* c, uint32_t count, bool rays, float* values_or_positions, float* normals, float* rgba, uint32_t* steps);
-void query_release(rr_ctx* c);
 // rr_cloud.cu: rr_extract_points over the sensors of `mask` (checked by the caller); cloud_download copies the last extraction
 // out and synchronises once
 int launch_extract_points(rr_ctx* c, uint32_t mask, uint32_t* out_n);
 int cloud_download(rr_ctx* c, float* positions, float* normals, float* colors, float* quality, uint32_t* pixels);
-void cloud_release(rr_ctx* c);
 // rr_parts.cu: rr_label_parts over the whole volume, ignoring the slab; the downloads copy out and synchronise once
 int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts);
 int parts_download(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels);
 int mesh_parts_download(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle_parts);   // the mesh and labelling of one epoch
-void parts_release(rr_ctx* c);
 int launch_unpack_frames(rr_ctx* c, int slot);
 int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4* d_out);
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines
@@ -349,3 +366,17 @@ uint32_t host_divide_box(const float bmin[3], const float bmax[3], float brick_s
     cudaError_t e__ = cudaGetLastError();                          \
     if (e__ != cudaSuccess) return rr::check((c), e__, (what));    \
   } while (0)
+
+// Grows to `need` elements plus 1/8 slack; a queued kernel or copy may still read the old memory, so the stream drains first.
+template <typename T>
+int rr::DeviceArray<T>::reserve(rr_ctx* c, size_t need, const char* what) {
+  if (need <= cap) return RR_OK;
+  if (ptr) {
+    RR_TRY_RC(rr::check(c, cudaStreamSynchronize(c->stream), what));
+    release();
+  }
+  const size_t n = need + need / 8 + 1;
+  RR_TRY_RC(rr::check(c, cudaMalloc((void**)&ptr, n * sizeof(T)), what));
+  cap = n;
+  return RR_OK;
+}

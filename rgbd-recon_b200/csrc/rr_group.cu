@@ -616,7 +616,7 @@ static int group_query(rr_group* g, bool rays, int space, const float* a, const 
       if (rc != RR_OK) return member_fail(g, i, rc);
       RR_G_TRY(g, cudaStreamWaitEvent(c->stream, g->ev_view[0], 0));
       // the directions follow the origins at offset 3 * count in both members' input arrays
-      RR_G_TRY(g, cudaMemcpyPeerAsync(c->d_q_in, c->device, c0->d_q_in, c0->device, bytes, c->stream));
+      RR_G_TRY(g, cudaMemcpyPeerAsync(c->d_q_in.ptr, c->device, c0->d_q_in.ptr, c0->device, bytes, c->stream));
     }
     rc = rays ? rr::launch_cast_rays(c, space, count) : rr::launch_sample_points(c, space, count);
     if (rc != RR_OK) return member_fail(g, i, rc);

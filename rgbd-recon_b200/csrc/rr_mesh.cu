@@ -328,36 +328,6 @@ __global__ void __launch_bounds__(256) k_mesh_triangles(const __grid_constant__ 
   }
 }
 
-template <typename T>
-int grow(rr_ctx* c, T** ptr, size_t* cap, size_t need, const char* what) {
-  if (need <= *cap && *ptr) return RR_OK;
-  if (*ptr) {
-    RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), what));   // the last extraction's kernels may still read it
-    cudaFree(*ptr);
-  }
-  *ptr = nullptr; *cap = 0;
-  const size_t n = need + need / 8 + 1;
-  RR_TRY_RC(check(c, cudaMalloc((void**)ptr, n * sizeof(T)), what));
-  *cap = n;
-  return RR_OK;
-}
-
-// the per-vertex arrays share one capacity (in vertices)
-int grow_vertices(rr_ctx* c, size_t nv) {
-  if (nv <= c->mesh_v_cap) return RR_OK;
-  RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "mesh vertex buffers"));
-  cudaFree(c->d_mesh_keys); cudaFree(c->d_mesh_pos); cudaFree(c->d_mesh_nrm); cudaFree(c->d_mesh_rgba);
-  c->d_mesh_keys = nullptr; c->d_mesh_pos = nullptr; c->d_mesh_nrm = nullptr; c->d_mesh_rgba = nullptr;
-  c->mesh_v_cap = 0;
-  const size_t n = nv + nv / 8 + 1;
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_mesh_keys, n * sizeof(unsigned long long)), "mesh keys"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_mesh_pos, n * 3 * sizeof(float)), "mesh positions"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_mesh_nrm, n * 3 * sizeof(float)), "mesh normals"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_mesh_rgba, n * sizeof(float4)), "mesh colours"));
-  c->mesh_v_cap = n;
-  return RR_OK;
-}
-
 }  // namespace
 
 bool mesh_rows_usable(const rr_ctx* c) {
@@ -375,14 +345,14 @@ int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt) {
   }
   const int X = (int)c->res[0], Y = (int)c->res[1], Z = (int)c->res[2];
   const size_t rows = (size_t)Y * Z;
-  RR_TRY_RC(grow(c, &c->d_mesh_rows, &c->mesh_rows_cap, 4 * (rows + 1), "mesh row counts"));
-  unsigned long long* cnt_v = c->d_mesh_rows;
+  RR_TRY_RC(c->d_mesh_rows.reserve(c, 4 * (rows + 1), "mesh row counts"));
+  unsigned long long* cnt_v = c->d_mesh_rows.ptr;
   unsigned long long* cnt_t = cnt_v + (rows + 1);
   unsigned long long* off_v = cnt_t + (rows + 1);
   unsigned long long* off_t = off_v + (rows + 1);
   size_t scan_bytes = 0;
   RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, cnt_v, off_v, (int)(rows + 1), c->stream), "mesh scan size"));
-  RR_TRY_RC(grow(c, &c->d_mesh_scratch, &c->mesh_scratch_cap, scan_bytes, "mesh scan scratch"));
+  RR_TRY_RC(c->d_mesh_scratch.reserve(c, scan_bytes, "mesh scan scratch"));
 
   MeshParams p{};
   p.tsdf = c->d_tsdf; p.X = X; p.Y = Y; p.Z = Z;
@@ -403,22 +373,26 @@ int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt) {
   RR_TRY_RC(check(c, cudaMemsetAsync(cnt_t + rows, 0, sizeof(unsigned long long), c->stream), "mesh counts"));
   k_mesh_count<<<row_blocks, 256, 0, c->stream>>>(p);
   RR_LAUNCH_CHECK(c, "k_mesh_count");
-  size_t bytes = c->mesh_scratch_cap;
-  RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(c->d_mesh_scratch, bytes, cnt_v, off_v, (int)(rows + 1), c->stream), "mesh vertex scan"));
-  bytes = c->mesh_scratch_cap;
-  RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(c->d_mesh_scratch, bytes, cnt_t, off_t, (int)(rows + 1), c->stream), "mesh triangle scan"));
+  size_t bytes = c->d_mesh_scratch.cap;
+  RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(c->d_mesh_scratch.ptr, bytes, cnt_v, off_v, (int)(rows + 1), c->stream), "mesh vertex scan"));
+  bytes = c->d_mesh_scratch.cap;
+  RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(c->d_mesh_scratch.ptr, bytes, cnt_t, off_t, (int)(rows + 1), c->stream), "mesh triangle scan"));
   c->launches += 2;
-  RR_TRY_RC(check(c, cudaMemcpyAsync(c->h_mesh_totals, off_v + rows, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream), "mesh totals"));
-  RR_TRY_RC(check(c, cudaMemcpyAsync(c->h_mesh_totals + 1, off_t + rows, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream), "mesh totals"));
+  unsigned long long* totals = c->pinned->mesh_totals;
+  RR_TRY_RC(check(c, cudaMemcpyAsync(totals, off_v + rows, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream), "mesh totals"));
+  RR_TRY_RC(check(c, cudaMemcpyAsync(totals + 1, off_t + rows, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream), "mesh totals"));
   RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "mesh count sync"));
-  const unsigned long long nv = c->h_mesh_totals[0], nt = c->h_mesh_totals[1];
+  const unsigned long long nv = totals[0], nt = totals[1];
   c->mesh_valid = false;
   // vertex and triangle indices are uint32 in the output and int-sized in the launches
   if (nv >= (1ull << 31) || nt >= (1ull << 31))
     return fail(c, RR_ERR_UNSUPPORTED, "rr_extract_mesh: meshes of 2^31 or more vertices or triangles are not supported");
-  RR_TRY_RC(grow_vertices(c, nv));
-  if (nt) RR_TRY_RC(grow(c, &c->d_mesh_tri, &c->mesh_t_cap, 3 * nt, "mesh triangles"));
-  p.keys = c->d_mesh_keys; p.pos = c->d_mesh_pos; p.nrm = c->d_mesh_nrm; p.rgba = c->d_mesh_rgba; p.tri = c->d_mesh_tri;
+  RR_TRY_RC(c->d_mesh_keys.reserve(c, nv, "mesh keys"));
+  RR_TRY_RC(c->d_mesh_pos.reserve(c, 3 * nv, "mesh positions"));
+  RR_TRY_RC(c->d_mesh_nrm.reserve(c, 3 * nv, "mesh normals"));
+  RR_TRY_RC(c->d_mesh_rgba.reserve(c, nv, "mesh colours"));
+  if (nt) RR_TRY_RC(c->d_mesh_tri.reserve(c, 3 * nt, "mesh triangles"));
+  p.keys = c->d_mesh_keys.ptr; p.pos = c->d_mesh_pos.ptr; p.nrm = c->d_mesh_nrm.ptr; p.rgba = c->d_mesh_rgba.ptr; p.tri = c->d_mesh_tri.ptr;
   p.nv = (uint32_t)nv;
   if (nv) {
     k_mesh_vertices<<<row_blocks, 256, 0, c->stream>>>(p);
@@ -436,12 +410,6 @@ int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt) {
   if (out_nv) *out_nv = c->mesh_nv;
   if (out_nt) *out_nt = c->mesh_nt;
   return RR_OK;
-}
-
-void mesh_release(rr_ctx* c) {
-  cudaFree(c->d_mesh_rows); cudaFree(c->d_mesh_scratch); cudaFree(c->d_mesh_keys); cudaFree(c->d_mesh_pos);
-  cudaFree(c->d_mesh_nrm); cudaFree(c->d_mesh_rgba); cudaFree(c->d_mesh_tri);
-  if (c->h_mesh_totals) cudaFreeHost(c->h_mesh_totals);
 }
 
 }  // namespace rr

@@ -259,54 +259,24 @@ __global__ void __launch_bounds__(128) k_mesh_triangle_parts(const uint32_t* __r
   if (t < nt) out[t] = vparts[tri[(size_t)t * 3]];
 }
 
-template <typename T>
-int grow(rr_ctx* c, T** ptr, size_t* cap, size_t need, const char* what) {
-  if (need <= *cap && *ptr) return RR_OK;
-  if (*ptr) {
-    RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), what));   // the last labelling's kernels or copies may still read it
-    cudaFree(*ptr);
-  }
-  *ptr = nullptr; *cap = 0;
-  const size_t n = need + need / 8 + 1;
-  RR_TRY_RC(check(c, cudaMalloc((void**)ptr, n * sizeof(T)), what));
-  *cap = n;
-  return RR_OK;
-}
-
-// the per-part arrays share one capacity (in parts)
-int grow_parts(rr_ctx* c, size_t np) {
-  if (np <= c->parts_cap && c->d_parts_voxels) return RR_OK;
-  RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "part buffers"));
-  cudaFree(c->d_parts_voxels); cudaFree(c->d_parts_boxes); cudaFree(c->d_parts_sums); cudaFree(c->d_parts_centroids);
-  c->d_parts_voxels = nullptr; c->d_parts_boxes = nullptr; c->d_parts_sums = nullptr; c->d_parts_centroids = nullptr;
-  c->parts_cap = 0;
-  const size_t n = np + np / 8 + 1;
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_parts_voxels, n * sizeof(uint32_t)), "part voxel counts"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_parts_boxes, n * 6 * sizeof(int32_t)), "part boxes"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_parts_sums, n * 3 * sizeof(unsigned long long)), "part index sums"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_parts_centroids, n * 3 * sizeof(float)), "part centroids"));
-  c->parts_cap = n;
-  return RR_OK;
-}
-
 }  // namespace
 
 int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
   const int X = (int)c->res[0], Y = (int)c->res[1], Z = (int)c->res[2];
   const size_t nvox = (size_t)X * Y * Z, rows = (size_t)Y * Z;
   c->parts_valid = false;
-  RR_TRY_RC(grow(c, &c->d_parts_labels, &c->parts_labels_cap, nvox, "part labels"));
-  RR_TRY_RC(grow(c, &c->d_parts_rows, &c->parts_rows_cap, 2 * (rows + 1), "part row counts"));
-  uint32_t* cnt = c->d_parts_rows;
+  RR_TRY_RC(c->d_parts_labels.reserve(c, nvox, "part labels"));
+  RR_TRY_RC(c->d_parts_rows.reserve(c, 2 * (rows + 1), "part row counts"));
+  uint32_t* cnt = c->d_parts_rows.ptr;
   uint32_t* off = cnt + (rows + 1);
   size_t scan_bytes = 0;
   RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, cnt, off, (int)(rows + 1), c->stream), "part scan size"));
-  RR_TRY_RC(grow(c, &c->d_parts_scratch, &c->parts_scratch_cap, scan_bytes, "part scan scratch"));
+  RR_TRY_RC(c->d_parts_scratch.reserve(c, scan_bytes, "part scan scratch"));
 
   PartsParams p{};
   p.tsdf = c->d_tsdf; p.X = X; p.Y = Y; p.Z = Z;
   p.half2 = c->cfg.store_weight == RR_VOXELS_HALF2 ? 1 : 0;
-  p.L = c->d_parts_labels;
+  p.L = c->d_parts_labels.ptr;
   p.use_rows = c->mesh_rows_ok ? 1 : 0;
   p.rby = (int)c->bricks.res[1]; p.mask_words = c->mask_words;
   p.rowmask = c->d_rowmask; p.rowany = c->d_rowany; p.cand_y = c->d_cand_y; p.cand_z = c->d_cand_z;
@@ -325,15 +295,18 @@ int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
   RR_LAUNCH_CHECK(c, "k_parts_merge");
   k_parts_compress<<<row_blocks, 256, 0, c->stream>>>(p);
   RR_LAUNCH_CHECK(c, "k_parts_compress");
-  size_t bytes = c->parts_scratch_cap;
-  RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(c->d_parts_scratch, bytes, cnt, off, (int)(rows + 1), c->stream), "part scan"));
+  size_t bytes = c->d_parts_scratch.cap;
+  RR_TRY_RC(check(c, cub::DeviceScan::ExclusiveSum(c->d_parts_scratch.ptr, bytes, cnt, off, (int)(rows + 1), c->stream), "part scan"));
   c->launches += 1;
-  RR_TRY_RC(check(c, cudaMemcpyAsync(c->h_parts_count, off + rows, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream), "part count"));
+  RR_TRY_RC(check(c, cudaMemcpyAsync(&c->pinned->parts_count, off + rows, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream), "part count"));
   RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "part count sync"));
-  const uint32_t np = *c->h_parts_count;
-  RR_TRY_RC(grow_parts(c, np));
+  const uint32_t np = c->pinned->parts_count;
+  RR_TRY_RC(c->d_parts_voxels.reserve(c, np, "part voxel counts"));
+  RR_TRY_RC(c->d_parts_boxes.reserve(c, 6 * (size_t)np, "part boxes"));
+  RR_TRY_RC(c->d_parts_sums.reserve(c, 3 * (size_t)np, "part index sums"));
+  RR_TRY_RC(c->d_parts_centroids.reserve(c, 3 * (size_t)np, "part centroids"));
   p.P = np;
-  p.voxels = c->d_parts_voxels; p.boxes = c->d_parts_boxes; p.sums = c->d_parts_sums; p.centroids = c->d_parts_centroids;
+  p.voxels = c->d_parts_voxels.ptr; p.boxes = c->d_parts_boxes.ptr; p.sums = c->d_parts_sums.ptr; p.centroids = c->d_parts_centroids.ptr;
   if (np) {
     k_parts_number<<<row_blocks, 256, 0, c->stream>>>(p);
     RR_LAUNCH_CHECK(c, "k_parts_number");
@@ -351,40 +324,29 @@ int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
 
 int parts_download(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels) {
   const size_t np = c->parts_n, nvox = (size_t)c->res[0] * c->res[1] * c->res[2];
-  if (voxels && np) RR_TRY_RC(check(c, cudaMemcpyAsync(voxels, c->d_parts_voxels, np * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "part download"));
-  if (boxes && np) RR_TRY_RC(check(c, cudaMemcpyAsync(boxes, c->d_parts_boxes, np * 6 * sizeof(int32_t), cudaMemcpyDefault, c->stream), "part download"));
-  if (centroids && np) RR_TRY_RC(check(c, cudaMemcpyAsync(centroids, c->d_parts_centroids, np * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "part download"));
-  if (labels) RR_TRY_RC(check(c, cudaMemcpyAsync(labels, c->d_parts_labels, nvox * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "label download"));
+  if (voxels && np) RR_TRY_RC(check(c, cudaMemcpyAsync(voxels, c->d_parts_voxels.ptr, np * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "part download"));
+  if (boxes && np) RR_TRY_RC(check(c, cudaMemcpyAsync(boxes, c->d_parts_boxes.ptr, np * 6 * sizeof(int32_t), cudaMemcpyDefault, c->stream), "part download"));
+  if (centroids && np) RR_TRY_RC(check(c, cudaMemcpyAsync(centroids, c->d_parts_centroids.ptr, np * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "part download"));
+  if (labels) RR_TRY_RC(check(c, cudaMemcpyAsync(labels, c->d_parts_labels.ptr, nvox * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "label download"));
   return check(c, cudaStreamSynchronize(c->stream), "part download sync");
 }
 
 int mesh_parts_download(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle_parts) {
   const uint32_t nv = c->mesh_nv, nt = c->mesh_nt;
-  RR_TRY_RC(grow(c, &c->d_mesh_parts, &c->mesh_parts_cap, (size_t)nv + nt, "mesh part buffers"));
-  uint32_t* vp = c->d_mesh_parts;
+  RR_TRY_RC(c->d_mesh_parts.reserve(c, (size_t)nv + nt, "mesh part buffers"));
+  uint32_t* vp = c->d_mesh_parts.ptr;
   uint32_t* tp = vp + nv;
   if (nv) {
-    k_mesh_vertex_parts<<<(nv + 127) / 128, 128, 0, c->stream>>>(c->d_mesh_keys, nv, (int)c->res[0], (int)c->res[1], c->d_parts_labels, vp);
+    k_mesh_vertex_parts<<<(nv + 127) / 128, 128, 0, c->stream>>>(c->d_mesh_keys.ptr, nv, (int)c->res[0], (int)c->res[1], c->d_parts_labels.ptr, vp);
     RR_LAUNCH_CHECK(c, "k_mesh_vertex_parts");
   }
   if (nt) {
-    k_mesh_triangle_parts<<<(nt + 127) / 128, 128, 0, c->stream>>>(c->d_mesh_tri, nt, vp, tp);
+    k_mesh_triangle_parts<<<(nt + 127) / 128, 128, 0, c->stream>>>(c->d_mesh_tri.ptr, nt, vp, tp);
     RR_LAUNCH_CHECK(c, "k_mesh_triangle_parts");
   }
   if (vertex_parts && nv) RR_TRY_RC(check(c, cudaMemcpyAsync(vertex_parts, vp, (size_t)nv * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "mesh part download"));
   if (triangle_parts && nt) RR_TRY_RC(check(c, cudaMemcpyAsync(triangle_parts, tp, (size_t)nt * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "mesh part download"));
   return check(c, cudaStreamSynchronize(c->stream), "mesh part download sync");
-}
-
-void parts_release(rr_ctx* c) {
-  cudaFree(c->d_parts_labels); cudaFree(c->d_parts_rows); cudaFree(c->d_parts_scratch);
-  cudaFree(c->d_parts_voxels); cudaFree(c->d_parts_boxes); cudaFree(c->d_parts_sums); cudaFree(c->d_parts_centroids);
-  cudaFree(c->d_mesh_parts);
-  c->d_parts_labels = nullptr; c->d_parts_rows = nullptr; c->d_parts_scratch = nullptr;
-  c->d_parts_voxels = nullptr; c->d_parts_boxes = nullptr; c->d_parts_sums = nullptr; c->d_parts_centroids = nullptr;
-  c->d_mesh_parts = nullptr;
-  c->parts_labels_cap = c->parts_rows_cap = c->parts_scratch_cap = c->parts_cap = c->mesh_parts_cap = 0;
-  c->parts_valid = false;
 }
 
 }  // namespace rr

@@ -187,36 +187,28 @@ QueryParams query_params(const rr_ctx* c, int space, uint32_t count) {
   set_march_params(p, c);
   for (int a = 0; a < 3; ++a) p.bmin[a] = c->bbox_min[a];
   p.world = space == RR_QUERY_WORLD ? 1 : 0;
-  p.in = c->d_q_in; p.n = count;
-  p.val = c->d_q_val; p.pos = c->d_q_pos; p.nrm = c->d_q_nrm; p.rgba = c->d_q_rgba; p.step = c->d_q_step;
+  p.in = c->d_q_in.ptr; p.n = count;
+  p.val = c->d_q_val.ptr; p.pos = c->d_q_pos.ptr; p.nrm = c->d_q_nrm.ptr; p.rgba = c->d_q_rgba.ptr; p.step = c->d_q_step.ptr;
   return p;
 }
 
 }  // namespace
 
-// the query arrays share one capacity (in entries), grown with 1/8 slack like the mesh buffers
 int query_reserve(rr_ctx* c, uint32_t count) {
-  if (count <= c->q_cap) return RR_OK;
-  RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "query buffers"));   // the last query's copies may still read them
-  cudaFree(c->d_q_in); cudaFree(c->d_q_val); cudaFree(c->d_q_pos); cudaFree(c->d_q_nrm); cudaFree(c->d_q_rgba); cudaFree(c->d_q_step);
-  c->d_q_in = nullptr; c->d_q_val = nullptr; c->d_q_pos = nullptr; c->d_q_nrm = nullptr; c->d_q_rgba = nullptr; c->d_q_step = nullptr;
-  c->q_cap = 0;
-  const size_t n = (size_t)count + count / 8 + 1;
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_q_in, n * 6 * sizeof(float)), "query inputs"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_q_val, n * sizeof(float)), "query values"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_q_pos, n * 3 * sizeof(float)), "query positions"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_q_nrm, n * 3 * sizeof(float)), "query normals"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_q_rgba, n * sizeof(float4)), "query colours"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_q_step, n * sizeof(uint32_t)), "query steps"));
-  c->q_cap = n;
-  return RR_OK;
+  const size_t n = count;
+  RR_TRY_RC(c->d_q_in.reserve(c, 6 * n, "query inputs"));
+  RR_TRY_RC(c->d_q_val.reserve(c, n, "query values"));
+  RR_TRY_RC(c->d_q_pos.reserve(c, 3 * n, "query positions"));
+  RR_TRY_RC(c->d_q_nrm.reserve(c, 3 * n, "query normals"));
+  RR_TRY_RC(c->d_q_rgba.reserve(c, n, "query colours"));
+  return c->d_q_step.reserve(c, n, "query steps");
 }
 
 int query_upload(rr_ctx* c, const float* a, const float* b, uint32_t count) {
   RR_TRY_RC(query_reserve(c, count));
   const size_t bytes = (size_t)count * 3 * sizeof(float);
-  RR_TRY_RC(check(c, cudaMemcpyAsync(c->d_q_in, a, bytes, cudaMemcpyDefault, c->stream), "query input copy"));
-  if (b) RR_TRY_RC(check(c, cudaMemcpyAsync(c->d_q_in + (size_t)count * 3, b, bytes, cudaMemcpyDefault, c->stream), "query input copy"));
+  RR_TRY_RC(check(c, cudaMemcpyAsync(c->d_q_in.ptr, a, bytes, cudaMemcpyDefault, c->stream), "query input copy"));
+  if (b) RR_TRY_RC(check(c, cudaMemcpyAsync(c->d_q_in.ptr + (size_t)count * 3, b, bytes, cudaMemcpyDefault, c->stream), "query input copy"));
   return RR_OK;
 }
 
@@ -240,7 +232,7 @@ int launch_query_composite(rr_ctx* const* members, int n, bool rays, int space, 
   pq.n = n;
   for (int m = 0; m < n; ++m) {
     const rr_ctx* c = members[m];
-    pq.val[m] = c->d_q_val; pq.pos[m] = c->d_q_pos; pq.nrm[m] = c->d_q_nrm; pq.rgba[m] = c->d_q_rgba; pq.step[m] = c->d_q_step;
+    pq.val[m] = c->d_q_val.ptr; pq.pos[m] = c->d_q_pos.ptr; pq.nrm[m] = c->d_q_nrm.ptr; pq.rgba[m] = c->d_q_rgba.ptr; pq.step[m] = c->d_q_step.ptr;
     pq.z1[m] = (int)c->slab_z1;
   }
   const QueryParams p = query_params(c0, space, count);
@@ -257,17 +249,13 @@ int launch_query_composite(rr_ctx* const* members, int n, bool rays, int space, 
 int query_download(rr_ctx* c, uint32_t count, bool rays, float* values_or_positions, float* normals, float* rgba, uint32_t* steps) {
   const size_t n = count;
   if (values_or_positions) {
-    const void* src = rays ? (const void*)c->d_q_pos : (const void*)c->d_q_val;
+    const void* src = rays ? (const void*)c->d_q_pos.ptr : (const void*)c->d_q_val.ptr;
     RR_TRY_RC(check(c, cudaMemcpyAsync(values_or_positions, src, n * (rays ? 3 : 1) * sizeof(float), cudaMemcpyDefault, c->stream), "query download"));
   }
-  if (normals) RR_TRY_RC(check(c, cudaMemcpyAsync(normals, c->d_q_nrm, n * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "query download"));
-  if (rgba) RR_TRY_RC(check(c, cudaMemcpyAsync(rgba, c->d_q_rgba, n * sizeof(float4), cudaMemcpyDefault, c->stream), "query download"));
-  if (rays && steps) RR_TRY_RC(check(c, cudaMemcpyAsync(steps, c->d_q_step, n * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "query download"));
+  if (normals) RR_TRY_RC(check(c, cudaMemcpyAsync(normals, c->d_q_nrm.ptr, n * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "query download"));
+  if (rgba) RR_TRY_RC(check(c, cudaMemcpyAsync(rgba, c->d_q_rgba.ptr, n * sizeof(float4), cudaMemcpyDefault, c->stream), "query download"));
+  if (rays && steps) RR_TRY_RC(check(c, cudaMemcpyAsync(steps, c->d_q_step.ptr, n * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "query download"));
   return check(c, cudaStreamSynchronize(c->stream), "query sync");
-}
-
-void query_release(rr_ctx* c) {
-  cudaFree(c->d_q_in); cudaFree(c->d_q_val); cudaFree(c->d_q_pos); cudaFree(c->d_q_nrm); cudaFree(c->d_q_rgba); cudaFree(c->d_q_step);
 }
 
 }  // namespace rr

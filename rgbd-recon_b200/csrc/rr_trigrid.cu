@@ -23,6 +23,7 @@
 #include "rr_draw.cuh"
 #include "rr_math.cuh"
 
+#include <algorithm>
 #include <cmath>
 
 namespace rr {
@@ -275,27 +276,6 @@ static void tg_matmul4(const double* a, const double* b, double* out) {
     }
 }
 
-template <typename T>
-static int tg_reserve(rr_ctx* c, T** ptr, size_t* have, size_t want, const char* what) {
-  if (*have >= want && *ptr) return RR_OK;
-  if (*ptr) { cudaFree(*ptr); *ptr = nullptr; *have = 0; }
-  RR_TRY_RC(check(c, cudaMalloc((void**)ptr, want * sizeof(T)), what));
-  *have = want;
-  return RR_OK;
-}
-
-// the fragment pool (colour contributions + list links) holds at least `want` fragments; it only ever grows
-static int tg_reserve_pool(rr_ctx* c, size_t want) {
-  if (c->tg_frag_cap >= want && c->d_tg_frag_rgba && c->d_tg_frag_pos && c->d_tg_frag_link) return RR_OK;
-  cudaFree(c->d_tg_frag_rgba); cudaFree(c->d_tg_frag_pos); cudaFree(c->d_tg_frag_link);
-  c->d_tg_frag_rgba = nullptr; c->d_tg_frag_pos = nullptr; c->d_tg_frag_link = nullptr; c->tg_frag_cap = 0;
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_tg_frag_rgba, want * sizeof(float4)), "trigrid fragments"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_tg_frag_pos, want * sizeof(float4)), "trigrid fragment positions"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_tg_frag_link, want * sizeof(uint2)), "trigrid fragment links"));
-  c->tg_frag_cap = want;
-  return RR_OK;
-}
-
 // The view images of the context (d_rgba, d_zbuf) receive the result, like a raymarch. One host synchronisation per draw: the
 // fragment count is read back, and the walk is repeated with a larger pool if the lists did not fit.
 int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length) {
@@ -318,12 +298,11 @@ int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length) {
   p.min_length = min_length; p.epsilon = 0.075f;                       // recon_trigrid.cpp:35
   const size_t n_vertices = (size_t)c->N * (c->W + 1) * (c->H + 1), n_triangles = (size_t)c->N * c->W * c->H * 2;
   if (n_triangles >= 0xFFFFFFFFull) return fail(c, RR_ERR_UNSUPPORTED, "rr_draw_trigrid: too many triangles");
-  RR_TRY_RC(tg_reserve(c, &c->d_tg_verts, &c->tg_verts_cap, n_vertices * 4, "trigrid vertices"));
-  RR_TRY_RC(tg_reserve(c, &c->d_tg_depth, &c->tg_depth_cap, (size_t)npx, "trigrid depth"));
-  RR_TRY_RC(tg_reserve(c, &c->d_tg_head, &c->tg_head_cap, (size_t)npx, "trigrid list heads"));
-  if (!c->d_tg_count) RR_TRY_RC(check(c, cudaMalloc((void**)&c->d_tg_count, sizeof(uint32_t)), "trigrid counter"));
-  RR_TRY_RC(tg_reserve_pool(c, (size_t)npx * (size_t)(tunables().trigrid_pool > 0 ? tunables().trigrid_pool : 1) / 16 + 16));
-  p.verts = c->d_tg_verts; p.depth1 = c->d_tg_depth; p.head = c->d_tg_head; p.frag_count = c->d_tg_count;
+  RR_TRY_RC(c->d_tg_verts.reserve(c, n_vertices * 4, "trigrid vertices"));
+  RR_TRY_RC(c->d_tg_depth.reserve(c, (size_t)npx, "trigrid depth"));
+  RR_TRY_RC(c->d_tg_head.reserve(c, (size_t)npx, "trigrid list heads"));
+  RR_TRY_RC(c->d_tg_count.reserve(c, 1, "trigrid counter"));
+  p.verts = c->d_tg_verts.ptr; p.depth1 = c->d_tg_depth.ptr; p.head = c->d_tg_head.ptr; p.frag_count = c->d_tg_count.ptr;
   p.out_rgba = c->d_rgba; p.out_depth = c->d_zbuf;
   timer_begin(c, "3recon");
   timer_begin(c, "draw");
@@ -331,9 +310,16 @@ int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length) {
   RR_LAUNCH_CHECK(c, "k_tg_clear");
   k_tg_vertices<<<(unsigned)((n_vertices + 255) / 256), 256, 0, c->stream>>>(p, (uint32_t)n_vertices);
   RR_LAUNCH_CHECK(c, "k_tg_vertices");
+  // the fragment pool (colour contributions + list links) holds at least `pool` fragments
+  size_t pool = (size_t)npx * (size_t)(tunables().trigrid_pool > 0 ? tunables().trigrid_pool : 1) / 16 + 16;
   for (int attempt = 0;; ++attempt) {
-    p.frag_rgba = c->d_tg_frag_rgba; p.frag_pos = c->d_tg_frag_pos; p.frag_link = c->d_tg_frag_link;
-    p.frag_cap = (uint32_t)(c->tg_frag_cap > 0xFFFFFFF0ull ? 0xFFFFFFF0ull : c->tg_frag_cap);
+    RR_TRY_RC(c->d_tg_frag_rgba.reserve(c, pool, "trigrid fragments"));
+    RR_TRY_RC(c->d_tg_frag_pos.reserve(c, pool, "trigrid fragment positions"));
+    RR_TRY_RC(c->d_tg_frag_link.reserve(c, pool, "trigrid fragment links"));
+    p.frag_rgba = c->d_tg_frag_rgba.ptr; p.frag_pos = c->d_tg_frag_pos.ptr; p.frag_link = c->d_tg_frag_link.ptr;
+    // the capacities are equal unless an earlier reserve failed part way
+    const size_t cap = std::min({c->d_tg_frag_rgba.cap, c->d_tg_frag_pos.cap, c->d_tg_frag_link.cap});
+    p.frag_cap = (uint32_t)(cap > 0xFFFFFFF0ull ? 0xFFFFFFF0ull : cap);
     k_tg_raster<<<(unsigned)((n_triangles + 127) / 128), 128, 0, c->stream>>>(p, (uint32_t)n_triangles);
     RR_LAUNCH_CHECK(c, "k_tg_raster");
     uint32_t count = 0;
@@ -343,7 +329,7 @@ int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length) {
     if (attempt > 0 || count >= 0xFFFFFFF0u) return fail(c, RR_ERR_UNSUPPORTED, "rr_draw_trigrid: fragment lists do not fit");
     // the lists did not fit: grow the pool to what this view needs (+ 1/8) and walk the triangles again (the depths the first
     // walk left are the final ones already: lowering them again changes nothing)
-    RR_TRY_RC(tg_reserve_pool(c, (size_t)count + (size_t)count / 8 + 1024));
+    pool = (size_t)count + (size_t)count / 8 + 1024;
     k_tg_clear_lists<<<(npx + 255) / 256, 256, 0, c->stream>>>(p.head, p.frag_count, npx);
     RR_LAUNCH_CHECK(c, "k_tg_clear_lists");
   }
@@ -352,12 +338,6 @@ int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length) {
   timer_end(c, "draw");
   timer_end(c, "3recon");
   return RR_OK;
-}
-
-void trigrid_release(rr_ctx* c) {
-  cudaFree(c->d_tg_verts); cudaFree(c->d_tg_depth); cudaFree(c->d_tg_head); cudaFree(c->d_tg_frag_rgba); cudaFree(c->d_tg_frag_pos); cudaFree(c->d_tg_frag_link); cudaFree(c->d_tg_count);
-  c->d_tg_verts = nullptr; c->d_tg_depth = nullptr; c->d_tg_head = nullptr; c->d_tg_frag_rgba = nullptr; c->d_tg_frag_pos = nullptr; c->d_tg_frag_link = nullptr; c->d_tg_count = nullptr;
-  c->tg_verts_cap = c->tg_depth_cap = c->tg_head_cap = c->tg_frag_cap = 0;
 }
 
 }  // namespace rr

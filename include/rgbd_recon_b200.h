@@ -320,6 +320,42 @@ int rr_extract_mesh(rr_ctx* ctx, uint32_t* out_num_vertices, uint32_t* out_num_t
 int rr_download_mesh(rr_ctx* ctx, float* positions, float* normals, float* rgba, uint32_t* triangles);
 int rr_group_extract_mesh(rr_group* g, uint32_t* out_num_vertices, uint32_t* out_num_triangles);
 
+/* ---- mesh simplification (no reference counterpart) --------------------------------------------------------------------
+ * A smaller indexed mesh from the last mesh of rr_extract_mesh / rr_group_extract_mesh, by vertex clustering with clusters
+ * of c = cluster_voxels voxels per side (c >= 1). Every vertex of the mesh has an edge key (lower corner (x, y, z), axis).
+ *   Cluster   of a vertex: (x / c, y / c, z / c) by integer division; id = (z/c * CY + y/c) * CX + x/c with CX = ceil(X / c),
+ *             likewise CY and CZ (ids stay below X*Y*Z < 2^31).
+ *   Triangles each mesh triangle (i, j, k) becomes (C(i), C(j), C(k)). It is dropped if two of the three are equal; otherwise
+ *             it is rotated so that the smallest comes first (cyclic order and orientation kept). Among triangles with the
+ *             same rotated triple only the one with the smallest source index is kept (opposite orientations are different
+ *             triples: both are kept). Order: ascending source triangle; sources uint32 [T'] = the index of each kept
+ *             triangle's source triangle in the last mesh (e.g. for rr_download_mesh_parts' triangle parts).
+ *   Vertices  one per cluster a kept triangle references, in ascending cluster id; a vertex's index is its rank in that list.
+ *             Position p_k = (float)(S_k / n): n = the number of mesh vertices in the cluster (all of them, also those whose
+ *             triangles were all dropped), S_k = the binary64 sum of their coordinate k, each widened from binary32, from +0.0
+ *             one vertex at a time in ascending edge key; IEEE binary64 division, rounded to nearest; no fused multiply-adds.
+ *             normal and rgba = exactly what rr_sample_points(RR_QUERY_WORLD) returns at p, evaluated over the whole volume
+ *             whatever rr_set_slab says (NaN normal and rgba 0 outside the unit cube).
+ * The order of every output depends neither on scheduling nor on the number of devices. Cost: one thread per cluster sums its
+ * members, and a cluster holds at most 3*c^3 vertices: c <= 8 is the intended range, a larger c is correct but slow.
+ *
+ * rr_simplify_mesh   simplifies on the context's stream and synchronises once; returns the counts (never more than the
+ *                   mesh's). RR_ERR_INVALID for cluster_voxels == 0, a NULL count pointer, no mesh, or a mesh of an older
+ *                   volume state (an integrate or a new volume since the extraction). Not a setting: the mesh
+ *                   (rr_download_mesh, rr_download_mesh_parts), volume, brick tables, view images (rr_fill_colors still
+ *                   fills the last view), cloud, parts, query results, captured frame graphs and rr_integrator_last stay as
+ *                   they are.
+ * rr_download_simplified_mesh  the last simplification: positions float32 [V'][3], normals float32 [V'][3], rgba float32
+ *                   [V'][4], triangles uint32 [T'][3], sources uint32 [T']; each pointer may be NULL, host memory (pageable or
+ *                   pinned) or device memory of the context's GPU. Returns after one synchronisation. RR_ERR_INVALID before
+ *                   any simplification of the current volume allocation.
+ * rr_group_simplify_mesh  the same on member 0 of a group right after rr_group_extract_mesh (member 0 then holds the gathered
+ *                   volume and the mesh), with no peer traffic, equal to a single context bit for bit; read it with
+ *                   rr_download_simplified_mesh(rr_group_member(g, 0), ...). */
+int rr_simplify_mesh(rr_ctx* ctx, uint32_t cluster_voxels, uint32_t* out_num_vertices, uint32_t* out_num_triangles);
+int rr_download_simplified_mesh(rr_ctx* ctx, float* positions, float* normals, float* rgba, uint32_t* triangles, uint32_t* sources);
+int rr_group_simplify_mesh(rr_group* g, uint32_t cluster_voxels, uint32_t* out_num_vertices, uint32_t* out_num_triangles);
+
 /* ---- connected parts (no reference counterpart) -------------------------------------------------------------------------
  * What is in the volume: its separate objects, where each is, and which mesh triangles belong to which.
  *   Values   the grid of the surface extraction: voxel (x, y, z) has the value v rr_raymarch reads there (R32F; the low

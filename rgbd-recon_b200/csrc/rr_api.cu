@@ -324,6 +324,7 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     c->volume_integrated = false;
     c->mesh_valid = false;
     c->parts_valid = false;
+    c->simp_valid = false;
     ++c->volume_epoch;
   }
   if (new_volume) {   // the label and row arrays are sized by the volume
@@ -932,6 +933,23 @@ int rr_download_mesh_parts(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle
              "with no integrate in between)");
   RR_SET_DEVICE(c);
   return mesh_parts_download(c, vertex_parts, triangle_parts);
+}
+
+int rr_simplify_mesh(rr_ctx* c, uint32_t cluster_voxels, uint32_t* out_num_vertices, uint32_t* out_num_triangles) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, out_num_vertices && out_num_triangles, "rr_simplify_mesh: null count pointer");
+  RR_REQUIRE(c, cluster_voxels >= 1, "rr_simplify_mesh: cluster_voxels must be at least 1");
+  RR_REQUIRE(c, c->mesh_valid && c->mesh_epoch == c->volume_epoch,
+             "rr_simplify_mesh: no mesh of the current volume state (rr_extract_mesh after the last integrate first)");
+  RR_SET_DEVICE(c);
+  return launch_simplify_mesh(c, cluster_voxels, out_num_vertices, out_num_triangles);
+}
+
+int rr_download_simplified_mesh(rr_ctx* c, float* positions, float* normals, float* rgba, uint32_t* triangles, uint32_t* sources) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, c->simp_valid, "rr_download_simplified_mesh: nothing simplified in the current volume (rr_simplify_mesh first)");
+  RR_SET_DEVICE(c);
+  return simplified_download(c, positions, normals, rgba, triangles, sources);
 }
 
 }  // extern "C"

@@ -82,6 +82,7 @@ struct PinnedScalars {
   uint32_t cloud_count;
   uint32_t parts_count;
   unsigned long long mesh_totals[2];   // vertices, triangles
+  uint32_t simplify_counts[2];         // vertices, triangles of rr_simplify_mesh
 };
 
 }  // namespace rr
@@ -262,6 +263,17 @@ struct rr_ctx {
   rr::DeviceArray<float> d_parts_centroids;          // [P][3]
   rr::DeviceArray<uint32_t> d_mesh_parts;            // [V] vertex parts, then [T] triangle parts
 
+  // mesh simplification (rr_simplify.cu): scratch sized by the mesh's V and T, outputs of at most V vertices and T triangles
+  bool simp_valid = false;         // d_simp_* hold a simplification of a mesh of the current volume allocation
+  uint32_t simp_nv = 0, simp_nt = 0;
+  rr::DeviceArray<uint32_t> d_simp_v;                // [10][V + 1] per-vertex cluster ids, orders, ranks and flags
+  rr::DeviceArray<uint32_t> d_simp_t;                // [10][T + 1] per-triangle rank triples, sort keys, orders and flags
+  rr::DeviceArray<unsigned long long> d_simp_k64;    // [2][T] 64-bit sort keys
+  rr::DeviceArray<uint8_t> d_simp_scratch;           // CUB sort and scan storage
+  rr::DeviceArray<float> d_simp_pos, d_simp_nrm;     // [V'][3]
+  rr::DeviceArray<float4> d_simp_rgba;               // [V']
+  rr::DeviceArray<uint32_t> d_simp_tri, d_simp_src;  // [T'][3], [T']
+
   // colour hole filling (rr_colorfill.cu): atlas right of column W, squeezed copy, filled colour
   int fill_w = 0, fill_h = 0;
   float4* d_fill_fc = nullptr; float* d_fill_fd = nullptr;
@@ -341,6 +353,10 @@ int cloud_download(rr_ctx* c, float* positions, float* normals, float* colors, f
 int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts);
 int parts_download(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels);
 int mesh_parts_download(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle_parts);   // the mesh and labelling of one epoch
+// rr_simplify.cu: rr_simplify_mesh of the last mesh (checked by the caller: current, cluster_voxels >= 1), synchronising once;
+// simplified_download copies the last simplification out and synchronises once
+int launch_simplify_mesh(rr_ctx* c, uint32_t cluster_voxels, uint32_t* out_nv, uint32_t* out_nt);
+int simplified_download(rr_ctx* c, float* positions, float* normals, float* rgba, uint32_t* triangles, uint32_t* sources);
 int launch_unpack_frames(rr_ctx* c, int slot);
 int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4* d_out);
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines

@@ -574,6 +574,13 @@ int rr_group_label_parts(rr_group* g, uint32_t* out_num_parts) {
   return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
 }
 
+// Right after rr_group_extract_mesh member 0 holds the gathered whole volume and the mesh: it simplifies, with no peer traffic.
+int rr_group_simplify_mesh(rr_group* g, uint32_t cluster_voxels, uint32_t* out_num_vertices, uint32_t* out_num_triangles) {
+  if (!g) return RR_ERR_INVALID;
+  const int rc = rr_simplify_mesh(g->m[0], cluster_voxels, out_num_vertices, out_num_triangles);
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
 // Pre-processing is replicated on every member (rr_group_preprocess / rr_group_fuse_frame), so member 0's stage images are
 // the whole frame set's: the cloud is extracted there, with no peer traffic.
 int rr_group_extract_points(rr_group* g, uint32_t sensor_mask, uint32_t* out_num_points) {

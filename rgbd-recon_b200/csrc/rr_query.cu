@@ -44,12 +44,6 @@ __device__ __forceinline__ bool finite3(float3 v) {
 __device__ __forceinline__ float3 ld3(const float* a, size_t i) { return make_float3(a[i * 3], a[i * 3 + 1], a[i * 3 + 2]); }
 __device__ __forceinline__ void st3(float* a, size_t i, float3 v) { a[i * 3] = v.x; a[i * 3 + 1] = v.y; a[i * 3 + 2] = v.z; }
 
-// q = (p - bbox_min) / (bbox_max - bbox_min): one IEEE division per component (built with --fmad=false: no contraction)
-__device__ __forceinline__ float3 to_volume(const QueryParams& p, float3 v) {
-  if (!p.world) return v;
-  return make_float3((v.x - p.bmin[0]) / p.dims[0], (v.y - p.bmin[1]) / p.dims[1], (v.z - p.bmin[2]) / p.dims[2]);
-}
-
 // Directions are normalised with the raymarch's normalize3 (v * (1 / sqrt(dot(v, v)))). Its dot product overflows for
 // |v| beyond ~1.8e19 (the result would be the zero vector, a ray of step 0) and loses precision below ~1e-15 (or becomes NaN),
 // so a finite non-zero direction outside that range is first scaled by an exact power of two; ordinary directions keep
@@ -82,16 +76,6 @@ __device__ __forceinline__ bool castable(float3 q0, float3 dir) {
 __device__ __forceinline__ float3 from_volume(const QueryParams& p, float3 q) {
   if (!p.world) return q;
   return make_float3(p.bmin[0] + q.x * p.dims[0], p.bmin[1] + q.y * p.dims[1], p.bmin[2] + q.z * p.dims[2]);
-}
-
-// the mesh vertex normal (rr_mesh.cu k_mesh_attributes): the raymarch's gradient, in world space
-__device__ __forceinline__ float3 world_normal(const QueryParams& p, float3 q) {
-  const float3 g = get_gradient(p, q, p.limit * 0.5f);
-  return normalize3(make_float3(g.x / p.dims[0], g.y / p.dims[1], g.z / p.dims[2]));
-}
-
-__device__ __forceinline__ bool in_unit_cube(float3 q) {   // false for NaN
-  return q.x >= 0.0f && q.x <= 1.0f && q.y >= 0.0f && q.y <= 1.0f && q.z >= 0.0f && q.z <= 1.0f;
 }
 
 __global__ void __launch_bounds__(128) k_sample_points(const __grid_constant__ QueryParams p) {

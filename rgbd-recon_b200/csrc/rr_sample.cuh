@@ -3,6 +3,8 @@
 // P is the caller's parameter block; it provides
 //   tsdf, X, Y, Z, half2                         the volume (R32F, or half2 voxels whose low half is the density)
 //   limit, N, inv, IX, IY, IZ, uv[], cx[], cy[], cz[], color, CW, CH, depth_b, quality, W, H   (blend_colors only)
+// to_volume and world_normal (the point-sample contract of rr_sample_points, shared by rr_query.cu and rr_simplify.cu) also
+// read world (1: positions in metres), bmin[3] and dims[3] = bbox_max - bbox_min.
 // Arithmetic as everywhere in the library: see rr_math.cuh.
 #pragma once
 
@@ -82,6 +84,24 @@ __device__ float4 blend_colors(const P& p, float3 q) {
   if (tw > 0.0f) { tc = tc / tw; return make_float4(tc.x, tc.y, tc.z, 1.0f); }
   tc2 = tc2 / tw2;
   return make_float4(tc2.x, tc2.y, tc2.z, -1.0f);
+}
+
+// q = (p - bbox_min) / (bbox_max - bbox_min): one IEEE division per component (built with --fmad=false: no contraction)
+template <class P>
+__device__ __forceinline__ float3 to_volume(const P& p, float3 v) {
+  if (!p.world) return v;
+  return make_float3((v.x - p.bmin[0]) / p.dims[0], (v.y - p.bmin[1]) / p.dims[1], (v.z - p.bmin[2]) / p.dims[2]);
+}
+
+// the mesh vertex normal (rr_mesh.cu k_mesh_attributes): the raymarch's gradient, in world space
+template <class P>
+__device__ __forceinline__ float3 world_normal(const P& p, float3 q) {
+  const float3 g = get_gradient(p, q, p.limit * 0.5f);
+  return normalize3(make_float3(g.x / p.dims[0], g.y / p.dims[1], g.z / p.dims[2]));
+}
+
+__device__ __forceinline__ bool in_unit_cube(float3 q) {   // false for NaN
+  return q.x >= 0.0f && q.x <= 1.0f && q.y >= 0.0f && q.y <= 1.0f && q.z >= 0.0f && q.z <= 1.0f;
 }
 
 }  // namespace rr

@@ -3,7 +3,7 @@
 // raymarches it. Prints the TimerDatabase stage means; optionally dumps the last TSDF volume, image and surface mesh.
 //   fusion_playback <file.ks> (--streams "s0;s1;..." | --messages file) [--depth W H --color CW CH] [--frames K] [--voxel m]
 //                   [--limit l] [--eye x y z | --matrices file] [--view W H] [--shade m] [--dump-tsdf file] [--dump-image file] [--dense]
-//                   [--dump-mesh file.ply [--min-part-voxels N]] [--dump-points file.ply] [--pick PX PY] [--parts]
+//                   [--dump-mesh file.ply [--simplify C] [--min-part-voxels N]] [--dump-points file.ply] [--pick PX PY] [--parts]
 //                   [--gpus N | --devices a,b,...] [--recon points|trigrid|calibs [--min-length m] [--dump-recon file]]
 // --recon: like kinect_client's reconstruction list (source/kinect_client.cpp:251-257, key-selected g_recon_mode), one of the
 // other reconstructions also draws the last frame set's maps - ReconPoints, ReconTrigrid (min_length from the sensor .yml
@@ -12,8 +12,11 @@
 // peer copies from the first device, per-slab integration, the view composited on the first device); after the first frame
 // the slabs are re-cut to equal integrate cost. A device may be named more than once (slabs sharing a GPU).
 // --dump-mesh: the last frame set's fused surface (ReconIntegration::extractMesh) as a binary PLY with normals and colours.
+// --simplify C: with --dump-mesh, the mesh simplified by vertex clustering with clusters of C voxels per side
+//   (ReconIntegration::simplifyMesh) instead of the full one.
 // --min-part-voxels N: with --dump-mesh, only the triangles of connected parts of at least N voxels, and the vertices they
 //   use, in their original order and re-indexed (drops the small floating blobs sensor noise leaves in front of the surface).
+//   With --simplify, a simplified triangle is in the part of its source triangle.
 // --parts: one line per connected part of the last frame set's volume (ReconIntegration::labelParts): index, voxels, box
 //   (x0 x1 y0 y1 z0 z1, half-open voxel ranges) and centroid (metres).
 // --dump-points: the last frame set's pre-processed sensor points (ReconPoints::extractPoints) as a binary PLY with normals,
@@ -107,6 +110,7 @@ int main(int argc, char** argv) {
   std::vector<int> devices(1, 0);
   bool print_parts = false;
   long long min_part_voxels = -1;
+  long long simplify = 0;
   for (int i = 1; i < argc; ++i) {
     auto next = [&](int k) { return std::atof(argv[i + k]); };
     if (!std::strcmp(argv[i], "--depth")) { W = (unsigned)next(1); H = (unsigned)next(2); i += 2; explicit_sizes = true; }
@@ -127,6 +131,7 @@ int main(int argc, char** argv) {
     else if (!std::strcmp(argv[i], "--dense")) dense = true;
     else if (!std::strcmp(argv[i], "--parts")) print_parts = true;
     else if (!std::strcmp(argv[i], "--min-part-voxels")) min_part_voxels = std::atoll(argv[++i]);
+    else if (!std::strcmp(argv[i], "--simplify")) simplify = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--gpus")) { devices.clear(); for (int d = 0, n = std::atoi(argv[++i]); d < n; ++d) devices.push_back(d); }
     else if (!std::strcmp(argv[i], "--devices")) {
       devices.clear();
@@ -219,12 +224,27 @@ int main(int argc, char** argv) {
     if (!dump_mesh.empty()) {
       Mesh mesh;
       recon.extractMesh(mesh);
+      std::vector<uint32_t> tparts;   // the part of each triangle of `mesh`
       if (min_part_voxels >= 0) {
-        std::vector<uint32_t> vparts, tparts;
+        std::vector<uint32_t> vparts;
         recon.meshParts(vparts, tparts);
+      }
+      if (simplify > 0) {
+        Mesh simple;
+        std::vector<uint32_t> sources;
+        recon.simplifyMesh((uint32_t)simplify, simple, &sources);
+        if (min_part_voxels >= 0) {   // a simplified triangle is in its source triangle's part
+          std::vector<uint32_t> sparts(sources.size());
+          for (std::size_t t = 0; t < sources.size(); ++t) sparts[t] = tparts[sources[t]];
+          tparts.swap(sparts);
+        }
+        std::swap(mesh, simple);
+      }
+      if (min_part_voxels >= 0) {
+        const std::size_t nv = mesh.positions.size() / 3;
         Mesh kept;
-        std::vector<uint32_t> index(vparts.size(), 0xFFFFFFFFu);
-        std::vector<char> used(vparts.size(), 0);
+        std::vector<uint32_t> index(nv, 0xFFFFFFFFu);
+        std::vector<char> used(nv, 0);
         for (std::size_t t = 0; t < tparts.size(); ++t)
           if (parts.voxels[tparts[t]] >= (unsigned long long)min_part_voxels)
             for (int j = 0; j < 3; ++j) used[mesh.triangles[t * 3 + j]] = 1;

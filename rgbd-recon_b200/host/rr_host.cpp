@@ -408,6 +408,17 @@ void ReconIntegration::labelParts(Parts& out) const {
   ck(rr_download_parts(ctx(), out.voxels.data(), out.boxes.data(), out.centroids.data(), nullptr), "rr_download_parts");
 }
 
+void ReconIntegration::simplifyMesh(uint32_t cluster_voxels, Mesh& out, std::vector<uint32_t>* sources) const {
+  uint32_t nv = 0, nt = 0;
+  if (gpu::Context::current().numDevices() > 1) gk(rr_group_simplify_mesh(grp(), cluster_voxels, &nv, &nt), "rr_group_simplify_mesh");
+  else ck(rr_simplify_mesh(ctx(), cluster_voxels, &nv, &nt), "rr_simplify_mesh");
+  out.positions.resize((std::size_t)nv * 3); out.normals.resize((std::size_t)nv * 3); out.rgba.resize((std::size_t)nv * 4);
+  out.triangles.resize((std::size_t)nt * 3);
+  if (sources) sources->resize(nt);
+  ck(rr_download_simplified_mesh(ctx(), out.positions.data(), out.normals.data(), out.rgba.data(), out.triangles.data(),
+                                 sources ? sources->data() : nullptr), "rr_download_simplified_mesh");
+}
+
 void ReconIntegration::meshParts(std::vector<uint32_t>& vertex_parts, std::vector<uint32_t>& triangle_parts) const {
   vertex_parts.resize(m_mesh_nv); triangle_parts.resize(m_mesh_nt);
   ck(rr_download_mesh_parts(ctx(), vertex_parts.data(), triangle_parts.data()), "rr_download_mesh_parts");

@@ -348,6 +348,9 @@ class ReconIntegration : public Reconstruction {
   // every vertex [V] and triangle [T] of the last extractMesh, which must come from the same volume state
   void labelParts(Parts& out) const;
   void meshParts(std::vector<uint32_t>& vertex_parts, std::vector<uint32_t>& triangle_parts) const;
+  // the last extractMesh simplified by vertex clustering with clusters of cluster_voxels voxels per side (rr_simplify_mesh;
+  // with several devices rr_group_simplify_mesh); sources: per simplified triangle, its source triangle in that mesh
+  void simplifyMesh(uint32_t cluster_voxels, Mesh& out, std::vector<uint32_t>* sources = nullptr) const;
   // Queries of the fused volume in metres (rr_sample_points / rr_cast_rays; with several devices their group forms).
   // points, origins, directions, normals, positions: [n][3]; values [n]; rgba [n][4]; steps [n] (0xFFFFFFFF: no hit, with
   // NaN positions and normals). The outputs are resized to n.

@@ -149,6 +149,9 @@ def lib():
     L.rr_download_parts.argtypes = [vp, vp, vp, vp, vp]
     L.rr_download_mesh_parts.argtypes = [vp, vp, vp]
     L.rr_group_label_parts.argtypes = [vp, u32]
+    L.rr_simplify_mesh.argtypes = [vp, C.c_uint32, u32, u32]
+    L.rr_download_simplified_mesh.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.rr_group_simplify_mesh.argtypes = [vp, C.c_uint32, u32, u32]
     L.rr_launch_count.argtypes = [vp]
     L.rr_launch_count.restype = C.c_uint64
     L.rr_version.restype = C.c_int
@@ -643,6 +646,31 @@ class Fusion:
         self._ck(self.L.rr_download_mesh_parts(self.h, *ptrs))
         return tuple(outs)
 
+    def simplify_mesh_counts(self, cluster_voxels):
+        """rr_simplify_mesh alone: simplifies the last mesh on the device and returns (vertices, triangles)."""
+        nv, nt = C.c_uint32(), C.c_uint32()
+        self._ck(self.L.rr_simplify_mesh(self.h, int(cluster_voxels), C.byref(nv), C.byref(nt)))
+        return int(nv.value), int(nt.value)
+
+    def download_simplified_mesh(self, nv, nt, device=False):
+        """rr_download_simplified_mesh of the last simplification (nv, nt: its counts), as numpy arrays or, with device,
+        CUDA tensors on the context's GPU: (positions [nv, 3], normals [nv, 3], rgba [nv, 4], triangles uint32 [nt, 3],
+        sources uint32 [nt])."""
+        dev = None
+        if device:
+            import torch
+            dev = torch.device("cuda", self.device)
+        outs, op = _query_outputs(dev, ((nv, 3), "f4"), ((nv, 3), "f4"), ((nv, 4), "f4"), ((nt, 3), "u4"), ((nt,), "u4"))
+        self._ck(self.L.rr_download_simplified_mesh(self.h, *op))
+        return tuple(outs)
+
+    def simplify_mesh(self, cluster_voxels, device=False):
+        """The last mesh simplified by vertex clustering with clusters of cluster_voxels voxels per side (rr_simplify_mesh +
+        rr_download_simplified_mesh): positions float32 [V', 3] (the clusters' mean positions, metres), normals float32
+        [V', 3] and rgba float32 [V', 4] (rr_sample_points at them), triangles uint32 [T', 3] and sources uint32 [T'] (each
+        triangle's source triangle in the last mesh); numpy arrays, or with device CUDA tensors."""
+        return self.download_simplified_mesh(*self.simplify_mesh_counts(cluster_voxels), device=device)
+
     def set_timing(self, level=1):
         self._ck(self.L.rr_set_timing(self.h, int(level)))
 
@@ -875,6 +903,13 @@ class Group:
     def mesh_parts(self, device=False):
         """As Fusion.mesh_parts, for the group's last extract_mesh and label_parts (member 0)."""
         return self.member(0).mesh_parts(device, getattr(self, "_mesh_n", (0, 0)))
+
+    def simplify_mesh(self, cluster_voxels, device=False):
+        """As Fusion.simplify_mesh (rr_group_simplify_mesh on member 0 after the group's extract_mesh; CUDA tensors on member
+        0's GPU), equal to a single context's bit for bit: (positions, normals, rgba, triangles, sources)."""
+        nv, nt = C.c_uint32(), C.c_uint32()
+        self._ck(self.L.rr_group_simplify_mesh(self.h, int(cluster_voxels), C.byref(nv), C.byref(nt)))
+        return self.member(0).download_simplified_mesh(int(nv.value), int(nt.value), device)
 
     def sample_points(self, points, space="world"):
         """As Fusion.sample_points (CUDA tensors on member 0's GPU), equal to a single context's bit for bit."""

@@ -67,7 +67,7 @@ void timer_end(rr_ctx* c, const char* name) {
 SensorTables sensor_tables(const rr_ctx* c) {
   SensorTables st{};
   for (int i = 0; i < c->N; ++i) {
-    st.xyz[i] = c->d_xyz[i]; st.uv[i] = c->d_uv[i];
+    st.xyz[i] = c->d_xyz[i].ptr; st.uv[i] = c->d_uv[i].ptr;
     st.cx[i] = (int)c->cres[i][0]; st.cy[i] = (int)c->cres[i][1]; st.cz[i] = (int)c->cres[i][2];
     st.dmin[i] = c->dlim[i][0]; st.dmax[i] = c->dlim[i][1];
     for (int a = 0; a < 3; ++a) st.cam[i][a] = c->cam_pos[i][a];
@@ -75,11 +75,13 @@ SensorTables sensor_tables(const rr_ctx* c) {
   return st;
 }
 
-template <typename T>
-static int dev_alloc(rr_ctx* c, T** p, size_t count, const char* what) {
-  if (*p) { cudaFree(*p); *p = nullptr; }
-  if (count == 0) return RR_OK;
-  return check(c, cudaMalloc((void**)p, count * sizeof(T)), what);
+// The read-back of a rendered view: rgba and / or depth of the current view, then one synchronise if either was asked for.
+int view_download(rr_ctx* c, float* out_rgba, float* out_depth, const char* what) {
+  const size_t n = (size_t)c->view_w * c->view_h;
+  if (out_rgba) RR_TRY_RC(check(c, cudaMemcpyAsync(out_rgba, c->d_rgba.ptr, n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), what));
+  if (out_depth) RR_TRY_RC(check(c, cudaMemcpyAsync(out_depth, c->d_zbuf.ptr, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream), what));
+  if (out_rgba || out_depth) RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), what));
+  return RR_OK;
 }
 
 __global__ void k_pad_xyz(const float* __restrict__ src, float4* __restrict__ dst, size_t n) {
@@ -121,34 +123,34 @@ int rr_create(rr_ctx** out, int device, int num_sensors, int depth_w, int depth_
   const size_t px = (size_t)c->N * c->W * c->H;
   int rc = RR_OK;
   for (int b = 0; b < 2; ++b) {
-    if (rc == RR_OK) rc = dev_alloc(c, &c->d_depth_slot[b], px, "depth");
-    if (rc == RR_OK) rc = dev_alloc(c, &c->d_color_slot[b], (size_t)c->N * c->CW * c->CH * 3, "color");
+    if (rc == RR_OK) rc = c->d_depth_slot[b].allocate(c, px, "depth");
+    if (rc == RR_OK) rc = c->d_color_slot[b].allocate(c, (size_t)c->N * c->CW * c->CH * 3, "color");
     if (rc == RR_OK) rc = check(c, cudaEventCreateWithFlags(&c->ev_free[b], cudaEventDisableTiming), "event");
   }
   if (rc == RR_OK) rc = check(c, cudaEventCreateWithFlags(&c->ev_staged, cudaEventDisableTiming), "event");
   if (rc == RR_OK) rc = check(c, cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking), "copy stream");
-  c->d_depth_raw = c->d_depth_slot[0]; c->d_color = c->d_color_slot[0];
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_morph, px, "morph");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_depth, px, "depth rg");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_lab, px, "lab");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_depth_b, px, "depth_b");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_sil, px, "silhouette");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_normal, px, "normal");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_quality, px, "quality");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_gather, (size_t)c->N * (c->W + 1) * (c->H + 1) * 2, "gather");
+  c->d_depth_raw = c->d_depth_slot[0].ptr; c->d_color = c->d_color_slot[0].ptr;
+  if (rc == RR_OK) rc = c->d_morph.allocate(c, px, "morph");
+  if (rc == RR_OK) rc = c->d_depth.allocate(c, px, "depth rg");
+  if (rc == RR_OK) rc = c->d_lab.allocate(c, px, "lab");
+  if (rc == RR_OK) rc = c->d_depth_b.allocate(c, px, "depth_b");
+  if (rc == RR_OK) rc = c->d_sil.allocate(c, px, "silhouette");
+  if (rc == RR_OK) rc = c->d_normal.allocate(c, px, "normal");
+  if (rc == RR_OK) rc = c->d_quality.allocate(c, px, "quality");
+  if (rc == RR_OK) rc = c->d_gather.allocate(c, (size_t)c->N * (c->W + 1) * (c->H + 1) * 2, "gather");
   c->pair_pitch = (c->W + 3) & ~1;
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_pairs, (size_t)c->N * (c->H + 2) * c->pair_pitch, "pair image");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_flags, 4, "flags");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_num_occ, 1, "num_occ");
-  if (rc == RR_OK) rc = dev_alloc(c, &c->d_work, 4, "work counters");
+  if (rc == RR_OK) rc = c->d_pairs.allocate(c, (size_t)c->N * (c->H + 2) * c->pair_pitch, "pair image");
+  if (rc == RR_OK) rc = c->d_flags.allocate(c, 4, "flags");
+  if (rc == RR_OK) rc = c->d_num_occ.allocate(c, 1, "num_occ");
+  if (rc == RR_OK) rc = c->d_work.allocate(c, 4, "work counters");
   if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->pinned, sizeof(rr::PinnedScalars)), "pinned scalars");
   if (rc == RR_OK) {
-    cudaMemsetAsync(c->d_flags, 0, 4 * sizeof(uint32_t), c->stream);
-    cudaMemsetAsync(c->d_pairs, 0, (size_t)c->N * (c->H + 2) * c->pair_pitch * sizeof(float2), c->stream);
-    cudaMemsetAsync(c->d_num_occ, 0, sizeof(uint32_t), c->stream);
+    cudaMemsetAsync(c->d_flags.ptr, 0, 4 * sizeof(uint32_t), c->stream);
+    cudaMemsetAsync(c->d_pairs.ptr, 0, (size_t)c->N * (c->H + 2) * c->pair_pitch * sizeof(float2), c->stream);
+    cudaMemsetAsync(c->d_num_occ.ptr, 0, sizeof(uint32_t), c->stream);
     for (int b = 0; b < 2; ++b) {
-      cudaMemsetAsync(c->d_color_slot[b], 0, (size_t)c->N * c->CW * c->CH * 3, c->stream);
-      cudaMemsetAsync(c->d_depth_slot[b], 0, px * sizeof(float), c->stream);
+      cudaMemsetAsync(c->d_color_slot[b].ptr, 0, (size_t)c->N * c->CW * c->CH * 3, c->stream);
+      cudaMemsetAsync(c->d_depth_slot[b].ptr, 0, px * sizeof(float), c->stream);
     }
     c->pinned->num_occ = 0;
     rc = check(c, cudaStreamSynchronize(c->stream), "create sync");
@@ -164,28 +166,18 @@ void rr_destroy(rr_ctx* c) {
   drop_frame_graphs(c);
   if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
   if (c->stream) cudaStreamSynchronize(c->stream);
-  for (int i = 0; i < RR_MAX_SENSORS; ++i) { cudaFree(c->d_xyz[i]); cudaFree(c->d_uv[i]); }
-  for (int b = 0; b < 2; ++b) { cudaFree(c->d_color_packed[b]); cudaFree(c->d_depth_packed[b]); }
-  for (int b = 0; b < 2; ++b) { cudaFree(c->d_depth_slot[b]); cudaFree(c->d_color_slot[b]); if (c->ev_free[b]) cudaEventDestroy(c->ev_free[b]); }
+  for (int b = 0; b < 2; ++b) if (c->ev_free[b]) cudaEventDestroy(c->ev_free[b]);
   if (c->ev_staged) cudaEventDestroy(c->ev_staged);
   if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-  cudaFree(c->d_inv); cudaFree(c->d_morph); cudaFree(c->d_depth);
-  cudaFree(c->d_lab); cudaFree(c->d_depth_b); cudaFree(c->d_sil); cudaFree(c->d_normal); cudaFree(c->d_quality);
-  staged_release(c);
   for (auto& v : c->ipc_views) { cudaIpcCloseMemHandle(v.step); cudaIpcCloseMemHandle(v.rgba); cudaIpcCloseMemHandle(v.zbuf); cudaIpcCloseMemHandle(v.nsamp); }
   cudaGetLastError();
-  cudaFree(c->d_pairs);
-  cudaFree(c->d_gather); cudaFree(c->d_flags); cudaFree(c->d_ranges); cudaFree(c->d_counters); cudaFree(c->d_occupied);
-  cudaFree(c->d_num_occ); cudaFree(c->d_work); cudaFree(c->d_ztab); cudaFree(c->d_rowmask); cudaFree(c->d_rowany); cudaFree(c->d_cand_y); cudaFree(c->d_cand_z); cudaFree(c->d_near_occ); cudaFree(c->d_occ_mask); cudaFree(c->d_pos); cudaFree(c->d_step); cudaFree(c->d_tsdf); cudaFree(c->d_weight);
-  cudaFree(c->d_rgba); cudaFree(c->d_zbuf); cudaFree(c->d_nsamples); cudaFree(c->d_point_keys);
-  cudaFree(c->d_fill_fc); cudaFree(c->d_fill_fd); cudaFree(c->d_fill_sc); cudaFree(c->d_fill_sd); cudaFree(c->d_filled);
   if (c->pinned) cudaFreeHost(c->pinned);
   for (auto& kv : c->timers) {
     for (cudaEvent_t e : kv.second.beg) cudaEventDestroy(e);
     for (cudaEvent_t e : kv.second.end) cudaEventDestroy(e);
   }
   if (c->stream) cudaStreamDestroy(c->stream);
-  delete c;
+  delete c;                    // the device arrays free their memory, on the context's device (current since the top)
 }
 
 const char* rr_last_error(const rr_ctx* c) {
@@ -229,17 +221,15 @@ int rr_calib_upload(rr_ctx* c, int sensor, const float* cv_xyz, const float* cv_
   RR_REQUIRE(c, res[0] >= 2 && res[1] >= 2 && res[2] >= 2, "rr_calib_upload: volume needs >= 2 voxels per axis");
   RR_SET_DEVICE(c);
   const size_t n = (size_t)res[0] * res[1] * res[2];
-  RR_TRY(dev_alloc(c, &c->d_xyz[sensor], n, "cv_xyz"));
-  RR_TRY(dev_alloc(c, &c->d_uv[sensor], n, "cv_uv"));
-  float* staging = nullptr;
-  RR_TRY(check(c, cudaMalloc((void**)&staging, n * 3 * sizeof(float)), "cv_xyz staging"));
-  cudaMemcpyAsync(staging, cv_xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream);
-  k_pad_xyz<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(staging, c->d_xyz[sensor], n);
+  RR_TRY(c->d_xyz[sensor].allocate(c, n, "cv_xyz"));
+  RR_TRY(c->d_uv[sensor].allocate(c, n, "cv_uv"));
+  DeviceArray<float> staging;
+  RR_TRY(staging.allocate(c, n * 3, "cv_xyz staging"));
+  cudaMemcpyAsync(staging.ptr, cv_xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream);
+  k_pad_xyz<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(staging.ptr, c->d_xyz[sensor].ptr, n);
   ++c->launches;
-  cudaMemcpyAsync(c->d_uv[sensor], cv_uv, n * 2 * sizeof(float), cudaMemcpyHostToDevice, c->stream);
-  int rc = check(c, cudaStreamSynchronize(c->stream), "calib upload");
-  cudaFree(staging);
-  RR_TRY(rc);
+  cudaMemcpyAsync(c->d_uv[sensor].ptr, cv_uv, n * 2 * sizeof(float), cudaMemcpyHostToDevice, c->stream);
+  RR_TRY(check(c, cudaStreamSynchronize(c->stream), "calib upload"));
   for (int a = 0; a < 3; ++a) c->cres[sensor][a] = res[a];
   c->dlim[sensor][0] = dl[0]; c->dlim[sensor][1] = dl[1];
   host_frustum(cv_xyz, res, c->planes[sensor], c->cam_pos[sensor]);
@@ -254,6 +244,17 @@ int rr_calib_upload(rr_ctx* c, int sensor, const float* cv_xyz, const float* cv_
   return RR_OK;
 }
 
+// All sensors share one inverse-volume resolution (CalibVolumes::getVolumeRes): a new one reallocates d_inv, and is refused
+// with `refusal` while another sensor's inverse volume is loaded.
+static int ensure_inv(rr_ctx* c, int sensor, const uint32_t res[3], const char* refusal) {
+  if (c->d_inv.ptr && c->ires[0] == res[0] && c->ires[1] == res[1] && c->ires[2] == res[2]) return RR_OK;
+  for (int i = 0; i < c->N; ++i) RR_REQUIRE(c, !c->have_inv[i] || i == sensor, refusal);
+  RR_TRY(c->d_inv.allocate(c, (size_t)res[0] * res[1] * res[2] * c->N, "cv_xyz_inv"));
+  for (int a = 0; a < 3; ++a) c->ires[a] = res[a];
+  for (int i = 0; i < c->N; ++i) c->have_inv[i] = false;
+  return RR_OK;
+}
+
 int rr_calib_upload_inv(rr_ctx* c, int sensor, const float* inv, const uint32_t res[3]) {
   if (!c) return RR_ERR_INVALID;
   drop_frame_graphs(c);
@@ -261,16 +262,8 @@ int rr_calib_upload_inv(rr_ctx* c, int sensor, const float* inv, const uint32_t 
   RR_REQUIRE(c, inv && res && res[0] && res[1] && res[2], "rr_calib_upload_inv: null pointer or empty volume");
   RR_SET_DEVICE(c);
   const size_t n = (size_t)res[0] * res[1] * res[2];
-  const bool same = c->d_inv && c->ires[0] == res[0] && c->ires[1] == res[1] && c->ires[2] == res[2];
-  if (!same) {
-    bool any = false;
-    for (int i = 0; i < c->N; ++i) any = any || (c->have_inv[i] && i != sensor);
-    RR_REQUIRE(c, !any, "rr_calib_upload_inv: all sensors must share one inverse-volume resolution (CalibVolumes::getVolumeRes)");
-    RR_TRY(dev_alloc(c, &c->d_inv, n * c->N, "cv_xyz_inv"));
-    for (int a = 0; a < 3; ++a) c->ires[a] = res[a];
-    for (int i = 0; i < c->N; ++i) c->have_inv[i] = false;
-  }
-  RR_TRY(check(c, cudaMemcpyAsync(c->d_inv + n * sensor, inv, n * sizeof(float4), cudaMemcpyHostToDevice, c->stream), "inv upload"));
+  RR_TRY(ensure_inv(c, sensor, res, "rr_calib_upload_inv: all sensors must share one inverse-volume resolution (CalibVolumes::getVolumeRes)"));
+  RR_TRY(check(c, cudaMemcpyAsync(c->d_inv.ptr + n * sensor, inv, n * sizeof(float4), cudaMemcpyHostToDevice, c->stream), "inv upload"));
   RR_TRY(check(c, cudaStreamSynchronize(c->stream), "inv upload sync"));
   c->have_inv[sensor] = true;
   c->sti.dirty = true;
@@ -308,15 +301,15 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
   const float bs = host_adjust_brick_size(cfg->voxel_size, cfg->brick_size);
   RR_REQUIRE(c, bs > 0.0f, "rr_configure: brick size rounds to zero voxels");
   const bool new_volume = !c->configured || res[0] != c->res[0] || res[1] != c->res[1] || res[2] != c->res[2] ||
-                          (cfg->store_weight == RR_VOXELS_F32_WEIGHT) != (c->d_weight != nullptr);
+                          (cfg->store_weight == RR_VOXELS_F32_WEIGHT) != (c->d_weight.ptr != nullptr);
   const bool new_bricks = new_volume || bs != c->bricks.brick_size;
   // the staged integrator's tables depend on the volume, the brick grid, bricks mode and the voxel format; plain setters
   // (limit, min_voxels, skip_space) keep them, and the next integrate needs no synchronising rebuild
   const bool restage = new_bricks || cfg->use_bricks != c->cfg.use_bricks || cfg->store_weight != c->cfg.store_weight;
   if (new_volume) {
     const size_t nvox = (size_t)res[0] * res[1] * res[2];
-    RR_TRY(dev_alloc(c, &c->d_tsdf, nvox, "tsdf volume"));
-    RR_TRY(dev_alloc(c, &c->d_weight, cfg->store_weight == RR_VOXELS_F32_WEIGHT ? nvox : 0, "weight volume"));
+    RR_TRY(c->d_tsdf.allocate(c, nvox, "tsdf volume"));
+    RR_TRY(c->d_weight.allocate(c, cfg->store_weight == RR_VOXELS_F32_WEIGHT ? nvox : 0, "weight volume"));
     for (int a = 0; a < 3; ++a) c->res[a] = res[a];
     c->slab_z0 = 0; c->slab_z1 = res[2];
   }
@@ -337,11 +330,11 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     const uint32_t nb = host_divide_box(c->bbox_min, c->bbox_max, bs, res, rb, &c->h_ranges);
     c->bricks.brick_size = bs; c->bricks.num = nb;
     for (int a = 0; a < 3; ++a) c->bricks.res[a] = rb[a];
-    RR_TRY(dev_alloc(c, &c->d_ranges, (size_t)nb * 6, "brick ranges"));
-    RR_TRY(dev_alloc(c, &c->d_counters, (size_t)nb + RR_CLASS_COUNTERS, "brick counters"));
-    RR_TRY(dev_alloc(c, &c->d_occupied, nb, "occupied list"));
-    RR_TRY(dev_alloc(c, &c->d_near_occ, nb, "near-occupied mask"));
-    RR_TRY(dev_alloc(c, &c->d_occ_mask, nb, "occupied mask"));
+    RR_TRY(c->d_ranges.allocate(c, (size_t)nb * 6, "brick ranges"));
+    RR_TRY(c->d_counters.allocate(c, (size_t)nb + RR_CLASS_COUNTERS, "brick counters"));
+    RR_TRY(c->d_occupied.allocate(c, nb, "occupied list"));
+    RR_TRY(c->d_near_occ.allocate(c, nb, "near-occupied mask"));
+    RR_TRY(c->d_occ_mask.allocate(c, nb, "occupied mask"));
     // per-axis candidate bricks of every voxel index (bricks may overlap by a voxel, or leave a gap)
     c->mask_words = (int)((res[0] + 31) / 32);
     c->fused_ok = rb[0] <= 32767 && rb[1] <= 32767 && rb[2] <= 32767;
@@ -359,21 +352,21 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
         }
       }
     }
-    RR_TRY(dev_alloc(c, &c->d_rowmask, (size_t)rb[2] * rb[1] * c->mask_words, "row masks"));
-    RR_TRY(dev_alloc(c, &c->d_rowany, (size_t)rb[2] * rb[1], "row flags"));
-    RR_TRY(dev_alloc(c, &c->d_cand_y, (size_t)res[1] * 2, "cand y"));
-    RR_TRY(dev_alloc(c, &c->d_cand_z, (size_t)res[2] * 2, "cand z"));
+    RR_TRY(c->d_rowmask.allocate(c, (size_t)rb[2] * rb[1] * c->mask_words, "row masks"));
+    RR_TRY(c->d_rowany.allocate(c, (size_t)rb[2] * rb[1], "row flags"));
+    RR_TRY(c->d_cand_y.allocate(c, (size_t)res[1] * 2, "cand y"));
+    RR_TRY(c->d_cand_z.allocate(c, (size_t)res[2] * 2, "cand z"));
     if (c->fused_ok) {
-      cudaMemcpyAsync(c->d_cand_y, cand[1].data(), cand[1].size() * sizeof(int16_t), cudaMemcpyHostToDevice, c->stream);
-      cudaMemcpyAsync(c->d_cand_z, cand[2].data(), cand[2].size() * sizeof(int16_t), cudaMemcpyHostToDevice, c->stream);
+      cudaMemcpyAsync(c->d_cand_y.ptr, cand[1].data(), cand[1].size() * sizeof(int16_t), cudaMemcpyHostToDevice, c->stream);
+      cudaMemcpyAsync(c->d_cand_z.ptr, cand[2].data(), cand[2].size() * sizeof(int16_t), cudaMemcpyHostToDevice, c->stream);
     }
-    cudaMemsetAsync(c->d_rowmask, 0, (size_t)rb[2] * rb[1] * c->mask_words * sizeof(uint32_t), c->stream);
-    cudaMemsetAsync(c->d_rowany, 0, (size_t)rb[2] * rb[1], c->stream);
-    cudaMemcpyAsync(c->d_ranges, c->h_ranges.data(), (size_t)nb * 6 * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream);
-    cudaMemsetAsync(c->d_counters, 0, ((size_t)nb + RR_CLASS_COUNTERS) * sizeof(uint32_t), c->stream);
-    cudaMemsetAsync(c->d_near_occ, 0, nb, c->stream);
-    cudaMemsetAsync(c->d_occ_mask, 0, nb, c->stream);
-    cudaMemsetAsync(c->d_num_occ, 0, sizeof(uint32_t), c->stream);
+    cudaMemsetAsync(c->d_rowmask.ptr, 0, (size_t)rb[2] * rb[1] * c->mask_words * sizeof(uint32_t), c->stream);
+    cudaMemsetAsync(c->d_rowany.ptr, 0, (size_t)rb[2] * rb[1], c->stream);
+    cudaMemcpyAsync(c->d_ranges.ptr, c->h_ranges.data(), (size_t)nb * 6 * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream);
+    cudaMemsetAsync(c->d_counters.ptr, 0, ((size_t)nb + RR_CLASS_COUNTERS) * sizeof(uint32_t), c->stream);
+    cudaMemsetAsync(c->d_near_occ.ptr, 0, nb, c->stream);
+    cudaMemsetAsync(c->d_occ_mask.ptr, 0, nb, c->stream);
+    cudaMemsetAsync(c->d_num_occ.ptr, 0, sizeof(uint32_t), c->stream);
     c->pinned->num_occ = 0;
     RR_TRY(check(c, cudaStreamSynchronize(c->stream), "brick table upload"));
   }
@@ -441,8 +434,8 @@ int rr_set_frame_format(rr_ctx* c, int color_format, int depth_format, const flo
   c->color_format = color_format; c->depth_format = depth_format;
   for (int b = 0; b < 2; ++b) {
     // sized for the larger block format (DXT5, 16 bytes per 4x4 block), so a later format switch needs no reallocation
-    if (color_format != RR_COLOR_RGB8 && !c->d_color_packed[b]) RR_TRY(dev_alloc(c, &c->d_color_packed[b], (size_t)c->N * c->CW * c->CH, "packed colour"));
-    if (depth_format == RR_DEPTH_U8 && !c->d_depth_packed[b]) RR_TRY(dev_alloc(c, &c->d_depth_packed[b], (size_t)c->N * c->W * c->H, "packed depth"));
+    if (color_format != RR_COLOR_RGB8 && !c->d_color_packed[b].ptr) RR_TRY(c->d_color_packed[b].allocate(c, (size_t)c->N * c->CW * c->CH, "packed colour"));
+    if (depth_format == RR_DEPTH_U8 && !c->d_depth_packed[b].ptr) RR_TRY(c->d_depth_packed[b].allocate(c, (size_t)c->N * c->W * c->H, "packed depth"));
   }
   for (int i = 0; i < c->N; ++i) {
     c->depth_near[i] = near_far ? near_far[2 * i] : 0.0f;
@@ -458,8 +451,8 @@ int rr_stage_frames(rr_ctx* c, const void* color, size_t cb, const void* depth, 
   const int t = c->cur_slot ^ 1;
   // the slot may still be read by kernels launched while it was current
   if (c->free_recorded[t]) RR_TRY(check(c, cudaStreamWaitEvent(c->copy_stream, c->ev_free[t], 0), "stage wait"));
-  void* dd = c->depth_format == RR_DEPTH_U8 ? (void*)c->d_depth_packed[t] : (void*)c->d_depth_slot[t];
-  void* dc = c->color_format != RR_COLOR_RGB8 ? (void*)c->d_color_packed[t] : (void*)c->d_color_slot[t];
+  void* dd = c->depth_format == RR_DEPTH_U8 ? (void*)c->d_depth_packed[t].ptr : (void*)c->d_depth_slot[t].ptr;
+  void* dc = c->color_format != RR_COLOR_RGB8 ? (void*)c->d_color_packed[t].ptr : (void*)c->d_color_slot[t].ptr;
   RR_TRY(check(c, cudaMemcpyAsync(dd, depth, db, cudaMemcpyHostToDevice, c->copy_stream), "depth upload"));
   if (color) RR_TRY(check(c, cudaMemcpyAsync(dc, color, cb, cudaMemcpyHostToDevice, c->copy_stream), "colour upload"));
   c->staged_color = color != nullptr;
@@ -477,7 +470,7 @@ int rr_swap_frames(rr_ctx* c) {
   c->free_recorded[old] = true;
   RR_TRY(check(c, cudaStreamWaitEvent(c->stream, c->ev_staged, 0), "swap wait"));
   c->cur_slot = t;
-  c->d_depth_raw = c->d_depth_slot[t]; c->d_color = c->d_color_slot[t];
+  c->d_depth_raw = c->d_depth_slot[t].ptr; c->d_color = c->d_color_slot[t].ptr;
   c->staged = false;
   // packed layers (DXT1 colour, 8-bit depth) are expanded here, once, behind the staged copy
   const int keep_color = c->color_format;
@@ -507,8 +500,8 @@ int rr_upload_frames_device(rr_ctx* c, const void* color, size_t cb, const void*
   // already on this GPU (e.g. the output of an NCCL broadcast ordered before the context's stream): straight into the
   // current slot, on the compute stream
   const int t = c->cur_slot;
-  void* dd = c->depth_format == RR_DEPTH_U8 ? (void*)c->d_depth_packed[t] : (void*)c->d_depth_slot[t];
-  void* dc = c->color_format != RR_COLOR_RGB8 ? (void*)c->d_color_packed[t] : (void*)c->d_color_slot[t];
+  void* dd = c->depth_format == RR_DEPTH_U8 ? (void*)c->d_depth_packed[t].ptr : (void*)c->d_depth_slot[t].ptr;
+  void* dc = c->color_format != RR_COLOR_RGB8 ? (void*)c->d_color_packed[t].ptr : (void*)c->d_color_slot[t].ptr;
   RR_TRY(check(c, cudaMemcpyAsync(dd, depth, db, cudaMemcpyDeviceToDevice, c->stream), "depth upload"));
   if (color) RR_TRY(check(c, cudaMemcpyAsync(dc, color, cb, cudaMemcpyDeviceToDevice, c->stream), "colour upload"));
   const int keep_color = c->color_format;
@@ -579,7 +572,7 @@ int rr_fuse_frame(rr_ctx* c, int filter_textures, int use_processed_depth, int r
   c->preprocessed = true;          // every path below pre-processes (direct, captured or replayed)
   // capture needs a launch sequence without allocations or event timers: the z table exists (first frame ran direct)
   // and stage timing is off
-  const bool ready = rr::tunables().graph != 0 && !c->graphs_broken && c->timing == 0 && c->d_ztab &&
+  const bool ready = rr::tunables().graph != 0 && !c->graphs_broken && c->timing == 0 && c->d_ztab.ptr &&
                      c->ztab_Z == (int)c->res[2] && c->ztab_IZ == (int)c->ires[2];
   if (!ready) return frame_direct(c, f, p, r);
   const uint64_t key = ((uint64_t)rr::tunables().generation << 8) | (uint64_t)(c->cur_slot << 3 | f << 2 | p << 1 | r);
@@ -629,12 +622,12 @@ int rr_bricks_count(rr_ctx* c, uint32_t* out_num, float* out_ratio) {
 int ensure_view(rr_ctx* c, int w, int h) {
   if (w == c->view_w && h == c->view_h) return RR_OK;
   RR_TRY(check(c, cudaStreamSynchronize(c->stream), "raymarch resize sync"));
-  RR_TRY(dev_alloc(c, &c->d_rgba, (size_t)w * h, "view rgba"));
-  RR_TRY(dev_alloc(c, &c->d_zbuf, (size_t)w * h, "view depth"));
-  RR_TRY(dev_alloc(c, &c->d_nsamples, (size_t)w * h, "view samples"));
-  RR_TRY(dev_alloc(c, &c->d_pos, (size_t)w * h, "view positions"));
-  RR_TRY(dev_alloc(c, &c->d_step, (size_t)w * h, "view steps"));
-  RR_TRY(dev_alloc(c, &c->d_point_keys, (size_t)w * h, "point keys"));
+  RR_TRY(c->d_rgba.allocate(c, (size_t)w * h, "view rgba"));
+  RR_TRY(c->d_zbuf.allocate(c, (size_t)w * h, "view depth"));
+  RR_TRY(c->d_nsamples.allocate(c, (size_t)w * h, "view samples"));
+  RR_TRY(c->d_pos.allocate(c, (size_t)w * h, "view positions"));
+  RR_TRY(c->d_step.allocate(c, (size_t)w * h, "view steps"));
+  RR_TRY(c->d_point_keys.allocate(c, (size_t)w * h, "point keys"));
   c->view_w = w; c->view_h = h;
   return RR_OK;
 }
@@ -645,26 +638,18 @@ int rr_raymarch(rr_ctx* c, const rr_view* view, float* out_rgba, float* out_dept
   RR_TRY(require_ready(c, true));
   RR_REQUIRE(c, view->viewport[2] > 0 && view->viewport[3] > 0, "rr_raymarch: empty viewport");
   RR_SET_DEVICE(c);
-  const int w = view->viewport[2], h = view->viewport[3];
-  RR_TRY(ensure_view(c, w, h));
+  RR_TRY(ensure_view(c, view->viewport[2], view->viewport[3]));
   RR_TRY(launch_raymarch(c, view));
-  if (out_rgba) RR_TRY(check(c, cudaMemcpyAsync(out_rgba, c->d_rgba, (size_t)w * h * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "rgba download"));
-  if (out_depth) RR_TRY(check(c, cudaMemcpyAsync(out_depth, c->d_zbuf, (size_t)w * h * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "depth download"));
-  if (out_rgba || out_depth) RR_TRY(check(c, cudaStreamSynchronize(c->stream), "raymarch sync"));
-  return RR_OK;
+  return view_download(c, out_rgba, out_depth, "rr_raymarch");
 }
 
 static int draw_points_common(rr_ctx* c, const rr_view* view, int mode, float limit, float* out_rgba, float* out_depth, const char* who) {
   RR_REQUIRE(c, view, "draw points: null view");
   RR_REQUIRE(c, view->viewport[2] > 0 && view->viewport[3] > 0, "draw points: empty viewport");
   RR_SET_DEVICE(c);
-  const int w = view->viewport[2], h = view->viewport[3];
-  RR_TRY(ensure_view(c, w, h));
+  RR_TRY(ensure_view(c, view->viewport[2], view->viewport[3]));
   RR_TRY(launch_draw_points(c, view, mode, limit));
-  if (out_rgba) RR_TRY(check(c, cudaMemcpyAsync(out_rgba, c->d_rgba, (size_t)w * h * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), who));
-  if (out_depth) RR_TRY(check(c, cudaMemcpyAsync(out_depth, c->d_zbuf, (size_t)w * h * sizeof(float), cudaMemcpyDeviceToHost, c->stream), who));
-  if (out_rgba || out_depth) RR_TRY(check(c, cudaStreamSynchronize(c->stream), who));
-  return RR_OK;
+  return view_download(c, out_rgba, out_depth, who);
 }
 
 int rr_draw_points(rr_ctx* c, const rr_view* view, float* out_rgba, float* out_depth) {
@@ -688,22 +673,18 @@ int rr_draw_trigrid(rr_ctx* c, const rr_view* view, float min_length, float* out
   RR_REQUIRE(c, min_length > 0.0f, "rr_draw_trigrid: min_length must be positive");
   for (int i = 0; i < c->N; ++i) RR_REQUIRE(c, c->have_calib[i], "rr_draw_trigrid: upload every sensor's calibration volumes first");
   RR_SET_DEVICE(c);
-  const int w = view->viewport[2], h = view->viewport[3];
-  RR_TRY(ensure_view(c, w, h));
+  RR_TRY(ensure_view(c, view->viewport[2], view->viewport[3]));
   RR_TRY(launch_draw_trigrid(c, view, min_length));
-  if (out_rgba) RR_TRY(check(c, cudaMemcpyAsync(out_rgba, c->d_rgba, (size_t)w * h * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "rr_draw_trigrid"));
-  if (out_depth) RR_TRY(check(c, cudaMemcpyAsync(out_depth, c->d_zbuf, (size_t)w * h * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "rr_draw_trigrid"));
-  if (out_rgba || out_depth) RR_TRY(check(c, cudaStreamSynchronize(c->stream), "rr_draw_trigrid"));
-  return RR_OK;
+  return view_download(c, out_rgba, out_depth, "rr_draw_trigrid");
 }
 
 int rr_fill_colors(rr_ctx* c, float* out_rgba) {
   if (!c) return RR_ERR_INVALID;
-  RR_REQUIRE(c, c->d_rgba && c->view_w > 0 && c->view_h > 0, "rr_fill_colors: no view yet (rr_raymarch / rr_composite / rr_upload_view first)");
+  RR_REQUIRE(c, c->d_rgba.ptr && c->view_w > 0 && c->view_h > 0, "rr_fill_colors: no view yet (rr_raymarch / rr_composite / rr_upload_view first)");
   RR_SET_DEVICE(c);
   RR_TRY(launch_fill_colors(c));
   if (out_rgba) {
-    RR_TRY(check(c, cudaMemcpyAsync(out_rgba, c->d_filled, (size_t)c->view_w * c->view_h * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "filled colour download"));
+    RR_TRY(check(c, cudaMemcpyAsync(out_rgba, c->d_filled.ptr, (size_t)c->view_w * c->view_h * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "filled colour download"));
     RR_TRY(check(c, cudaStreamSynchronize(c->stream), "fill sync"));
   }
   return RR_OK;
@@ -715,8 +696,8 @@ int rr_upload_view(rr_ctx* c, int width, int height, const float* rgba, const fl
   RR_SET_DEVICE(c);
   RR_TRY(ensure_view(c, width, height));
   const size_t n = (size_t)width * height;
-  RR_TRY(check(c, cudaMemcpyAsync(c->d_rgba, rgba, n * sizeof(float4), cudaMemcpyHostToDevice, c->stream), "view upload"));
-  RR_TRY(check(c, cudaMemcpyAsync(c->d_zbuf, depth, n * sizeof(float), cudaMemcpyHostToDevice, c->stream), "view upload"));
+  RR_TRY(check(c, cudaMemcpyAsync(c->d_rgba.ptr, rgba, n * sizeof(float4), cudaMemcpyHostToDevice, c->stream), "view upload"));
+  RR_TRY(check(c, cudaMemcpyAsync(c->d_zbuf.ptr, depth, n * sizeof(float), cudaMemcpyHostToDevice, c->stream), "view upload"));
   return check(c, cudaStreamSynchronize(c->stream), "view upload sync");
 }
 
@@ -753,11 +734,7 @@ int rr_composite(rr_ctx* c, const void* d_records, int n_parts, int width, int h
   timer_begin(c, "composite");
   RR_TRY(launch_composite(c, (const float4*)d_records, n_parts));
   timer_end(c, "composite");
-  const size_t n = (size_t)width * height;
-  if (out_rgba) RR_TRY(check(c, cudaMemcpyAsync(out_rgba, c->d_rgba, n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "rgba download"));
-  if (out_depth) RR_TRY(check(c, cudaMemcpyAsync(out_depth, c->d_zbuf, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "depth download"));
-  if (out_rgba || out_depth) RR_TRY(check(c, cudaStreamSynchronize(c->stream), "composite sync"));
-  return RR_OK;
+  return view_download(c, out_rgba, out_depth, "rr_composite");
 }
 
 int rr_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float* host_out, int keep) {
@@ -768,29 +745,20 @@ int rr_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float* hos
   RR_REQUIRE(c, out_res && out_res[0] && out_res[1] && out_res[2], "rr_calib_invert: empty output resolution");
   RR_SET_DEVICE(c);
   const size_t n = (size_t)out_res[0] * out_res[1] * out_res[2];
+  DeviceArray<float4> own;     // the output when it is not kept
   float4* d_out = nullptr;
-  bool own = true;
   if (keep) {
-    const bool same = c->d_inv && c->ires[0] == out_res[0] && c->ires[1] == out_res[1] && c->ires[2] == out_res[2];
-    if (!same) {
-      bool any = false;
-      for (int i = 0; i < c->N; ++i) any = any || (c->have_inv[i] && i != sensor);
-      RR_REQUIRE(c, !any, "rr_calib_invert: all sensors must share one inverse-volume resolution");
-      RR_TRY(dev_alloc(c, &c->d_inv, n * c->N, "cv_xyz_inv"));
-      for (int a = 0; a < 3; ++a) c->ires[a] = out_res[a];
-      for (int i = 0; i < c->N; ++i) c->have_inv[i] = false;
-    }
-    d_out = c->d_inv + n * sensor;
-    own = false;
+    RR_TRY(ensure_inv(c, sensor, out_res, "rr_calib_invert: all sensors must share one inverse-volume resolution"));
+    d_out = c->d_inv.ptr + n * sensor;
   } else {
-    RR_TRY(check(c, cudaMalloc((void**)&d_out, n * sizeof(float4)), "inverse volume"));
+    RR_TRY(own.allocate(c, n, "inverse volume"));
+    d_out = own.ptr;
   }
-  int rc = launch_calib_invert(c, sensor, out_res, d_out);
-  if (rc == RR_OK && host_out) rc = check(c, cudaMemcpyAsync(host_out, d_out, n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "inverse download");
-  if (rc == RR_OK) rc = check(c, cudaStreamSynchronize(c->stream), "invert sync");
-  if (own) cudaFree(d_out);
-  if (rc == RR_OK && keep) { c->have_inv[sensor] = true; c->sti.dirty = true; }
-  return rc;
+  RR_TRY(launch_calib_invert(c, sensor, out_res, d_out));
+  if (host_out) RR_TRY(check(c, cudaMemcpyAsync(host_out, d_out, n * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "inverse download"));
+  RR_TRY(check(c, cudaStreamSynchronize(c->stream), "invert sync"));
+  if (keep) { c->have_inv[sensor] = true; c->sti.dirty = true; }
+  return RR_OK;
 }
 
 static int download(rr_ctx* c, void* dst, const void* src, size_t bytes, const char* what) {
@@ -825,7 +793,7 @@ static float half_bits_to_float(uint16_t h) {
 // half2 voxels are 4 bytes like R32F ones: download raw, then widen the chosen half in place
 static int download_half2(rr_ctx* c, float* out, int which) {
   const size_t n = (size_t)c->res[0] * c->res[1] * c->res[2];
-  RR_TRY(download(c, out, c->d_tsdf, n * sizeof(float), "voxel download"));
+  RR_TRY(download(c, out, c->d_tsdf.ptr, n * sizeof(float), "voxel download"));
   for (size_t i = 0; i < n; ++i) {
     uint32_t u;
     std::memcpy(&u, out + i, sizeof(u));
@@ -838,15 +806,15 @@ int rr_download_tsdf(rr_ctx* c, float* out) {
   if (!c) return RR_ERR_INVALID;
   RR_REQUIRE(c, out && c->configured, "rr_download_tsdf: not configured or null pointer");
   if (c->cfg.store_weight == RR_VOXELS_HALF2) return download_half2(c, out, 0);
-  return download(c, out, c->d_tsdf, (size_t)c->res[0] * c->res[1] * c->res[2] * sizeof(float), "tsdf download");
+  return download(c, out, c->d_tsdf.ptr, (size_t)c->res[0] * c->res[1] * c->res[2] * sizeof(float), "tsdf download");
 }
 
 int rr_download_weight(rr_ctx* c, float* out) {
   if (!c) return RR_ERR_INVALID;
   RR_REQUIRE(c, out && c->configured, "rr_download_weight: not configured or null pointer");
   if (c->cfg.store_weight == RR_VOXELS_HALF2) return download_half2(c, out, 1);
-  RR_REQUIRE(c, c->d_weight, "rr_download_weight: store_weight is off");
-  return download(c, out, c->d_weight, (size_t)c->res[0] * c->res[1] * c->res[2] * sizeof(float), "weight download");
+  RR_REQUIRE(c, c->d_weight.ptr, "rr_download_weight: store_weight is off");
+  return download(c, out, c->d_weight.ptr, (size_t)c->res[0] * c->res[1] * c->res[2] * sizeof(float), "weight download");
 }
 
 int rr_download_stage(rr_ctx* c, int stage, float* out) {
@@ -854,21 +822,19 @@ int rr_download_stage(rr_ctx* c, int stage, float* out) {
   RR_REQUIRE(c, out, "rr_download_stage: null pointer");
   const size_t px = (size_t)c->N * c->W * c->H;
   switch (stage) {
-    case RR_STAGE_MORPH: return download(c, out, c->d_morph, px * sizeof(float), "stage download");
-    case RR_STAGE_DEPTH: return download(c, out, c->d_depth, px * sizeof(float2), "stage download");
-    case RR_STAGE_DEPTH_B: return download(c, out, c->d_depth_b, px * sizeof(float2), "stage download");
-    case RR_STAGE_SILHOUETTE: return download(c, out, c->d_sil, px * sizeof(float), "stage download");
-    case RR_STAGE_QUALITY: return download(c, out, c->d_quality, px * sizeof(float), "stage download");
+    case RR_STAGE_MORPH: return download(c, out, c->d_morph.ptr, px * sizeof(float), "stage download");
+    case RR_STAGE_DEPTH: return download(c, out, c->d_depth.ptr, px * sizeof(float2), "stage download");
+    case RR_STAGE_DEPTH_B: return download(c, out, c->d_depth_b.ptr, px * sizeof(float2), "stage download");
+    case RR_STAGE_SILHOUETTE: return download(c, out, c->d_sil.ptr, px * sizeof(float), "stage download");
+    case RR_STAGE_QUALITY: return download(c, out, c->d_quality.ptr, px * sizeof(float), "stage download");
     case RR_STAGE_LAB:
     case RR_STAGE_NORMAL: {
       RR_SET_DEVICE(c);
-      float* tmp = nullptr;
-      RR_TRY(check(c, cudaMalloc((void**)&tmp, px * 3 * sizeof(float)), "stage staging"));
-      k_unpad3<<<(unsigned)((px + 255) / 256), 256, 0, c->stream>>>(stage == RR_STAGE_LAB ? c->d_lab : c->d_normal, tmp, px);
+      DeviceArray<float> tmp;
+      RR_TRY(tmp.allocate(c, px * 3, "stage staging"));
+      k_unpad3<<<(unsigned)((px + 255) / 256), 256, 0, c->stream>>>(stage == RR_STAGE_LAB ? c->d_lab.ptr : c->d_normal.ptr, tmp.ptr, px);
       ++c->launches;
-      int rc = download(c, out, tmp, px * 3 * sizeof(float), "stage download");
-      cudaFree(tmp);
-      return rc;
+      return download(c, out, tmp.ptr, px * 3 * sizeof(float), "stage download");
     }
     default: return fail(c, RR_ERR_INVALID, "rr_download_stage: unknown stage");
   }
@@ -880,23 +846,23 @@ int rr_download_bricks(rr_ctx* c, uint32_t* counters, uint32_t* occupied, uint32
   RR_SET_DEVICE(c);
   RR_TRY(check(c, cudaStreamSynchronize(c->stream), "bricks download sync"));
   uint32_t n = 0;
-  RR_TRY(download(c, &n, c->d_num_occ, sizeof(uint32_t), "count download"));
-  if (counters) RR_TRY(download(c, counters, c->d_counters, c->bricks.num * sizeof(uint32_t), "counters download"));
-  if (occupied && n) RR_TRY(download(c, occupied, c->d_occupied, n * sizeof(uint32_t), "occupied download"));
+  RR_TRY(download(c, &n, c->d_num_occ.ptr, sizeof(uint32_t), "count download"));
+  if (counters) RR_TRY(download(c, counters, c->d_counters.ptr, c->bricks.num * sizeof(uint32_t), "counters download"));
+  if (occupied && n) RR_TRY(download(c, occupied, c->d_occupied.ptr, n * sizeof(uint32_t), "occupied download"));
   if (num_occupied) *num_occupied = n;
   return RR_OK;
 }
 
 int rr_download_num_samples(rr_ctx* c, float* out) {
   if (!c) return RR_ERR_INVALID;
-  RR_REQUIRE(c, out && c->d_nsamples, "rr_download_num_samples: no raymarch yet");
-  return download(c, out, c->d_nsamples, (size_t)c->view_w * c->view_h * sizeof(float), "samples download");
+  RR_REQUIRE(c, out && c->d_nsamples.ptr, "rr_download_num_samples: no raymarch yet");
+  return download(c, out, c->d_nsamples.ptr, (size_t)c->view_w * c->view_h * sizeof(float), "samples download");
 }
 
 int rr_download_hit_positions(rr_ctx* c, float* out) {
   if (!c) return RR_ERR_INVALID;
-  RR_REQUIRE(c, out && c->d_pos, "rr_download_hit_positions: no raymarch yet");
-  return download(c, out, c->d_pos, (size_t)c->view_w * c->view_h * sizeof(float4), "positions download");
+  RR_REQUIRE(c, out && c->d_pos.ptr, "rr_download_hit_positions: no raymarch yet");
+  return download(c, out, c->d_pos.ptr, (size_t)c->view_w * c->view_h * sizeof(float4), "positions download");
 }
 
 int rr_extract_mesh(rr_ctx* c, uint32_t* out_num_vertices, uint32_t* out_num_triangles) {
@@ -1075,10 +1041,10 @@ int rr_integrator_info(rr_ctx* c, uint32_t* out) {
   out[1] = (uint32_t)s.T; out[2] = (uint32_t)s.BX; out[3] = (uint32_t)s.BY; out[4] = (uint32_t)s.BZ;
   out[5] = (uint32_t)s.cy; out[6] = (uint32_t)s.cz; out[7] = (uint32_t)s.n_yc; out[8] = (uint32_t)s.n_zc;
   out[9] = s.n_oversize; out[10] = s.smem_bytes; out[11] = (uint32_t)s.cwarps; out[12] = (uint32_t)s.fwarps; out[14] = s.n_slots; out[15] = s.slot_bytes;
-  if (s.d_err) {
+  if (s.d_err.ptr) {
     uint32_t e[4] = {0, 0, 0, 0};
     RR_TRY(check(c, cudaStreamSynchronize(c->stream), "integrator info sync"));
-    RR_TRY(check(c, cudaMemcpy(e, s.d_err, sizeof(e), cudaMemcpyDeviceToHost), "integrator flags"));
+    RR_TRY(check(c, cudaMemcpy(e, s.d_err.ptr, sizeof(e), cudaMemcpyDeviceToHost), "integrator flags"));
     out[13] = (e[0] ? 1u : 0u) | (e[1] ? 2u : 0u);
   }
   return RR_OK;
@@ -1094,10 +1060,10 @@ int rr_integrator_profile(rr_ctx* c, uint64_t* out) {
   if (!c || !out) return RR_ERR_INVALID;
   RR_SET_DEVICE(c);
   std::memset(out, 0, 16 * sizeof(uint64_t));
-  if (!c->sti.d_err) return RR_OK;
+  if (!c->sti.d_err.ptr) return RR_OK;
   RR_TRY(check(c, cudaStreamSynchronize(c->stream), "integrator profile sync"));
-  RR_TRY(check(c, cudaMemcpy(out, c->sti.d_err + 4, 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost), "integrator profile"));
-  RR_TRY(check(c, cudaMemset(c->sti.d_err + 4, 0, 16 * sizeof(uint64_t)), "integrator profile reset"));
+  RR_TRY(check(c, cudaMemcpy(out, c->sti.d_err.ptr + 4, 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost), "integrator profile"));
+  RR_TRY(check(c, cudaMemset(c->sti.d_err.ptr + 4, 0, 16 * sizeof(uint64_t)), "integrator profile reset"));
   return RR_OK;
 }
 

@@ -98,7 +98,7 @@ __global__ void __launch_bounds__(1024) k_bricks_update(const uint32_t* __restri
 }
 
 int launch_bricks_clear(rr_ctx* c) {
-  cudaError_t e = cudaMemsetAsync(c->d_counters, 0, sizeof(uint32_t) * ((size_t)c->bricks.num + RR_CLASS_COUNTERS), c->stream);
+  cudaError_t e = cudaMemsetAsync(c->d_counters.ptr, 0, sizeof(uint32_t) * ((size_t)c->bricks.num + RR_CLASS_COUNTERS), c->stream);
   c->sti.lists_key = 0;
   return check(c, e, "bricks clear");
 }
@@ -116,15 +116,15 @@ int launch_bricks_update(rr_ctx* c) {
   const uint32_t cls_blocks = classify ? (nb * (uint32_t)cq.per_brick + 31u) / 32u : 0u;
   timer_begin(c, "bricks");
   k_bricks_update<<<1 + mask_blocks + cls_blocks, 1024, 0, c->stream>>>(
-      c->d_counters, nb, c->bricks.res[0], c->bricks.res[1], c->bricks.res[2], c->cfg.min_voxels_per_brick, c->d_ranges, c->mask_words,
-      c->d_occupied, c->d_num_occ, grid_ok ? c->d_near_occ : nullptr, c->d_occ_mask, (grid_ok && c->fused_ok) ? c->d_rowmask : nullptr, c->d_rowany,
-      c->d_work, mask_blocks, cq);
+      c->d_counters.ptr, nb, c->bricks.res[0], c->bricks.res[1], c->bricks.res[2], c->cfg.min_voxels_per_brick, c->d_ranges.ptr, c->mask_words,
+      c->d_occupied.ptr, c->d_num_occ.ptr, grid_ok ? c->d_near_occ.ptr : nullptr, c->d_occ_mask.ptr, (grid_ok && c->fused_ok) ? c->d_rowmask.ptr : nullptr, c->d_rowany.ptr,
+      c->d_work.ptr, mask_blocks, cq);
   RR_LAUNCH_CHECK(c, "k_bricks_update");
   timer_end(c, "bricks");
   c->work_fresh = true;
   c->mesh_rows_ok = false;     // new row tables: the volume was cleared by the previous ones
   if (classify) c->sti.lists_key = staged_lists_key(c);
-  cudaError_t e = cudaMemcpyAsync(&c->pinned->num_occ, c->d_num_occ, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream);
+  cudaError_t e = cudaMemcpyAsync(&c->pinned->num_occ, c->d_num_occ.ptr, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream);
   return check(c, e, "bricks count copy");
 }
 

@@ -187,32 +187,31 @@ int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4
   g.inv_cell = 1.0 / g.cell;
   const size_t ncell = (size_t)g.dim[0] * g.dim[1] * g.dim[2];
 
-  uint32_t *d_count = nullptr, *d_start = nullptr;
-  float4* d_sorted = nullptr;
-  void* d_tmp = nullptr;
+  DeviceArray<uint32_t> count, start;
+  DeviceArray<float4> sorted;
+  DeviceArray<uint8_t> tmp;
   size_t tmp_bytes = 0;
   cudaStream_t s = c->stream;
-  int rc = RR_OK;
-  auto cleanup = [&]() { cudaFree(d_count); cudaFree(d_start); cudaFree(d_sorted); cudaFree(d_tmp); };
-  if ((rc = check(c, cudaMalloc((void**)&d_count, (ncell + 1) * sizeof(uint32_t)), "invert: cell counters")) != RR_OK ||
-      (rc = check(c, cudaMalloc((void**)&d_start, (ncell + 1) * sizeof(uint32_t)), "invert: cell starts")) != RR_OK ||
-      (rc = check(c, cudaMalloc((void**)&d_sorted, n * sizeof(float4)), "invert: binned samples")) != RR_OK) { cleanup(); return rc; }
+  RR_TRY_RC(count.allocate(c, ncell + 1, "invert: cell counters"));
+  RR_TRY_RC(start.allocate(c, ncell + 1, "invert: cell starts"));
+  RR_TRY_RC(sorted.allocate(c, n, "invert: binned samples"));
+  uint32_t *d_count = count.ptr, *d_start = start.ptr;
   cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_count, d_start, (int)(ncell + 1), s);
-  if ((rc = check(c, cudaMalloc(&d_tmp, tmp_bytes), "invert: scan scratch")) != RR_OK) { cleanup(); return rc; }
+  RR_TRY_RC(tmp.allocate(c, tmp_bytes, "invert: scan scratch"));
 
   timer_begin(c, "calib_invert");
   cudaMemsetAsync(d_count, 0, (ncell + 1) * sizeof(uint32_t), s);
   const unsigned nb = (unsigned)((n + 255) / 256);
-  k_invert_bin<<<nb, 256, 0, s>>>(c->d_xyz[sensor], X, Y, Z, g, d_count, nullptr);
+  k_invert_bin<<<nb, 256, 0, s>>>(c->d_xyz[sensor].ptr, X, Y, Z, g, d_count, nullptr);
   ++c->launches;
-  cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, d_count, d_start, (int)(ncell + 1), s);
+  cub::DeviceScan::ExclusiveSum(tmp.ptr, tmp_bytes, d_count, d_start, (int)(ncell + 1), s);
   ++c->launches;
   cudaMemcpyAsync(d_count, d_start, (ncell + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s);   // scatter cursors
-  k_invert_bin<<<nb, 256, 0, s>>>(c->d_xyz[sensor], X, Y, Z, g, d_count, d_sorted);
+  k_invert_bin<<<nb, 256, 0, s>>>(c->d_xyz[sensor].ptr, X, Y, Z, g, d_count, sorted.ptr);
   ++c->launches;
 
   InvertParams p{};
-  p.sorted = d_sorted; p.cell_start = d_start; p.g = g; p.xyz = c->d_xyz[sensor];
+  p.sorted = sorted.ptr; p.cell_start = d_start; p.g = g; p.xyz = c->d_xyz[sensor].ptr;
   for (int i = 0; i < 6; ++i) for (int k = 0; k < 4; ++k) p.planes[i][k] = c->planes[sensor][i][k];
   for (int a = 0; a < 3; ++a) {
     // calibration_inverter.cpp:100-108, single precision as written
@@ -225,15 +224,13 @@ int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4
   p.cX = X; p.cY = Y; p.cZ = Z;
   p.ox = (int)out_res[0]; p.oy = (int)out_res[1]; p.oz = (int)out_res[2];
   p.out = d_out;
-  if (p.oy > 65535 || p.oz > 65535) { cleanup(); return fail(c, RR_ERR_UNSUPPORTED, "rr_calib_invert: output resolution too large"); }
+  if (p.oy > 65535 || p.oz > 65535) return fail(c, RR_ERR_UNSUPPORTED, "rr_calib_invert: output resolution too large");
   const dim3 grd((p.ox + 127) / 128, p.oy, p.oz);
   k_invert<<<grd, 128, 0, s>>>(p);
   ++c->launches;
   timer_end(c, "calib_invert");
-  rc = check(c, cudaGetLastError(), "k_invert");
-  if (rc == RR_OK) rc = check(c, cudaStreamSynchronize(s), "invert sync");
-  cleanup();
-  return rc;
+  RR_TRY_RC(check(c, cudaGetLastError(), "k_invert"));
+  return check(c, cudaStreamSynchronize(s), "invert sync");
 }
 
 }  // namespace rr

@@ -70,7 +70,7 @@ int launch_extract_points(rr_ctx* c, uint32_t mask, uint32_t* out_n) {
 
   CloudParams p{};
   p.st = sensor_tables(c);
-  p.depth_b = c->d_depth_b; p.normal = c->d_normal; p.quality = c->d_quality; p.color = c->d_color;
+  p.depth_b = c->d_depth_b.ptr; p.normal = c->d_normal.ptr; p.quality = c->d_quality.ptr; p.color = c->d_color;
   p.W = c->W; p.H = c->H; p.CW = c->CW; p.CH = c->CH;
   p.mask = mask; p.n_px = n_px;
   for (int a = 0; a < 3; ++a) { p.bmin[a] = c->bbox_min[a]; p.bmax[a] = c->bbox_max[a]; }

@@ -239,19 +239,17 @@ int launch_fill_colors(rr_ctx* c) {
   make_lods(p, W, H);
   if (p.FW <= W) return fail(c, RR_ERR_INVALID, "fill colours: view too small");
   if (c->fill_w != W || c->fill_h != H) {
-    cudaStreamSynchronize(c->stream);
-    cudaFree(c->d_fill_fc); cudaFree(c->d_fill_fd); cudaFree(c->d_fill_sc); cudaFree(c->d_fill_sd); cudaFree(c->d_filled);
-    c->d_fill_fc = nullptr; c->d_fill_fd = nullptr; c->d_fill_sc = nullptr; c->d_fill_sd = nullptr; c->d_filled = nullptr;
     c->fill_w = c->fill_h = 0;
     const size_t nf = (size_t)(p.FW - W) * H, ns = (size_t)W * H;
-    if (cudaMalloc((void**)&c->d_fill_fc, nf * sizeof(float4)) != cudaSuccess || cudaMalloc((void**)&c->d_fill_fd, nf * sizeof(float)) != cudaSuccess ||
-        cudaMalloc((void**)&c->d_fill_sc, ns * sizeof(float4)) != cudaSuccess || cudaMalloc((void**)&c->d_fill_sd, ns * sizeof(float)) != cudaSuccess ||
-        cudaMalloc((void**)&c->d_filled, ns * sizeof(float4)) != cudaSuccess)
+    const char* what = "fill colours";
+    if (c->d_fill_fc.allocate(c, nf, what) != RR_OK || c->d_fill_fd.allocate(c, nf, what) != RR_OK ||
+        c->d_fill_sc.allocate(c, ns, what) != RR_OK || c->d_fill_sd.allocate(c, ns, what) != RR_OK ||
+        c->d_filled.allocate(c, ns, what) != RR_OK)
       return fail(c, RR_ERR_CUDA, "fill colours: allocation failed");
     c->fill_w = W; c->fill_h = H;
   }
-  p.rgba = c->d_rgba; p.zbuf = c->d_zbuf;
-  p.fc = c->d_fill_fc; p.fd = c->d_fill_fd; p.sc = c->d_fill_sc; p.sd = c->d_fill_sd; p.out = c->d_filled;
+  p.rgba = c->d_rgba.ptr; p.zbuf = c->d_zbuf.ptr;
+  p.fc = c->d_fill_fc.ptr; p.fd = c->d_fill_fd.ptr; p.sc = c->d_fill_sc.ptr; p.sd = c->d_fill_sd.ptr; p.out = c->d_filled.ptr;
   timer_begin(c, "holefill");
   const dim3 blk(32, 8, 1);
   const dim3 grd((W + 31) / 32, (H + 7) / 8, 1);

@@ -1,6 +1,10 @@
 // Internal state behind the opaque rr_ctx of include/rgbd_recon_b200.h. One context = one GPU, one stream.
 //
-// Device memory layout (all allocations live for the context's lifetime; sized for 180 GB HBM3e, nothing is paged):
+// Ownership: every device allocation is an rr::DeviceArray (a context field, or a local for a call's temporaries), and
+// nothing outside this header calls cudaMalloc / cudaFree. An array frees its memory when it is reallocated or destroyed;
+// the context's destructor, run by rr_destroy on the context's device, is what releases the context's buffers.
+//
+// Device memory layout (sized for 180 GB HBM3e, nothing is paged):
 //   frames     depth float[N][H][W], colour uint8[N][CH][CW][3]                       (written by rr_upload_frames)
 //   calib      per sensor cv_xyz as float4[Z][Y][X] (xyz padded to 16 B so a corner is one LDG.128),
 //              cv_uv float2[Z][Y][X]; cv_xyz_inv float4[N][IZ][IY][IX] in one allocation
@@ -61,8 +65,9 @@ struct StageTimer {            // one CUDA-event pair per recorded interval; sum
   float last_ms = 0.0f;        // the newest folded interval (rr_get_stage_ms right after a fold)
 };
 
-// A device array of the context that grows on demand to the size of a result (reserve, defined below rr_ctx); freed by the
-// context's destructor, on the context's device.
+// The one owner of device memory: a fixed-size buffer (allocate) or one that grows on demand to the size of a result
+// (reserve), both defined below rr_ctx. Freed by its destructor on the current device, which must be the device it was
+// allocated on.
 template <typename T>
 struct DeviceArray {
   T* ptr = nullptr;
@@ -70,7 +75,12 @@ struct DeviceArray {
   DeviceArray() = default;
   DeviceArray(const DeviceArray&) = delete;
   DeviceArray& operator=(const DeviceArray&) = delete;
+  DeviceArray& operator=(DeviceArray&& o) {
+    if (this != &o) { release(); ptr = o.ptr; cap = o.cap; o.ptr = nullptr; o.cap = 0; }
+    return *this;
+  }
   ~DeviceArray() { cudaFree(ptr); }
+  int allocate(rr_ctx* c, size_t count, const char* what);
   int reserve(rr_ctx* c, size_t need, const char* what);
   void release() { cudaFree(ptr); ptr = nullptr; cap = 0; }
 };
@@ -101,24 +111,24 @@ struct rr_ctx {
   // calibration
   float bbox_min[3] = {0, 0, 0}, bbox_max[3] = {0, 0, 0};
   bool have_bbox = false;
-  float4* d_xyz[RR_MAX_SENSORS] = {};
-  float2* d_uv[RR_MAX_SENSORS] = {};
+  rr::DeviceArray<float4> d_xyz[RR_MAX_SENSORS];
+  rr::DeviceArray<float2> d_uv[RR_MAX_SENSORS];
   uint32_t cres[RR_MAX_SENSORS][3] = {};
   float dlim[RR_MAX_SENSORS][2] = {};
   float cam_pos[RR_MAX_SENSORS][3] = {};
   float planes[RR_MAX_SENSORS][6][4] = {};
   float xyz_min[RR_MAX_SENSORS][3] = {}, xyz_max[RR_MAX_SENSORS][3] = {};   // bounding box of the cv_xyz samples
   bool have_calib[RR_MAX_SENSORS] = {};
-  float4* d_inv = nullptr;
+  rr::DeviceArray<float4> d_inv;
   uint32_t ires[3] = {0, 0, 0};
   bool have_inv[RR_MAX_SENSORS] = {};
 
   // frames + stages. Two device frame slots (the reference's double PBO, double_pixel_buffer.cpp): d_depth_raw / d_color
-  // alias the CURRENT slot (read by the kernels); rr_stage_frames copies into the other one on copy_stream.
+  // alias the CURRENT slot (read by the kernels; they own nothing); rr_stage_frames copies into the other one on copy_stream.
   float* d_depth_raw = nullptr;
   uint8_t* d_color = nullptr;
-  float* d_depth_slot[2] = {nullptr, nullptr};
-  uint8_t* d_color_slot[2] = {nullptr, nullptr};
+  rr::DeviceArray<float> d_depth_slot[2];
+  rr::DeviceArray<uint8_t> d_color_slot[2];
   int cur_slot = 0;
   bool staged = false;                       // the other slot holds a frame set that has not been swapped in yet
   bool staged_color = false;                 // ... and it came with colour
@@ -128,21 +138,21 @@ struct rr_ctx {
   bool free_recorded[2] = {false, false};
   // compressed ingest (rr_set_frame_format): packed layers per slot, expanded by launch_unpack_frames at the swap
   int color_format = 0, depth_format = 0;
-  uint8_t* d_color_packed[2] = {nullptr, nullptr};
-  uint8_t* d_depth_packed[2] = {nullptr, nullptr};
+  rr::DeviceArray<uint8_t> d_color_packed[2];
+  rr::DeviceArray<uint8_t> d_depth_packed[2];
   float depth_near[RR_MAX_SENSORS] = {}, depth_far[RR_MAX_SENSORS] = {};
-  float* d_morph = nullptr;
-  float2* d_depth = nullptr;
-  float4* d_lab = nullptr;
-  float2* d_depth_b = nullptr;
-  float* d_sil = nullptr;
-  float4* d_normal = nullptr;
-  float* d_quality = nullptr;
-  float4* d_gather = nullptr;
+  rr::DeviceArray<float> d_morph;
+  rr::DeviceArray<float2> d_depth;
+  rr::DeviceArray<float4> d_lab;
+  rr::DeviceArray<float2> d_depth_b;
+  rr::DeviceArray<float> d_sil;
+  rr::DeviceArray<float4> d_normal;
+  rr::DeviceArray<float> d_quality;
+  rr::DeviceArray<float4> d_gather;
   bool gather_packed = false;      // d_gather holds the texels of the last rr_preprocess (k_pack_gather ran for it)
-  float2* d_pairs = nullptr;       // [N][H+2][pair_pitch]
+  rr::DeviceArray<float2> d_pairs;   // [N][H+2][pair_pitch]
   int pair_pitch = 0;              // W+2 rounded up to even (TMA strides are multiples of 16 bytes)
-  uint32_t* d_flags = nullptr;     // [0] pack-encoding violation counter
+  rr::DeviceArray<uint32_t> d_flags; // [0] pack-encoding violation counter
 
   // settings + bricks + volume
   rr_config cfg{};
@@ -151,22 +161,20 @@ struct rr_ctx {
   uint32_t slab_z0 = 0, slab_z1 = 0;
   rr::BrickGrid bricks{};
   std::vector<int32_t> h_ranges;
-  int32_t* d_ranges = nullptr;
-  uint32_t* d_counters = nullptr;  // [bricks.num] voxels seen per brick, then RR_CLASS_COUNTERS item-class counters of the staged integrator
-  uint32_t* d_occupied = nullptr;
-  uint32_t* d_num_occ = nullptr;
-  uint8_t* d_near_occ = nullptr;
-  uint8_t* d_occ_mask = nullptr;
+  rr::DeviceArray<int32_t> d_ranges;
+  rr::DeviceArray<uint32_t> d_counters;   // [bricks.num] voxels seen per brick, then RR_CLASS_COUNTERS item-class counters of the staged integrator
+  rr::DeviceArray<uint32_t> d_occupied, d_num_occ;
+  rr::DeviceArray<uint8_t> d_near_occ, d_occ_mask;
   // fused clear+integrate support: per brick row (bz, by) the x bitmask of voxels inside occupied bricks, a byte that
   // says whether the row has any, and per voxel y / z index the (at most two) brick indices whose range contains it
-  uint32_t* d_rowmask = nullptr;   // [nbz][nby][mask_words]
-  uint8_t* d_rowany = nullptr;     // [nbz][nby]
-  int16_t* d_cand_y = nullptr;     // [Y][2], -1 = none
-  int16_t* d_cand_z = nullptr;     // [Z][2]
-  uint32_t* d_work = nullptr;      // [4] work-item counters of the persistent fused kernel
+  rr::DeviceArray<uint32_t> d_rowmask;   // [nbz][nby][mask_words]
+  rr::DeviceArray<uint8_t> d_rowany;      // [nbz][nby]
+  rr::DeviceArray<int16_t> d_cand_y;      // [Y][2], -1 = none
+  rr::DeviceArray<int16_t> d_cand_z;      // [Z][2]
+  rr::DeviceArray<uint32_t> d_work;       // [4] work-item counters of the persistent fused kernel
   bool work_fresh = false;         // k_bricks_update has reset them and no integrate launch has drawn from them since
   int mask_words = 0;
-  float4* d_ztab = nullptr;        // [Z] (k0, k1, g, 1-g) of the z filter tap against the inverse volume (k_build_ztab)
+  rr::DeviceArray<float4> d_ztab;  // [Z] (k0, k1, g, 1-g) of the z filter tap against the inverse volume (k_build_ztab)
   int ztab_Z = 0, ztab_IZ = 0;
   bool fused_ok = false;           // brick table is separable with <= 2 bricks per voxel and axis
   // rr_fuse_frame: captured launch sequences, keyed by (frame slot, pre-process flags, tunable generation)
@@ -191,29 +199,28 @@ struct rr_ctx {
     int cwarps = 0, fwarps = 0;    // consumer / fill warps per CTA
     uint32_t inv_bytes = 0, tile_bytes = 0, inv_span = 0, smem_bytes = 0, fill_src_bytes = 0, fill_src_off = 0, tables_off = 0;
     uint32_t slot_bytes = 0, n_slots = 0, slots_off = 0;   // ring of per-sensor operand slots (inverse-volume box + tile)
-    uint2* d_fp = nullptr;         // [items][N]: tile origin tx0 | ty0 << 16, footprint rectangle inside the tile (bit 7 of .y: exceeds the tile)
+    rr::DeviceArray<uint2> d_fp;   // [items][N]: tile origin tx0 | ty0 << 16, footprint rectangle inside the tile (bit 7 of .y: exceeds the tile)
     uint32_t n_oversize = 0;       // (item, sensor) pairs of the whole brick grid whose footprint exceeds the tile
-    uint2* d_list = nullptr;       // [N + 1][list_stride]: this frame's occupied items by cost class (item, verdict), k_bricks_update
+    rr::DeviceArray<uint2> d_list; // [N + 1][list_stride]: this frame's occupied items by cost class (item, verdict), k_bricks_update
     unsigned tables = 0;           // bumped by every table rebuild
     uint64_t lists_key = 0;        // staged_lists_key() the lists were classified for; 0: no valid lists (cleared by a table
                                    // rebuild, rr_bricks_clear and rr_preprocess, whose new pair image the verdicts do not describe)
     uint32_t list_stride = 0;
-    float2* d_zr = nullptr;        // [items][N]: exact range of pos_calib.z over the item (k_footprints)
-    uint32_t* d_err = nullptr;     // [4] device-side consistency flags (must stay 0)
+    rr::DeviceArray<float2> d_zr;  // [items][N]: exact range of pos_calib.z over the item (k_footprints)
+    rr::DeviceArray<uint32_t> d_err;   // [4] device-side consistency flags (must stay 0), then 16 profile counters (uint64)
     CUtensorMap map_inv, map_pairs;
   } sti;
   rr::PinnedScalars* pinned = nullptr;   // one cudaMallocHost allocation for the context's lifetime
-  float* d_tsdf = nullptr;
-  float* d_weight = nullptr;
+  rr::DeviceArray<float> d_tsdf;
+  rr::DeviceArray<float> d_weight;   // empty unless rr_config.store_weight is RR_VOXELS_F32_WEIGHT
 
   // raymarch outputs
   int view_w = 0, view_h = 0;
-  float4* d_rgba = nullptr;
-  float* d_zbuf = nullptr;
-  float* d_nsamples = nullptr;
-  float4* d_pos = nullptr;         // hit position in volume space (w = 1 on a hit)
-  uint32_t* d_step = nullptr;      // step index of the hit, 0xFFFFFFFF = none (multi-GPU compositing key)
-  unsigned long long* d_point_keys = nullptr;   // rr_draw_points / rr_draw_calibs: per pixel (depth bits << 32 | vertex id), atomicMin
+  rr::DeviceArray<float4> d_rgba;
+  rr::DeviceArray<float> d_zbuf, d_nsamples;
+  rr::DeviceArray<float4> d_pos;         // hit position in volume space (w = 1 on a hit)
+  rr::DeviceArray<uint32_t> d_step;      // step index of the hit, 0xFFFFFFFF = none (multi-GPU compositing key)
+  rr::DeviceArray<unsigned long long> d_point_keys;   // rr_draw_points / rr_draw_calibs: per pixel (depth bits << 32 | vertex id), atomicMin
 
   // rr_draw_trigrid (rr_trigrid.cu): vertex records, pass-1 depth bits, per-pixel fragment lists (grown on demand)
   rr::DeviceArray<float4> d_tg_verts;
@@ -276,9 +283,8 @@ struct rr_ctx {
 
   // colour hole filling (rr_colorfill.cu): atlas right of column W, squeezed copy, filled colour
   int fill_w = 0, fill_h = 0;
-  float4* d_fill_fc = nullptr; float* d_fill_fd = nullptr;
-  float4* d_fill_sc = nullptr; float* d_fill_sd = nullptr;
-  float4* d_filled = nullptr;
+  rr::DeviceArray<float4> d_fill_fc, d_fill_sc, d_filled;
+  rr::DeviceArray<float> d_fill_fd, d_fill_sd;
 };
 
 namespace rr {
@@ -318,6 +324,7 @@ int check(rr_ctx* c, cudaError_t e, const char* what);
 void timer_begin(rr_ctx* c, const char* name);
 void timer_end(rr_ctx* c, const char* name);
 SensorTables sensor_tables(const rr_ctx* c);
+int view_download(rr_ctx* c, float* out_rgba, float* out_depth, const char* what);   // d_rgba / d_zbuf out, one synchronise
 
 // kernels' host launchers (one translation unit each)
 int launch_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, int refine);
@@ -360,7 +367,6 @@ int simplified_download(rr_ctx* c, float* positions, float* normals, float* rgba
 int launch_unpack_frames(rr_ctx* c, int slot);
 int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4* d_out);
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines
-void staged_release(rr_ctx* c);
 bool staged_selected(const rr_ctx* c); // after staged_prepare: the next bricks-mode integrate runs the staged kernel
 uint64_t staged_lists_key(const rr_ctx* c);   // what the item lists depend on besides the frame: table rebuild, limit
 void drop_frame_graphs(rr_ctx* c);
@@ -383,16 +389,24 @@ uint32_t host_divide_box(const float bmin[3], const float bmax[3], float brick_s
     if (e__ != cudaSuccess) return rr::check((c), e__, (what));    \
   } while (0)
 
-// Grows to `need` elements plus 1/8 slack; a queued kernel or copy may still read the old memory, so the stream drains first.
+// Both methods free the old memory before allocating the new; a queued kernel or copy may still read it, so the context's
+// stream drains first.
+// Exactly `count` elements, no slack (count == 0: empty, ptr == nullptr).
 template <typename T>
-int rr::DeviceArray<T>::reserve(rr_ctx* c, size_t need, const char* what) {
-  if (need <= cap) return RR_OK;
+int rr::DeviceArray<T>::allocate(rr_ctx* c, size_t count, const char* what) {
   if (ptr) {
     RR_TRY_RC(rr::check(c, cudaStreamSynchronize(c->stream), what));
     release();
   }
-  const size_t n = need + need / 8 + 1;
-  RR_TRY_RC(rr::check(c, cudaMalloc((void**)&ptr, n * sizeof(T)), what));
-  cap = n;
+  if (count == 0) return RR_OK;
+  RR_TRY_RC(rr::check(c, cudaMalloc((void**)&ptr, count * sizeof(T)), what));
+  cap = count;
   return RR_OK;
+}
+
+// Grows to `need` elements plus 1/8 slack.
+template <typename T>
+int rr::DeviceArray<T>::reserve(rr_ctx* c, size_t need, const char* what) {
+  if (need <= cap) return RR_OK;
+  return allocate(c, need + need / 8 + 1, what);
 }

@@ -26,7 +26,8 @@ struct rr_group {
   std::vector<char> peer;              // member 0's kernels may load from member i's memory
   std::string error;
   // fallback for members member 0 cannot address: their view is copied into these (device 0) before compositing
-  std::vector<uint32_t*> f_step; std::vector<float4*> f_rgba; std::vector<float*> f_zbuf; std::vector<float*> f_nsamp;
+  struct FallbackView { rr::DeviceArray<uint32_t> step; rr::DeviceArray<float4> rgba; rr::DeviceArray<float> zbuf, nsamp; };
+  std::vector<FallbackView> fallback;  // per member
   size_t f_pixels = 0;
   std::vector<cudaEvent_t> ev_view;    // member i's view (or its fallback copy) is complete
   std::vector<cudaEvent_t> ev_copied[2];   // [slot][i]: member i has copied its parent's frame slot `slot` (the parent may overwrite it)
@@ -145,7 +146,7 @@ int rr_group_create(rr_group** out, const int* devices, int n_devices, int num_s
     cudaEventCreateWithFlags(&g->ev_copied[0][i], cudaEventDisableTiming);
     cudaEventCreateWithFlags(&g->ev_copied[1][i], cudaEventDisableTiming);
   }
-  g->f_step.assign(n_devices, nullptr); g->f_rgba.assign(n_devices, nullptr); g->f_zbuf.assign(n_devices, nullptr); g->f_nsamp.assign(n_devices, nullptr);
+  g->fallback = std::vector<rr_group::FallbackView>(n_devices);
   *out = g;
   return RR_OK;
 }
@@ -160,7 +161,7 @@ void rr_group_destroy(rr_group* g) {
     for (int b = 0; b < 2; ++b) if (g->ev_copied[b][i]) cudaEventDestroy(g->ev_copied[b][i]);
   }
   cudaSetDevice(g->dev[0]);
-  for (size_t i = 0; i < g->m.size(); ++i) { cudaFree(g->f_step[i]); cudaFree(g->f_rgba[i]); cudaFree(g->f_zbuf[i]); cudaFree(g->f_nsamp[i]); }
+  g->fallback.clear();
   for (rr_ctx* c : g->m) rr_destroy(c);
   delete g;
 }
@@ -313,12 +314,12 @@ static int stage_from_peer(rr_group* g, size_t self, bool color, size_t cb, size
   if (c->free_recorded[t]) RR_G_TRY(g, cudaStreamWaitEvent(c->copy_stream, c->ev_free[t], 0));
   RR_G_TRY_RC(wait_for_children(g, self, t));
   RR_G_TRY(g, cudaStreamWaitEvent(c->copy_stream, s->ev_staged, 0));
-  void* dd = c->depth_format == RR_DEPTH_U8 ? (void*)c->d_depth_packed[t] : (void*)c->d_depth_slot[t];
-  const void* sd = s->depth_format == RR_DEPTH_U8 ? (const void*)s->d_depth_packed[ts] : (const void*)s->d_depth_slot[ts];
+  void* dd = c->depth_format == RR_DEPTH_U8 ? (void*)c->d_depth_packed[t].ptr : (void*)c->d_depth_slot[t].ptr;
+  const void* sd = s->depth_format == RR_DEPTH_U8 ? (const void*)s->d_depth_packed[ts].ptr : (const void*)s->d_depth_slot[ts].ptr;
   RR_G_TRY(g, cudaMemcpyPeerAsync(dd, c->device, sd, s->device, db, c->copy_stream));
   if (color) {
-    void* dc = c->color_format != RR_COLOR_RGB8 ? (void*)c->d_color_packed[t] : (void*)c->d_color_slot[t];
-    const void* sc = s->color_format != RR_COLOR_RGB8 ? (const void*)s->d_color_packed[ts] : (const void*)s->d_color_slot[ts];
+    void* dc = c->color_format != RR_COLOR_RGB8 ? (void*)c->d_color_packed[t].ptr : (void*)c->d_color_slot[t].ptr;
+    const void* sc = s->color_format != RR_COLOR_RGB8 ? (const void*)s->d_color_packed[ts].ptr : (const void*)s->d_color_slot[ts].ptr;
     RR_G_TRY(g, cudaMemcpyPeerAsync(dc, c->device, sc, s->device, cb, c->copy_stream));
   }
   c->staged_color = color;
@@ -414,23 +415,23 @@ int rr_group_raymarch(rr_group* g, const rr_view* view, float* out_rgba, float* 
     rr_ctx* c = g->m[i];
     if (i > 0 && !g->peer[i]) {
       // no peer addressing between the two devices: copy the member's view to the display device first
-      if (g->f_pixels < px || !g->f_step[i]) {
+      rr_group::FallbackView& f = g->fallback[i];
+      if (g->f_pixels < px || !f.step.ptr) {
         RR_G_TRY(g, cudaSetDevice(c0->device));
-        RR_G_TRY(g, cudaStreamSynchronize(c0->stream));
-        cudaFree(g->f_step[i]); cudaFree(g->f_rgba[i]); cudaFree(g->f_zbuf[i]); cudaFree(g->f_nsamp[i]);
-        RR_G_TRY(g, cudaMalloc((void**)&g->f_step[i], px * sizeof(uint32_t)));
-        RR_G_TRY(g, cudaMalloc((void**)&g->f_rgba[i], px * sizeof(float4)));
-        RR_G_TRY(g, cudaMalloc((void**)&g->f_zbuf[i], px * sizeof(float)));
-        RR_G_TRY(g, cudaMalloc((void**)&g->f_nsamp[i], px * sizeof(float)));
+        int rc = f.step.allocate(c0, px, "group view steps");
+        if (rc == RR_OK) rc = f.rgba.allocate(c0, px, "group view rgba");
+        if (rc == RR_OK) rc = f.zbuf.allocate(c0, px, "group view depth");
+        if (rc == RR_OK) rc = f.nsamp.allocate(c0, px, "group view samples");
+        if (rc != RR_OK) return member_fail(g, 0, rc);
       }
       RR_G_TRY(g, cudaSetDevice(c->device));
-      RR_G_TRY(g, cudaMemcpyPeerAsync(g->f_step[i], c0->device, c->d_step, c->device, px * sizeof(uint32_t), c->stream));
-      RR_G_TRY(g, cudaMemcpyPeerAsync(g->f_rgba[i], c0->device, c->d_rgba, c->device, px * sizeof(float4), c->stream));
-      RR_G_TRY(g, cudaMemcpyPeerAsync(g->f_zbuf[i], c0->device, c->d_zbuf, c->device, px * sizeof(float), c->stream));
-      RR_G_TRY(g, cudaMemcpyPeerAsync(g->f_nsamp[i], c0->device, c->d_nsamples, c->device, px * sizeof(float), c->stream));
-      pv.step[i] = g->f_step[i]; pv.rgba[i] = g->f_rgba[i]; pv.zbuf[i] = g->f_zbuf[i]; pv.nsamp[i] = g->f_nsamp[i];
+      RR_G_TRY(g, cudaMemcpyPeerAsync(f.step.ptr, c0->device, c->d_step.ptr, c->device, px * sizeof(uint32_t), c->stream));
+      RR_G_TRY(g, cudaMemcpyPeerAsync(f.rgba.ptr, c0->device, c->d_rgba.ptr, c->device, px * sizeof(float4), c->stream));
+      RR_G_TRY(g, cudaMemcpyPeerAsync(f.zbuf.ptr, c0->device, c->d_zbuf.ptr, c->device, px * sizeof(float), c->stream));
+      RR_G_TRY(g, cudaMemcpyPeerAsync(f.nsamp.ptr, c0->device, c->d_nsamples.ptr, c->device, px * sizeof(float), c->stream));
+      pv.step[i] = f.step.ptr; pv.rgba[i] = f.rgba.ptr; pv.zbuf[i] = f.zbuf.ptr; pv.nsamp[i] = f.nsamp.ptr;
     } else {
-      pv.step[i] = c->d_step; pv.rgba[i] = c->d_rgba; pv.zbuf[i] = c->d_zbuf; pv.nsamp[i] = c->d_nsamples;
+      pv.step[i] = c->d_step.ptr; pv.rgba[i] = c->d_rgba.ptr; pv.zbuf[i] = c->d_zbuf.ptr; pv.nsamp[i] = c->d_nsamples.ptr;
     }
     if (i > 0) {
       RR_G_TRY(g, cudaSetDevice(c->device));
@@ -443,7 +444,7 @@ int rr_group_raymarch(rr_group* g, const rr_view* view, float* out_rgba, float* 
   RR_G_TRY(g, cudaSetDevice(c0->device));
   for (size_t i = 1; i < n; ++i) RR_G_TRY(g, cudaStreamWaitEvent(c0->stream, g->ev_view[i], 0));
   rr::timer_begin(c0, "composite");
-  rr::k_composite_peers<<<(unsigned)((px + 255) / 256), 256, 0, c0->stream>>>(pv, (int)px, c0->d_rgba, c0->d_zbuf, c0->d_step, c0->d_nsamples);
+  rr::k_composite_peers<<<(unsigned)((px + 255) / 256), 256, 0, c0->stream>>>(pv, (int)px, c0->d_rgba.ptr, c0->d_zbuf.ptr, c0->d_step.ptr, c0->d_nsamples.ptr);
   ++c0->launches;
   RR_G_TRY(g, cudaGetLastError());
   rr::timer_end(c0, "composite");
@@ -454,10 +455,8 @@ int rr_group_raymarch(rr_group* g, const rr_view* view, float* out_rgba, float* 
     RR_G_TRY(g, cudaStreamWaitEvent(g->m[i]->stream, g->ev_view[0], 0));
   }
   RR_G_TRY(g, cudaSetDevice(c0->device));
-  if (out_rgba) RR_G_TRY(g, cudaMemcpyAsync(out_rgba, c0->d_rgba, px * sizeof(float4), cudaMemcpyDeviceToHost, c0->stream));
-  if (out_depth) RR_G_TRY(g, cudaMemcpyAsync(out_depth, c0->d_zbuf, px * sizeof(float), cudaMemcpyDeviceToHost, c0->stream));
-  if (out_rgba || out_depth) RR_G_TRY(g, cudaStreamSynchronize(c0->stream));
-  return RR_OK;
+  const int rc = rr::view_download(c0, out_rgba, out_depth, "rr_group_raymarch");
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
 }
 
 int rr_group_fill_colors(rr_group* g, float* out_rgba) {
@@ -476,7 +475,7 @@ int rr_view_export(rr_ctx* c, int width, int height, void* out_handle) {
   RR_TRY_RC(ensure_view(c, width, height));
   cudaIpcMemHandle_t h[4];
   static_assert(sizeof(h) == RR_VIEW_HANDLE_BYTES, "four IPC handles");
-  void* ptrs[4] = {c->d_step, c->d_rgba, c->d_zbuf, c->d_nsamples};
+  void* ptrs[4] = {c->d_step.ptr, c->d_rgba.ptr, c->d_zbuf.ptr, c->d_nsamples.ptr};
   for (int i = 0; i < 4; ++i) {
     const cudaError_t e = cudaIpcGetMemHandle(&h[i], ptrs[i]);
     if (e != cudaSuccess) return rr::check(c, e, "rr_view_export: cudaIpcGetMemHandle");
@@ -487,12 +486,12 @@ int rr_view_export(rr_ctx* c, int width, int height, void* out_handle) {
 
 int rr_composite_peers(rr_ctx* c, const void* peer_handles, int n_peers, int width, int height, float* out_rgba, float* out_depth) {
   if (!c) return RR_ERR_INVALID;
-  if (n_peers < 0 || n_peers >= RR_MAX_GROUP || (n_peers > 0 && !peer_handles) || width != c->view_w || height != c->view_h || !c->d_step)
+  if (n_peers < 0 || n_peers >= RR_MAX_GROUP || (n_peers > 0 && !peer_handles) || width != c->view_w || height != c->view_h || !c->d_step.ptr)
     return rr::fail(c, RR_ERR_INVALID, "rr_composite_peers: march this context's own view at this size first; at most 15 peers");
   if (cudaSetDevice(c->device) != cudaSuccess) return rr::check(c, cudaGetLastError(), "rr_composite_peers");
   rr::PeerViews pv{};
   pv.n = n_peers + 1;
-  pv.step[0] = c->d_step; pv.rgba[0] = c->d_rgba; pv.zbuf[0] = c->d_zbuf; pv.nsamp[0] = c->d_nsamples;
+  pv.step[0] = c->d_step.ptr; pv.rgba[0] = c->d_rgba.ptr; pv.zbuf[0] = c->d_zbuf.ptr; pv.nsamp[0] = c->d_nsamples.ptr;
   for (int p = 0; p < n_peers; ++p) {
     const std::string key(static_cast<const char*>(peer_handles) + (size_t)p * RR_VIEW_HANDLE_BYTES, RR_VIEW_HANDLE_BYTES);
     const rr_ctx::IpcView* v = nullptr;
@@ -515,13 +514,10 @@ int rr_composite_peers(rr_ctx* c, const void* peer_handles, int n_peers, int wid
   }
   const size_t px = (size_t)width * height;
   rr::timer_begin(c, "composite");
-  rr::k_composite_peers<<<(unsigned)((px + 255) / 256), 256, 0, c->stream>>>(pv, (int)px, c->d_rgba, c->d_zbuf, c->d_step, c->d_nsamples);
+  rr::k_composite_peers<<<(unsigned)((px + 255) / 256), 256, 0, c->stream>>>(pv, (int)px, c->d_rgba.ptr, c->d_zbuf.ptr, c->d_step.ptr, c->d_nsamples.ptr);
   RR_LAUNCH_CHECK(c, "k_composite_peers");
   rr::timer_end(c, "composite");
-  if (out_rgba) RR_TRY_RC(rr::check(c, cudaMemcpyAsync(out_rgba, c->d_rgba, px * sizeof(float4), cudaMemcpyDeviceToHost, c->stream), "rgba download"));
-  if (out_depth) RR_TRY_RC(rr::check(c, cudaMemcpyAsync(out_depth, c->d_zbuf, px * sizeof(float), cudaMemcpyDeviceToHost, c->stream), "depth download"));
-  if (out_rgba || out_depth) RR_TRY_RC(rr::check(c, cudaStreamSynchronize(c->stream), "composite sync"));
-  return RR_OK;
+  return rr::view_download(c, out_rgba, out_depth, "rr_composite_peers");
 }
 
 // Member 0 receives every other member's owned slices by peer copies (one volume over NVLink per call), so that it holds
@@ -549,7 +545,7 @@ static int group_gather_volume(rr_group* g, const std::string& who, bool need_ca
     RR_G_TRY(g, cudaStreamWaitEvent(c0->stream, g->ev_view[i], 0));
     const size_t z0 = g->bounds[i], z1 = g->bounds[i + 1];
     if (z1 > z0)
-      RR_G_TRY(g, cudaMemcpyPeerAsync(c0->d_tsdf + plane * z0, c0->device, c->d_tsdf + plane * z0, c->device, plane * (z1 - z0) * sizeof(float), c0->stream));
+      RR_G_TRY(g, cudaMemcpyPeerAsync(c0->d_tsdf.ptr + plane * z0, c0->device, c->d_tsdf.ptr + plane * z0, c->device, plane * (z1 - z0) * sizeof(float), c0->stream));
   }
   RR_G_TRY(g, cudaSetDevice(c0->device));
   return RR_OK;
@@ -660,7 +656,7 @@ int rr_group_download_tsdf(rr_group* g, float* out) {
     rr_ctx* c = g->m[i];
     RR_G_TRY(g, cudaSetDevice(c->device));
     const size_t z0 = g->bounds[i], z1 = g->bounds[i + 1];
-    RR_G_TRY(g, cudaMemcpyAsync(out + plane * z0, c->d_tsdf + plane * z0, plane * (z1 - z0) * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    RR_G_TRY(g, cudaMemcpyAsync(out + plane * z0, c->d_tsdf.ptr + plane * z0, plane * (z1 - z0) * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   }
   const int rc = rr_group_synchronize(g);
   if (rc != RR_OK || g->m[0]->cfg.store_weight != RR_VOXELS_HALF2) return rc;

@@ -58,14 +58,14 @@ __global__ void __launch_bounds__(256) k_depth8(const uint8_t* __restrict__ in, 
 int launch_unpack_frames(rr_ctx* c, int slot) {
   if (c->color_format == RR_COLOR_DXT1 || c->color_format == RR_COLOR_DXT5) {
     const dim3 blk(32, 8, 1), grd((c->CW / 4 + 31) / 32, (c->CH / 4 + 7) / 8, c->N);
-    const uint2* src = reinterpret_cast<const uint2*>(c->d_color_packed[slot]);
-    if (c->color_format == RR_COLOR_DXT5) k_decode_dxt<true><<<grd, blk, 0, c->stream>>>(src, c->d_color_slot[slot], c->CW, c->CH);
-    else k_decode_dxt<false><<<grd, blk, 0, c->stream>>>(src, c->d_color_slot[slot], c->CW, c->CH);
+    const uint2* src = reinterpret_cast<const uint2*>(c->d_color_packed[slot].ptr);
+    if (c->color_format == RR_COLOR_DXT5) k_decode_dxt<true><<<grd, blk, 0, c->stream>>>(src, c->d_color_slot[slot].ptr, c->CW, c->CH);
+    else k_decode_dxt<false><<<grd, blk, 0, c->stream>>>(src, c->d_color_slot[slot].ptr, c->CW, c->CH);
     RR_LAUNCH_CHECK(c, "k_decode_dxt");
   }
   if (c->depth_format == RR_DEPTH_U8) {
     const size_t n = (size_t)c->N * c->W * c->H;
-    k_depth8<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->d_depth_packed[slot], c->d_depth_slot[slot], n);
+    k_depth8<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->d_depth_packed[slot].ptr, c->d_depth_slot[slot].ptr, n);
     RR_LAUNCH_CHECK(c, "k_depth8");
   }
   return RR_OK;

@@ -194,9 +194,9 @@ Tunables& tunables() {
 
 void setup_fill(const rr_ctx* c, const IntegrateParams& p, int mode, int fill_rows, FusedParams& f) {
   f.ip = p;
-  f.rowmask = c->d_rowmask; f.rowany = c->d_rowany; f.cand_y = c->d_cand_y; f.cand_z = c->d_cand_z;
+  f.rowmask = c->d_rowmask.ptr; f.rowany = c->d_rowany.ptr; f.cand_y = c->d_cand_y.ptr; f.cand_z = c->d_cand_z.ptr;
   f.mask_words = c->mask_words; f.nby = (int)c->bricks.res[1];
-  f.work = c->d_work;
+  f.work = c->d_work.ptr;
   f.fill_rows = std::min(32, std::max(1, fill_rows));
   f.row_begin = (uint32_t)p.z_begin * (uint32_t)p.Y; f.row_end = (uint32_t)p.z_end * (uint32_t)p.Y;
   f.fill_items = (f.row_end - f.row_begin + (uint32_t)f.fill_rows - 1u) / (uint32_t)f.fill_rows;
@@ -251,7 +251,7 @@ static int launch_n(rr_ctx* c, const IntegrateParams& p, bool bricks, int mode, 
       f.fill_warps = tn.fill_warps;
       // chunk <= 0: one z-chunk of one brick (all its column blocks) per draw
       f.chunk = tn.chunk > 0 ? tn.chunk : (max_cols + 31) / 32;
-      cudaMemsetAsync(c->d_work, 0, 4 * sizeof(uint32_t), c->stream);
+      cudaMemsetAsync(c->d_work.ptr, 0, 4 * sizeof(uint32_t), c->stream);
       const dim3 grd(148 * std::min(2, std::max(1, tn.ctas)), 1, 1);
       c->last_integrate[0] = 2;
       c->last_integrate[3] = N > 4 ? 256u : (mode == 0 && tn.threads != 384 ? 512u : 384u);
@@ -285,10 +285,9 @@ static int launch_n(rr_ctx* c, const IntegrateParams& p, bool bricks, int mode, 
 // (k0, k1, g, 1-g) of every fine z against the inverse volume's z axis; rebuilt when either resolution changes
 int build_ztab(rr_ctx* c) {
   const int Z = (int)c->res[2], IZ = (int)c->ires[2];
-  if (c->d_ztab && c->ztab_Z == Z && c->ztab_IZ == IZ) return RR_OK;
-  if (c->d_ztab) { cudaStreamSynchronize(c->stream); cudaFree(c->d_ztab); c->d_ztab = nullptr; }
-  if (cudaMalloc((void**)&c->d_ztab, sizeof(float4) * (size_t)Z) != cudaSuccess) return fail(c, RR_ERR_CUDA, "integrate: z table allocation failed");
-  k_build_ztab<<<(Z + 127) / 128, 128, 0, c->stream>>>(c->d_ztab, Z, IZ);
+  if (c->d_ztab.ptr && c->ztab_Z == Z && c->ztab_IZ == IZ) return RR_OK;
+  RR_TRY_RC(c->d_ztab.allocate(c, (size_t)Z, "integrate: z table"));
+  k_build_ztab<<<(Z + 127) / 128, 128, 0, c->stream>>>(c->d_ztab.ptr, Z, IZ);
   RR_LAUNCH_CHECK(c, "k_build_ztab");
   c->ztab_Z = Z; c->ztab_IZ = IZ;
   return RR_OK;
@@ -296,8 +295,8 @@ int build_ztab(rr_ctx* c) {
 
 int launch_integrate(rr_ctx* c) {
   IntegrateParams p{};
-  p.inv = c->d_inv; p.gather = c->d_gather; p.tsdf = c->d_tsdf; p.weight = c->d_weight;
-  p.ranges = c->d_ranges; p.occupied = c->d_occupied; p.num_occupied = c->d_num_occ;
+  p.inv = c->d_inv.ptr; p.gather = c->d_gather.ptr; p.tsdf = c->d_tsdf.ptr; p.weight = c->d_weight.ptr;
+  p.ranges = c->d_ranges.ptr; p.occupied = c->d_occupied.ptr; p.num_occupied = c->d_num_occ.ptr;
   p.IX = (int)c->ires[0]; p.IY = (int)c->ires[1]; p.IZ = (int)c->ires[2];
   p.W = c->W; p.H = c->H; p.X = (int)c->res[0]; p.Y = (int)c->res[1]; p.Z = (int)c->res[2];
   p.z_begin = (int)c->slab_z0; p.z_end = (int)c->slab_z1;
@@ -313,8 +312,8 @@ int launch_integrate(rr_ctx* c) {
   p.z_chunk = 32;
   p.fW = (float)c->W; p.fH = (float)c->H; p.exmax = (float)(c->W - 1); p.eymax = (float)(c->H - 1);
   RR_TRY_RC(build_ztab(c));
-  p.ztab = c->d_ztab;
-  p.pairs = c->d_pairs; p.pair_pitch = c->pair_pitch;
+  p.ztab = c->d_ztab.ptr;
+  p.pairs = c->d_pairs.ptr; p.pair_pitch = c->pair_pitch;
   p.limit = c->cfg.limit;
   p.wide_loads = tunables().ldg256;
   const int mode = c->cfg.store_weight == RR_VOXELS_HALF2 ? 2 : (c->cfg.store_weight != 0 ? 1 : 0);
@@ -340,11 +339,11 @@ int launch_integrate(rr_ctx* c) {
   if (!done && rc == RR_OK) {
     if (bricks && !fused && nslab) {
       // dense mode overwrites every voxel, so only the brick path needs the clear
-      float* t0 = c->d_tsdf + plane * p.z_begin;
+      float* t0 = c->d_tsdf.ptr + plane * p.z_begin;
       k_fill<<<148 * 8, 256, 0, c->stream>>>(t0, nslab, cleared_voxel(mode, p.limit));
       RR_LAUNCH_CHECK(c, "k_fill");
       if (weight) {
-        k_fill<<<148 * 8, 256, 0, c->stream>>>(c->d_weight + plane * p.z_begin, nslab, 0.0f);
+        k_fill<<<148 * 8, 256, 0, c->stream>>>(c->d_weight.ptr + plane * p.z_begin, nslab, 0.0f);
         RR_LAUNCH_CHECK(c, "k_fill");
       }
     }

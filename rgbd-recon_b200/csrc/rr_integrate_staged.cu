@@ -20,6 +20,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstring>
+#include <utility>
 #include <vector>
 
 // Role-level cycle counters (rr_integrator_profile): compiled in only for `make prof` (librr_b200_prof.so), so that the
@@ -623,13 +624,6 @@ static int footprints(rr_ctx* c, const IntegrateParams& p, int cy, int cz, int n
   return RR_OK;
 }
 
-void staged_release(rr_ctx* c) {
-  cudaFree(c->sti.d_fp); cudaFree(c->sti.d_list); cudaFree(c->sti.d_err); cudaFree(c->sti.d_zr);
-  c->sti.d_fp = nullptr; c->sti.d_list = nullptr; c->sti.d_err = nullptr; c->sti.d_zr = nullptr;
-  c->sti.ok = false; c->sti.dirty = true;
-  c->sti.lists_key = 0;
-}
-
 uint64_t staged_lists_key(const rr_ctx* c) {
   uint32_t limit;
   std::memcpy(&limit, &c->cfg.limit, sizeof(limit));
@@ -653,8 +647,8 @@ bool staged_selected(const rr_ctx* c) {
 bool staged_classify_params(const rr_ctx* c, ClassifyParams& q) {
   if (!staged_selected(c)) return false;
   const auto& st = c->sti;
-  q.fp = st.d_fp; q.zr = st.d_zr; q.pairs = c->d_pairs; q.pair_pitch = c->pair_pitch; q.H2 = c->H + 2;
-  q.list = st.d_list; q.class_count = c->d_counters + c->bricks.num; q.list_stride = st.list_stride;
+  q.fp = st.d_fp.ptr; q.zr = st.d_zr.ptr; q.pairs = c->d_pairs.ptr; q.pair_pitch = c->pair_pitch; q.H2 = c->H + 2;
+  q.list = st.d_list.ptr; q.class_count = c->d_counters.ptr + c->bricks.num; q.list_stride = st.list_stride;
   q.per_brick = st.n_yc * st.n_zc; q.N = c->N; q.limit = c->cfg.limit;
   return true;
 }
@@ -672,7 +666,7 @@ int staged_prepare(rr_ctx* c) {
   st.n_oversize = 0;
   // declined before any table is built: stay dirty, so that returning to the current tunables rebuilds the tables
   st.dirty = true;
-  if (!c->configured || !c->cfg.use_bricks || !c->fused_ok || !tn.staged || !tn.fused || !c->d_inv) return RR_OK;
+  if (!c->configured || !c->cfg.use_bricks || !c->fused_ok || !tn.staged || !tn.fused || !c->d_inv.ptr) return RR_OK;
   for (int i = 0; i < c->N; ++i) if (!c->have_inv[i]) return RR_OK;
   st.dirty = false;
   st.generation = staged_key();
@@ -748,23 +742,26 @@ int staged_prepare(rr_ctx* c) {
 
   // footprints of every item of the brick grid
   IntegrateParams p{};
-  p.inv = c->d_inv; p.ranges = c->d_ranges;
+  p.inv = c->d_inv.ptr; p.ranges = c->d_ranges.ptr;
   p.IX = IX; p.IY = IY; p.IZ = IZ; p.W = c->W; p.H = c->H; p.X = X; p.Y = Y; p.Z = Z;
   p.fW = (float)c->W; p.fH = (float)c->H; p.exmax = (float)(c->W - 1); p.eymax = (float)(c->H - 1);
   RR_TRY_RC(build_ztab(c));
-  p.ztab = c->d_ztab;
+  p.ztab = c->d_ztab.ptr;
   const size_t items = nb * (size_t)n_yc * n_zc;
   if (items == 0 || items > 0x3fffffffull) return RR_OK;
-  int4* d_ext = nullptr;
-  float2* d_zr = nullptr;
-  if (cudaMalloc((void**)&d_ext, items * N * sizeof(int4)) != cudaSuccess) { cudaGetLastError(); return RR_OK; }
-  if (cudaMalloc((void**)&d_zr, items * N * sizeof(float2)) != cudaSuccess) { cudaGetLastError(); cudaFree(d_ext); return RR_OK; }
-  int rc = footprints(c, p, cy, cz, n_yc, n_zc, d_ext, d_zr, (uint32_t)items);
   std::vector<int4> ext(items * N);
-  if (rc == RR_OK) rc = check(c, cudaMemcpyAsync(ext.data(), d_ext, ext.size() * sizeof(int4), cudaMemcpyDeviceToHost, c->stream), "footprint download");
-  if (rc == RR_OK) rc = check(c, cudaStreamSynchronize(c->stream), "footprint sync");
-  cudaFree(d_ext);
-  if (rc != RR_OK) { cudaFree(d_zr); return rc; }
+  DeviceArray<float2> d_zr;
+  {
+    DeviceArray<int4> d_ext;
+    // a failed allocation declines: the direct kernels run
+    if (d_ext.allocate(c, items * N, "footprint extents") != RR_OK || d_zr.allocate(c, items * N, "footprint z ranges") != RR_OK) {
+      cudaGetLastError();
+      return RR_OK;
+    }
+    RR_TRY_RC(footprints(c, p, cy, cz, n_yc, n_zc, d_ext.ptr, d_zr.ptr, (uint32_t)items));
+    RR_TRY_RC(check(c, cudaMemcpyAsync(ext.data(), d_ext.ptr, ext.size() * sizeof(int4), cudaMemcpyDeviceToHost, c->stream), "footprint download"));
+    RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "footprint sync"));
+  }
   // Tile edge: a smaller tile leaves more slots in the ring (more items in flight), a larger one sends fewer (item, sensor)
   // pairs to the global-memory path, which costs several times a staged item: the largest tile that keeps two items' worth
   // of slots plus one, and no larger than the largest footprint of the grid.
@@ -772,7 +769,7 @@ int staged_prepare(rr_ctx* c) {
   need.reserve(ext.size());
   for (const int4& e : ext)
     if (e.z >= e.x) need.push_back(std::max(e.z - (e.x & ~1), e.w - e.y) + 2);
-  if (need.empty()) { cudaFree(d_zr); return RR_OK; }
+  if (need.empty()) return RR_OK;
   std::sort(need.begin(), need.end());
   auto even = [](long v) { return (v + 1) & ~1L; };
   long T;
@@ -784,7 +781,7 @@ int staged_prepare(rr_ctx* c) {
   T = std::max(T, 8L);
   const long slot_bytes = slot_bytes_for(T);
   const long n_slots = std::min(budget / slot_bytes, 64L);
-  if (n_slots < N) { cudaFree(d_zr); return RR_OK; }
+  if (n_slots < N) return RR_OK;
   std::vector<uint2> fp(items * N, make_uint2(0u, 0u));
   for (size_t i = 0; i < items; ++i)
     for (int s = 0; s < N; ++s) {
@@ -797,17 +794,16 @@ int staged_prepare(rr_ctx* c) {
       fp[i * N + s] = make_uint2((uint32_t)(e.x & ~1) | ((uint32_t)e.y << 16), rx | over | (rw << 8) | (rh << 20));
       st.n_oversize += over ? 1u : 0u;
     }
-  staged_release(c);
-  st.dirty = false;
+  st.lists_key = 0;
   ++st.tables;
-  st.d_zr = d_zr;
+  st.d_zr = std::move(d_zr);
   st.list_stride = (uint32_t)items;
-  RR_TRY_RC(check(c, cudaMalloc((void**)&st.d_list, (size_t)(N + 1) * items * sizeof(uint2)), "item lists"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&st.d_fp, fp.size() * sizeof(uint2)), "footprint table"));
-  RR_TRY_RC(check(c, cudaMalloc((void**)&st.d_err, 4 * sizeof(uint32_t) + 16 * sizeof(unsigned long long)), "staged flags"));
-  cudaMemcpyAsync(st.d_fp, fp.data(), fp.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream);
-  cudaMemsetAsync(st.d_err, 0, 4 * sizeof(uint32_t) + 16 * sizeof(unsigned long long), c->stream);
-  cudaMemsetAsync(c->d_counters + nb, 0, RR_CLASS_COUNTERS * sizeof(uint32_t), c->stream);
+  RR_TRY_RC(st.d_list.allocate(c, (size_t)(N + 1) * items, "item lists"));
+  RR_TRY_RC(st.d_fp.allocate(c, fp.size(), "footprint table"));
+  RR_TRY_RC(st.d_err.allocate(c, 4 + 16 * sizeof(unsigned long long) / sizeof(uint32_t), "staged flags"));
+  cudaMemcpyAsync(st.d_fp.ptr, fp.data(), fp.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream);
+  cudaMemsetAsync(st.d_err.ptr, 0, 4 * sizeof(uint32_t) + 16 * sizeof(unsigned long long), c->stream);
+  cudaMemsetAsync(c->d_counters.ptr + nb, 0, RR_CLASS_COUNTERS * sizeof(uint32_t), c->stream);
   RR_TRY_RC(check(c, cudaStreamSynchronize(c->stream), "staged tables upload"));
 
   // tensor maps: inverse volumes as (xyzw, IX, IY, IZ, N) float32 with a one-sensor box, pair image as (pitch, H+2, N) 8-byte pixels.
@@ -817,7 +813,7 @@ int staged_prepare(rr_ctx* c) {
     const cuuint64_t strides[4] = {16, (cuuint64_t)IX * 16, (cuuint64_t)IX * IY * 16, (cuuint64_t)IX * IY * IZ * 16};
     const cuuint32_t box[5] = {4, (cuuint32_t)BX, (cuuint32_t)BY, (cuuint32_t)BZ, 1};
     const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    if (enc(&st.map_inv, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, c->d_inv, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    if (enc(&st.map_inv, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, c->d_inv.ptr, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) return RR_OK;
   }
   {
@@ -825,7 +821,7 @@ int staged_prepare(rr_ctx* c) {
     const cuuint64_t strides[2] = {(cuuint64_t)c->pair_pitch * 8, (cuuint64_t)c->pair_pitch * (c->H + 2) * 8};
     const cuuint32_t box[3] = {(cuuint32_t)T, (cuuint32_t)T, 1};
     const cuuint32_t es[3] = {1, 1, 1};
-    if (enc(&st.map_pairs, CU_TENSOR_MAP_DATA_TYPE_INT64, 3, c->d_pairs, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    if (enc(&st.map_pairs, CU_TENSOR_MAP_DATA_TYPE_INT64, 3, c->d_pairs.ptr, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) return RR_OK;
   }
   st.cy = cy; st.cz = cz; st.n_yc = n_yc; st.n_zc = n_zc;
@@ -857,12 +853,12 @@ int launch_integrate_staged(rr_ctx* c, const IntegrateParams& p, int mode, bool*
   setup_fill(c, p, mode, tunables().stage_fill_rows, sp.f);
   sp.cy = st.cy; sp.cz = st.cz; sp.n_yc = st.n_yc; sp.n_zc = st.n_zc;
   sp.BX = st.BX; sp.BY = st.BY; sp.BZ = st.BZ; sp.T = st.T;
-  sp.fp = st.d_fp;
-  sp.list = st.d_list; sp.class_count = c->d_counters + c->bricks.num; sp.list_stride = st.list_stride;
+  sp.fp = st.d_fp.ptr;
+  sp.list = st.d_list.ptr; sp.class_count = c->d_counters.ptr + c->bricks.num; sp.list_stride = st.list_stride;
   sp.inv_bytes = st.inv_bytes; sp.tile_bytes = st.tile_bytes; sp.inv_span = st.inv_span;
   sp.slot_bytes = st.slot_bytes; sp.n_slots = st.n_slots; sp.slots_off = st.slots_off;
-  sp.err = st.d_err;
-  sp.prof = (tunables().stage_debug & 128) ? reinterpret_cast<unsigned long long*>(st.d_err + 4) : nullptr;
+  sp.err = st.d_err.ptr;
+  sp.prof = (tunables().stage_debug & 128) ? reinterpret_cast<unsigned long long*>(st.d_err.ptr + 4) : nullptr;
   sp.fill_src_off = st.fill_src_off; sp.fill_src_bytes = st.fill_src_bytes;
   sp.tables_off = st.tables_off; sp.n_rowany = c->bricks.res[1] * c->bricks.res[2];
   if (tunables().stage_debug & 1) sp.f.fill_items = 0;
@@ -871,7 +867,7 @@ int launch_integrate_staged(rr_ctx* c, const IntegrateParams& p, int mode, bool*
   sp.tail_cap = tunables().stage_tail_cap;
   // The work counters are reset and this frame's item lists written by k_bricks_update; a second integrate of the same
   // frame set (another slab, a repeated call) finds the lists intact and only needs fresh counters.
-  if (!c->work_fresh) cudaMemsetAsync(c->d_work, 0, 4 * sizeof(uint32_t), c->stream);
+  if (!c->work_fresh) cudaMemsetAsync(c->d_work.ptr, 0, 4 * sizeof(uint32_t), c->stream);
   c->work_fresh = false;
   int rc;
   switch (c->N) {

@@ -163,12 +163,12 @@ __device__ __forceinline__ void march_ray(const P& p, float3 cam, float3 dir, Do
 template <class P>
 inline void set_sample_params(P& p, const rr_ctx* c) {
   p.half2 = c->cfg.store_weight == RR_VOXELS_HALF2 ? 1 : 0;
-  p.tsdf = c->d_tsdf; p.X = (int)c->res[0]; p.Y = (int)c->res[1]; p.Z = (int)c->res[2];
+  p.tsdf = c->d_tsdf.ptr; p.X = (int)c->res[0]; p.Y = (int)c->res[1]; p.Z = (int)c->res[2];
   p.limit = c->cfg.limit;
-  p.N = c->N; p.inv = c->d_inv; p.IX = (int)c->ires[0]; p.IY = (int)c->ires[1]; p.IZ = (int)c->ires[2];
-  for (int i = 0; i < c->N; ++i) { p.uv[i] = c->d_uv[i]; p.cx[i] = (int)c->cres[i][0]; p.cy[i] = (int)c->cres[i][1]; p.cz[i] = (int)c->cres[i][2]; }
+  p.N = c->N; p.inv = c->d_inv.ptr; p.IX = (int)c->ires[0]; p.IY = (int)c->ires[1]; p.IZ = (int)c->ires[2];
+  for (int i = 0; i < c->N; ++i) { p.uv[i] = c->d_uv[i].ptr; p.cx[i] = (int)c->cres[i][0]; p.cy[i] = (int)c->cres[i][1]; p.cz[i] = (int)c->cres[i][2]; }
   p.color = c->d_color; p.CW = c->CW; p.CH = c->CH;
-  p.depth_b = c->d_depth_b; p.quality = c->d_quality; p.W = c->W; p.H = c->H;
+  p.depth_b = c->d_depth_b.ptr; p.quality = c->d_quality.ptr; p.W = c->W; p.H = c->H;
 }
 
 // The march fields of P (after set_sample_params) as rr_raymarch sets them from the context's current settings and brick tables.
@@ -177,7 +177,7 @@ inline void set_march_params(P& p, const rr_ctx* c) {
   const float dx = c->bbox_max[0] - c->bbox_min[0], dy = c->bbox_max[1] - c->bbox_min[1], dz = c->bbox_max[2] - c->bbox_min[2];
   const bool grid_ok = c->bricks.num == c->bricks.res[0] * c->bricks.res[1] * c->bricks.res[2];
   p.skip_space = (c->cfg.skip_space && c->cfg.use_bricks && grid_ok) ? 1 : 0;   // drawF: m_skip_space && m_use_bricks
-  p.occ_mask = c->d_occ_mask; p.near_occ = c->d_near_occ;
+  p.occ_mask = c->d_occ_mask.ptr; p.near_occ = c->d_near_occ.ptr;
   for (int a = 0; a < 3; ++a) p.rb[a] = (int)c->bricks.res[a];
   p.brick_size = c->bricks.brick_size;
   p.dims[0] = dx; p.dims[1] = dy; p.dims[2] = dz;

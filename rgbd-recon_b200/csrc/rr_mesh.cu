@@ -333,7 +333,7 @@ __global__ void __launch_bounds__(256) k_mesh_triangles(const __grid_constant__ 
 bool mesh_rows_usable(const rr_ctx* c) {
   const bool grid_ok = c->bricks.num == c->bricks.res[0] * c->bricks.res[1] * c->bricks.res[2];
   const uint32_t path = c->last_integrate[0];
-  return c->cfg.use_bricks && grid_ok && c->fused_ok && c->d_rowany && c->d_cand_y && c->d_cand_z && path >= 1 && path <= 3;
+  return c->cfg.use_bricks && grid_ok && c->fused_ok && c->d_rowany.ptr && c->d_cand_y.ptr && c->d_cand_z.ptr && path >= 1 && path <= 3;
 }
 
 int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt) {
@@ -355,17 +355,17 @@ int launch_extract_mesh(rr_ctx* c, uint32_t* out_nv, uint32_t* out_nt) {
   RR_TRY_RC(c->d_mesh_scratch.reserve(c, scan_bytes, "mesh scan scratch"));
 
   MeshParams p{};
-  p.tsdf = c->d_tsdf; p.X = X; p.Y = Y; p.Z = Z;
+  p.tsdf = c->d_tsdf.ptr; p.X = X; p.Y = Y; p.Z = Z;
   p.half2 = c->cfg.store_weight == RR_VOXELS_HALF2 ? 1 : 0;
   p.limit = c->cfg.limit;
-  p.N = c->N; p.inv = c->d_inv; p.IX = (int)c->ires[0]; p.IY = (int)c->ires[1]; p.IZ = (int)c->ires[2];
-  for (int i = 0; i < c->N; ++i) { p.uv[i] = c->d_uv[i]; p.cx[i] = (int)c->cres[i][0]; p.cy[i] = (int)c->cres[i][1]; p.cz[i] = (int)c->cres[i][2]; }
+  p.N = c->N; p.inv = c->d_inv.ptr; p.IX = (int)c->ires[0]; p.IY = (int)c->ires[1]; p.IZ = (int)c->ires[2];
+  for (int i = 0; i < c->N; ++i) { p.uv[i] = c->d_uv[i].ptr; p.cx[i] = (int)c->cres[i][0]; p.cy[i] = (int)c->cres[i][1]; p.cz[i] = (int)c->cres[i][2]; }
   p.color = c->d_color; p.CW = c->CW; p.CH = c->CH;
-  p.depth_b = c->d_depth_b; p.quality = c->d_quality; p.W = c->W; p.H = c->H;
+  p.depth_b = c->d_depth_b.ptr; p.quality = c->d_quality.ptr; p.W = c->W; p.H = c->H;
   for (int a = 0; a < 3; ++a) { p.bmin[a] = c->bbox_min[a]; p.size[a] = c->bbox_max[a] - c->bbox_min[a]; }
   p.use_rows = c->mesh_rows_ok ? 1 : 0;
   p.rby = (int)c->bricks.res[1];
-  p.rowany = c->d_rowany; p.cand_y = c->d_cand_y; p.cand_z = c->d_cand_z;
+  p.rowany = c->d_rowany.ptr; p.cand_y = c->d_cand_y.ptr; p.cand_z = c->d_cand_z.ptr;
   p.cnt_v = cnt_v; p.cnt_t = cnt_t; p.off_v = off_v; p.off_t = off_t;
 
   const unsigned row_blocks = (unsigned)((rows + 7) / 8);

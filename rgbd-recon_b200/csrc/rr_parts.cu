@@ -274,12 +274,12 @@ int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
   RR_TRY_RC(c->d_parts_scratch.reserve(c, scan_bytes, "part scan scratch"));
 
   PartsParams p{};
-  p.tsdf = c->d_tsdf; p.X = X; p.Y = Y; p.Z = Z;
+  p.tsdf = c->d_tsdf.ptr; p.X = X; p.Y = Y; p.Z = Z;
   p.half2 = c->cfg.store_weight == RR_VOXELS_HALF2 ? 1 : 0;
   p.L = c->d_parts_labels.ptr;
   p.use_rows = c->mesh_rows_ok ? 1 : 0;
   p.rby = (int)c->bricks.res[1]; p.mask_words = c->mask_words;
-  p.rowmask = c->d_rowmask; p.rowany = c->d_rowany; p.cand_y = c->d_cand_y; p.cand_z = c->d_cand_z;
+  p.rowmask = c->d_rowmask.ptr; p.rowany = c->d_rowany.ptr; p.cand_y = c->d_cand_y.ptr; p.cand_z = c->d_cand_z.ptr;
   p.cnt = cnt; p.off = off;
   for (int a = 0; a < 3; ++a) {
     p.bmin[a] = (double)c->bbox_min[a];

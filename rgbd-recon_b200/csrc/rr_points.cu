@@ -179,13 +179,13 @@ int launch_draw_points(rr_ctx* c, const rr_view* v, int mode, float calib_limit)
   p.vw = vw; p.vh = vh; p.shade_mode = v->shade_mode; p.mode = mode;
   p.N = c->N; p.W = c->W; p.H = c->H; p.CW = c->CW; p.CH = c->CH;
   p.st = sensor_tables(c);
-  p.depth_b = c->d_depth_b; p.normal = c->d_normal; p.color = c->d_color;
+  p.depth_b = c->d_depth_b.ptr; p.normal = c->d_normal.ptr; p.color = c->d_color;
   for (int a = 0; a < 3; ++a) { p.bmin[a] = c->bbox_min[a]; p.bmax[a] = c->bbox_max[a]; }
   p.IX = (int)c->ires[0]; p.IY = (int)c->ires[1]; p.IZ = (int)c->ires[2];
-  p.tsdf = c->d_tsdf; p.X = (int)c->res[0]; p.Y = (int)c->res[1]; p.Z = (int)c->res[2];
+  p.tsdf = c->d_tsdf.ptr; p.X = (int)c->res[0]; p.Y = (int)c->res[1]; p.Z = (int)c->res[2];
   p.half2 = c->cfg.store_weight == RR_VOXELS_HALF2 ? 1 : 0;
   p.limit = calib_limit;
-  p.keys = c->d_point_keys; p.out_rgba = c->d_rgba; p.out_depth = c->d_zbuf;
+  p.keys = c->d_point_keys.ptr; p.out_rgba = c->d_rgba.ptr; p.out_depth = c->d_zbuf.ptr;
   const uint32_t n_vertices = mode == 0 ? (uint32_t)c->N * c->W * c->H : (uint32_t)(p.IX * p.IY * p.IZ);
   const int npx = vw * vh;
   timer_begin(c, "3recon");

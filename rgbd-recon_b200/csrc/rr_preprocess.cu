@@ -542,7 +542,7 @@ int launch_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, i
   timer_begin(c, "1preprocess");
 
   timer_begin(c, "morph");
-  k_morph<<<grd, blk, 0, s>>>(c->d_depth_raw, c->d_morph, W, H);
+  k_morph<<<grd, blk, 0, s>>>(c->d_depth_raw, c->d_morph.ptr, W, H);
   RR_LAUNCH_CHECK(c, "k_morph");
   timer_end(c, "morph");
 
@@ -557,13 +557,13 @@ int launch_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, i
     dp.scale[i] = c->depth_far[i] - c->depth_near[i];
     dp.scaled_near[i] = dp.scale[i] / 255.0f;
   }
-  k_bilateral<<<grd, blk, 0, s>>>(use_processed_depth ? c->d_morph : c->d_depth_raw, c->d_color, c->d_depth, c->d_lab,
+  k_bilateral<<<grd, blk, 0, s>>>(use_processed_depth ? c->d_morph.ptr : c->d_depth_raw, c->d_color, c->d_depth.ptr, c->d_lab.ptr,
                                   W, H, c->CW, c->CH, st, dp);
   RR_LAUNCH_CHECK(c, "k_bilateral");
   timer_end(c, "bilateral");
 
   timer_begin(c, "boundary");
-  k_boundary<<<grd, blk, 0, s>>>(c->d_depth, c->d_lab, c->d_depth_b, c->d_sil, W, H, refine);
+  k_boundary<<<grd, blk, 0, s>>>(c->d_depth.ptr, c->d_lab.ptr, c->d_depth_b.ptr, c->d_sil.ptr, W, H, refine);
   RR_LAUNCH_CHECK(c, "k_boundary");
   timer_end(c, "boundary");
 
@@ -578,16 +578,16 @@ int launch_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, i
   c->gather_packed = false;
   if (tunables().fuse_nq) {
     timer_begin(c, "quality");
-    k_normal_quality<<<grd, blk, 0, s>>>(c->d_depth_b, c->d_normal, c->d_counters, c->d_quality, c->d_sil, c->d_pairs, c->pair_pitch,
-                                         c->d_flags, W, H, st, bp);
+    k_normal_quality<<<grd, blk, 0, s>>>(c->d_depth_b.ptr, c->d_normal.ptr, c->d_counters.ptr, c->d_quality.ptr, c->d_sil.ptr, c->d_pairs.ptr, c->pair_pitch,
+                                         c->d_flags.ptr, W, H, st, bp);
     RR_LAUNCH_CHECK(c, "k_normal_quality");
   } else {
     timer_begin(c, "normal");
-    k_normal<<<grd, blk, 0, s>>>(c->d_depth_b, c->d_normal, c->d_counters, W, H, st, bp);
+    k_normal<<<grd, blk, 0, s>>>(c->d_depth_b.ptr, c->d_normal.ptr, c->d_counters.ptr, W, H, st, bp);
     RR_LAUNCH_CHECK(c, "k_normal");
     timer_end(c, "normal");
     timer_begin(c, "quality");
-    k_quality<<<grd, blk, 0, s>>>(c->d_depth_b, c->d_normal, c->d_quality, c->d_sil, c->d_pairs, c->pair_pitch, c->d_flags, W, H, st);
+    k_quality<<<grd, blk, 0, s>>>(c->d_depth_b.ptr, c->d_normal.ptr, c->d_quality.ptr, c->d_sil.ptr, c->d_pairs.ptr, c->pair_pitch, c->d_flags.ptr, W, H, st);
     RR_LAUNCH_CHECK(c, "k_quality");
   }
   if (!staged) RR_TRY_RC(launch_pack_gather(c));
@@ -600,7 +600,7 @@ int launch_preprocess(rr_ctx* c, int filter_textures, int use_processed_depth, i
 int launch_pack_gather(rr_ctx* c) {
   const dim3 blk(TILE_X, TILE_Y, 1);
   const dim3 grd_g((c->W + 1 + TILE_X - 1) / TILE_X, (c->H + 1 + TILE_Y - 1) / TILE_Y, c->N);
-  k_pack_gather<<<grd_g, blk, 0, c->stream>>>(c->d_depth_b, c->d_quality, c->d_sil, c->d_gather, c->d_flags, c->W, c->H);
+  k_pack_gather<<<grd_g, blk, 0, c->stream>>>(c->d_depth_b.ptr, c->d_quality.ptr, c->d_sil.ptr, c->d_gather.ptr, c->d_flags.ptr, c->W, c->H);
   RR_LAUNCH_CHECK(c, "k_pack_gather");
   c->gather_packed = true;
   return RR_OK;

@@ -199,14 +199,14 @@ int launch_partial_keep(rr_ctx* c, float4* d_rec, const long long* d_keys_min, i
 
 int launch_pack_partial(rr_ctx* c, float4* d_rec) {
   const int n = c->view_w * c->view_h;
-  k_pack_partial<<<(n + 255) / 256, 256, 0, c->stream>>>(c->d_rgba, c->d_zbuf, c->d_step, c->d_nsamples, d_rec, n);
+  k_pack_partial<<<(n + 255) / 256, 256, 0, c->stream>>>(c->d_rgba.ptr, c->d_zbuf.ptr, c->d_step.ptr, c->d_nsamples.ptr, d_rec, n);
   RR_LAUNCH_CHECK(c, "k_pack_partial");
   return RR_OK;
 }
 
 int launch_composite(rr_ctx* c, const float4* d_rec, int n_parts) {
   const int n = c->view_w * c->view_h;
-  k_composite<<<(n + 255) / 256, 256, 0, c->stream>>>(d_rec, n_parts, n, c->d_rgba, c->d_zbuf, c->d_step, c->d_nsamples);
+  k_composite<<<(n + 255) / 256, 256, 0, c->stream>>>(d_rec, n_parts, n, c->d_rgba.ptr, c->d_zbuf.ptr, c->d_step.ptr, c->d_nsamples.ptr);
   RR_LAUNCH_CHECK(c, "k_composite");
   return RR_OK;
 }
@@ -281,7 +281,7 @@ int launch_raymarch(rr_ctx* c, const rr_view* v) {
   set_sample_params(p, c);
   p.vw = vw; p.vh = vh; p.shade_mode = v->shade_mode;
   set_march_params(p, c);
-  p.out_rgba = c->d_rgba; p.out_depth = c->d_zbuf; p.out_samples = c->d_nsamples; p.out_pos = c->d_pos; p.out_step = c->d_step;
+  p.out_rgba = c->d_rgba.ptr; p.out_depth = c->d_zbuf.ptr; p.out_samples = c->d_nsamples.ptr; p.out_pos = c->d_pos.ptr; p.out_step = c->d_step.ptr;
   timer_begin(c, "3recon");
   timer_begin(c, "draw");
   const dim3 blk(8, 8, 1), grd((vw + 7) / 8, (vh + 7) / 8, 1);

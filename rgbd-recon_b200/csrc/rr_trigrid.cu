@@ -293,7 +293,7 @@ int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length) {
   p.vw = vw; p.vh = vh; p.shade_mode = v->shade_mode;
   p.N = c->N; p.W = c->W; p.H = c->H; p.CW = c->CW; p.CH = c->CH;
   p.st = sensor_tables(c);
-  p.depth_b = c->d_depth_b; p.quality = c->d_quality; p.color = c->d_color;
+  p.depth_b = c->d_depth_b.ptr; p.quality = c->d_quality.ptr; p.color = c->d_color;
   for (int a = 0; a < 3; ++a) { p.bmin[a] = c->bbox_min[a]; p.bmax[a] = c->bbox_max[a]; }
   p.min_length = min_length; p.epsilon = 0.075f;                       // recon_trigrid.cpp:35
   const size_t n_vertices = (size_t)c->N * (c->W + 1) * (c->H + 1), n_triangles = (size_t)c->N * c->W * c->H * 2;
@@ -303,7 +303,7 @@ int launch_draw_trigrid(rr_ctx* c, const rr_view* v, float min_length) {
   RR_TRY_RC(c->d_tg_head.reserve(c, (size_t)npx, "trigrid list heads"));
   RR_TRY_RC(c->d_tg_count.reserve(c, 1, "trigrid counter"));
   p.verts = c->d_tg_verts.ptr; p.depth1 = c->d_tg_depth.ptr; p.head = c->d_tg_head.ptr; p.frag_count = c->d_tg_count.ptr;
-  p.out_rgba = c->d_rgba; p.out_depth = c->d_zbuf;
+  p.out_rgba = c->d_rgba.ptr; p.out_depth = c->d_zbuf.ptr;
   timer_begin(c, "3recon");
   timer_begin(c, "draw");
   k_tg_clear<<<(npx + 255) / 256, 256, 0, c->stream>>>(p.depth1, p.head, p.frag_count, npx);

@@ -511,8 +511,15 @@ int rr_integrator_info(rr_ctx* ctx, uint32_t* out);
  *  [3] CTA threads, or consumer warps of the staged kernel;
  *  [4] repairs: bit 0 the staged kernel declined because its item lists were not built for the current tables, limit and
  *      stage images (a direct kernel ran instead), bit 1 the gather texels were packed by this call because the last
- *      rr_preprocess had left them to the staged kernel; [5..7] 0. */
+ *      rr_preprocess had left them to the staged kernel;
+ *  [5] clear: 0 none (dense mode, or nothing launched), 1 the whole slab outside the occupied bricks, 2 incremental: only
+ *      the bricks that left the occupied set since the last integrate (the staged kernel, when the volume outside the
+ *      bricks that integrate evaluated is known to hold the cleared value); [6..7] 0. */
 int rr_integrator_last(const rr_ctx* ctx, uint32_t* out);
+/* Bricks the incremental clear of the last integrate reset to the cleared value (evaluated by the integrate before it, not
+ * occupied now); 0 when the last integrate did not clear incrementally. The count is kept by the device past later
+ * rr_bricks_update calls, until the next integrate. Waits for the stream. out[1]. */
+int rr_integrator_cleared(rr_ctx* ctx, uint32_t* out);
 /* Cycle counters of the staged integrator's warp roles, accumulated while the tunable "stage_debug" has bit 7 set and reset
  * by this call (diagnostics, no reference counterpart). out[16], SM clock cycles summed over warps / producer threads:
  *  [0] consumer warps waiting for a staged item, [1] evaluating one, [2] items a consumer warp had no columns of,

@@ -142,10 +142,11 @@ int rr_create(rr_ctx** out, int device, int num_sensors, int depth_w, int depth_
   if (rc == RR_OK) rc = c->d_pairs.allocate(c, (size_t)c->N * (c->H + 2) * c->pair_pitch, "pair image");
   if (rc == RR_OK) rc = c->d_flags.allocate(c, 4, "flags");
   if (rc == RR_OK) rc = c->d_num_occ.allocate(c, 1, "num_occ");
-  if (rc == RR_OK) rc = c->d_work.allocate(c, 4, "work counters");
+  if (rc == RR_OK) rc = c->d_work.allocate(c, 8, "work counters");
   if (rc == RR_OK) rc = check(c, cudaMallocHost((void**)&c->pinned, sizeof(rr::PinnedScalars)), "pinned scalars");
   if (rc == RR_OK) {
     cudaMemsetAsync(c->d_flags.ptr, 0, 4 * sizeof(uint32_t), c->stream);
+    cudaMemsetAsync(c->d_work.ptr, 0, 8 * sizeof(uint32_t), c->stream);
     cudaMemsetAsync(c->d_pairs.ptr, 0, (size_t)c->N * (c->H + 2) * c->pair_pitch * sizeof(float2), c->stream);
     cudaMemsetAsync(c->d_num_occ.ptr, 0, sizeof(uint32_t), c->stream);
     for (int b = 0; b < 2; ++b) {
@@ -313,6 +314,8 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     for (int a = 0; a < 3; ++a) c->res[a] = res[a];
     c->slab_z0 = 0; c->slab_z1 = res[2];
   }
+  // the incremental clear knows nothing about a new allocation, a new brick grid or a volume last written in another mode
+  if (new_bricks || !c->configured || cfg->store_weight != c->cfg.store_weight || cfg->use_bricks != c->cfg.use_bricks) c->clear.valid = false;
   if (new_volume || cfg->store_weight != c->cfg.store_weight) {   // a new volume allocation as far as extraction goes
     c->volume_integrated = false;
     c->mesh_valid = false;
@@ -335,6 +338,7 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     RR_TRY(c->d_occupied.allocate(c, nb, "occupied list"));
     RR_TRY(c->d_near_occ.allocate(c, nb, "near-occupied mask"));
     RR_TRY(c->d_occ_mask.allocate(c, nb, "occupied mask"));
+    RR_TRY(c->d_written.allocate(c, 2 * (size_t)nb, "written bricks"));
     // per-axis candidate bricks of every voxel index (bricks may overlap by a voxel, or leave a gap)
     c->mask_words = (int)((res[0] + 31) / 32);
     c->fused_ok = rb[0] <= 32767 && rb[1] <= 32767 && rb[2] <= 32767;
@@ -366,6 +370,7 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     cudaMemsetAsync(c->d_counters.ptr, 0, ((size_t)nb + RR_CLASS_COUNTERS) * sizeof(uint32_t), c->stream);
     cudaMemsetAsync(c->d_near_occ.ptr, 0, nb, c->stream);
     cudaMemsetAsync(c->d_occ_mask.ptr, 0, nb, c->stream);
+    cudaMemsetAsync(c->d_written.ptr, 0, 2 * (size_t)nb, c->stream);
     cudaMemsetAsync(c->d_num_occ.ptr, 0, sizeof(uint32_t), c->stream);
     c->pinned->num_occ = 0;
     RR_TRY(check(c, cudaStreamSynchronize(c->stream), "brick table upload"));
@@ -402,6 +407,7 @@ int rr_set_slab(rr_ctx* c, uint32_t z0, uint32_t z1) {
   RR_REQUIRE(c, c->configured, "rr_set_slab: call rr_configure first");
   RR_REQUIRE(c, z0 <= z1 && z1 <= c->res[2], "rr_set_slab: slab outside the volume");
   c->slab_z0 = z0; c->slab_z1 = z1;
+  c->clear.valid = false;
   return RR_OK;
 }
 
@@ -575,17 +581,26 @@ int rr_fuse_frame(rr_ctx* c, int filter_textures, int use_processed_depth, int r
   const bool ready = rr::tunables().graph != 0 && !c->graphs_broken && c->timing == 0 && c->d_ztab.ptr &&
                      c->ztab_Z == (int)c->res[2] && c->ztab_IZ == (int)c->ires[2];
   if (!ready) return frame_direct(c, f, p, r);
-  const uint64_t key = ((uint64_t)rr::tunables().generation << 8) | (uint64_t)(c->cur_slot << 3 | f << 2 | p << 1 | r);
+  // a graph captured with the incremental clear must not run while the volume needs the whole slab cleared, nor the other
+  // way round: whether the integrate clears incrementally is part of the key
+  const int inc = rr::clear_incremental(c) ? 1 : 0;
+  const uint64_t key = ((uint64_t)rr::tunables().generation << 8) | (uint64_t)(inc << 4 | c->cur_slot << 3 | f << 2 | p << 1 | r);
   for (auto& g : c->frame_graphs)
     if (g.key == key) {
       c->launches += g.launches;
       c->volume_integrated = true;                 // the captured frame ends with the integrate launch_integrate recorded
       ++c->volume_epoch;
+      c->clear = g.clear;
+      std::memcpy(c->last_integrate, g.last, sizeof(g.last));
       c->mesh_rows_ok = mesh_rows_usable(c);
       return check(c, cudaGraphLaunch(g.exec, c->stream), "frame graph launch");
     }
   if (c->frame_graphs.size() >= 16) drop_frame_graphs(c);          // stale tunable generations
   const uint64_t l0 = c->launches;
+  // a capture runs nothing: what launch_integrate records on the host while capturing must not survive a failed capture
+  const rr::ClearState clear0 = c->clear;
+  uint32_t last0[8];
+  std::memcpy(last0, c->last_integrate, sizeof(last0));
   if (cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
     cudaGetLastError();
     c->graphs_broken = true;
@@ -602,9 +617,12 @@ int rr_fuse_frame(rr_ctx* c, int filter_textures, int use_processed_depth, int r
   if (rc != RR_OK || e != cudaSuccess || !exec) {
     cudaGetLastError();
     c->graphs_broken = true;
+    c->clear = clear0;
+    std::memcpy(c->last_integrate, last0, sizeof(last0));
     return frame_direct(c, f, p, r);
   }
-  c->frame_graphs.push_back({key, exec, captured});
+  c->frame_graphs.push_back({key, exec, captured, c->clear, {}});
+  std::memcpy(c->frame_graphs.back().last, c->last_integrate, sizeof(c->last_integrate));
   c->launches += captured;
   return check(c, cudaGraphLaunch(exec, c->stream), "frame graph launch");
 }
@@ -1046,6 +1064,7 @@ int rr_integrator_info(rr_ctx* c, uint32_t* out) {
     RR_TRY(check(c, cudaStreamSynchronize(c->stream), "integrator info sync"));
     RR_TRY(check(c, cudaMemcpy(e, s.d_err.ptr, sizeof(e), cudaMemcpyDeviceToHost), "integrator flags"));
     out[13] = (e[0] ? 1u : 0u) | (e[1] ? 2u : 0u);
+    if (out[13]) c->clear.valid = false;       // an item may have been left out: clear the whole slab next time
   }
   return RR_OK;
 }
@@ -1054,6 +1073,15 @@ int rr_integrator_last(const rr_ctx* c, uint32_t* out) {
   if (!c || !out) return RR_ERR_INVALID;
   std::memcpy(out, c->last_integrate, sizeof(c->last_integrate));
   return RR_OK;
+}
+
+int rr_integrator_cleared(rr_ctx* c, uint32_t* out) {
+  if (!c || !out) return RR_ERR_INVALID;
+  RR_SET_DEVICE(c);
+  out[0] = 0;
+  if (c->last_integrate[0] != 1 || c->last_integrate[5] != 2 || !c->d_work.ptr) return RR_OK;
+  RR_TRY(check(c, cudaStreamSynchronize(c->stream), "integrator cleared sync"));
+  return check(c, cudaMemcpy(out, c->d_work.ptr + 6, sizeof(uint32_t), cudaMemcpyDeviceToHost), "cleared bricks");
 }
 
 int rr_integrator_profile(rr_ctx* c, uint64_t* out) {

@@ -53,6 +53,17 @@ struct BrickGrid {
 
 #define RR_CLASS_COUNTERS 16      // >= RR_MAX_SENSORS + 1
 
+// What the volume holds outside the bricks of rr_ctx::d_written: after a staged integrate into slab rows [z0, z1) with the
+// cleared voxel `fill` (voxel format `mode`), every voxel of those rows outside the bricks it evaluated holds `fill`, so
+// the next staged integrate with the same key only has to clear the bricks that left the occupied set (incremental clear).
+// valid = false: nothing is known, the next integrate clears its whole slab.
+struct ClearState {
+  bool valid = false;
+  int z0 = 0, z1 = 0, mode = 0;
+  uint32_t fill = 0;
+  bool same(const ClearState& o) const { return valid && o.valid && z0 == o.z0 && z1 == o.z1 && mode == o.mode && fill == o.fill; }
+};
+
 struct StageTimer {            // one CUDA-event pair per recorded interval; summed and recycled by rr_get_stage_stats
   std::vector<cudaEvent_t> beg, end;
   size_t used = 0;             // intervals recorded since the last reset / fold
@@ -171,21 +182,30 @@ struct rr_ctx {
   rr::DeviceArray<uint8_t> d_rowany;      // [nbz][nby]
   rr::DeviceArray<int16_t> d_cand_y;      // [Y][2], -1 = none
   rr::DeviceArray<int16_t> d_cand_z;      // [Z][2]
-  rr::DeviceArray<uint32_t> d_work;       // [4] work-item counters of the persistent fused kernel
+  // [0..3] work-item counters of the persistent integrators (reset per launch); the staged kernel's own state behind them:
+  // [4] which half of d_written holds the last evaluated set, [5] CTAs finished, [6] bricks the last incremental clear reset
+  rr::DeviceArray<uint32_t> d_work;       // [8]
   bool work_fresh = false;         // k_bricks_update has reset them and no integrate launch has drawn from them since
   int mask_words = 0;
   rr::DeviceArray<float4> d_ztab;  // [Z] (k0, k1, g, 1-g) of the z filter tap against the inverse volume (k_build_ztab)
   int ztab_Z = 0, ztab_IZ = 0;
   bool fused_ok = false;           // brick table is separable with <= 2 bricks per voxel and axis
-  // rr_fuse_frame: captured launch sequences, keyed by (frame slot, pre-process flags, tunable generation)
-  struct FrameGraph { uint64_t key; cudaGraphExec_t exec; uint64_t launches; };
+  // incremental clear (rr_integrate_staged.cu): the bricks the last staged integrate evaluated (its d_occ_mask; two halves,
+  // the kernel reads one and writes the other, d_work[4] says which) and the state of the volume around them. Everything
+  // else that writes the volume resets `clear`.
+  rr::DeviceArray<uint8_t> d_written;     // [2][nb]
+  rr::ClearState clear;
+  // rr_fuse_frame: captured launch sequences, keyed by (frame slot, pre-process flags, full / incremental clear, tunable
+  // generation), with the clear state and rr_integrator_last record the captured integrate left (restored by a replay)
+  struct FrameGraph { uint64_t key; cudaGraphExec_t exec; uint64_t launches; rr::ClearState clear; uint32_t last[8]; };
   std::vector<FrameGraph> frame_graphs;
   // view images of other processes' contexts opened through CUDA IPC (rr_composite_peers); key = the 256-byte handle blob
   struct IpcView { std::string key; uint32_t* step; float4* rgba; float* zbuf; float* nsamp; };
   std::vector<IpcView> ipc_views;
   bool graphs_broken = false;      // a capture failed once: stay on direct launches
   // the last launch_integrate (rr_integrator_last): path (0 none, 1 staged, 2 fused, 3 k_fill + k_integrate_bricks, 4 dense),
-  // sensors, voxel mode, CTA threads or consumer warps, repairs (bit 0 stale item lists declined, bit 1 gather packed late)
+  // sensors, voxel mode, CTA threads or consumer warps, repairs (bit 0 stale item lists declined, bit 1 gather packed late),
+  // clear (0 none, 1 whole slab, 2 incremental)
   uint32_t last_integrate[8] = {};
   // staged (TMA) integrator, rr_integrate_staged.cu. `dirty` is set by everything its tables depend on (inverse volumes,
   // volume / brick grid, bricks mode, voxel format, tunables); they are rebuilt lazily by the next integrate or pre-process call.
@@ -194,6 +214,7 @@ struct rr_ctx {
     bool ok = false;               // the configuration fits the staged kernel
     unsigned generation = 0;       // key of the tunables the tables were built for (staged_key)
     int cy = 0, cz = 0, n_yc = 0, n_zc = 0;   // work item = brick x y-chunk x z-chunk (voxels per chunk, chunks per brick)
+    int max_nz = 0;                // largest z extent of a brick (voxels): z planes per brick of the incremental clear
     int BX = 0, BY = 0, BZ = 0;    // inverse-volume box staged per item (coarse texels)
     int T = 0;                     // pair-image tile edge staged per item and sensor (pixels, even)
     int cwarps = 0, fwarps = 0;    // consumer / fill warps per CTA
@@ -366,6 +387,8 @@ int launch_simplify_mesh(rr_ctx* c, uint32_t cluster_voxels, uint32_t* out_nv, u
 int simplified_download(rr_ctx* c, float* positions, float* normals, float* rgba, uint32_t* triangles, uint32_t* sources);
 int launch_unpack_frames(rr_ctx* c, int slot);
 int launch_calib_invert(rr_ctx* c, int sensor, const uint32_t out_res[3], float4* d_out);
+ClearState integrate_clear_key(const rr_ctx* c);   // rr_integrate.cu: the clear state an integrate now would leave
+bool clear_incremental(const rr_ctx* c);          // the next staged integrate clears only the bricks that left the occupied set
 int staged_prepare(rr_ctx* c);        // (re)builds the staged integrator's tables when dirty; RR_OK also when it declines
 bool staged_selected(const rr_ctx* c); // after staged_prepare: the next bricks-mode integrate runs the staged kernel
 uint64_t staged_lists_key(const rr_ctx* c);   // what the item lists depend on besides the frame: table rebuild, limit

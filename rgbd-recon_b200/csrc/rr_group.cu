@@ -547,6 +547,7 @@ static int group_gather_volume(rr_group* g, const std::string& who, bool need_ca
     if (z1 > z0)
       RR_G_TRY(g, cudaMemcpyPeerAsync(c0->d_tsdf.ptr + plane * z0, c0->device, c->d_tsdf.ptr + plane * z0, c->device, plane * (z1 - z0) * sizeof(float), c0->stream));
   }
+  c0->clear.valid = false;      // member 0's volume was written outside an integrate: its next integrate clears the whole slab
   RR_G_TRY(g, cudaSetDevice(c0->device));
   return RR_OK;
 }

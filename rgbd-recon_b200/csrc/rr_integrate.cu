@@ -293,22 +293,44 @@ int build_ztab(rr_ctx* c) {
   return RR_OK;
 }
 
+// Voxel rows an integrate writes: the slab, and for a slab owner a read-only halo: the raymarcher's refinement and gradient
+// taps reach at most 2 * (limit/2) * Z voxels (+1 for the trilinear tap) past the owned samples; integration is pure, so
+// the halo is recomputed locally instead of exchanged
+static void integrate_rows(const rr_ctx* c, int& z0, int& z1) {
+  z0 = (int)c->slab_z0; z1 = (int)c->slab_z1;
+  if (c->slab_z0 > 0 || c->slab_z1 < c->res[2]) {
+    const int halo = (int)std::ceil(c->cfg.limit * (float)c->res[2]) + 2;
+    z0 = std::max(0, z0 - halo);
+    z1 = std::min((int)c->res[2], z1 + halo);
+  }
+}
+
+static int voxel_mode(const rr_ctx* c) {
+  return c->cfg.store_weight == RR_VOXELS_HALF2 ? 2 : (c->cfg.store_weight != 0 ? 1 : 0);
+}
+
+ClearState integrate_clear_key(const rr_ctx* c) {
+  ClearState k;
+  k.valid = true;
+  integrate_rows(c, k.z0, k.z1);
+  k.mode = voxel_mode(c);
+  const float f = cleared_voxel(k.mode, c->cfg.limit);
+  std::memcpy(&k.fill, &f, sizeof(f));
+  return k;
+}
+
+bool clear_incremental(const rr_ctx* c) {
+  return c->d_written.ptr && c->bricks.num == c->bricks.res[0] * c->bricks.res[1] * c->bricks.res[2] && c->clear.same(integrate_clear_key(c));
+}
+
 int launch_integrate(rr_ctx* c) {
   IntegrateParams p{};
   p.inv = c->d_inv.ptr; p.gather = c->d_gather.ptr; p.tsdf = c->d_tsdf.ptr; p.weight = c->d_weight.ptr;
   p.ranges = c->d_ranges.ptr; p.occupied = c->d_occupied.ptr; p.num_occupied = c->d_num_occ.ptr;
   p.IX = (int)c->ires[0]; p.IY = (int)c->ires[1]; p.IZ = (int)c->ires[2];
   p.W = c->W; p.H = c->H; p.X = (int)c->res[0]; p.Y = (int)c->res[1]; p.Z = (int)c->res[2];
-  p.z_begin = (int)c->slab_z0; p.z_end = (int)c->slab_z1;
+  integrate_rows(c, p.z_begin, p.z_end);
   p.plane_elems = (unsigned)(c->res[0] * c->res[1]);
-  if (c->slab_z0 > 0 || c->slab_z1 < c->res[2]) {
-    // a slab owner also computes a read-only halo: the raymarcher's refinement and gradient taps reach at most
-    // 2 * (limit/2) * Z voxels (+1 for the trilinear tap) past the owned samples; integration is pure, so the halo is
-    // recomputed locally instead of exchanged
-    const int halo = (int)std::ceil(c->cfg.limit * (float)c->res[2]) + 2;
-    p.z_begin = std::max(0, p.z_begin - halo);
-    p.z_end = std::min((int)c->res[2], p.z_end + halo);
-  }
   p.z_chunk = 32;
   p.fW = (float)c->W; p.fH = (float)c->H; p.exmax = (float)(c->W - 1); p.eymax = (float)(c->H - 1);
   RR_TRY_RC(build_ztab(c));
@@ -316,7 +338,7 @@ int launch_integrate(rr_ctx* c) {
   p.pairs = c->d_pairs.ptr; p.pair_pitch = c->pair_pitch;
   p.limit = c->cfg.limit;
   p.wide_loads = tunables().ldg256;
-  const int mode = c->cfg.store_weight == RR_VOXELS_HALF2 ? 2 : (c->cfg.store_weight != 0 ? 1 : 0);
+  const int mode = voxel_mode(c);
   const bool weight = mode == 1;
   const bool bricks = c->cfg.use_bricks != 0;
   std::memset(c->last_integrate, 0, sizeof(c->last_integrate));
@@ -337,6 +359,10 @@ int launch_integrate(rr_ctx* c) {
     c->last_integrate[4] |= 2u;
   }
   if (!done && rc == RR_OK) {
+    // the direct kernels clear the whole slab (bricks mode) or write every voxel of it (dense, gaps between bricks
+    // included), and keep no record of what they wrote: the next staged integrate clears its whole slab
+    if (nslab) c->clear.valid = false;
+    if (bricks && nslab) c->last_integrate[5] = 1;
     if (bricks && !fused && nslab) {
       // dense mode overwrites every voxel, so only the brick path needs the clear
       float* t0 = c->d_tsdf.ptr + plane * p.z_begin;

@@ -13,11 +13,14 @@
 // (depth_b.x, quality | silhouette sign; 8 bytes per pixel, border replicated so CLAMP_TO_EDGE needs no clamping).
 // A persistent CTA per SM runs a two-stage mbarrier pipeline: one producer thread draws items from a global counter and
 // issues the copies for item i+1 while CWARPS consumer warps evaluate item i out of shared memory (LDS only, no global
-// loads in the voxel loop); FWARPS warps stream the clear (-limit) over every voxel outside the occupied bricks the whole
-// time, and every warp that runs out of its own work helps with the clear.
+// loads in the voxel loop); FWARPS warps clear the voxels that must hold -limit from the start, and every warp that runs out
+// of its own work helps with the clear. The clear is incremental when the host knows the volume outside the bricks the
+// last integrate evaluated still holds -limit (rr_ctx::clear): only the bricks that left the occupied set are cleared, a few
+// MB instead of the whole slab. Otherwise it streams -limit over every voxel outside the occupied bricks.
 #include "rr_integrate.cuh"
 
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstring>
 #include <utility>
@@ -52,6 +55,12 @@ struct StagedParams {
   int tail_cap;             // tunable stage_tail_cap: items in flight per CTA once the list runs out (0: no limit)
   unsigned long long* prof; // stage_debug bit 7: cycle counters per role (rr_integrator_profile), else nullptr
   int debug;
+  // incremental clear: bricks occupied now (k_bricks_update) and [2][nb] the ones the last integrate evaluated (half
+  // work[4]); this launch writes the set it evaluates into the other half. full = 1: clear the whole slab instead
+  const uint8_t* occ; uint8_t* written;
+  uint32_t nb, rx, ry;      // bricks, brick grid x / y resolution
+  int max_nz;               // largest z extent of a brick (voxels)
+  int full;
 };
 
 // An item in flight = one header of the header ring + one operand slot per sensor that is evaluated voxel by voxel.
@@ -225,6 +234,98 @@ __device__ __forceinline__ void march_staged(const IntegrateParams& p, const uin
 template <int N, int MODE>
 __device__ __noinline__ void march_direct(const IntegrateParams& p, int x, int y, int zb, int ze) {
   march_column<N, MODE, true>(p, x, y, zb, ze);
+}
+
+// ---- incremental clear -----------------------------------------------------------------------------------------------
+// One z plane of brick b, which the last integrate evaluated and which is not occupied now: every voxel of it that no
+// occupied brick contains gets the cleared value (the voxels an occupied brick shares are the integration's). Bricks overlap
+// their neighbours by a voxel at most and the grid is separable (fused_ok), so only the 26 neighbours can share a voxel, and
+// only where the voxel lies inside the neighbour's range on every axis the neighbour is offset on.
+template <bool WEIGHT>
+__device__ __forceinline__ void clear_plane(const StagedParams& p, uint32_t b, int z, int lane) {
+  const IntegrateParams& ip = p.f.ip;
+  const int bx = (int)(b % p.rx), by = (int)((b / p.rx) % p.ry), bz = (int)(b / (p.rx * p.ry));
+  const int rz = (int)(p.nb / (p.rx * p.ry));
+  // lane l < 27: neighbour (l % 3 - 1, l / 3 % 3 - 1, l / 9 - 1) is occupied
+  bool nocc = false;
+  if (lane < 27) {
+    const int dx = lane % 3 - 1, dy = lane / 3 % 3 - 1, dz = lane / 9 - 1;
+    const int x = bx + dx, y = by + dy, zz = bz + dz;
+    if ((dx | dy | dz) != 0 && x >= 0 && y >= 0 && zz >= 0 && x < (int)p.rx && y < (int)p.ry && zz < rz)
+      nocc = p.occ[((size_t)zz * p.ry + y) * p.rx + x] != 0;
+  }
+  const uint32_t nbr = __ballot_sync(0xffffffffu, nocc);
+  const int32_t* rg = ip.ranges + (size_t)b * 6;
+  const int x0 = rg[0], x1 = rg[1], y0 = rg[2], y1 = rg[3];
+  // voxels below `lo_end` lie in the range of the lower neighbour too, voxels from `hi_beg` on in that of the upper one
+  const int sx = 1, sy = (int)p.rx, sz = (int)(p.rx * p.ry);
+  const int xlo = bx > 0 ? ip.ranges[(size_t)(b - sx) * 6 + 1] : INT_MIN, xhi = bx + 1 < (int)p.rx ? ip.ranges[(size_t)(b + sx) * 6 + 0] : INT_MAX;
+  const int ylo = by > 0 ? ip.ranges[(size_t)(b - sy) * 6 + 3] : INT_MIN, yhi = by + 1 < (int)p.ry ? ip.ranges[(size_t)(b + sy) * 6 + 2] : INT_MAX;
+  const int zlo = bz > 0 ? ip.ranges[(size_t)(b - sz) * 6 + 5] : INT_MIN, zhi = bz + 1 < rz ? ip.ranges[(size_t)(b + sz) * 6 + 4] : INT_MAX;
+  // axis offsets a voxel coordinate can take: bit 0 the lower neighbour, bit 1 the brick's own row, bit 2 the upper one
+  auto offsets = [](int v, int lo, int hi) -> uint32_t { return 2u | (v < lo ? 1u : 0u) | (v >= hi ? 4u : 0u); };
+  const uint32_t az = offsets(z, zlo, zhi);
+  // per y offset: the x offsets of occupied neighbours over the z offsets of this plane
+  uint32_t yrow[3];
+#pragma unroll
+  for (int dy = 0; dy < 3; ++dy) {
+    uint32_t m = 0;
+#pragma unroll
+    for (int dz = 0; dz < 3; ++dz)
+      if ((az >> dz) & 1u) m |= (nbr >> (dz * 9 + dy * 3)) & 7u;
+    yrow[dy] = m;
+  }
+  const int nx = x1 - x0, n = nx * (y1 - y0);
+  const float fill = p.f.fill_value;
+  float* plane_t = ip.tsdf + (size_t)z * ip.plane_elems;
+  float* plane_w = WEIGHT ? ip.weight + (size_t)z * ip.plane_elems : nullptr;
+  for (int i = lane; i < n; i += 32) {
+    const int yy = i / nx, x = x0 + (i - yy * nx), y = y0 + yy;
+    const uint32_t ax = offsets(x, xlo, xhi), ay = offsets(y, ylo, yhi);
+    uint32_t cover = 0;
+#pragma unroll
+    for (int dy = 0; dy < 3; ++dy)
+      if ((ay >> dy) & 1u) cover |= yrow[dy] & ax;
+    if (cover == 0) {
+      const size_t o = (size_t)y * ip.X + x;
+      plane_t[o] = fill;
+      if (WEIGHT) plane_w[o] = 0.0f;
+    }
+  }
+}
+
+// Work item = 32 (brick, z plane) pairs, plane-major, so that the planes of one brick spread over many warps. Counts the
+// bricks that left the occupied set in work[3] (rr_integrator_cleared).
+// Run by the clear warps only: the consumer warps help with the whole-slab clear, not with this one (a few bricks), so that
+// its registers do not shape the consumers' allocation.
+template <bool WEIGHT>
+__device__ __forceinline__ void clear_left(const StagedParams& p, const uint8_t* __restrict__ written, int lane) {
+  const IntegrateParams& ip = p.f.ip;
+  const uint32_t total = p.nb * (uint32_t)p.max_nz;
+  for (;;) {
+    uint32_t it = 0;
+    if (lane == 0) it = atomicAdd(p.f.work + 2, 1u);
+    it = __shfl_sync(0xffffffffu, it, 0);
+    if (it * 32u >= total) break;
+    const uint32_t v = it * 32u + (uint32_t)lane;
+    uint32_t b = 0;
+    int z = 0;
+    bool left = false;
+    if (v < total) {
+      const uint32_t k = v / p.nb;
+      b = v - k * p.nb;
+      if (written[b] && !p.occ[b]) {
+        const int32_t* rg = ip.ranges + (size_t)b * 6;
+        z = rg[4] + (int)k;
+        left = z < rg[5] && z >= ip.z_begin && z < ip.z_end;
+        if (k == 0) atomicAdd(p.f.work + 3, 1u);
+      }
+    }
+    for (uint32_t m = __ballot_sync(0xffffffffu, left); m; m &= m - 1u) {
+      const int l = __ffs((int)m) - 1;
+      clear_plane<WEIGHT>(p, __shfl_sync(0xffffffffu, b, l), __shfl_sync(0xffffffffu, z, l), lane);
+    }
+  }
 }
 
 // ---- the kernel ------------------------------------------------------------------------------------------------------
@@ -453,7 +554,7 @@ k_integrate_staged(const __grid_constant__ StagedParams p, const __grid_constant
       atomicAdd(p.prof + 12, (unsigned long long)(clock64() - t_start));
     })
   };
-  const bool helpers_clear = !(p.debug & 16);
+  const bool helpers_clear = p.full && !(p.debug & 16);
   // each role's code sits behind its own setmaxnreg, so that ptxas allocates it against that budget
   if (warp < PWARP) {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(Shape::kConsumerRegs));
@@ -466,7 +567,29 @@ k_integrate_staged(const __grid_constant__ StagedParams p, const __grid_constant
       __syncwarp();
       if (helpers_clear) clear();
     } else {
-      clear();
+      // the half of p.written that holds the last evaluated set (the last CTA to finish flips it, below, so every CTA reads
+      // the same); the clear warps record the set this launch evaluates in the other half
+      const uint32_t half = *reinterpret_cast<volatile const uint32_t*>(p.f.work + 4) & 1u;
+      const int fw = (int)(blockDim.x >> 5) - PWARP - 1;
+      if (p.written) {
+        uint8_t* next = p.written + (size_t)(half ^ 1u) * p.nb;
+        for (uint32_t b = (blockIdx.x * (uint32_t)fw + (uint32_t)(warp - PWARP - 1)) * 32u + (uint32_t)lane; b < p.nb; b += gridDim.x * (uint32_t)fw * 32u)
+          next[b] = p.occ[b];
+      }
+      if (p.full) clear();
+      else clear_left<MODE == 1>(p, p.written + (size_t)half * p.nb, lane);
+    }
+  }
+  // The last CTA to finish makes the new set current (every CTA has read the old one by then) and keeps this launch's count
+  // of cleared bricks for rr_integrator_cleared, which the next launch's counter reset would lose.
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    if (atomicAdd(p.f.work + 5, 1u) == gridDim.x - 1u) {
+      __threadfence();
+      atomicExch(p.f.work + 6, atomicAdd(p.f.work + 3, 0u));
+      if (p.written) atomicXor(p.f.work + 4, 1u);
+      atomicExch(p.f.work + 5, 0u);
     }
   }
 }
@@ -824,7 +947,7 @@ int staged_prepare(rr_ctx* c) {
     if (enc(&st.map_pairs, CU_TENSOR_MAP_DATA_TYPE_INT64, 3, c->d_pairs.ptr, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) return RR_OK;
   }
-  st.cy = cy; st.cz = cz; st.n_yc = n_yc; st.n_zc = n_zc;
+  st.cy = cy; st.cz = cz; st.n_yc = n_yc; st.n_zc = n_zc; st.max_nz = max_nz;
   st.BX = BX; st.BY = BY; st.BZ = BZ; st.T = (int)T;
   st.inv_bytes = (uint32_t)inv_bytes;
   st.tile_bytes = (uint32_t)(T * T * 8);
@@ -861,7 +984,16 @@ int launch_integrate_staged(rr_ctx* c, const IntegrateParams& p, int mode, bool*
   sp.prof = (tunables().stage_debug & 128) ? reinterpret_cast<unsigned long long*>(st.d_err.ptr + 4) : nullptr;
   sp.fill_src_off = st.fill_src_off; sp.fill_src_bytes = st.fill_src_bytes;
   sp.tables_off = st.tables_off; sp.n_rowany = c->bricks.res[1] * c->bricks.res[2];
-  if (tunables().stage_debug & 1) sp.f.fill_items = 0;
+  // incremental clear: needs d_occ_mask, which k_bricks_update writes for a complete brick grid only
+  const bool grid_ok = c->bricks.num == c->bricks.res[0] * c->bricks.res[1] * c->bricks.res[2];
+  const bool incremental = clear_incremental(c);
+  sp.occ = c->d_occ_mask.ptr; sp.written = c->d_written.ptr;
+  sp.nb = c->bricks.num; sp.rx = c->bricks.res[0]; sp.ry = c->bricks.res[1];
+  sp.max_nz = st.max_nz;
+  sp.full = incremental ? 0 : 1;
+  const bool no_clear = (tunables().stage_debug & 1) != 0;
+  if (no_clear) { sp.f.fill_items = 0; sp.max_nz = 0; }
+  if (!grid_ok) sp.written = nullptr;     // d_occ_mask is not maintained: no set to record
   sp.debug = tunables().stage_debug;
   sp.fill_depth = tunables().stage_fill_depth; sp.fill_lsu = tunables().stage_fill_lsu;
   sp.tail_cap = tunables().stage_tail_cap;
@@ -881,8 +1013,11 @@ int launch_integrate_staged(rr_ctx* c, const IntegrateParams& p, int mode, bool*
     case 8: rc = st.cwarps == 11 ? launch_staged_n<8, 11>(c, sp, mode) : launch_staged_n<8, 16>(c, sp, mode); break;
     default: return fail(c, RR_ERR_UNSUPPORTED, "integrate: 1..8 sensors supported");
   }
-  if (rc != RR_OK) return rc;
-  c->last_integrate[0] = 1; c->last_integrate[3] = (uint32_t)st.cwarps;
+  if (rc != RR_OK) { c->clear.valid = false; return rc; }
+  // the kernel recorded the bricks it evaluated; with the clear switched off (measurement only) the volume outside them is unknown
+  c->clear.valid = false;
+  if (grid_ok && c->d_written.ptr && !no_clear) c->clear = integrate_clear_key(c);
+  c->last_integrate[0] = 1; c->last_integrate[3] = (uint32_t)st.cwarps; c->last_integrate[5] = incremental ? 2u : 1u;
   *done = true;
   return RR_OK;
 }

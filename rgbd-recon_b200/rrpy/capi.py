@@ -29,6 +29,8 @@ VOXELS_F32, VOXELS_F32_WEIGHT, VOXELS_HALF2 = 0, 1, 2
 
 # rr_integrator_last()[0]
 INTEGRATE_PATHS = ("none", "staged", "fused", "two_kernel", "dense")
+# rr_integrator_last()[5]
+INTEGRATE_CLEARS = ("none", "full", "incremental")
 
 
 class View(C.Structure):
@@ -98,6 +100,7 @@ def lib():
     L.rr_integrator_info.argtypes = [vp, u32]
     L.rr_integrator_profile.argtypes = [vp, C.POINTER(C.c_uint64)]
     L.rr_integrator_last.argtypes = [vp, u32]
+    L.rr_integrator_cleared.argtypes = [vp, u32]
     L.rr_draw_points.argtypes = [vp, C.POINTER(View), f32, f32]
     L.rr_draw_calibs.argtypes = [vp, C.POINTER(View), C.c_int, C.c_float, f32, f32]
     L.rr_draw_trigrid.argtypes = [vp, C.POINTER(View), C.c_float, f32, f32]
@@ -695,10 +698,18 @@ class Fusion:
 
     def integrator_last(self):
         """rr_integrator_last as a dict: the kernel the last integrate launched (path name), its sensors, voxel format, CTA
-        threads (consumer warps for the staged kernel) and repair bits (1: stale staged item lists, 2: gather packed late)."""
+        threads (consumer warps for the staged kernel), repair bits (1: stale staged item lists, 2: gather packed late) and the
+        clear it did ("none", "full" or "incremental")."""
         out = np.zeros(8, np.uint32)
         self._ck(self.L.rr_integrator_last(self.h, _u32(out)))
-        return dict(path=INTEGRATE_PATHS[int(out[0])], sensors=int(out[1]), voxel_mode=int(out[2]), threads=int(out[3]), repairs=int(out[4]))
+        return dict(path=INTEGRATE_PATHS[int(out[0])], sensors=int(out[1]), voxel_mode=int(out[2]), threads=int(out[3]), repairs=int(out[4]),
+                    clear=INTEGRATE_CLEARS[int(out[5])])
+
+    def integrator_cleared(self):
+        """rr_integrator_cleared: bricks the last integrate's incremental clear reset (0 unless it cleared incrementally)."""
+        out = np.zeros(1, np.uint32)
+        self._ck(self.L.rr_integrator_cleared(self.h, _u32(out)))
+        return int(out[0])
 
     def integrator_profile(self):
         """rr_integrator_profile: cycle counters of the staged integrator's roles (stage_debug bit 7), reset on read."""

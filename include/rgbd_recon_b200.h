@@ -394,6 +394,53 @@ int rr_download_parts(rr_ctx* ctx, uint32_t* voxels, int32_t* boxes, float* cent
 int rr_download_mesh_parts(rr_ctx* ctx, uint32_t* vertex_parts, uint32_t* triangle_parts);
 int rr_group_label_parts(rr_group* g, uint32_t* out_num_parts);
 
+/* ---- part tracking (no reference counterpart) ---------------------------------------------------------------------------
+ * Persistent identities for the connected parts from one frame set to the next: a part's number depends on what else is in
+ * the volume, a track id follows the object by voxel overlap.
+ *   State    a context holds optional tracking state: the tracked labelling (the labels and per-part track ids of the last
+ *            rr_track_parts) and next_id, which starts at 0. A context that never tracks allocates nothing for it.
+ *            rr_reset_part_tracks and a new volume allocation as far as extraction goes (a new resolution or voxel format
+ *            in rr_configure) empty it and set next_id to 0; other settings (limit, brick size, rr_set_slab, bbox) leave it.
+ *   Labels   the current volume is labelled exactly as rr_label_parts does: rr_download_parts and rr_download_mesh_parts
+ *            then return, bit for bit, what they return after rr_label_parts, epoch rule included.
+ *   Pairs    a current part p is tracked iff voxels[p] >= min_voxels; a previous part q is a candidate iff it received a
+ *            track id in the previous call; O(q, p) counts the voxels labelled q in the tracked labelling and p now. The
+ *            candidate pairs are those with q a candidate, p tracked and O(q, p) > 0.
+ *   Matching greedy in the strict total order O descending, then q ascending, then p ascending: a pair is accepted iff
+ *            neither its q nor its p is accepted already. An accepted p inherits q's track id, prev_parts[p] = q and
+ *            overlaps[p] = O(q, p). Tracked parts left unmatched get new ids next_id, next_id + 1, ... in ascending part
+ *            index, with prev_parts 0xFFFFFFFF and overlaps 0. Untracked parts get track id 0xFFFFFFFF, prev_parts
+ *            0xFFFFFFFF, overlaps 0. Ids are never reused before a reset.
+ *   Ended    ended[E]: the track ids of the candidate previous parts that were not accepted, by ascending previous part.
+ *            The labelling and its ids then become the tracked labelling; the first call after a reset has no candidates
+ *            (every tracked part is new, E = 0).
+ *   Overlaps are exact counts and the order is total: no output depends on scheduling, the brick shortcut or the number of
+ *   devices. Tracking the same volume twice keeps every id with overlaps == voxels and ends nothing. Matching is by overlap
+ *   only: a caller that skips frame sets over which an object moves further than its own extent gets a new id for it.
+ *
+ * rr_track_parts   labels and tracks on the context's stream, with at most three synchronisations (the part count, the
+ *                  pair-record count, the counts returned); returns the part count P and the ended count E.
+ *                  RR_ERR_INVALID for min_voxels == 0, a NULL count pointer, before any integrate into the current volume
+ *                  and on a context restricted by rr_set_slab (use rr_group_track_parts). RR_ERR_UNSUPPORTED when the call
+ *                  would need track id 0xFFFFFFFF; the tracking state then stays as it was. Not a setting: the volume,
+ *                  brick tables, view images (rr_fill_colors still fills the last view), mesh, simplified mesh, cloud,
+ *                  query buffers, captured frame graphs and rr_integrator_last stay as they are. rr_label_parts keeps its
+ *                  results and cost, and a call of it between two rr_track_parts does not change what the second compares
+ *                  against.
+ * rr_download_part_tracks  the last tracking: track_ids, prev_parts and overlaps uint32 [P], ended uint32 [E]. Each pointer may
+ *                  be NULL, host memory (pageable or pinned) or device memory of the context's GPU; returns after one
+ *                  synchronisation. Valid until the next rr_track_parts, reset or new volume, whatever rr_label_parts calls
+ *                  come in between; RR_ERR_INVALID before any tracking of the current volume allocation (or after a reset).
+ * rr_reset_part_tracks  empties the tracking state: the next rr_track_parts starts ids at 0 with no candidates.
+ * rr_group_track_parts  the same for a group, bit for bit equal to a single context over the same sequence of frame sets:
+ *                  member 0 receives the other members' slabs by peer copies (as rr_group_label_parts) and tracks there;
+ *                  read with rr_download_part_tracks(rr_group_member(g, 0), ...), reset with rr_reset_part_tracks on
+ *                  member 0. */
+int rr_track_parts(rr_ctx* ctx, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended);
+int rr_download_part_tracks(rr_ctx* ctx, uint32_t* track_ids, uint32_t* prev_parts, uint32_t* overlaps, uint32_t* ended);
+int rr_reset_part_tracks(rr_ctx* ctx);
+int rr_group_track_parts(rr_group* g, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended);
+
 /* ---- point clouds (no reference counterpart: a reference user draws the points and reads pixels back) -------------------
  * The pre-processed, registered sensor points: every kept depth pixel of the sensors in sensor_mask, lifted to the world.
  * For sensor i (bit i of sensor_mask) and pixel (x, y) of its W x H depth image, id = i*W*H + y*W + x:

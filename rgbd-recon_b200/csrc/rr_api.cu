@@ -321,10 +321,12 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     c->mesh_valid = false;
     c->parts_valid = false;
     c->simp_valid = false;
+    track_reset(c);                // labels of another grid or voxel format are not comparable
     ++c->volume_epoch;
   }
   if (new_volume) {   // the label and row arrays are sized by the volume
-    c->d_parts_labels.release();
+    c->d_parts_labels[0].release();
+    c->d_parts_labels[1].release();
     c->d_parts_rows.release();
   }
   if (new_bricks) {
@@ -900,7 +902,31 @@ int rr_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
   RR_REQUIRE(c, c->slab_z0 == 0 && c->slab_z1 == c->res[2],
              "rr_label_parts: this context holds only its z-slab (rr_set_slab); label through rr_group_label_parts");
   RR_SET_DEVICE(c);
-  return launch_label_parts(c, out_num_parts);
+  return launch_label_parts(c, label_dest(c), out_num_parts);
+}
+
+int rr_track_parts(rr_ctx* c, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, out_num_parts && out_num_ended, "rr_track_parts: null count pointer");
+  RR_REQUIRE(c, min_voxels >= 1, "rr_track_parts: min_voxels must be at least 1");
+  RR_REQUIRE(c, c->configured && c->volume_integrated, "rr_track_parts: nothing has been integrated into the current volume");
+  RR_REQUIRE(c, c->slab_z0 == 0 && c->slab_z1 == c->res[2],
+             "rr_track_parts: this context holds only its z-slab (rr_set_slab); track through rr_group_track_parts");
+  RR_SET_DEVICE(c);
+  return launch_track_parts(c, min_voxels, out_num_parts, out_num_ended);
+}
+
+int rr_download_part_tracks(rr_ctx* c, uint32_t* track_ids, uint32_t* prev_parts, uint32_t* overlaps, uint32_t* ended) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, c->track_valid, "rr_download_part_tracks: nothing tracked in the current volume (rr_track_parts first)");
+  RR_SET_DEVICE(c);
+  return track_download(c, track_ids, prev_parts, overlaps, ended);
+}
+
+int rr_reset_part_tracks(rr_ctx* c) {
+  if (!c) return RR_ERR_INVALID;
+  track_reset(c);
+  return RR_OK;
 }
 
 int rr_download_parts(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels) {

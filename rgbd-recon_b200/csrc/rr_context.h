@@ -104,6 +104,7 @@ struct PinnedScalars {
   uint32_t parts_count;
   unsigned long long mesh_totals[2];   // vertices, triangles
   uint32_t simplify_counts[2];         // vertices, triangles of rr_simplify_mesh
+  uint32_t track_counts[3];            // rr_track_parts: pair records, then new ids and ended tracks
 };
 
 }  // namespace rr
@@ -282,7 +283,10 @@ struct rr_ctx {
   uint64_t volume_epoch = 0, mesh_epoch = 0, parts_epoch = 0;
   bool parts_valid = false;        // d_parts_* hold the last labelling (parts_n parts)
   uint32_t parts_n = 0;
-  rr::DeviceArray<uint32_t> d_parts_labels;          // [Z][Y][X]: union-find forest, then part labels
+  // [2][Z][Y][X]: union-find forest, then part labels. A labelling writes the array that does not hold the tracked
+  // labelling (array 0 while nothing is tracked); parts_cur is the one holding the last labelling.
+  rr::DeviceArray<uint32_t> d_parts_labels[2];
+  int parts_cur = 0;
   rr::DeviceArray<uint32_t> d_parts_rows;            // [2][rows + 1]: roots per row, their offsets
   rr::DeviceArray<uint8_t> d_parts_scratch;          // CUB scan storage
   rr::DeviceArray<uint32_t> d_parts_voxels;          // per part
@@ -290,6 +294,20 @@ struct rr_ctx {
   rr::DeviceArray<unsigned long long> d_parts_sums;  // [P][3]
   rr::DeviceArray<float> d_parts_centroids;          // [P][3]
   rr::DeviceArray<uint32_t> d_mesh_parts;            // [V] vertex parts, then [T] triangle parts
+
+  // part tracking (rr_track.cu). track_slot: the label array holding the tracked labelling (-1: none); the per-part
+  // outputs of a call live in the slot of the labelling it tracked, so a refused call leaves the last call's outputs.
+  int track_slot = -1;
+  bool track_valid = false;        // the outputs of slot track_slot are a tracking of the current volume allocation
+  uint64_t track_next_id = 0;      // the next new track id
+  uint32_t track_n[2] = {0, 0}, track_e[2] = {0, 0};   // parts and ended tracks of each slot
+  rr::DeviceArray<uint32_t> d_track_ids[2], d_track_prev[2], d_track_overlaps[2];   // [P] per slot
+  rr::DeviceArray<uint32_t> d_track_ended[2];        // [E] per slot
+  rr::DeviceArray<unsigned long long> d_track_keys;  // [4][R]: pair records q << 32 | p, sorted, distinct; then ordered
+  rr::DeviceArray<uint32_t> d_track_counts;          // [4][R]: voxels per record, sorted, per distinct pair (O); ordered
+  rr::DeviceArray<uint32_t> d_track_flags;           // [P + 1] new-id flags, offsets; [Pprev + 1] ended flags, offsets;
+                                                     // [Pprev] accepted previous parts; [1] distinct pairs
+  rr::DeviceArray<uint8_t> d_track_scratch;          // CUB sort, reduce and scan storage
 
   // mesh simplification (rr_simplify.cu): scratch sized by the mesh's V and T, outputs of at most V vertices and T triangles
   bool simp_valid = false;         // d_simp_* hold a simplification of a mesh of the current volume allocation
@@ -378,9 +396,15 @@ int query_download(rr_ctx* c, uint32_t count, bool rays, float* values_or_positi
 int launch_extract_points(rr_ctx* c, uint32_t mask, uint32_t* out_n);
 int cloud_download(rr_ctx* c, float* positions, float* normals, float* colors, float* quality, uint32_t* pixels);
 // rr_parts.cu: rr_label_parts over the whole volume, ignoring the slab; the downloads copy out and synchronise once
-int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts);
+int launch_label_parts(rr_ctx* c, int dest, uint32_t* out_num_parts);   // into d_parts_labels[dest]
+int label_dest(const rr_ctx* c);   // the label array a labelling writes: the one not holding the tracked labelling
 int parts_download(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels);
 int mesh_parts_download(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle_parts);   // the mesh and labelling of one epoch
+// rr_track.cu: rr_track_parts (checked by the caller: whole volume, integrated, min_voxels >= 1); track_download copies the
+// last tracking out and synchronises once; track_reset empties the tracking state
+int launch_track_parts(rr_ctx* c, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended);
+int track_download(rr_ctx* c, uint32_t* track_ids, uint32_t* prev_parts, uint32_t* overlaps, uint32_t* ended);
+void track_reset(rr_ctx* c);
 // rr_simplify.cu: rr_simplify_mesh of the last mesh (checked by the caller: current, cluster_voxels >= 1), synchronising once;
 // simplified_download copies the last simplification out and synchronises once
 int launch_simplify_mesh(rr_ctx* c, uint32_t cluster_voxels, uint32_t* out_nv, uint32_t* out_nt);

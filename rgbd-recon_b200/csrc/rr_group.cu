@@ -566,7 +566,19 @@ int rr_group_label_parts(rr_group* g, uint32_t* out_num_parts) {
   if (!g) return RR_ERR_INVALID;
   RR_G_REQUIRE(g, out_num_parts, "rr_group_label_parts: null count pointer");
   RR_TRY_RC(group_gather_volume(g, "rr_group_label_parts", false));
-  const int rc = rr::launch_label_parts(g->m[0], out_num_parts);
+  const int rc = rr::launch_label_parts(g->m[0], rr::label_dest(g->m[0]), out_num_parts);
+  RR_G_TRY(g, cudaStreamSynchronize(g->m[0]->stream));
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
+// The same gather, then member 0 tracks the whole volume against its tracked labelling; read the tracks with
+// rr_download_part_tracks(rr_group_member(g, 0), ...), reset them with rr_reset_part_tracks on member 0.
+int rr_group_track_parts(rr_group* g, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended) {
+  if (!g) return RR_ERR_INVALID;
+  RR_G_REQUIRE(g, out_num_parts && out_num_ended, "rr_group_track_parts: null count pointer");
+  RR_G_REQUIRE(g, min_voxels >= 1, "rr_group_track_parts: min_voxels must be at least 1");
+  RR_TRY_RC(group_gather_volume(g, "rr_group_track_parts", false));
+  const int rc = rr::launch_track_parts(g->m[0], min_voxels, out_num_parts, out_num_ended);
   RR_G_TRY(g, cudaStreamSynchronize(g->m[0]->stream));
   return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
 }

@@ -7,7 +7,7 @@
 // smaller index (Playne & Hawick, "A new algorithm for parallel connected-component labelling on GPUs", 2018): a root is
 // hooked to the smaller root with atomicMin, so a finished root is its part's smallest index, the part's key. Every pass
 // is one voxel row (y, z) per warp, lanes along x; in bricks mode only the voxels inside occupied bricks are visited (each
-// once: the x masks of the brick rows that contain the row), otherwise every voxel:
+// once: the x masks of the brick rows that contain the row; rr_rows.cuh), otherwise every voxel:
 //   memset             L = 0xFFFFFFFF (outside)
 //   k_parts_init       L[i] = i for every inside voxel
 //   k_parts_merge      union with the inside -x, -y and -z neighbours
@@ -18,6 +18,7 @@
 //   k_parts_finish     per part: half-open box and the centroid in binary64
 // Volumes hold fewer than 2^31 voxels (rr_configure), so bit 31 of an index is free for the root mark.
 #include "rr_context.h"
+#include "rr_rows.cuh"
 #include "rr_sample.cuh"
 
 #include <cub/device/device_scan.cuh>
@@ -48,36 +49,6 @@ struct PartsParams {
 
 __device__ __forceinline__ bool inside_voxel(float v) { return v > 0.0f && v <= 3.402823466e38f; }
 
-// the candidate voxels of word w (x = 32 w + lane) of row (y, z)
-__device__ __forceinline__ uint32_t row_word(const PartsParams& p, int y, int z, int w) {
-  const int rem = p.X - 32 * w;
-  const uint32_t all = rem >= 32 ? 0xFFFFFFFFu : ((1u << rem) - 1u);
-  if (!p.use_rows) return all;
-  uint32_t m = 0;
-  for (int a = 0; a < 2; ++a) {
-    const int by = p.cand_y[2 * y + a];
-    if (by < 0) continue;
-    for (int b = 0; b < 2; ++b) {
-      const int bz = p.cand_z[2 * z + b];
-      if (bz >= 0) m |= p.rowmask[((size_t)bz * p.rby + by) * p.mask_words + w];
-    }
-  }
-  return m & all;
-}
-
-__device__ __forceinline__ bool row_any(const PartsParams& p, int y, int z) {
-  if (!p.use_rows) return true;
-  for (int a = 0; a < 2; ++a) {
-    const int by = p.cand_y[2 * y + a];
-    if (by < 0) continue;
-    for (int b = 0; b < 2; ++b) {
-      const int bz = p.cand_z[2 * z + b];
-      if (bz >= 0 && p.rowany[bz * p.rby + by]) return true;
-    }
-  }
-  return false;
-}
-
 __device__ __forceinline__ uint32_t find_root(const uint32_t* L, uint32_t i) {
   uint32_t n = L[i];
   while (n != i) { i = n; n = L[i]; }
@@ -92,22 +63,6 @@ __device__ void unite(uint32_t* L, uint32_t a, uint32_t b) {
     const uint32_t old = atomicMin(L + a, b);
     if (old == a) return;
     a = find_root(L, old); b = find_root(L, b);
-  }
-}
-
-// Each pass: warp = row r, the body runs for every lane (all 32 lanes, uniform control flow) with the lane's voxel and
-// whether it is a candidate.
-template <class F>
-__device__ __forceinline__ void walk_row(const PartsParams& p, unsigned r, F&& body) {
-  const unsigned lane = threadIdx.x & 31u;
-  const int y = (int)(r % (unsigned)p.Y), z = (int)(r / (unsigned)p.Y);
-  if (!row_any(p, y, z)) return;
-  const unsigned nw = ((unsigned)p.X + 31u) / 32u;
-  for (unsigned w = 0; w < nw; ++w) {
-    const uint32_t m = row_word(p, y, z, (int)w);
-    if (!m) continue;
-    const int x = (int)(w * 32u + lane);
-    body(x, y, z, ((unsigned)z * (unsigned)p.Y + (unsigned)y) * (unsigned)p.X + (unsigned)x, ((m >> lane) & 1u) != 0, w * 32u);
   }
 }
 
@@ -261,11 +216,11 @@ __global__ void __launch_bounds__(128) k_mesh_triangle_parts(const uint32_t* __r
 
 }  // namespace
 
-int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
+int launch_label_parts(rr_ctx* c, int dest, uint32_t* out_num_parts) {
   const int X = (int)c->res[0], Y = (int)c->res[1], Z = (int)c->res[2];
   const size_t nvox = (size_t)X * Y * Z, rows = (size_t)Y * Z;
   c->parts_valid = false;
-  RR_TRY_RC(c->d_parts_labels.reserve(c, nvox, "part labels"));
+  RR_TRY_RC(c->d_parts_labels[dest].reserve(c, nvox, "part labels"));
   RR_TRY_RC(c->d_parts_rows.reserve(c, 2 * (rows + 1), "part row counts"));
   uint32_t* cnt = c->d_parts_rows.ptr;
   uint32_t* off = cnt + (rows + 1);
@@ -276,7 +231,7 @@ int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
   PartsParams p{};
   p.tsdf = c->d_tsdf.ptr; p.X = X; p.Y = Y; p.Z = Z;
   p.half2 = c->cfg.store_weight == RR_VOXELS_HALF2 ? 1 : 0;
-  p.L = c->d_parts_labels.ptr;
+  p.L = c->d_parts_labels[dest].ptr;
   p.use_rows = c->mesh_rows_ok ? 1 : 0;
   p.rby = (int)c->bricks.res[1]; p.mask_words = c->mask_words;
   p.rowmask = c->d_rowmask.ptr; p.rowany = c->d_rowany.ptr; p.cand_y = c->d_cand_y.ptr; p.cand_z = c->d_cand_z.ptr;
@@ -316,6 +271,7 @@ int launch_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
     RR_LAUNCH_CHECK(c, "k_parts_finish");
   }
   c->parts_n = np;
+  c->parts_cur = dest;
   c->parts_epoch = c->volume_epoch;
   c->parts_valid = true;
   *out_num_parts = np;
@@ -327,7 +283,7 @@ int parts_download(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids
   if (voxels && np) RR_TRY_RC(check(c, cudaMemcpyAsync(voxels, c->d_parts_voxels.ptr, np * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "part download"));
   if (boxes && np) RR_TRY_RC(check(c, cudaMemcpyAsync(boxes, c->d_parts_boxes.ptr, np * 6 * sizeof(int32_t), cudaMemcpyDefault, c->stream), "part download"));
   if (centroids && np) RR_TRY_RC(check(c, cudaMemcpyAsync(centroids, c->d_parts_centroids.ptr, np * 3 * sizeof(float), cudaMemcpyDefault, c->stream), "part download"));
-  if (labels) RR_TRY_RC(check(c, cudaMemcpyAsync(labels, c->d_parts_labels.ptr, nvox * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "label download"));
+  if (labels) RR_TRY_RC(check(c, cudaMemcpyAsync(labels, c->d_parts_labels[c->parts_cur].ptr, nvox * sizeof(uint32_t), cudaMemcpyDefault, c->stream), "label download"));
   return check(c, cudaStreamSynchronize(c->stream), "part download sync");
 }
 
@@ -337,7 +293,8 @@ int mesh_parts_download(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle_pa
   uint32_t* vp = c->d_mesh_parts.ptr;
   uint32_t* tp = vp + nv;
   if (nv) {
-    k_mesh_vertex_parts<<<(nv + 127) / 128, 128, 0, c->stream>>>(c->d_mesh_keys.ptr, nv, (int)c->res[0], (int)c->res[1], c->d_parts_labels.ptr, vp);
+    k_mesh_vertex_parts<<<(nv + 127) / 128, 128, 0, c->stream>>>(c->d_mesh_keys.ptr, nv, (int)c->res[0], (int)c->res[1],
+                                                                 c->d_parts_labels[c->parts_cur].ptr, vp);
     RR_LAUNCH_CHECK(c, "k_mesh_vertex_parts");
   }
   if (nt) {

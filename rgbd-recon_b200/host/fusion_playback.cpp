@@ -4,6 +4,7 @@
 //   fusion_playback <file.ks> (--streams "s0;s1;..." | --messages file) [--depth W H --color CW CH] [--frames K] [--voxel m]
 //                   [--limit l] [--eye x y z | --matrices file] [--view W H] [--shade m] [--dump-tsdf file] [--dump-image file] [--dense]
 //                   [--dump-mesh file.ply [--simplify C] [--min-part-voxels N]] [--dump-points file.ply] [--pick PX PY] [--parts]
+//                   [--track-parts N]
 //                   [--gpus N | --devices a,b,...] [--recon points|trigrid|calibs [--min-length m] [--dump-recon file]]
 // --recon: like kinect_client's reconstruction list (source/kinect_client.cpp:251-257, key-selected g_recon_mode), one of the
 // other reconstructions also draws the last frame set's maps - ReconPoints, ReconTrigrid (min_length from the sensor .yml
@@ -19,6 +20,10 @@
 //   With --simplify, a simplified triangle is in the part of its source triangle.
 // --parts: one line per connected part of the last frame set's volume (ReconIntegration::labelParts): index, voxels, box
 //   (x0 x1 y0 y1 z0 z1, half-open voxel ranges) and centroid (metres).
+// --track-parts N: after every frame set, its connected parts with track ids that persist across frame sets
+//   (ReconIntegration::trackParts with min_voxels N, matched by voxel overlap): one line "frame F part K track T voxels V
+//   prev Q overlap O" per part of at least N voxels (Q = 4294967295 and O = 0 for a new track), then one line
+//   "frame F ended T" per track that ended; F counts frame sets from 0.
 // --dump-points: the last frame set's pre-processed sensor points (ReconPoints::extractPoints) as a binary PLY with normals,
 // colours and quality (with --gpus N through the group call: pre-processing is replicated on every member).
 // --pick PX PY: picking as kinect_client's view would do it - the world ray through the centre of view pixel (PX, PY) (GL window
@@ -111,6 +116,7 @@ int main(int argc, char** argv) {
   bool print_parts = false;
   long long min_part_voxels = -1;
   long long simplify = 0;
+  long long track_min_voxels = 0;
   for (int i = 1; i < argc; ++i) {
     auto next = [&](int k) { return std::atof(argv[i + k]); };
     if (!std::strcmp(argv[i], "--depth")) { W = (unsigned)next(1); H = (unsigned)next(2); i += 2; explicit_sizes = true; }
@@ -132,6 +138,7 @@ int main(int argc, char** argv) {
     else if (!std::strcmp(argv[i], "--parts")) print_parts = true;
     else if (!std::strcmp(argv[i], "--min-part-voxels")) min_part_voxels = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--simplify")) simplify = std::atoll(argv[++i]);
+    else if (!std::strcmp(argv[i], "--track-parts")) track_min_voxels = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--gpus")) { devices.clear(); for (int d = 0, n = std::atoi(argv[++i]); d < n; ++d) devices.push_back(d); }
     else if (!std::strcmp(argv[i], "--devices")) {
       devices.clear();
@@ -200,6 +207,16 @@ int main(int argc, char** argv) {
       recon.integrate();
       recon.drawF();
       if (done == 0 && devices.size() > 1) gpu.balanceSlabs();                        // occupied bricks cluster around the subject
+      if (track_min_voxels > 0) {                                                      // persistent part ids, per frame set
+        Parts parts;
+        PartTracks tracks;
+        recon.trackParts((uint32_t)track_min_voxels, parts, tracks);
+        for (std::size_t k = 0; k < parts.voxels.size(); ++k)
+          if (tracks.track_ids[k] != 0xFFFFFFFFu)
+            std::printf("frame %d part %zu track %u voxels %u prev %u overlap %u\n", done, k, (unsigned)tracks.track_ids[k],
+                        (unsigned)parts.voxels[k], (unsigned)tracks.prev_parts[k], (unsigned)tracks.overlaps[k]);
+        for (uint32_t t : tracks.ended) std::printf("frame %d ended %u\n", done, (unsigned)t);
+      }
       ++done;
     }
     if (!messages.empty()) std::cout << "last frame time " << nka.getCurrentFrameTime() << std::endl;

@@ -408,6 +408,19 @@ void ReconIntegration::labelParts(Parts& out) const {
   ck(rr_download_parts(ctx(), out.voxels.data(), out.boxes.data(), out.centroids.data(), nullptr), "rr_download_parts");
 }
 
+void ReconIntegration::trackParts(uint32_t min_voxels, Parts& parts, PartTracks& tracks) const {
+  uint32_t n = 0, e = 0;
+  if (gpu::Context::current().numDevices() > 1) gk(rr_group_track_parts(grp(), min_voxels, &n, &e), "rr_group_track_parts");
+  else ck(rr_track_parts(ctx(), min_voxels, &n, &e), "rr_track_parts");
+  parts.voxels.resize(n); parts.boxes.resize((std::size_t)n * 6); parts.centroids.resize((std::size_t)n * 3);
+  ck(rr_download_parts(ctx(), parts.voxels.data(), parts.boxes.data(), parts.centroids.data(), nullptr), "rr_download_parts");
+  tracks.track_ids.resize(n); tracks.prev_parts.resize(n); tracks.overlaps.resize(n); tracks.ended.resize(e);
+  ck(rr_download_part_tracks(ctx(), tracks.track_ids.data(), tracks.prev_parts.data(), tracks.overlaps.data(), tracks.ended.data()),
+     "rr_download_part_tracks");
+}
+
+void ReconIntegration::resetPartTracks() const { ck(rr_reset_part_tracks(ctx()), "rr_reset_part_tracks"); }
+
 void ReconIntegration::simplifyMesh(uint32_t cluster_voxels, Mesh& out, std::vector<uint32_t>* sources) const {
   uint32_t nv = 0, nt = 0;
   if (gpu::Context::current().numDevices() > 1) gk(rr_group_simplify_mesh(grp(), cluster_voxels, &nv, &nt), "rr_group_simplify_mesh");

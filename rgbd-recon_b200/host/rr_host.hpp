@@ -304,6 +304,14 @@ struct Parts {
   std::vector<float> centroids;      // [P][3] metres
 };
 
+// The tracks of rr_download_part_tracks, per part of the Parts they come with (the header states the matching).
+struct PartTracks {
+  std::vector<uint32_t> track_ids;   // [P] persistent id; 0xFFFFFFFF for a part below min_voxels
+  std::vector<uint32_t> prev_parts;  // [P] the previous part it continues; 0xFFFFFFFF for a new track or an untracked part
+  std::vector<uint32_t> overlaps;    // [P] voxels shared with that previous part; 0 for none
+  std::vector<uint32_t> ended;       // [E] ids of the tracks that ended, by ascending previous part
+};
+
 // ---- point clouds (no reference counterpart): the pre-processed, registered sensor points --------------------------------
 // The arrays of rr_download_points (include/rgbd_recon_b200.h states what they hold).
 struct PointCloud {
@@ -348,6 +356,10 @@ class ReconIntegration : public Reconstruction {
   // every vertex [V] and triangle [T] of the last extractMesh, which must come from the same volume state
   void labelParts(Parts& out) const;
   void meshParts(std::vector<uint32_t>& vertex_parts, std::vector<uint32_t>& triangle_parts) const;
+  // the parts of the fused volume with track ids persistent across frame sets, matched by voxel overlap against the last
+  // trackParts (rr_track_parts; with several devices rr_group_track_parts); resetPartTracks starts ids at 0 again
+  void trackParts(uint32_t min_voxels, Parts& parts, PartTracks& tracks) const;
+  void resetPartTracks() const;
   // the last extractMesh simplified by vertex clustering with clusters of cluster_voxels voxels per side (rr_simplify_mesh;
   // with several devices rr_group_simplify_mesh); sources: per simplified triangle, its source triangle in that mesh
   void simplifyMesh(uint32_t cluster_voxels, Mesh& out, std::vector<uint32_t>* sources = nullptr) const;

@@ -152,6 +152,10 @@ def lib():
     L.rr_download_parts.argtypes = [vp, vp, vp, vp, vp]
     L.rr_download_mesh_parts.argtypes = [vp, vp, vp]
     L.rr_group_label_parts.argtypes = [vp, u32]
+    L.rr_track_parts.argtypes = [vp, C.c_uint32, u32, u32]
+    L.rr_download_part_tracks.argtypes = [vp, vp, vp, vp, vp]
+    L.rr_reset_part_tracks.argtypes = [vp]
+    L.rr_group_track_parts.argtypes = [vp, C.c_uint32, u32, u32]
     L.rr_simplify_mesh.argtypes = [vp, C.c_uint32, u32, u32]
     L.rr_download_simplified_mesh.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rr_group_simplify_mesh.argtypes = [vp, C.c_uint32, u32, u32]
@@ -649,6 +653,36 @@ class Fusion:
         self._ck(self.L.rr_download_mesh_parts(self.h, *ptrs))
         return tuple(outs)
 
+    def track_parts_counts(self, min_voxels=1):
+        """rr_track_parts alone: labels the volume, tracks its parts against the tracked labelling and returns (parts P,
+        ended tracks E)."""
+        n, e = C.c_uint32(), C.c_uint32()
+        self._ck(self.L.rr_track_parts(self.h, int(min_voxels), C.byref(n), C.byref(e)))
+        return int(n.value), int(e.value)
+
+    def download_part_tracks(self, n, e, device=False):
+        """rr_download_part_tracks of the last tracking (n, e: its counts): (track_ids uint32 [n], prev_parts uint32 [n],
+        overlaps uint32 [n], ended uint32 [e]), as numpy arrays or, with device, CUDA tensors on the context's GPU."""
+        dev = None
+        if device:
+            import torch
+            dev = torch.device("cuda", self.device)
+        outs, op = _query_outputs(dev, ((n,), "u4"), ((n,), "u4"), ((n,), "u4"), ((e,), "u4"))
+        self._ck(self.L.rr_download_part_tracks(self.h, *op))
+        return tuple(outs)
+
+    def track_parts(self, min_voxels=1, device=False):
+        """The parts of the volume with persistent track ids (rr_track_parts + rr_download_parts + rr_download_part_tracks):
+        (voxels, boxes, centroids) as label_parts, then track_ids, prev_parts and overlaps uint32 [P] (0xFFFFFFFF, 0xFFFFFFFF
+        and 0 for parts below min_voxels voxels; prev_parts 0xFFFFFFFF and overlaps 0 for a new track) and ended uint32 [E],
+        the ids of the tracks that ended. device: the four tracking arrays as CUDA tensors on the context's GPU."""
+        n, e = self.track_parts_counts(min_voxels)
+        return self.download_parts(n) + self.download_part_tracks(n, e, device)
+
+    def reset_part_tracks(self):
+        """rr_reset_part_tracks: forget the tracked labelling; the next track_parts starts ids at 0."""
+        self._ck(self.L.rr_reset_part_tracks(self.h))
+
     def simplify_mesh_counts(self, cluster_voxels):
         """rr_simplify_mesh alone: simplifies the last mesh on the device and returns (vertices, triangles)."""
         nv, nt = C.c_uint32(), C.c_uint32()
@@ -914,6 +948,18 @@ class Group:
     def mesh_parts(self, device=False):
         """As Fusion.mesh_parts, for the group's last extract_mesh and label_parts (member 0)."""
         return self.member(0).mesh_parts(device, getattr(self, "_mesh_n", (0, 0)))
+
+    def track_parts(self, min_voxels=1, device=False):
+        """As Fusion.track_parts (rr_group_track_parts: the whole volume, labelled and tracked on member 0), equal to a
+        single context over the same sequence of frame sets."""
+        n, e = C.c_uint32(), C.c_uint32()
+        self._ck(self.L.rr_group_track_parts(self.h, int(min_voxels), C.byref(n), C.byref(e)))
+        m0 = self.member(0)
+        return m0.download_parts(int(n.value)) + m0.download_part_tracks(int(n.value), int(e.value), device)
+
+    def reset_part_tracks(self):
+        """rr_reset_part_tracks on member 0, which holds the group's tracking state."""
+        self.member(0).reset_part_tracks()
 
     def simplify_mesh(self, cluster_voxels, device=False):
         """As Fusion.simplify_mesh (rr_group_simplify_mesh on member 0 after the group's extract_mesh; CUDA tensors on member

@@ -69,6 +69,9 @@ def context_lifecycle(x, device):
     fu.label_parts()
     fu.mesh_parts(counts=(nv, nt))
     fu.simplify_mesh(2)
+    fu.track_parts()
+    fu.label_parts()
+    fu.track_parts()
     fu.extract_points()
     fu.sample_points(x["pts"])
     fu.cast_rays(x["origins"], x["dirs"])
@@ -96,6 +99,8 @@ def group_lifecycle(x, devices):
     g.extract_mesh()
     g.label_parts()
     g.simplify_mesh(2)
+    g.track_parts()
+    g.track_parts()
     g.extract_points()
     g.sample_points(x["pts"])
     g.cast_rays(x["origins"], x["dirs"])

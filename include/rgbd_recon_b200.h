@@ -441,6 +441,61 @@ int rr_download_part_tracks(rr_ctx* ctx, uint32_t* track_ids, uint32_t* prev_par
 int rr_reset_part_tracks(rr_ctx* ctx);
 int rr_group_track_parts(rr_group* g, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended);
 
+/* ---- distances (no reference counterpart) -------------------------------------------------------------------------------
+ * How far a point is from the captured surface, and the nearest point on it: the volume itself only answers within +-limit
+ * of the surface (every voxel farther out holds -limit in bricks mode).
+ *   Grid     the grid and inside rule of the connected parts: v is the value rr_raymarch reads (R32F; the low half of a half2
+ *            voxel, widened; F32_WEIGHT: the tsdf volume), a voxel is inside iff v > 0 and v is finite, and every voxel of
+ *            the volume counts, whatever rr_set_slab says.
+ *   Field    nearest uint32 [Z][Y][X]: for every voxel a = (x, y, z), the linear index z*X*Y + y*X + x of an inside voxel s
+ *            minimising d^2(a, s) = dx^2 + dy^2 + dz^2 in voxel index units (exact integers); on ties the smallest linear
+ *            index. An inside voxel is its own nearest voxel; with no inside voxel every entry is 0xFFFFFFFF. The rule is
+ *            total: the field depends neither on scheduling, on the occupied-brick shortcut nor on the number of devices.
+ *            Index units: the voxel spacing (bmax_k - bmin_k) / R_k may differ slightly between axes (R_k = ceil(size_k /
+ *            voxel_size)), so in an anisotropic box the index-metric nearest voxel can differ from the metric one.
+ *   Query    points [n][3] in RR_QUERY_WORLD or RR_QUERY_VOLUME, converted as rr_sample_points does (to_volume). For q in the
+ *            closed unit cube the query voxel is a = (floor(q_x X), floor(q_y Y), floor(q_z Z)), each clamped to [0, R_k - 1]
+ *            (the nearest-texel rule), and f = nearest[a]:
+ *              nearest_voxels uint32 [n]   f;
+ *              nearest_points float32 [n][3]  f's voxel centre in the input's space: volume ((float)f_k + 0.5f) / (float)R_k,
+ *                                          world c_k = bmin_k + (((float)f_k + 0.5f) / (float)R_k) * (bmax_k - bmin_k);
+ *              distances float32 [n]       metres, always: p = the point in world space (a volume-space input q becomes
+ *                                          bmin + q * (bmax - bmin)), d = sqrtf((dx*dx + dy*dy) + dz*dz) with dx = p_x - c_x,
+ *                                          ... (binary32, no fused multiply-add, sqrtf correctly rounded).
+ *            d is the distance from p to the centre of the nearest inside voxel of p's voxel: within one voxel diagonal of
+ *            p's distance to the nearest inside-voxel centre. No inside voxel: distance +inf, nearest point NaN, voxel
+ *            0xFFFFFFFF. Outside the closed unit cube or non-finite input: distance NaN, nearest point NaN, voxel 0xFFFFFFFF
+ *            (as rr_sample_points).
+ *   Parts    the part of the nearest voxel is part_labels[nearest_voxels] when a labelling of the same volume state exists.
+ *
+ * rr_distance_field  computes the field of the current volume on the context's stream and synchronises once; returns the
+ *                  number of inside voxels. RR_ERR_INVALID for a NULL count pointer, before any integrate into the current
+ *                  volume (as rr_extract_mesh) and on a context restricted by rr_set_slab (use rr_group_distance_field);
+ *                  RR_ERR_UNSUPPORTED for a volume with an axis of more than 2048 voxels. The field records the volume
+ *                  state (epoch) it was computed from. Not a setting: the volume, brick tables, view images (rr_fill_colors
+ *                  still fills the last view), mesh, simplified mesh, cloud, part labels and tracking state, query buffers,
+ *                  captured frame graphs and rr_integrator_last stay as they are. A new volume allocation (a new resolution
+ *                  or voxel format in rr_configure) releases the field's two volume-sized arrays.
+ * rr_download_distance_field  the last field of the current volume allocation (also after later integrates); nearest may be
+ *                  NULL, host memory (pageable or pinned) or device memory of the context's GPU; returns after one
+ *                  synchronisation. RR_ERR_INVALID before any field of the current volume allocation.
+ * rr_sample_distance  the query above against the last field, which must be of the current volume state: a query after an
+ *                  integrate is refused until the next rr_distance_field, so it never answers about a previous frame set.
+ *                  points and each output may be host (pageable or pinned) or device memory, outputs may be NULL; one
+ *                  synchronisation. count 0 does nothing; RR_ERR_INVALID for a bad space, NULL points with count > 0, or no
+ *                  field of the current volume state; RR_ERR_UNSUPPORTED for count >= 2^31.
+ * rr_group_distance_field  the same for a group, bit for bit: member 0 receives the other members' slabs by peer copies (as
+ *                  rr_group_label_parts) and computes the field there; read it with
+ *                  rr_download_distance_field(rr_group_member(g, 0), ...).
+ * rr_group_sample_distance  rr_sample_distance on member 0 against the group's field, whatever member 0's slab. */
+int rr_distance_field(rr_ctx* ctx, uint32_t* out_num_inside);
+int rr_download_distance_field(rr_ctx* ctx, uint32_t* nearest);
+int rr_sample_distance(rr_ctx* ctx, int space, const float* points, uint32_t count, float* distances, float* nearest_points,
+                       uint32_t* nearest_voxels);
+int rr_group_distance_field(rr_group* g, uint32_t* out_num_inside);
+int rr_group_sample_distance(rr_group* g, int space, const float* points, uint32_t count, float* distances,
+                             float* nearest_points, uint32_t* nearest_voxels);
+
 /* ---- point clouds (no reference counterpart: a reference user draws the points and reads pixels back) -------------------
  * The pre-processed, registered sensor points: every kept depth pixel of the sensors in sensor_mask, lifted to the world.
  * For sensor i (bit i of sensor_mask) and pixel (x, y) of its W x H depth image, id = i*W*H + y*W + x:

@@ -321,13 +321,16 @@ int rr_configure(rr_ctx* c, const rr_config* cfg) {
     c->mesh_valid = false;
     c->parts_valid = false;
     c->simp_valid = false;
+    c->dist_valid = false;
     track_reset(c);                // labels of another grid or voxel format are not comparable
     ++c->volume_epoch;
   }
-  if (new_volume) {   // the label and row arrays are sized by the volume
+  if (new_volume) {   // the label, row and distance arrays are sized by the volume
     c->d_parts_labels[0].release();
     c->d_parts_labels[1].release();
     c->d_parts_rows.release();
+    c->d_dist[0].release();
+    c->d_dist[1].release();
   }
   if (new_bricks) {
     c->mesh_rows_ok = false;
@@ -927,6 +930,36 @@ int rr_reset_part_tracks(rr_ctx* c) {
   if (!c) return RR_ERR_INVALID;
   track_reset(c);
   return RR_OK;
+}
+
+int rr_distance_field(rr_ctx* c, uint32_t* out_num_inside) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, out_num_inside, "rr_distance_field: null count pointer");
+  RR_REQUIRE(c, c->configured && c->volume_integrated, "rr_distance_field: nothing has been integrated into the current volume");
+  RR_REQUIRE(c, c->slab_z0 == 0 && c->slab_z1 == c->res[2],
+             "rr_distance_field: this context holds only its z-slab (rr_set_slab); compute through rr_group_distance_field");
+  RR_SET_DEVICE(c);
+  return launch_distance_field(c, out_num_inside);
+}
+
+int rr_download_distance_field(rr_ctx* c, uint32_t* nearest) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, c->dist_valid, "rr_download_distance_field: no distance field of the current volume (rr_distance_field first)");
+  RR_SET_DEVICE(c);
+  return distance_download(c, nearest);
+}
+
+int rr_sample_distance(rr_ctx* c, int space, const float* points, uint32_t count, float* distances, float* nearest_points,
+                       uint32_t* nearest_voxels) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, space == RR_QUERY_WORLD || space == RR_QUERY_VOLUME, "rr_sample_distance: space must be RR_QUERY_WORLD or RR_QUERY_VOLUME");
+  if (count == 0) return RR_OK;
+  RR_REQUIRE(c, points, "rr_sample_distance: null points");
+  if (count >= (1u << 31)) return fail(c, RR_ERR_UNSUPPORTED, "rr_sample_distance: 2^31 or more entries are not supported");
+  RR_REQUIRE(c, c->dist_valid && c->dist_epoch == c->volume_epoch,
+             "rr_sample_distance: no distance field of the current volume state (rr_distance_field after the last integrate first)");
+  RR_SET_DEVICE(c);
+  return sample_distance(c, space, points, count, distances, nearest_points, nearest_voxels);
 }
 
 int rr_download_parts(rr_ctx* c, uint32_t* voxels, int32_t* boxes, float* centroids, uint32_t* labels) {

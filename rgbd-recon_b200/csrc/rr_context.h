@@ -105,6 +105,7 @@ struct PinnedScalars {
   unsigned long long mesh_totals[2];   // vertices, triangles
   uint32_t simplify_counts[2];         // vertices, triangles of rr_simplify_mesh
   uint32_t track_counts[3];            // rr_track_parts: pair records, then new ids and ended tracks
+  uint32_t dist_inside;                // inside voxels of rr_distance_field
 };
 
 }  // namespace rr
@@ -309,6 +310,15 @@ struct rr_ctx {
                                                      // [Pprev] accepted previous parts; [1] distinct pairs
   rr::DeviceArray<uint8_t> d_track_scratch;          // CUB sort, reduce and scan storage
 
+  // distance field (rr_distance.cu): d_dist[0] holds the last field, d_dist[1] is the other half of the passes' ping-pong
+  // pair; both are exactly a volume and are released by a new volume allocation
+  bool dist_valid = false;         // d_dist[0] holds a field of the current volume allocation (of dist_epoch)
+  uint64_t dist_epoch = 0;
+  rr::DeviceArray<uint32_t> d_dist[2];               // [Z][Y][X] nearest inside voxel
+  rr::DeviceArray<uint32_t> d_dist_count;            // [1] inside voxels
+  rr::DeviceArray<float> d_dq;                       // rr_sample_distance: [n][3] inputs, [n] distances, [n][3] points
+  rr::DeviceArray<uint32_t> d_dq_vox;                // [n] nearest voxels
+
   // mesh simplification (rr_simplify.cu): scratch sized by the mesh's V and T, outputs of at most V vertices and T triangles
   bool simp_valid = false;         // d_simp_* hold a simplification of a mesh of the current volume allocation
   uint32_t simp_nv = 0, simp_nt = 0;
@@ -405,6 +415,13 @@ int mesh_parts_download(rr_ctx* c, uint32_t* vertex_parts, uint32_t* triangle_pa
 int launch_track_parts(rr_ctx* c, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended);
 int track_download(rr_ctx* c, uint32_t* track_ids, uint32_t* prev_parts, uint32_t* overlaps, uint32_t* ended);
 void track_reset(rr_ctx* c);
+// rr_distance.cu: rr_distance_field over the whole volume (checked by the caller: integrated, whole volume), synchronising
+// once; distance_download and sample_distance (checked by the caller: a field of the current epoch, count > 0) copy out
+// and synchronise once
+int launch_distance_field(rr_ctx* c, uint32_t* out_num_inside);
+int distance_download(rr_ctx* c, uint32_t* nearest);
+int sample_distance(rr_ctx* c, int space, const float* points, uint32_t count, float* distances, float* nearest_points,
+                    uint32_t* nearest_voxels);
 // rr_simplify.cu: rr_simplify_mesh of the last mesh (checked by the caller: current, cluster_voxels >= 1), synchronising once;
 // simplified_download copies the last simplification out and synchronises once
 int launch_simplify_mesh(rr_ctx* c, uint32_t cluster_voxels, uint32_t* out_nv, uint32_t* out_nt);

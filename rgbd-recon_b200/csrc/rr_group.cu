@@ -583,6 +583,25 @@ int rr_group_track_parts(rr_group* g, uint32_t min_voxels, uint32_t* out_num_par
   return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
 }
 
+// The same gather, then member 0 computes the field of the whole volume; read it with
+// rr_download_distance_field(rr_group_member(g, 0), ...).
+int rr_group_distance_field(rr_group* g, uint32_t* out_num_inside) {
+  if (!g) return RR_ERR_INVALID;
+  RR_G_REQUIRE(g, out_num_inside, "rr_group_distance_field: null count pointer");
+  RR_TRY_RC(group_gather_volume(g, "rr_group_distance_field", false));
+  const int rc = rr::launch_distance_field(g->m[0], out_num_inside);
+  RR_G_TRY(g, cudaStreamSynchronize(g->m[0]->stream));
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
+// Member 0 holds the group's field (rr_group_distance_field), which covers the whole volume whatever its slab: it answers.
+int rr_group_sample_distance(rr_group* g, int space, const float* points, uint32_t count, float* distances, float* nearest_points,
+                             uint32_t* nearest_voxels) {
+  if (!g) return RR_ERR_INVALID;
+  const int rc = rr_sample_distance(g->m[0], space, points, count, distances, nearest_points, nearest_voxels);
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
 // Right after rr_group_extract_mesh member 0 holds the gathered whole volume and the mesh: it simplifies, with no peer traffic.
 int rr_group_simplify_mesh(rr_group* g, uint32_t cluster_voxels, uint32_t* out_num_vertices, uint32_t* out_num_triangles) {
   if (!g) return RR_ERR_INVALID;

@@ -4,7 +4,7 @@
 //   fusion_playback <file.ks> (--streams "s0;s1;..." | --messages file) [--depth W H --color CW CH] [--frames K] [--voxel m]
 //                   [--limit l] [--eye x y z | --matrices file] [--view W H] [--shade m] [--dump-tsdf file] [--dump-image file] [--dense]
 //                   [--dump-mesh file.ply [--simplify C] [--min-part-voxels N]] [--dump-points file.ply] [--pick PX PY] [--parts]
-//                   [--track-parts N]
+//                   [--track-parts N] [--distance X Y Z]
 //                   [--gpus N | --devices a,b,...] [--recon points|trigrid|calibs [--min-length m] [--dump-recon file]]
 // --recon: like kinect_client's reconstruction list (source/kinect_client.cpp:251-257, key-selected g_recon_mode), one of the
 // other reconstructions also draws the last frame set's maps - ReconPoints, ReconTrigrid (min_length from the sensor .yml
@@ -24,6 +24,9 @@
 //   (ReconIntegration::trackParts with min_voxels N, matched by voxel overlap): one line "frame F part K track T voxels V
 //   prev Q overlap O" per part of at least N voxels (Q = 4294967295 and O = 0 for a new track), then one line
 //   "frame F ended T" per track that ended; F counts frame sets from 0.
+// --distance X Y Z: after every frame set, how far the world point (X, Y, Z) (metres) is from the fused surface
+//   (ReconIntegration::distanceField, then sampleDistance): one line "frame F distance D nearest x y z voxel V" (%.9g, so
+//   every binary32 value is exact; D = inf when nothing is inside, nan with voxel 4294967295 outside the bbox).
 // --dump-points: the last frame set's pre-processed sensor points (ReconPoints::extractPoints) as a binary PLY with normals,
 // colours and quality (with --gpus N through the group call: pre-processing is replicated on every member).
 // --pick PX PY: picking as kinect_client's view would do it - the world ray through the centre of view pixel (PX, PY) (GL window
@@ -117,6 +120,7 @@ int main(int argc, char** argv) {
   long long min_part_voxels = -1;
   long long simplify = 0;
   long long track_min_voxels = 0;
+  std::vector<float> distance_point;
   for (int i = 1; i < argc; ++i) {
     auto next = [&](int k) { return std::atof(argv[i + k]); };
     if (!std::strcmp(argv[i], "--depth")) { W = (unsigned)next(1); H = (unsigned)next(2); i += 2; explicit_sizes = true; }
@@ -139,6 +143,7 @@ int main(int argc, char** argv) {
     else if (!std::strcmp(argv[i], "--min-part-voxels")) min_part_voxels = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--simplify")) simplify = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--track-parts")) track_min_voxels = std::atoll(argv[++i]);
+    else if (!std::strcmp(argv[i], "--distance")) { distance_point = {(float)next(1), (float)next(2), (float)next(3)}; i += 3; }
     else if (!std::strcmp(argv[i], "--gpus")) { devices.clear(); for (int d = 0, n = std::atoi(argv[++i]); d < n; ++d) devices.push_back(d); }
     else if (!std::strcmp(argv[i], "--devices")) {
       devices.clear();
@@ -216,6 +221,14 @@ int main(int argc, char** argv) {
             std::printf("frame %d part %zu track %u voxels %u prev %u overlap %u\n", done, k, (unsigned)tracks.track_ids[k],
                         (unsigned)parts.voxels[k], (unsigned)tracks.prev_parts[k], (unsigned)tracks.overlaps[k]);
         for (uint32_t t : tracks.ended) std::printf("frame %d ended %u\n", done, (unsigned)t);
+      }
+      if (!distance_point.empty()) {                                                   // distance to the surface, per frame set
+        std::vector<float> dist, nearest;
+        std::vector<uint32_t> voxel;
+        recon.distanceField();
+        recon.sampleDistance(distance_point, dist, nearest, voxel);
+        std::printf("frame %d distance %.9g nearest %.9g %.9g %.9g voxel %u\n", done, dist[0], nearest[0], nearest[1], nearest[2],
+                    (unsigned)voxel[0]);
       }
       ++done;
     }

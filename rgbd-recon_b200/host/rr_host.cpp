@@ -449,6 +449,27 @@ void ReconIntegration::samplePoints(std::vector<float> const& points, std::vecto
     ck(rr_sample_points(ctx(), RR_QUERY_WORLD, points.data(), (uint32_t)n, values.data(), normals.data(), rgba.data()), "rr_sample_points");
 }
 
+uint32_t ReconIntegration::distanceField() const {
+  uint32_t n = 0;
+  if (gpu::Context::current().numDevices() > 1) gk(rr_group_distance_field(grp(), &n), "rr_group_distance_field");
+  else ck(rr_distance_field(ctx(), &n), "rr_distance_field");
+  return n;
+}
+
+void ReconIntegration::sampleDistance(std::vector<float> const& points, std::vector<float>& distances, std::vector<float>& nearest_points,
+                                      std::vector<uint32_t>& nearest_voxels) const {
+  if (points.size() % 3) throw std::runtime_error("sampleDistance: points must hold whole [x, y, z] triples");
+  const std::size_t n = points.size() / 3;
+  if (n >= (std::size_t(1) << 31)) throw std::runtime_error("sampleDistance: 2^31 or more points");
+  distances.resize(n); nearest_points.resize(n * 3); nearest_voxels.resize(n);
+  if (gpu::Context::current().numDevices() > 1)
+    gk(rr_group_sample_distance(grp(), RR_QUERY_WORLD, points.data(), (uint32_t)n, distances.data(), nearest_points.data(),
+                                nearest_voxels.data()), "rr_group_sample_distance");
+  else
+    ck(rr_sample_distance(ctx(), RR_QUERY_WORLD, points.data(), (uint32_t)n, distances.data(), nearest_points.data(),
+                          nearest_voxels.data()), "rr_sample_distance");
+}
+
 void ReconIntegration::castRays(std::vector<float> const& origins, std::vector<float> const& directions, std::vector<float>& positions,
                                 std::vector<float>& normals, std::vector<float>& rgba, std::vector<uint32_t>& steps) const {
   if (origins.size() % 3 || origins.size() != directions.size()) throw std::runtime_error("castRays: origins and directions must be equal-length [n][3]");

@@ -367,6 +367,13 @@ class ReconIntegration : public Reconstruction {
   // points, origins, directions, normals, positions: [n][3]; values [n]; rgba [n][4]; steps [n] (0xFFFFFFFF: no hit, with
   // NaN positions and normals). The outputs are resized to n.
   void samplePoints(std::vector<float> const& points, std::vector<float>& values, std::vector<float>& normals, std::vector<float>& rgba) const;
+  // distances to the surface: distanceField computes the nearest inside voxel of every voxel of the fused volume and returns
+  // the inside count (rr_distance_field; with several devices rr_group_distance_field); sampleDistance queries that field at
+  // world points (rr_sample_distance, which refuses a field older than the last integrate): distances [n] in metres, the
+  // nearest inside-voxel centres [n][3] in metres and their linear voxel indices [n]
+  uint32_t distanceField() const;
+  void sampleDistance(std::vector<float> const& points, std::vector<float>& distances, std::vector<float>& nearest_points,
+                      std::vector<uint32_t>& nearest_voxels) const;
   void castRays(std::vector<float> const& origins, std::vector<float> const& directions, std::vector<float>& positions,
                 std::vector<float>& normals, std::vector<float>& rgba, std::vector<uint32_t>& steps) const;
  private:

@@ -156,6 +156,11 @@ def lib():
     L.rr_download_part_tracks.argtypes = [vp, vp, vp, vp, vp]
     L.rr_reset_part_tracks.argtypes = [vp]
     L.rr_group_track_parts.argtypes = [vp, C.c_uint32, u32, u32]
+    L.rr_distance_field.argtypes = [vp, u32]
+    L.rr_download_distance_field.argtypes = [vp, vp]
+    L.rr_sample_distance.argtypes = [vp, C.c_int, vp, C.c_uint32, vp, vp, vp]
+    L.rr_group_distance_field.argtypes = [vp, u32]
+    L.rr_group_sample_distance.argtypes = [vp, C.c_int, vp, C.c_uint32, vp, vp, vp]
     L.rr_simplify_mesh.argtypes = [vp, C.c_uint32, u32, u32]
     L.rr_download_simplified_mesh.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rr_group_simplify_mesh.argtypes = [vp, C.c_uint32, u32, u32]
@@ -232,6 +237,13 @@ def _cast_rays(call, origins, directions, space):
     ptrs, n, keep, device = _query_inputs(origins, directions)
     outs, op = _query_outputs(device, ((n, 3), "f4"), ((n, 3), "f4"), ((n, 4), "f4"), ((n,), "u4"))
     call(QUERY_SPACES[space], ptrs[0], ptrs[1], n, *op)
+    return tuple(outs)
+
+
+def _sample_distance(call, points, space):
+    ptrs, n, keep, device = _query_inputs(points)
+    outs, op = _query_outputs(device, ((n,), "f4"), ((n, 3), "f4"), ((n,), "u4"))
+    call(QUERY_SPACES[space], ptrs[0], n, *op)
     return tuple(outs)
 
 
@@ -683,6 +695,31 @@ class Fusion:
         """rr_reset_part_tracks: forget the tracked labelling; the next track_parts starts ids at 0."""
         self._ck(self.L.rr_reset_part_tracks(self.h))
 
+    def distance_field(self):
+        """rr_distance_field: the nearest inside voxel of every voxel of the current volume, computed on the device; returns
+        the number of inside voxels."""
+        n = C.c_uint32()
+        self._ck(self.L.rr_distance_field(self.h, C.byref(n)))
+        return int(n.value)
+
+    def nearest_voxels(self, device=False):
+        """rr_download_distance_field: uint32 [Z, Y, X], the linear index of every voxel's nearest inside voxel (0xFFFFFFFF
+        when nothing is inside); a numpy array, or with device a CUDA tensor on the context's GPU."""
+        X, Y, Z = (int(v) for v in self.volume_res())
+        dev = None
+        if device:
+            import torch
+            dev = torch.device("cuda", self.device)
+        (nearest,), (ptr,) = _query_outputs(dev, ((Z, Y, X), "u4"))
+        self._ck(self.L.rr_download_distance_field(self.h, ptr))
+        return nearest
+
+    def sample_distance(self, points, space="world"):
+        """rr_sample_distance at points [n, 3] ("world": metres, "volume": texture coordinates over the bbox) against the
+        last distance_field, which must be of the current volume state: (distances float32 [n] in metres, nearest_points
+        float32 [n, 3] in the input's space, nearest_voxels uint32 [n]); CUDA tensors when the points are."""
+        return _sample_distance(lambda *a: self._ck(self.L.rr_sample_distance(self.h, *a)), points, space)
+
     def simplify_mesh_counts(self, cluster_voxels):
         """rr_simplify_mesh alone: simplifies the last mesh on the device and returns (vertices, triangles)."""
         nv, nt = C.c_uint32(), C.c_uint32()
@@ -960,6 +997,21 @@ class Group:
     def reset_part_tracks(self):
         """rr_reset_part_tracks on member 0, which holds the group's tracking state."""
         self.member(0).reset_part_tracks()
+
+    def distance_field(self):
+        """As Fusion.distance_field (rr_group_distance_field: the whole volume, on member 0), equal to a single context;
+        read the field with member(0).nearest_voxels()."""
+        n = C.c_uint32()
+        self._ck(self.L.rr_group_distance_field(self.h, C.byref(n)))
+        return int(n.value)
+
+    def nearest_voxels(self, device=False):
+        """The group's last distance field (member 0's)."""
+        return self.member(0).nearest_voxels(device)
+
+    def sample_distance(self, points, space="world"):
+        """As Fusion.sample_distance (rr_group_sample_distance: member 0, against the group's field)."""
+        return _sample_distance(lambda *a: self._ck(self.L.rr_group_sample_distance(self.h, *a)), points, space)
 
     def simplify_mesh(self, cluster_voxels, device=False):
         """As Fusion.simplify_mesh (rr_group_simplify_mesh on member 0 after the group's extract_mesh; CUDA tensors on member

@@ -72,6 +72,9 @@ def context_lifecycle(x, device):
     fu.track_parts()
     fu.label_parts()
     fu.track_parts()
+    fu.distance_field()
+    fu.nearest_voxels()
+    fu.sample_distance(x["pts"])
     fu.extract_points()
     fu.sample_points(x["pts"])
     fu.cast_rays(x["origins"], x["dirs"])
@@ -101,6 +104,8 @@ def group_lifecycle(x, devices):
     g.simplify_mesh(2)
     g.track_parts()
     g.track_parts()
+    g.distance_field()
+    g.sample_distance(x["pts"])
     g.extract_points()
     g.sample_points(x["pts"])
     g.cast_rays(x["origins"], x["dirs"])

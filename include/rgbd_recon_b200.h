@@ -394,6 +394,41 @@ int rr_download_parts(rr_ctx* ctx, uint32_t* voxels, int32_t* boxes, float* cent
 int rr_download_mesh_parts(rr_ctx* ctx, uint32_t* vertex_parts, uint32_t* triangle_parts);
 int rr_group_label_parts(rr_group* g, uint32_t* out_num_parts);
 
+/* ---- removing parts (no reference counterpart) --------------------------------------------------------------------------
+ * Takes chosen parts out of the volume itself - the small floating blobs sensor noise leaves in front of the surface, or
+ * everything but the objects a client wants to show - so that every output (views, colour fill, meshes, queries, distances,
+ * parts and tracks) sees the cleaned volume through its own code path.
+ *   Labelling  the context's last labelling (rr_label_parts, or the labelling inside rr_track_parts), which must be of the
+ *            current volume state: no integrate, no new volume and no other removal since.
+ *   Parts    part p of that labelling (P parts) is removed iff voxels[p] < min_voxels, or keep != NULL and keep[p] == 0.
+ *            keep: uint8 [P], host memory (pageable or pinned) or device memory of the context's GPU; it must hold P entries.
+ *            min_voxels == 0 with keep == NULL removes nothing.
+ *   Voxels   every voxel labelled with a removed part becomes exactly the voxel the bricks-mode clear writes with the limit in
+ *            effect now: R32F -limit; F32_WEIGHT tsdf -limit and weight 0; HALF2 half2(-limit, 0). Every other voxel of the
+ *            volume and of the weight volume stays bit for bit as it was. The outside band (-limit < v <= 0) around a removed
+ *            part stays: it produces no hit, no mesh vertex and no part.
+ *
+ * rr_remove_parts  rewrites on the context's stream and synchronises once; returns the number of removed parts and the exact
+ *                  sum of their voxel counts. RR_ERR_INVALID for a NULL count pointer, no labelling of the current volume
+ *                  state, and on a context restricted by rr_set_slab (use rr_group_remove_parts). When a part was removed
+ *                  the volume epoch advances (a new volume state): a mesh, labelling or distance field taken before is of
+ *                  the previous state under the rules above (rr_download_mesh_parts pairs only a mesh and a labelling of one
+ *                  state, rr_sample_distance refuses until the next rr_distance_field, and a second rr_remove_parts needs a
+ *                  new labelling); the labelling is not renumbered. Not a setting: brick tables, stage images, view images
+ *                  (rr_fill_colors still fills the last view), cloud, query buffers, tracking state, captured frame graphs,
+ *                  rr_integrator_last and rr_integrator_cleared stay as they are, and the next integrates clear and write
+ *                  exactly what they would have (the incremental clear stays valid: a removed voxel was inside, so it lay in
+ *                  a brick the last integrate evaluated).
+ * rr_group_remove_parts  the same for a group with member 0's last labelling (rr_group_label_parts / rr_group_track_parts):
+ *                  every member rewrites the rows its integrate writes (its slab and halo), so that every member's slab
+ *                  and halo, and the group's views, queries and meshes, equal a single context's bit for bit. Member 0
+ *                  writes the other members' volumes through peer memory: RR_ERR_UNSUPPORTED when its device cannot address
+ *                  a member's memory. */
+int rr_remove_parts(rr_ctx* ctx, uint32_t min_voxels, const uint8_t* keep, uint32_t* out_removed_parts,
+                    uint32_t* out_removed_voxels);
+int rr_group_remove_parts(rr_group* g, uint32_t min_voxels, const uint8_t* keep, uint32_t* out_removed_parts,
+                          uint32_t* out_removed_voxels);
+
 /* ---- part tracking (no reference counterpart) ---------------------------------------------------------------------------
  * Persistent identities for the connected parts from one frame set to the next: a part's number depends on what else is in
  * the volume, a track id follows the object by voxel overlap.

@@ -908,6 +908,18 @@ int rr_label_parts(rr_ctx* c, uint32_t* out_num_parts) {
   return launch_label_parts(c, label_dest(c), out_num_parts);
 }
 
+int rr_remove_parts(rr_ctx* c, uint32_t min_voxels, const uint8_t* keep, uint32_t* out_removed_parts, uint32_t* out_removed_voxels) {
+  if (!c) return RR_ERR_INVALID;
+  RR_REQUIRE(c, out_removed_parts && out_removed_voxels, "rr_remove_parts: null count pointer");
+  RR_REQUIRE(c, c->configured && c->slab_z0 == 0 && c->slab_z1 == c->res[2],
+             "rr_remove_parts: this context holds only its z-slab (rr_set_slab); remove through rr_group_remove_parts");
+  RR_REQUIRE(c, c->parts_valid && c->parts_epoch == c->volume_epoch,
+             "rr_remove_parts: no labelling of the current volume state (rr_label_parts or rr_track_parts after the last integrate "
+             "or removal first)");
+  RR_SET_DEVICE(c);
+  return remove_parts(c, &c, 1, min_voxels, keep, out_removed_parts, out_removed_voxels);
+}
+
 int rr_track_parts(rr_ctx* c, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended) {
   if (!c) return RR_ERR_INVALID;
   RR_REQUIRE(c, out_num_parts && out_num_ended, "rr_track_parts: null count pointer");

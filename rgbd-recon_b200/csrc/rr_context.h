@@ -106,6 +106,7 @@ struct PinnedScalars {
   uint32_t simplify_counts[2];         // vertices, triangles of rr_simplify_mesh
   uint32_t track_counts[3];            // rr_track_parts: pair records, then new ids and ended tracks
   uint32_t dist_inside;                // inside voxels of rr_distance_field
+  uint32_t remove_counts[2];           // rr_remove_parts: removed parts, their voxels
 };
 
 }  // namespace rr
@@ -319,6 +320,12 @@ struct rr_ctx {
   rr::DeviceArray<float> d_dq;                       // rr_sample_distance: [n][3] inputs, [n] distances, [n][3] points
   rr::DeviceArray<uint32_t> d_dq_vox;                // [n] nearest voxels
 
+  // part removal (rr_remove.cu): per part of the labelling it acts on
+  rr::DeviceArray<uint8_t> d_remove_keep;            // [P] the caller's keep flags, staged
+  rr::DeviceArray<unsigned long long> d_remove_rows; // [2][P + 1] rows of each removed part's box (0: kept), their offsets
+  rr::DeviceArray<uint32_t> d_remove_counts;         // [2] removed parts, their voxels
+  rr::DeviceArray<uint8_t> d_remove_scratch;         // CUB scan storage
+
   // mesh simplification (rr_simplify.cu): scratch sized by the mesh's V and T, outputs of at most V vertices and T triangles
   bool simp_valid = false;         // d_simp_* hold a simplification of a mesh of the current volume allocation
   uint32_t simp_nv = 0, simp_nt = 0;
@@ -422,6 +429,11 @@ int launch_distance_field(rr_ctx* c, uint32_t* out_num_inside);
 int distance_download(rr_ctx* c, uint32_t* nearest);
 int sample_distance(rr_ctx* c, int space, const float* points, uint32_t count, float* distances, float* nearest_points,
                     uint32_t* nearest_voxels);
+// rr_remove.cu: rr_remove_parts with the last labelling of c (checked by the caller: of the current volume state), rewriting
+// the integrate rows of each of the n member volumes (c itself, or a group's members, which c's device can address) on c's
+// stream; synchronises once
+int remove_parts(rr_ctx* c, rr_ctx* const* members, int n, uint32_t min_voxels, const uint8_t* keep, uint32_t* out_parts,
+                 uint32_t* out_voxels);
 // rr_simplify.cu: rr_simplify_mesh of the last mesh (checked by the caller: current, cluster_voxels >= 1), synchronising once;
 // simplified_download copies the last simplification out and synchronises once
 int launch_simplify_mesh(rr_ctx* c, uint32_t cluster_voxels, uint32_t* out_nv, uint32_t* out_nt);

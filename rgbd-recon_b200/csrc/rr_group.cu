@@ -571,6 +571,32 @@ int rr_group_label_parts(rr_group* g, uint32_t* out_num_parts) {
   return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
 }
 
+// Member 0's last labelling (of the gathered volume) says which voxels go; member 0 rewrites them in every member's slab and
+// halo rows, the other members' through peer memory, on its own stream after the members' queued work.
+int rr_group_remove_parts(rr_group* g, uint32_t min_voxels, const uint8_t* keep, uint32_t* out_removed_parts,
+                          uint32_t* out_removed_voxels) {
+  if (!g) return RR_ERR_INVALID;
+  RR_G_REQUIRE(g, out_removed_parts && out_removed_voxels, "rr_group_remove_parts: null count pointer");
+  RR_G_REQUIRE(g, g->bounds.size() == g->m.size() + 1, "rr_group_remove_parts: configure the group first");
+  rr_ctx* c0 = g->m[0];
+  RR_G_REQUIRE(g, c0->parts_valid && c0->parts_epoch == c0->volume_epoch,
+               "rr_group_remove_parts: no labelling of the current volume state (rr_group_label_parts or rr_group_track_parts "
+               "after the last integrate or removal first)");
+  for (size_t i = 1; i < g->m.size(); ++i)
+    if (!g->peer[i])
+      return gfail(g, RR_ERR_UNSUPPORTED, "rr_group_remove_parts: member 0's device cannot address member " + std::to_string(i) + "'s memory");
+  for (size_t i = 1; i < g->m.size(); ++i) {
+    rr_ctx* c = g->m[i];
+    RR_G_TRY(g, cudaSetDevice(c->device));
+    RR_G_TRY(g, cudaEventRecord(g->ev_view[i], c->stream));
+    RR_G_TRY(g, cudaSetDevice(c0->device));
+    RR_G_TRY(g, cudaStreamWaitEvent(c0->stream, g->ev_view[i], 0));
+  }
+  RR_G_TRY(g, cudaSetDevice(c0->device));
+  const int rc = rr::remove_parts(c0, g->m.data(), (int)g->m.size(), min_voxels, keep, out_removed_parts, out_removed_voxels);
+  return rc == RR_OK ? RR_OK : member_fail(g, 0, rc);
+}
+
 // The same gather, then member 0 tracks the whole volume against its tracked labelling; read the tracks with
 // rr_download_part_tracks(rr_group_member(g, 0), ...), reset them with rr_reset_part_tracks on member 0.
 int rr_group_track_parts(rr_group* g, uint32_t min_voxels, uint32_t* out_num_parts, uint32_t* out_num_ended) {

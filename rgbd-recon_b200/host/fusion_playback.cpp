@@ -4,7 +4,7 @@
 //   fusion_playback <file.ks> (--streams "s0;s1;..." | --messages file) [--depth W H --color CW CH] [--frames K] [--voxel m]
 //                   [--limit l] [--eye x y z | --matrices file] [--view W H] [--shade m] [--dump-tsdf file] [--dump-image file] [--dense]
 //                   [--dump-mesh file.ply [--simplify C] [--min-part-voxels N]] [--dump-points file.ply] [--pick PX PY] [--parts]
-//                   [--track-parts N] [--distance X Y Z]
+//                   [--track-parts N] [--distance X Y Z] [--remove-parts N]
 //                   [--gpus N | --devices a,b,...] [--recon points|trigrid|calibs [--min-length m] [--dump-recon file]]
 // --recon: like kinect_client's reconstruction list (source/kinect_client.cpp:251-257, key-selected g_recon_mode), one of the
 // other reconstructions also draws the last frame set's maps - ReconPoints, ReconTrigrid (min_length from the sensor .yml
@@ -18,6 +18,9 @@
 // --min-part-voxels N: with --dump-mesh, only the triangles of connected parts of at least N voxels, and the vertices they
 //   use, in their original order and re-indexed (drops the small floating blobs sensor noise leaves in front of the surface).
 //   With --simplify, a simplified triangle is in the part of its source triangle.
+// --remove-parts N: after every frame set's fuse, before anything reads the volume (the view, --recon, the dumps, --pick,
+//   --parts, --track-parts, --distance), its connected parts of fewer than N voxels are taken out of the volume
+//   (ReconIntegration::labelParts, then removeParts): one line "frame F removed K parts V voxels" per frame set.
 // --parts: one line per connected part of the last frame set's volume (ReconIntegration::labelParts): index, voxels, box
 //   (x0 x1 y0 y1 z0 z1, half-open voxel ranges) and centroid (metres).
 // --track-parts N: after every frame set, its connected parts with track ids that persist across frame sets
@@ -120,6 +123,7 @@ int main(int argc, char** argv) {
   long long min_part_voxels = -1;
   long long simplify = 0;
   long long track_min_voxels = 0;
+  long long remove_min_voxels = -1;
   std::vector<float> distance_point;
   for (int i = 1; i < argc; ++i) {
     auto next = [&](int k) { return std::atof(argv[i + k]); };
@@ -143,6 +147,7 @@ int main(int argc, char** argv) {
     else if (!std::strcmp(argv[i], "--min-part-voxels")) min_part_voxels = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--simplify")) simplify = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--track-parts")) track_min_voxels = std::atoll(argv[++i]);
+    else if (!std::strcmp(argv[i], "--remove-parts")) remove_min_voxels = std::atoll(argv[++i]);
     else if (!std::strcmp(argv[i], "--distance")) { distance_point = {(float)next(1), (float)next(2), (float)next(3)}; i += 3; }
     else if (!std::strcmp(argv[i], "--gpus")) { devices.clear(); for (int d = 0, n = std::atoi(argv[++i]); d < n; ++d) devices.push_back(d); }
     else if (!std::strcmp(argv[i], "--devices")) {
@@ -210,6 +215,12 @@ int main(int argc, char** argv) {
       nka.processTextures();
       recon.updateOccupiedBricks();
       recon.integrate();
+      if (remove_min_voxels >= 0) {                                                    // floaters out of the volume, per frame set
+        Parts labelled;
+        recon.labelParts(labelled);
+        const std::pair<uint32_t, uint32_t> removed = recon.removeParts((uint32_t)remove_min_voxels);
+        std::printf("frame %d removed %u parts %u voxels\n", done, (unsigned)removed.first, (unsigned)removed.second);
+      }
       recon.drawF();
       if (done == 0 && devices.size() > 1) gpu.balanceSlabs();                        // occupied bricks cluster around the subject
       if (track_min_voxels > 0) {                                                      // persistent part ids, per frame set

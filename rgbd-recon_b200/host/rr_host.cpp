@@ -408,6 +408,14 @@ void ReconIntegration::labelParts(Parts& out) const {
   ck(rr_download_parts(ctx(), out.voxels.data(), out.boxes.data(), out.centroids.data(), nullptr), "rr_download_parts");
 }
 
+std::pair<uint32_t, uint32_t> ReconIntegration::removeParts(uint32_t min_voxels, const std::vector<uint8_t>* keep) const {
+  uint32_t parts = 0, voxels = 0;
+  const uint8_t* k = keep ? keep->data() : nullptr;
+  if (gpu::Context::current().numDevices() > 1) gk(rr_group_remove_parts(grp(), min_voxels, k, &parts, &voxels), "rr_group_remove_parts");
+  else ck(rr_remove_parts(ctx(), min_voxels, k, &parts, &voxels), "rr_remove_parts");
+  return {parts, voxels};
+}
+
 void ReconIntegration::trackParts(uint32_t min_voxels, Parts& parts, PartTracks& tracks) const {
   uint32_t n = 0, e = 0;
   if (gpu::Context::current().numDevices() > 1) gk(rr_group_track_parts(grp(), min_voxels, &n, &e), "rr_group_track_parts");

@@ -355,6 +355,10 @@ class ReconIntegration : public Reconstruction {
   // the 6-connected parts of the fused volume (rr_label_parts; with several devices rr_group_label_parts), and the part of
   // every vertex [V] and triangle [T] of the last extractMesh, which must come from the same volume state
   void labelParts(Parts& out) const;
+  // takes parts of the last labelParts / trackParts (of the current volume state) out of the fused volume: those of fewer
+  // than min_voxels voxels and, with keep (one entry per part), those whose entry is 0 (rr_remove_parts; with several devices
+  // rr_group_remove_parts); returns (removed parts, removed voxels)
+  std::pair<uint32_t, uint32_t> removeParts(uint32_t min_voxels, const std::vector<uint8_t>* keep = nullptr) const;
   void meshParts(std::vector<uint32_t>& vertex_parts, std::vector<uint32_t>& triangle_parts) const;
   // the parts of the fused volume with track ids persistent across frame sets, matched by voxel overlap against the last
   // trackParts (rr_track_parts; with several devices rr_group_track_parts); resetPartTracks starts ids at 0 again

@@ -152,6 +152,8 @@ def lib():
     L.rr_download_parts.argtypes = [vp, vp, vp, vp, vp]
     L.rr_download_mesh_parts.argtypes = [vp, vp, vp]
     L.rr_group_label_parts.argtypes = [vp, u32]
+    L.rr_remove_parts.argtypes = [vp, C.c_uint32, vp, u32, u32]
+    L.rr_group_remove_parts.argtypes = [vp, C.c_uint32, vp, u32, u32]
     L.rr_track_parts.argtypes = [vp, C.c_uint32, u32, u32]
     L.rr_download_part_tracks.argtypes = [vp, vp, vp, vp, vp]
     L.rr_reset_part_tracks.argtypes = [vp]
@@ -245,6 +247,37 @@ def _sample_distance(call, points, space):
     outs, op = _query_outputs(device, ((n,), "f4"), ((n, 3), "f4"), ((n,), "u4"))
     call(QUERY_SPACES[space], ptrs[0], n, *op)
     return tuple(outs)
+
+
+def _remove_parts(call, min_voxels, keep, n_parts):
+    """rr_remove_parts / rr_group_remove_parts with keep None, or one bool / uint8 entry per part of the last labelling
+    (n_parts, recorded by this object's label_parts / track_parts): a numpy array or a torch tensor (host, or on the context's
+    GPU: the caller's stream is synchronised first, as the library reads it on its own stream). The library reads exactly
+    n_parts bytes, so any other length or element type is refused here."""
+    ref = None
+    if keep is None:
+        ptr = None
+    else:
+        if n_parts is None:
+            raise ValueError("keep needs the part count of the last labelling: label_parts or track_parts through this object first")
+        if type(keep).__module__.startswith("torch"):
+            import torch
+            if keep.dtype not in (torch.bool, torch.uint8):
+                raise ValueError("keep must be a bool or uint8 tensor")
+            ref = keep.detach().reshape(-1).contiguous()
+            if ref.is_cuda:
+                torch.cuda.current_stream(ref.device).synchronize()
+            ptr, count = ref.data_ptr(), ref.numel()
+        else:
+            ref = np.ascontiguousarray(keep).reshape(-1)
+            if ref.dtype not in (np.bool_, np.uint8):
+                raise ValueError("keep must be a bool or uint8 array")
+            ptr, count = ref.ctypes.data, ref.size
+        if count != n_parts:
+            raise ValueError(f"keep holds {count} entries, the last labelling {n_parts} parts")
+    parts, voxels = C.c_uint32(), C.c_uint32()
+    call(int(min_voxels), ptr, C.byref(parts), C.byref(voxels))
+    return int(parts.value), int(voxels.value)
 
 
 def _sensor_mask(sensors, n_sensors):
@@ -625,7 +658,8 @@ class Fusion:
         """rr_label_parts alone: labels the connected parts of the volume on the device and returns their count."""
         n = C.c_uint32()
         self._ck(self.L.rr_label_parts(self.h, C.byref(n)))
-        return int(n.value)
+        self._parts_n = int(n.value)
+        return self._parts_n
 
     def download_parts(self, n):
         """rr_download_parts of the last labelling (n: its part count): (voxels uint32 [n], boxes int32 [n, 6], centroids
@@ -665,11 +699,19 @@ class Fusion:
         self._ck(self.L.rr_download_mesh_parts(self.h, *ptrs))
         return tuple(outs)
 
+    def remove_parts(self, min_voxels=0, keep=None):
+        """rr_remove_parts: rewrites the voxels of the parts of the last labelling (label_parts / track_parts of the current
+        volume state) that have fewer than min_voxels voxels or whose keep entry is 0 to the cleared voxel, on the device.
+        keep: None, or one bool / uint8 per part (numpy array or torch tensor, on the host or the context's GPU). Returns
+        (removed_parts, removed_voxels)."""
+        return _remove_parts(lambda *a: self._ck(self.L.rr_remove_parts(self.h, *a)), min_voxels, keep, getattr(self, "_parts_n", None))
+
     def track_parts_counts(self, min_voxels=1):
         """rr_track_parts alone: labels the volume, tracks its parts against the tracked labelling and returns (parts P,
         ended tracks E)."""
         n, e = C.c_uint32(), C.c_uint32()
         self._ck(self.L.rr_track_parts(self.h, int(min_voxels), C.byref(n), C.byref(e)))
+        self._parts_n = int(n.value)
         return int(n.value), int(e.value)
 
     def download_part_tracks(self, n, e, device=False):
@@ -976,6 +1018,7 @@ class Group:
         bit for bit: (voxels, boxes, centroids)."""
         n = C.c_uint32()
         self._ck(self.L.rr_group_label_parts(self.h, C.byref(n)))
+        self._parts_n = int(n.value)
         return self.member(0).download_parts(int(n.value))
 
     def part_labels(self, device=False):
@@ -991,8 +1034,14 @@ class Group:
         single context over the same sequence of frame sets."""
         n, e = C.c_uint32(), C.c_uint32()
         self._ck(self.L.rr_group_track_parts(self.h, int(min_voxels), C.byref(n), C.byref(e)))
+        self._parts_n = int(n.value)
         m0 = self.member(0)
         return m0.download_parts(int(n.value)) + m0.download_part_tracks(int(n.value), int(e.value), device)
+
+    def remove_parts(self, min_voxels=0, keep=None):
+        """As Fusion.remove_parts (rr_group_remove_parts: member 0's last labelling, every member's slab and halo), equal to
+        a single context bit for bit: (removed_parts, removed_voxels)."""
+        return _remove_parts(lambda *a: self._ck(self.L.rr_group_remove_parts(self.h, *a)), min_voxels, keep, getattr(self, "_parts_n", None))
 
     def reset_part_tracks(self):
         """rr_reset_part_tracks on member 0, which holds the group's tracking state."""

@@ -75,6 +75,10 @@ def context_lifecycle(x, device):
     fu.distance_field()
     fu.nearest_voxels()
     fu.sample_distance(x["pts"])
+    fu.label_parts()
+    fu.remove_parts(50)
+    fu.track_parts()
+    fu.remove_parts(0, np.ones(fu.label_parts_count(), np.uint8))
     fu.extract_points()
     fu.sample_points(x["pts"])
     fu.cast_rays(x["origins"], x["dirs"])
@@ -106,6 +110,8 @@ def group_lifecycle(x, devices):
     g.track_parts()
     g.distance_field()
     g.sample_distance(x["pts"])
+    g.label_parts()
+    g.remove_parts(50)
     g.extract_points()
     g.sample_points(x["pts"])
     g.cast_rays(x["origins"], x["dirs"])
